@@ -10,6 +10,10 @@ with global ids rank*B .. rank*B+B-1 (weak scaling, no collective inside the ste
 statistics are summed on the device and all-reduced over NCCL once per episode and once at the end of
 the timed region.  Rank 0 prints ONE JSON line.
 
+--dump-outputs DIR writes what the last of the K timed steps returned to the caller as DIR/<name>.npy.  The
+inputs (env seed, pre-generated actions) depend on the arguments only, so two builds run with the same arguments
+can be compared output for output.
+
 --impl reference times the reference's own CPU implementation on all host cores: the unmodified Python
 ``GridworldCtf`` (one env per process; /root/reference, or its byte-compiled copy oracle/_ref on the GPU box),
 falling back to the C port of the oracle only where neither exists.
@@ -37,6 +41,7 @@ OBS_ELEM_BYTES = {"float32": 4, "uint8": 1, "float16": 2, "bfloat16": 2}
 DTYPE_TAG = {"float32": "f32", "uint8": "u8", "float16": "f16", "bfloat16": "bf16"}
 KERNEL_T = {"float32": "float", "uint8": "uint8_t", "float16": "__half", "bfloat16": "__nv_bfloat16"}
 REF_ENV_STEPS_PER_PASS = 100  # --impl reference: env steps every process advances per bench "step"
+DUMP_BYTES = 60_000_000  # --dump-outputs stays below 64 MB: larger batches are written for a fixed, seeded sample of envs
 
 
 def host_threads() -> int:
@@ -267,6 +272,42 @@ def workload_config(args, envs_per_gpu: int, n_gpus: int, experiment: str | None
 
 
 # -----------------------------------------------------------------------------------------------------
+def dump_env_index(env, torch):
+    """Envs whose step outputs --dump-outputs writes: every env when they fit DUMP_BYTES, else a sample drawn with a
+    fixed seed, so that two builds run with the same arguments write the same envs."""
+    import numpy as np
+
+    per_env = 8 + env.rewards[0].numel() * 4 + 4 + env.meta[0].numel() * 4
+    if env.obs is not None:
+        per_env += env.obs[0].numel() * 4
+    if env.obs_bits is not None:
+        per_env += env.obs_bits[0].numel() * 8
+    n = min(env.num_envs, DUMP_BYTES // per_env)
+    idx = np.sort(np.random.default_rng(0).choice(env.num_envs, n, replace=False))
+    return torch.from_numpy(idx).to(env.device)
+
+
+def take_outputs(env, idx) -> dict:
+    """What env.step returned in the step just launched (observations, metadata, rewards, dones and the packed
+    observations if enabled), gathered on the device at the envs `idx`."""
+    outs = {"obs": env.obs, "meta": env.meta, "rewards": env.rewards, "dones": env.dones, "obs_bits": env.obs_bits}
+    return {name: t.index_select(0, idx) for name, t in outs.items() if t is not None}
+
+
+def write_outputs(path, idx, outs, torch) -> list:
+    """DIR/<name>.npy per array: integer arrays as float64 (exact), everything else as float32 (exact for the
+    float32, float16, bfloat16 and uint8 buffers).  env_index.npy names the env of every row."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    names = []
+    for name, t in dict(outs, env_index=idx).items():
+        t = t.double() if t.dtype in (torch.int32, torch.int64) else t.float()
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+        names.append(name)
+    return sorted(names)
+
+
 def time_steps(env, actions, steps, dev, torch):
     """ms per step of `steps` back-to-back step launches (CUDA events on the launching stream)."""
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -342,6 +383,8 @@ def run_ours(args) -> dict | None:
     n_act = 8  # distinct pre-generated action tensors, resident in HBM before the timed region
     actions = torch.randint(0, 9, (n_act, B, N), dtype=torch.uint8, device=dev, generator=gen)
     stats_total = torch.zeros((13, N), dtype=torch.int64, device=dev)
+    dump_idx = dump_env_index(env, torch) if args.dump_outputs and rank == 0 else None
+    last_outputs = None
 
     launches = 0
 
@@ -351,11 +394,13 @@ def run_ours(args) -> dict | None:
             stats_total.add_(env.stats_sum(all_reduce=world > 1))   # k_stats_sum + (N > 1) one NCCL all-reduce of 13*N int64
             launches += 1
 
-    def one_step(k):
-        nonlocal launches
+    def one_step(k, keep_outputs=False):
+        nonlocal launches, last_outputs
         env.step(actions[k % n_act])
         launches += 1
         if (k + 1) % env.GAME_STEPS == 0:  # episode over: reduce its statistics, start the next one
+            if keep_outputs:   # the reset below overwrites the output buffers: gather them first, inside the timed region
+                last_outputs = take_outputs(env, dump_idx)
             reduce_stats()
             env.reset()
             launches += 1
@@ -382,6 +427,8 @@ def run_ours(args) -> dict | None:
     for _ in range(W):
         one_step(step_idx)
         step_idx += 1
+    if dump_idx is not None:
+        take_outputs(env, dump_idx)   # loads the gather kernels and caches their buffers before the timed region
     graph = None
     if args.graph_steps > 0:
         graph = env.make_step_graph(actions[0], steps_per_replay=args.graph_steps)
@@ -395,22 +442,26 @@ def run_ours(args) -> dict | None:
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     if graph is None:
-        for _ in range(K):
-            one_step(step_idx)
+        for i in range(K):
+            one_step(step_idx, keep_outputs=dump_idx is not None and i == K - 1)
             step_idx += 1
     else:
         for _ in range(K // args.graph_steps):
             graph.replay()
-        launches = (K // args.graph_steps) * args.graph_steps
-        K = launches
+        for _ in range(K % args.graph_steps):   # the same step as the captured one, so that exactly K steps are timed
+            env.step(actions[0])
+        launches = K
     if step_idx % env.GAME_STEPS != 0:
         reduce_stats()
     e1.record()
+    if dump_idx is not None and last_outputs is None:
+        last_outputs = take_outputs(env, dump_idx)   # nothing has touched the output buffers since the last step
     barrier()
     sampler.sample()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop()
     gpu_launches = launches
+    dumped = write_outputs(args.dump_outputs, dump_idx, last_outputs, torch) if dump_idx is not None else None
 
     # ---- e2e: the same steps through the host-buffer entry point (ctf_step_host): H2D actions from pinned
     # memory and D2H rewards + dones inside the timed region; observations stay in the policy's device buffer
@@ -474,6 +525,9 @@ def run_ours(args) -> dict | None:
             },
             "episode_stats_checksum": int(stats_total.sum().item()),
         }
+        if dumped is not None:
+            result["dump_outputs"] = {"dir": args.dump_outputs, "arrays": dumped, "envs": int(dump_idx.numel()),
+                                      "step": "last timed step"}
         if world == 1 and not args.no_side:
             # the write-only ceiling of this GPU, measured now: torch.fill_ of the observation buffer
             if env.obs is not None:
@@ -549,7 +603,14 @@ def main():
     ap.add_argument("--prewarm-s", type=float, default=0.6, help="seconds of untimed steps before the warm-up steps")
     ap.add_argument("--obs-dtype", choices=["float32", "uint8", "float16", "bfloat16"], default="float32",
                     help="float32 is the drop-in default and the headline; the narrower buffers are reported separately")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (obs, meta, rewards, dones; packed obs with --packed) as "
+                         "DIR/<name>.npy, for all envs or a fixed seeded sample of them (< 64 MB in all); rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU step path (--impl ours)")
     args.warmup = max(3, args.warmup)
     global EXPERIMENT
     EXPERIMENT = args.experiment

@@ -2,12 +2,14 @@
 (tests/golden/callers/) against (a) the same loops on the CPU oracle — pins the oracle-side loops — and, where the
 reference is importable (this container, or oracle/_ref), (b) a fresh run of the unmodified callers — pins the
 generator — plus the state_dict compatibility of CtfPolicy with the reference Agent."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
 import caller_cases as cc
-from helpers import bits, compiled
+from helpers import GOLDEN, bits, compiled
 from oracle import ref_shim as rs
 
 needs_reference = pytest.mark.skipif(not rs.available(), reason="reference neither under /root/reference nor in oracle/_ref")
@@ -114,3 +116,62 @@ def test_ctf_policy_loads_the_reference_agent_state_dict_bit_for_bit():
     b_ref = batched_action(ref, g, m, flags)
     torch.manual_seed(5)
     assert torch.equal(b_ref, batched_action(ours, g, m, flags))
+
+
+# ------------------------------------------------------------------------------------------------------------------
+POLICY_RECORD = os.path.join(GOLDEN, "ctf_policy_outputs.npz")
+
+
+def _policy_case():
+    """A small network (9 actions, 4 channels, 6x6 grid, 10 metadata) with weights and inputs from a fixed numpy seed."""
+    from marl_ctf_development_b200.policy import CtfPolicy
+
+    rng = np.random.default_rng(3)
+    shapes = {k: v.shape for k, v in CtfPolicy(9, 4, 6, 10).state_dict().items()}
+    sd = {k: torch.from_numpy(rng.uniform(-0.3, 0.3, shape).astype(np.float32)) for k, shape in shapes.items()}
+    g = torch.from_numpy((rng.random((37, 4, 6, 6)) < 0.2).astype(np.float32))
+    m = torch.from_numpy(rng.random((37, 10)).astype(np.float32))
+    flags = (torch.arange(37) % 2).float()
+    actions = torch.from_numpy(np.where(flags.numpy() == 1, rng.integers(0, 5, 37), rng.integers(0, 9, 37)))
+    return sd, g, m, flags, actions
+
+
+def _policy_outputs(net, g, m, flags, actions) -> dict:
+    with torch.no_grad():
+        value, logits = net(g, m)
+        _, log_prob, entropy, _ = net.get_action_and_value(g, m, flags, actions)
+    return {"value": value.numpy(), "logits": logits.numpy(), "log_prob": log_prob.numpy(), "entropy": entropy.numpy()}
+
+
+def test_ctf_policy_outputs_match_the_stored_agent_outputs():
+    """CtfPolicy's values, logits, masked log-probs and entropies for fixed weights and inputs, against
+    tests/golden/ctf_policy_outputs.npz.  The record was written from CtfPolicy (PYTHONPATH=.:tests python
+    tests/test_callers_fixtures.py) at a commit where test_ctf_policy_loads_the_reference_agent_state_dict_bit_for_bit
+    passed; where the reference is importable, agent_network.Agent with the same weights is checked against the
+    record bit for bit as well."""
+    from marl_ctf_development_b200.policy import CtfPolicy
+
+    sd, g, m, flags, actions = _policy_case()
+    ours = CtfPolicy(9, 4, 6, 10)
+    ours.load_state_dict(sd, strict=True)
+    got = _policy_outputs(ours, g, m, flags, actions)
+    want = dict(np.load(POLICY_RECORD))
+    assert sorted(got) == sorted(want)
+    for k in want:   # float32 convolutions and matmuls: summation order may differ between CPU kernels
+        np.testing.assert_allclose(got[k], want[k], rtol=1e-5, atol=1e-6, err_msg=k)
+    masked = _policy_outputs(ours, g, m, flags, torch.full((37,), 6))["log_prob"]
+    assert (masked[flags.numpy() == 1] < -1e6).all() and (masked[flags.numpy() == 0] > -1e6).all()   # only 0..4 when masked
+    if rs.available():
+        ref = rs.caller_modules()["agent_network"].Agent(9, 4, 6, 10)
+        ref.load_state_dict(sd, strict=True)
+        for k, v in _policy_outputs(ref, g, m, flags, actions).items():
+            assert np.array_equal(bits(v), bits(want[k])), k
+
+
+if __name__ == "__main__":
+    from marl_ctf_development_b200.policy import CtfPolicy
+
+    sd, g, m, flags, actions = _policy_case()
+    net = CtfPolicy(9, 4, 6, 10)
+    net.load_state_dict(sd, strict=True)
+    np.savez_compressed(POLICY_RECORD, **_policy_outputs(net, g, m, flags, actions))
