@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """BASELINE config 5: self-play rollout on 8_arena with the GPU env feeding the agent_network-style policy.
 
-    python bench_rollout.py [--envs B] [--steps K] [--warmup W] [--policy-dtype bf16|fp32] [--chunk S]
+    python bench_rollout.py [--envs B] [--steps K] [--warmup W] [--policy-dtype bf16|fp32] [--chunk S] [--fused]
     torchrun --nproc-per-node N bench_rollout.py ...      (env sharding, one rank per GPU)
 
 Reports, as one JSON line from rank 0, agent-steps/s of the whole loop — policy forward for both teams on the
@@ -9,7 +9,8 @@ observation buffers the step kernel wrote, action sampling, env.step, and the pa
 trained team's observations stored into a rollout ring buffer — next to the env-only and the policy-only figures.
 With --graph the whole loop body (both policy forwards + step + store) is captured in ONE CUDA graph and replayed.
 This is a functional integration of SURVEY §8f row N1: the policy is stock torch/cuDNN (≈3.9 MFLOP per agent-step)
-and dominates the time; it is outside the hot path this repo accelerates, so this number is not the headline.
+and dominates the time.  With --fused the env is created packed-only and both teams run through FusedPolicy
+(k_policy_trunk from the packed observations, then fc1 .. heads in bf16 on cuBLAS), one forward per team.
 """
 from __future__ import annotations
 
@@ -35,6 +36,9 @@ def parse_args(argv=None):
     ap.add_argument("--channels-last", action="store_true", help="run the convolutions in NHWC (stock torch option)")
     ap.add_argument("--obs-dtype", choices=["float32", "bfloat16"], default=None,
                     help="env observation buffer type (default: bfloat16 when the policy runs in bf16)")
+    ap.add_argument("--fused", action="store_true",
+                    help="packed-only env, both teams through FusedPolicy (bf16; --chunk, --channels-last, --obs-dtype "
+                         "and --policy-dtype do not apply)")
     return ap.parse_args(argv)
 
 
@@ -54,19 +58,35 @@ def measure(args):
     B = args.envs
     obs_dtype = args.obs_dtype or ("bfloat16" if args.policy_dtype == "bf16" else "float32")
     torch.backends.cudnn.benchmark = True
-    env = GridworldCtfGPU(**experiment_env_config("8_arena"), num_envs=B, device=dev, seed=0, env_id_base=rank * B,
-                          reverse_team1_actions=True, stats="counters", obs_dtype=getattr(torch, obs_dtype), packed_obs=True)
+    if args.fused:
+        from marl_ctf_development_b200.fused_policy import FusedPolicy
+
+        obs_dtype = "packed-only"
+        env = GridworldCtfGPU(**experiment_env_config("8_arena"), num_envs=B, device=dev, seed=0, env_id_base=rank * B,
+                              reverse_team1_actions=True, stats="counters", dense_obs=False, packed_obs=True)
+    else:
+        env = GridworldCtfGPU(**experiment_env_config("8_arena"), num_envs=B, device=dev, seed=0, env_id_base=rank * B,
+                              reverse_team1_actions=True, stats="counters", obs_dtype=getattr(torch, obs_dtype),
+                              packed_obs=True)
     N, C, G, M = env.N_AGENTS, env.n_channels, env.GRID_SIZE, env.meta_size
     torch.manual_seed(rank)
     pols = [CtfPolicy(9, C, G, M).to(dev).eval() for _ in range(2)]
     if args.channels_last:
         pols = [p.to(memory_format=torch.channels_last) for p in pols]
     teams = [torch.tensor([i for i in range(N) if env.AGENT_TEAMS[i] == t], device=dev) for t in (0, 1)]
+    team_ids = [[i for i in range(N) if env.AGENT_TEAMS[i] == t] for t in (0, 1)]   # host lists: capturable
+    fused = [FusedPolicy(env, p) for p in pols] if args.fused else None
     actions = torch.empty((B, N), dtype=torch.uint8, device=dev)
     amp = torch.autocast("cuda", dtype=torch.bfloat16, enabled=args.policy_dtype == "bf16")
 
     @torch.no_grad()
     def policy_step(obs, meta):
+        if fused is not None:
+            for idx, ids, fp in zip(teams, team_ids, fused):
+                k = len(ids)
+                f = env.use_action_mask[idx].unsqueeze(0).expand(B, k).reshape(B * k)
+                actions[:, idx] = fp.get_action(f, agent_ids=ids).reshape(B, k).to(torch.uint8)
+            return
         for idx, pol in zip(teams, pols):
             k = idx.numel()
             g = obs[:, idx].reshape(B * k, C, G, G)
@@ -147,16 +167,20 @@ def measure(args):
             "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": ms_full / args.steps, "env_ms_per_step": ms_env / args.steps, "policy_ms_per_step": ms_pol / args.steps,
             "cuda_graph": bool(args.graph),
+            "policy_path": "fused" if args.fused else "cudnn",
             "rollout_storage": f"packed observations of the trained team, ring of {args.store_steps} steps: "
                                f"{ring.numel() * 4 / 1e6:.0f} MB (float32 would be {ring.numel() * 4 * 32 / 1e9:.1f} GB)",
             "config": {"workload": f"8_arena self-play rollout, B={B} envs/GPU, CtfPolicy (agent_network.py architecture) "
-                                   f"for both teams, policy dtype {args.policy_dtype}, {obs_dtype} observations"
-                                   f"{', channels_last' if args.channels_last else ''}; env-only = step + packed rollout store",
+                                   f"for both teams, "
+                                   + ("FusedPolicy (k_policy_trunk + bf16 cuBLAS heads), packed-only env" if args.fused else
+                                      f"policy dtype {args.policy_dtype}, {obs_dtype} observations"
+                                      f"{', channels_last' if args.channels_last else ''}")
+                                   + "; env-only = step + packed rollout store",
                        "envs_per_gpu": B},
             "data": "synthetic (random-init policies)",
         })
     env.close()
-    del env, ring, ring_meta, pols, graphs
+    del env, ring, ring_meta, pols, graphs, fused
     torch.cuda.empty_cache()
     return result
 

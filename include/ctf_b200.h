@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 4
+#define CTF_ABI_VERSION 5
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -260,6 +260,35 @@ typedef struct ctf_kernel_info {
     int reserved;
 } ctf_kernel_info_t;
 int ctf_get_kernel_info(ctf_handle_t h, ctf_kernel_info_t* out);
+
+/*
+ * Policy inference from packed observations (no reference counterpart: the reference feeds agent_network.Agent a dense
+ * float32 grid).  Weights of the convolutional trunk of policy.CtfPolicy; all pointers are device memory.
+ */
+typedef struct ctf_policy_weights {
+    const float* conv1_w;   /* [16][C][3][3] fp32 (conv1.weight as stored by torch) */
+    const float* conv1_b;   /* [16] */
+    const void*  conv2_w;   /* bf16 [9 taps][4 n-tiles][32 lanes][4], the mma.sync B-fragment order that
+                               fused_policy.conv2_kernel_layout_index() gives from conv2.weight [32][16][3][3] */
+    const float* conv2_b;   /* [32] */
+} ctf_policy_weights_t;
+
+/*
+ * Trunk of CtfPolicy (conv1 -> tanh -> conv2 -> tanh -> flatten, then the metadata) computed from packed
+ * observations: writes one bf16 feature row per sample, [32*(G-4)^2 conv2 outputs in (c, y, x) order | M metadata
+ * values | zeros up to feature_stride], i.e. the fc1 input.  Sample s = e*k + j (e < n_envs, j < k) reads packed
+ * block e*agents_per_env + agent_ids[j] ([bits_words_per_agent] uint32, outputs.obs_bits layout) and the metadata row
+ * ([M] float32) with the same index: agents_per_env = N with a team's ids reads outputs.obs_bits / outputs.meta in
+ * place, agents_per_env = 1 with id 0 reads contiguous rows (e.g. a rollout buffer).
+ * conv1 is exact fp32 sparse accumulation over the set bits (any {0,1} input), tanhf, rounded to bf16; conv2 runs on
+ * tensor cores (bf16 inputs and weights, fp32 accumulation, fp32 bias, tanhf, rounded to bf16).  Deterministic (no
+ * atomics), no allocation and no host synchronisation: capturable in a CUDA graph.
+ * agent_ids: host array of k (1..8) ids < agents_per_env.  features: 16-byte aligned; feature_stride: elements per
+ * row, a multiple of 8 and >= 32*(G-4)^2 + M.
+ */
+int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uint32_t* packed, const float* meta,
+                        int64_t n_envs, int agents_per_env, const uint8_t* agent_ids, int k,
+                        void* features, int64_t feature_stride, void* stream);
 
 #ifdef __cplusplus
 }

@@ -3,6 +3,7 @@
 Public surface:
     GridworldCtfGPU   batched env (B envs per GPU), device tensors in / out
     GridworldCtf      single-env view with the reference's exact methods (drop-in for ppo.py / utils.py)
+    FusedPolicy       CtfPolicy inference from packed observations (fused_policy.py)
     compile_config    (AGENT_CONFIG, SCENARIO, kwargs) -> ctf_config_t
     experiment_env_config / experiment_names   the reference's nine experiment configs as data
 """
@@ -16,4 +17,8 @@ def __getattr__(name):
         from . import env
 
         return getattr(env, name)
+    if name == "FusedPolicy":
+        from .fused_policy import FusedPolicy
+
+        return FusedPolicy
     raise AttributeError(name)

@@ -26,8 +26,9 @@ EXPORTS = (
     "ctf_take_faults",
     "ctf_step_host",
     "ctf_get_kernel_info",
+    "ctf_policy_features",
 )
-ABI_VERSION = 4
+ABI_VERSION = 5
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
 
 
@@ -74,6 +75,10 @@ class CtfKernelInfo(C.Structure):
                 ("min_envs_for_persistent", C.c_int64), ("warp_per_env_ctas_per_sm", C.c_int), ("reserved", C.c_int)]
 
 
+class CtfPolicyWeights(C.Structure):
+    _fields_ = [("conv1_w", C.c_void_p), ("conv1_b", C.c_void_p), ("conv2_w", C.c_void_p), ("conv2_b", C.c_void_p)]
+
+
 class NativeError(RuntimeError):
     pass
 
@@ -118,6 +123,8 @@ def load():
     L.ctf_take_faults.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
     L.ctf_get_kernel_info.argtypes = [C.c_void_p, C.POINTER(CtfKernelInfo)]
     L.ctf_step_host.argtypes = [C.c_void_p, CtfState, C.c_void_p, CtfOutputs, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.ctf_policy_features.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
+                                      C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]
     if L.ctf_abi_version() != ABI_VERSION:
         raise NativeError(f"ABI version mismatch: library {L.ctf_abi_version()}, binding {ABI_VERSION}")
     if L.ctf_config_size() != C.sizeof(CtfConfig):

@@ -1145,6 +1145,184 @@ __global__ void k_stats_sum(const uint32_t* __restrict__ stats, long long B, int
     if (acc) atomicAdd(&out[k], acc);
 }
 
+// ------------------------------------------------------------------------------------------------
+// policy trunk from packed observations: conv1 (sparse, fp32) -> tanh -> conv2 (mma.sync bf16) -> tanh -> fc1 input rows
+// ------------------------------------------------------------------------------------------------
+// One warp owns one sample at a time (grid-stride over samples); the CTA's warps share the conv weights in shared memory.
+// Per sample: the wpa packed words are staged, a per-cell channel mask is built from them, conv1 accumulates for every
+// output position the bias plus the weight columns of the set (cell, channel) pairs of its 3x3 window (exact for any
+// {0,1} input; cost grows with the number of set bits), and stores tanh as bf16 in a [position][16 channels] tile.
+// conv2 is an implicit GEMM on that tile: M = (G-4)^2 positions, N = 32 channels, K = 9 taps x 16 channels, one
+// m16n8k16 k-step per tap.  The epilogue writes one n-tile (8 channels = a contiguous 8*(G-4)^2 run of the (c, y, x)
+// feature row) at a time through shared memory so that the row is written with 16-byte stores.
+constexpr int kTrunkWarps = 8;
+constexpr int kTrunkThreads = kTrunkWarps * 32;
+constexpr int kTrunkW2Words = 9 * 4 * 32 * 2;   // conv2 B fragments: [tap][n-tile][lane][2 x bf16x2]
+
+struct TrunkArgs {
+    const float* conv1_w;
+    const float* conv1_b;
+    const uint2* conv2_w;
+    const float* conv2_b;
+    const uint32_t* packed;
+    const float* meta;
+    __nv_bfloat16* features;
+    long long n_samples;
+    long long stride;
+    int ape, k;
+    int G, C, GG, wpa, M;
+    int S1, S2;              // conv1 / conv2 output side
+    int warp_words;          // shared-memory words per warp
+    int off_mask, off_act, off_stage;   // word offsets inside a warp's region
+    unsigned char ids[CTF_MAX_AGENTS];
+};
+
+__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
+    const __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
+    return *reinterpret_cast<const uint32_t*>(&v);
+}
+
+__global__ void __launch_bounds__(kTrunkThreads) k_policy_trunk(const __grid_constant__ TrunkArgs A) {
+    extern __shared__ uint4 smem_raw[];
+    float* w1 = reinterpret_cast<float*>(smem_raw);                      // [C*9][16]: column of one (c, dy, dx) tap
+    float* b1 = w1 + A.C * 9 * 16;                                        // [16]
+    float* b2 = b1 + 16;                                                  // [32]
+    uint2* w2 = reinterpret_cast<uint2*>(b2 + 32);                        // [9][4][32]
+    uint32_t* warp_base = reinterpret_cast<uint32_t*>(w2 + kTrunkW2Words / 2);
+    const int C = A.C, G = A.G, GG = A.GG, S1 = A.S1, S2 = A.S2, M2 = S2 * S2;
+    for (int i = threadIdx.x; i < C * 9 * 16; i += kTrunkThreads) {
+        const int o = i & 15, tap = i >> 4;                              // tap = c*9 + dy*3 + dx
+        w1[i] = A.conv1_w[o * C * 9 + tap];
+    }
+    if (threadIdx.x < 16) b1[threadIdx.x] = A.conv1_b[threadIdx.x];
+    if (threadIdx.x < 32) b2[threadIdx.x] = A.conv2_b[threadIdx.x];
+    for (int i = threadIdx.x; i < kTrunkW2Words / 2; i += kTrunkThreads) w2[i] = A.conv2_w[i];
+    __syncthreads();
+
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t* bits = warp_base + (size_t)warp * A.warp_words;                           // [wpa]
+    uint16_t* cmask = reinterpret_cast<uint16_t*>(bits + A.off_mask);                   // [GG] channel mask per cell
+    uint32_t* act = bits + A.off_act;                                                    // [S1*S1][8] bf16x2
+    __nv_bfloat16* stage = reinterpret_cast<__nv_bfloat16*>(bits + A.off_stage);        // [8][M2]
+    const int g = lane >> 2, t = lane & 3;
+    const int n_mt = (M2 + 15) >> 4;
+    const long long conv_elems = 32LL * M2;
+
+    for (long long s = (long long)blockIdx.x * kTrunkWarps + warp; s < A.n_samples; s += (long long)gridDim.x * kTrunkWarps) {
+        const long long e = s / A.k;
+        const int j = (int)(s - e * A.k);
+        const long long blk = e * A.ape + A.ids[j];
+        const uint32_t* src = A.packed + blk * A.wpa;
+        for (int i = lane; i < A.wpa; i += 32) bits[i] = __ldg(src + i);
+        __syncwarp();
+        // channel mask of every cell: bit c = element c*GG + p
+        for (int p = lane; p < GG; p += 32) {
+            uint32_t m = 0;
+            for (int c = 0; c < C; ++c) {
+                const int el = c * GG + p;
+                m |= ((bits[el >> 5] >> (el & 31)) & 1u) << c;
+            }
+            cmask[p] = (uint16_t)m;
+        }
+        __syncwarp();
+        // conv1: bias + the weight columns of the set (cell, channel) pairs, fixed order (dy, dx, c ascending)
+        for (int q = lane; q < S1 * S1; q += 32) {
+            const int y = q / S1, x = q - y * S1;
+            float acc[16];
+#pragma unroll
+            for (int o = 0; o < 16; ++o) acc[o] = b1[o];
+            for (int dy = 0; dy < 3; ++dy) {
+                for (int dx = 0; dx < 3; ++dx) {
+                    uint32_t m = cmask[(y + dy) * G + x + dx];
+                    while (m) {
+                        const int c = __ffs(m) - 1;
+                        m &= m - 1;
+                        const float4* col = reinterpret_cast<const float4*>(w1 + ((c * 3 + dy) * 3 + dx) * 16);
+#pragma unroll
+                        for (int v = 0; v < 4; ++v) {
+                            const float4 wv = col[v];
+                            acc[4 * v] += wv.x; acc[4 * v + 1] += wv.y; acc[4 * v + 2] += wv.z; acc[4 * v + 3] += wv.w;
+                        }
+                    }
+                }
+            }
+            uint4 lo, hi;
+            lo.x = pack_bf16x2(tanhf(acc[0]), tanhf(acc[1]));   lo.y = pack_bf16x2(tanhf(acc[2]), tanhf(acc[3]));
+            lo.z = pack_bf16x2(tanhf(acc[4]), tanhf(acc[5]));   lo.w = pack_bf16x2(tanhf(acc[6]), tanhf(acc[7]));
+            hi.x = pack_bf16x2(tanhf(acc[8]), tanhf(acc[9]));   hi.y = pack_bf16x2(tanhf(acc[10]), tanhf(acc[11]));
+            hi.z = pack_bf16x2(tanhf(acc[12]), tanhf(acc[13])); hi.w = pack_bf16x2(tanhf(acc[14]), tanhf(acc[15]));
+            reinterpret_cast<uint4*>(act)[2 * q] = lo;
+            reinterpret_cast<uint4*>(act)[2 * q + 1] = hi;
+        }
+        __syncwarp();
+        __nv_bfloat16* row = A.features + s * A.stride;
+        // conv2: n-tile (8 output channels) outer, m-tile (16 positions) inner, one k-step per tap
+        for (int nt = 0; nt < 4; ++nt) {
+            const float bias0 = b2[8 * nt + 2 * t], bias1 = b2[8 * nt + 2 * t + 1];
+            for (int mt = 0; mt < n_mt; ++mt) {
+                const int m0 = min(mt * 16 + g, M2 - 1), m1 = min(mt * 16 + g + 8, M2 - 1);   // pad rows: any valid position
+                const int y0 = m0 / S2, y1 = m1 / S2;
+                const int p0 = y0 * S1 + (m0 - y0 * S2), p1 = y1 * S1 + (m1 - y1 * S2);
+                float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f;
+#pragma unroll
+                for (int tap = 0; tap < 9; ++tap) {
+                    const int off = (tap / 3) * S1 + (tap % 3);
+                    const uint32_t a0 = act[(p0 + off) * 8 + t], a1 = act[(p1 + off) * 8 + t];
+                    const uint32_t a2 = act[(p0 + off) * 8 + t + 4], a3 = act[(p1 + off) * 8 + t + 4];
+                    const uint2 b = w2[(tap * 4 + nt) * 32 + lane];
+                    asm volatile(
+                        "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
+                        "{%0,%1,%2,%3};\n"
+                        : "+f"(d0), "+f"(d1), "+f"(d2), "+f"(d3)
+                        : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b.x), "r"(b.y));
+                }
+                const int r0 = mt * 16 + g, r1 = r0 + 8;
+                if (r0 < M2) {
+                    stage[(2 * t) * M2 + r0] = __float2bfloat16_rn(tanhf(d0 + bias0));
+                    stage[(2 * t + 1) * M2 + r0] = __float2bfloat16_rn(tanhf(d1 + bias1));
+                }
+                if (r1 < M2) {
+                    stage[(2 * t) * M2 + r1] = __float2bfloat16_rn(tanhf(d2 + bias0));
+                    stage[(2 * t + 1) * M2 + r1] = __float2bfloat16_rn(tanhf(d3 + bias1));
+                }
+            }
+            __syncwarp();
+            // channels 8nt .. 8nt+7 are elements [8nt*M2, 8(nt+1)*M2) of the row: 16*M2 bytes, 16-byte aligned
+            uint4* dst = reinterpret_cast<uint4*>(row + (long long)8 * nt * M2);
+            const uint4* sv = reinterpret_cast<const uint4*>(stage);
+            for (int i = lane; i < M2; i += 32) dst[i] = sv[i];
+            __syncwarp();
+        }
+        // metadata as bf16, then zeros up to the stride (8 elements per 16-byte store)
+        const float* mrow = A.meta + blk * A.M;
+        const int tail = (int)((A.stride - conv_elems) >> 3);
+        uint4* dst = reinterpret_cast<uint4*>(row + conv_elems);
+        for (int i = lane; i < tail; i += 32) {
+            float v[8];
+#pragma unroll
+            for (int u = 0; u < 8; ++u) {
+                const int c = 8 * i + u;
+                v[u] = c < A.M ? __ldg(mrow + c) : 0.f;
+            }
+            dst[i] = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+        }
+        __syncwarp();
+    }
+}
+
+// shared-memory layout of k_policy_trunk for a plan: bytes of the CTA-wide weights, words per warp and the offsets
+static __host__ void trunk_layout(const DevPlan& P, TrunkArgs& A, size_t& smem) {
+    const int S1 = P.G - 2, S2 = P.G - 4;
+    const auto up4 = [](int w) { return (w + 3) & ~3; };                 // 16-byte alignment in words
+    A.G = P.G; A.C = P.C; A.GG = P.GG; A.wpa = P.wpa; A.M = P.M; A.S1 = S1; A.S2 = S2;
+    A.off_mask = up4(P.wpa);
+    A.off_act = A.off_mask + up4((P.GG + 1) / 2);
+    A.off_stage = A.off_act + S1 * S1 * 8;
+    A.warp_words = A.off_stage + up4(4 * S2 * S2);                       // 8 channels x S2^2 bf16
+    const size_t shared_words = (size_t)P.C * 9 * 16 + 16 + 32 + kTrunkW2Words;
+    smem = (shared_words + (size_t)kTrunkWarps * A.warp_words) * 4;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -1171,6 +1349,8 @@ struct ctf_env {
     int n_sm;
     int k_step_ctas_per_sm;  // resident-CTA cap of the warp-per-env kernels (0: whatever fits)
     size_t ws_smem_bytes;
+    size_t trunk_smem_bytes; // k_policy_trunk: dynamic shared memory for this plan
+    int trunk_ctas;          // k_policy_trunk: CTAs that fit on the device at once
 };
 
 // cudaSetDevice for the duration of an entry point; the caller's current device is restored on return
@@ -1430,6 +1610,16 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
     CTF_SET_SMEM((k_step_ws<T, false, true>), ws_smem); CTF_SET_SMEM((k_step_ws<T, true, true>), ws_smem);     \
     CTF_SET_SMEM((k_unpack<T>), smem)
     CTF_SET_SMEM_T(float); CTF_SET_SMEM_T(uint8_t); CTF_SET_SMEM_T(__half); CTF_SET_SMEM_T(__nv_bfloat16);
+    // k_policy_trunk needs at most 94 KB (G = 16, C = 14); the ceiling is per kernel, so it covers every plan
+    CTF_SET_SMEM(k_policy_trunk, 100 * 1024);
+    {
+        TrunkArgs ta;
+        trunk_layout(h->plan, ta, h->trunk_smem_bytes);
+        int per_sm = 0;
+        if (e == cudaSuccess && h->plan.G >= 5)
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk, kTrunkThreads, h->trunk_smem_bytes);
+        h->trunk_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
+    }
 #undef CTF_SET_SMEM_T
 #undef CTF_SET_SMEM
     if (e != cudaSuccess) {
@@ -1611,6 +1801,45 @@ extern "C" int ctf_unpack_obs(ctf_handle_t h, const uint32_t* packed, void* out,
         using T = decltype(tag);
         k_unpack<T><<<grid, kUnpackThreads, smem, s>>>(packed, static_cast<T*>(out), n_agent_blocks, nbits, wpa, chunk, bits_words);
     });
+    CTF_CUDA(cudaGetLastError());
+    return CTF_OK;
+}
+
+extern "C" int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uint32_t* packed, const float* meta,
+                                   int64_t n_envs, int agents_per_env, const uint8_t* agent_ids, int k, void* features,
+                                   int64_t feature_stride, void* stream) {
+    if (!h || !w || !packed || !meta || !agent_ids || !features) return fail(CTF_ERR_INVALID, "ctf_policy_features: null argument");
+    if (!w->conv1_w || !w->conv1_b || !w->conv2_w || !w->conv2_b)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features: null weight pointer");
+    const DevPlan& P = h->plan;
+    if (P.G < 5) return fail(CTF_ERR_INVALID, "ctf_policy_features: the policy needs grid_size >= 5 (two valid 3x3 convolutions)");
+    if (k < 1 || k > CTF_MAX_AGENTS) return fail(CTF_ERR_INVALID, "ctf_policy_features: k must be in 1..8");
+    if (agents_per_env < 1) return fail(CTF_ERR_INVALID, "ctf_policy_features: agents_per_env must be >= 1");
+    if (n_envs < 0) return fail(CTF_ERR_INVALID, "ctf_policy_features: negative n_envs");
+    for (int j = 0; j < k; ++j)
+        if (agent_ids[j] >= agents_per_env) return fail(CTF_ERR_INVALID, "ctf_policy_features: an agent id is >= agents_per_env");
+    const long long k1 = 32LL * (P.G - 4) * (P.G - 4) + P.M;
+    if (feature_stride < k1 || (feature_stride & 7))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features: feature_stride must be a multiple of 8 and >= 32*(G-4)^2 + M");
+    if (reinterpret_cast<uintptr_t>(features) & 15) return fail(CTF_ERR_INVALID, "ctf_policy_features: features must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(w->conv1_w) & 15) || (reinterpret_cast<uintptr_t>(w->conv2_w) & 7) ||
+        (reinterpret_cast<uintptr_t>(packed) & 3) || (reinterpret_cast<uintptr_t>(meta) & 3))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features: misaligned weights or inputs");
+    const long long n = (long long)n_envs * k;
+    if (n == 0) return CTF_OK;
+    TrunkArgs A;
+    memset(&A, 0, sizeof(A));
+    size_t smem = 0;
+    trunk_layout(P, A, smem);
+    A.conv1_w = w->conv1_w; A.conv1_b = w->conv1_b; A.conv2_w = static_cast<const uint2*>(w->conv2_w); A.conv2_b = w->conv2_b;
+    A.packed = packed; A.meta = meta; A.features = static_cast<__nv_bfloat16*>(features);
+    A.n_samples = n; A.stride = feature_stride; A.ape = agents_per_env; A.k = k;
+    for (int j = 0; j < k; ++j) A.ids[j] = agent_ids[j];
+    DeviceGuard guard(h->device);
+    CTF_CUDA(guard.err);
+    const long long want = (n + kTrunkWarps - 1) / kTrunkWarps;
+    const unsigned grid = (unsigned)(want < h->trunk_ctas ? want : h->trunk_ctas);
+    k_policy_trunk<<<grid, kTrunkThreads, smem, static_cast<cudaStream_t>(stream)>>>(A);
     CTF_CUDA(cudaGetLastError());
     return CTF_OK;
 }

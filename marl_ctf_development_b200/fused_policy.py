@@ -1,0 +1,249 @@
+"""Policy inference from packed observations: the trunk of ``CtfPolicy`` as one CUDA kernel.
+
+``FusedPolicy(env, policy)`` runs a ``CtfPolicy`` (or the reference ``Agent``'s weights loaded into one) for rollouts,
+duels and league evaluation without dense observations.  ``ctf_policy_features`` (``k_policy_trunk`` in
+csrc/ctf_kernels.cu) reads the env's packed 1-bit observations (``env.obs_bits``) and metadata in place and writes
+one bf16 fc1 input row per sample: conv1 by sparse fp32 accumulation over the set bits, tanh, bf16, conv2 on tensor
+cores with fp32 accumulation, tanh, bf16, then the metadata.  fc1 -> tanh -> fc2 -> tanh -> heads run in torch
+(cuBLAS, bf16 weights, fp32 accumulation) on those rows: fc1 runs over the whole stride with fc1.weight zero-padded
+to it (the pad columns of the rows are exact zeros), which keeps K a multiple of 8 for cuBLAS.  The env can then be created packed-only
+(``dense_obs=False, packed_obs=True``) and never writes the dense observation tensor.
+
+Precision: this is a bf16 path, like running ``CtfPolicy`` under ``torch.autocast(dtype=torch.bfloat16)``; it is not
+bit-equal to fp32 ``CtfPolicy``.  ``reference_features`` states in torch exactly what the kernel computes.
+Inference only: the PPO update keeps using ``CtfPolicy`` on ``env.unpack_obs`` output.
+"""
+from __future__ import annotations
+
+import ctypes as C
+
+import torch
+import torch.nn.functional as F
+from torch.distributions.categorical import Categorical
+
+from . import _native
+
+N_ACTIONS = 9
+MAX_IDS = 8
+
+
+def trunk_dims(n_channels: int, grid_size: int, metadata_size: int):
+    """(K1, feature_stride): fc1 input width 32*(G-4)^2 + M and the row stride of the kernel's output (multiple of 8)."""
+    side = grid_size - 4
+    k1 = 32 * side * side + metadata_size
+    return k1, (k1 + 7) // 8 * 8
+
+
+def conv2_kernel_layout_index(device=None) -> torch.Tensor:
+    """Index into ``conv2.weight.reshape(-1)`` ([32][16][3][3]) that gives the kernel's bf16 layout
+    [tap 9][n-tile 4][lane 32][4]: the two mma.sync m16n8k16 B registers of every lane.  Lane 4*g + t of n-tile j holds,
+    for output channel 8*j + g, input channels (2t, 2t+1, 2t+8, 2t+9) of the tap (K = the 16 input channels of a tap)."""
+    tap = torch.arange(9).view(9, 1, 1, 1)
+    nt = torch.arange(4).view(1, 4, 1, 1)
+    lane = torch.arange(32).view(1, 1, 32, 1)
+    g, t = lane // 4, lane % 4
+    ci = 2 * t + torch.tensor([0, 1, 8, 9]).view(1, 1, 1, 4)
+    return ((8 * nt + g) * 144 + ci * 9 + tap).reshape(-1).to(device)
+
+
+@torch.no_grad()
+def reference_conv1(policy, dense_obs: torch.Tensor, round_bf16: bool = True) -> torch.Tensor:
+    """conv1 -> tanh as ``k_policy_trunk`` computes it: [S, 16, G-2, G-2] float32.  Every output starts at its fp32 bias
+    and adds ``x * W1[:, c, dy, dx]`` in the kernel's order (dy, dx, then c ascending), one fp32 rounding per term; for
+    {0,1} inputs the products are exact and the sum is bit-for-bit the kernel's.  Then tanh, and bf16 if round_bf16."""
+    x = dense_obs.float()
+    S, Cn, G, _ = x.shape
+    S1 = G - 2
+    w1 = policy.conv1.weight.float()
+    acc = policy.conv1.bias.float().view(1, 16, 1, 1).expand(S, 16, S1, S1).clone()
+    for dy in range(3):
+        for dx in range(3):
+            for c in range(Cn):
+                acc += x[:, c : c + 1, dy : dy + S1, dx : dx + S1] * w1[:, c, dy, dx].view(1, 16, 1, 1)
+    h1 = torch.tanh(acc)
+    return h1.bfloat16().float() if round_bf16 else h1
+
+
+@torch.no_grad()
+def reference_features(policy, dense_obs: torch.Tensor, meta: torch.Tensor, round_bf16: bool = True) -> torch.Tensor:
+    """What ``k_policy_trunk`` computes, in torch: [S, K1] float32 (bf16 values when ``round_bf16``).
+
+    conv1 summed in fp32 in the kernel's order (``reference_conv1``), tanh, bf16; conv2 of those bf16 activations with
+    bf16 weights, summed exactly and rounded to fp32 (the kernel accumulates in fp32 on tensor cores, in an order of the
+    hardware's), + fp32 bias, tanh, bf16; flattened in (c, y, x) order, then the metadata as bf16.  With
+    round_bf16=False every rounding to bf16 is skipped, and the rows fed through fc1 ... heads reproduce
+    ``CtfPolicy.forward`` in fp32.
+    """
+    bf = (lambda x: x.bfloat16().float()) if round_bf16 else (lambda x: x)
+    h1 = reference_conv1(policy, dense_obs, round_bf16)
+    w2 = bf(policy.conv2.weight.float()).double()
+    h2 = F.conv2d(h1.double(), w2).float() + policy.conv2.bias.float().view(1, -1, 1, 1)
+    h2 = bf(torch.tanh(h2))
+    return torch.cat((h2.reshape(h2.shape[0], -1), bf(meta.float())), dim=1)
+
+
+class FusedPolicy:
+    """Inference-only view of a ``CtfPolicy`` that reads packed observations (see the module docstring).
+
+    ``refresh()`` copies the module's current weights into persistent device buffers in place (called once here;
+    call it again after every optimiser step): a CUDA graph captured around ``forward_*`` stays valid.
+    """
+
+    def __init__(self, env, policy):
+        self.env, self.policy = env, policy
+        Cn, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
+        if G < 5:
+            raise ValueError(f"the policy needs GRID_SIZE >= 5 (two valid 3x3 convolutions), env has {G}")
+        self.k1, self.stride = trunk_dims(Cn, G, M)
+        want = {
+            "conv1.weight": (16, Cn, 3, 3), "conv2.weight": (32, 16, 3, 3), "fc1.weight": (256, self.k1),
+            "fc2.weight": (128, 256), "action_head.weight": (N_ACTIONS, 128), "value_head.weight": (1, 128),
+        }
+        for name, shape in want.items():
+            mod, attr = name.split(".")
+            got = tuple(getattr(getattr(policy, mod, None), attr, torch.empty(0)).shape)
+            if got != shape:
+                raise ValueError(f"policy {name} has shape {got}; this env (C={Cn}, G={G}, M={M}, {N_ACTIONS} actions) "
+                                 f"needs {shape}")
+        if policy.conv1.weight.device != env.device:
+            raise ValueError(f"policy is on {policy.conv1.weight.device}, env on {env.device}")
+        dev = env.device
+        bf = dict(dtype=torch.bfloat16, device=dev)
+        self._c1w = torch.empty((16, Cn, 3, 3), dtype=torch.float32, device=dev)
+        self._c1b = torch.empty(16, dtype=torch.float32, device=dev)
+        self._c2w = torch.empty(9 * 4 * 32 * 4, **bf)
+        self._c2b = torch.empty(32, dtype=torch.float32, device=dev)
+        self._c2_index = conv2_kernel_layout_index(dev)
+        # fc1.weight in columns :K1, zeros up to the row stride
+        self._fc1w, self._fc1b = torch.zeros((256, self.stride), **bf), torch.empty(256, **bf)
+        self._fc2w, self._fc2b = torch.empty((128, 256), **bf), torch.empty(128, **bf)
+        self._hw, self._hb = torch.empty((1 + N_ACTIONS, 128), **bf), torch.empty(1 + N_ACTIONS, **bf)  # value | logits
+        self._weights = _native.CtfPolicyWeights(self._c1w.data_ptr(), self._c1b.data_ptr(), self._c2w.data_ptr(),
+                                                 self._c2b.data_ptr())
+        self._features = None   # bf16 [S_max, stride] rows, reused by every call (see features())
+        self._ids = {}
+        self.refresh()
+
+    @torch.no_grad()
+    def refresh(self):
+        """Copies the policy's current weights into the persistent buffers, on the device (no host round trip)."""
+        p = self.policy
+        self._c1w.copy_(p.conv1.weight)
+        self._c1b.copy_(p.conv1.bias)
+        self._c2w.copy_(p.conv2.weight.reshape(-1)[self._c2_index])
+        self._c2b.copy_(p.conv2.bias)
+        self._fc1w[:, : self.k1].copy_(p.fc1.weight)
+        self._fc1b.copy_(p.fc1.bias)
+        self._fc2w.copy_(p.fc2.weight)
+        self._fc2b.copy_(p.fc2.bias)
+        self._hw[:1].copy_(p.value_head.weight)
+        self._hw[1:].copy_(p.action_head.weight)
+        self._hb[:1].copy_(p.value_head.bias)
+        self._hb[1:].copy_(p.action_head.bias)
+
+    # ------------------------------------------------------------------ plumbing
+    def _env_for(self, env):
+        if env is None:
+            return self.env
+        mine = (self.env.n_channels, self.env.GRID_SIZE, self.env.meta_size, self.env.bits_words_per_agent)
+        if (env.n_channels, env.GRID_SIZE, env.meta_size, env.bits_words_per_agent) != mine or env.device != self.env.device:
+            raise ValueError("env does not have the shapes (C, G, M) or the device this FusedPolicy was built for")
+        return env
+
+    def _id_array(self, agent_ids, n_per_env):
+        ids = tuple(int(i) for i in (agent_ids.tolist() if isinstance(agent_ids, torch.Tensor) else agent_ids))
+        if not 1 <= len(ids) <= MAX_IDS:
+            raise ValueError(f"agent_ids must name 1..{MAX_IDS} agents, got {len(ids)}")
+        if any(i < 0 or i >= n_per_env for i in ids):
+            raise ValueError(f"agent_ids {ids} out of range for {n_per_env} agents per env")
+        arr = self._ids.get(ids)
+        if arr is None:
+            arr = self._ids[ids] = (C.c_uint8 * len(ids))(*ids)
+        return arr, len(ids)
+
+    def features(self, n_samples: int) -> torch.Tensor:
+        """bf16 [n_samples, stride] feature rows: the first rows of ONE buffer per FusedPolicy, sized for the largest
+        sample count seen so far (8_arena, B = 65 536, one team: 2 GB).  A call with more samples than ever before
+        replaces the buffer, so warm up with the largest forward before capturing a CUDA graph around this policy."""
+        if self._features is None or self._features.shape[0] < n_samples:
+            self._features = None   # release the old rows before allocating the larger ones
+            self._features = torch.empty((n_samples, self.stride), dtype=torch.bfloat16, device=self.env.device)
+        return self._features[:n_samples]
+
+    def _trunk(self, env, packed_ptr, meta_ptr, n_envs, agents_per_env, ids, k):
+        feat = self.features(n_envs * k)
+        stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
+        _native.check(env._lib.ctf_policy_features(
+            env._handle, C.byref(self._weights), C.c_void_p(packed_ptr), C.c_void_p(meta_ptr), n_envs, agents_per_env,
+            ids, k, C.c_void_p(feat.data_ptr()), self.stride, stream))
+        return feat
+
+    def _head(self, feat):
+        x = torch.tanh(F.linear(feat, self._fc1w, self._fc1b))
+        x = torch.tanh(F.linear(x, self._fc2w, self._fc2b))
+        out = F.linear(x, self._hw, self._hb).float()
+        return out[:, :1], out[:, 1:]
+
+    # ------------------------------------------------------------------ trunk and forwards
+    def trunk_from_env(self, agent_ids, env=None, envs=None) -> torch.Tensor:
+        """bf16 feature rows [S, stride] (the fc1 input in columns :K1, zeros after) for the agents ``agent_ids`` of
+        every env (or of ``envs``, a slice of env indices), read in place from ``env.obs_bits`` / ``env.meta``; sample
+        s = e*k + j is agent agent_ids[j] of env e.  ``env`` defaults to the one given at construction (any env of the
+        same shapes may be passed).  The rows live in a buffer that the next call overwrites (see ``features``)."""
+        env = self._env_for(env)
+        if env.obs_bits is None:
+            raise ValueError("FusedPolicy reads env.obs_bits: create the env with packed_obs=True")
+        N, wpa, M = env.N_AGENTS, env.bits_words_per_agent, env.meta_size
+        e0, e1, step = (envs if envs is not None else slice(None)).indices(env.num_envs)
+        if step != 1 or e1 < e0:
+            raise ValueError("envs must be a contiguous slice of env indices")
+        ids, k = self._id_array(agent_ids, N)
+        return self._trunk(env, env.obs_bits.data_ptr() + e0 * N * wpa * 4, env.meta.data_ptr() + e0 * N * M * 4,
+                           e1 - e0, N, ids, k)
+
+    def trunk_packed(self, bits: torch.Tensor, meta: torch.Tensor) -> torch.Tensor:
+        """Feature rows (as ``trunk_from_env``) for packed observations ``bits`` int32 [S, wpa] and ``meta`` [S, M]."""
+        env = self.env
+        wpa, M = env.bits_words_per_agent, env.meta_size
+        if bits.dtype != torch.int32 or bits.dim() != 2 or bits.shape[1] != wpa or bits.device != env.device:
+            raise ValueError(f"bits must be an int32 tensor [S, {wpa}] on {env.device}")
+        if meta.dtype != torch.float32 or tuple(meta.shape) != (bits.shape[0], M) or meta.device != env.device:
+            raise ValueError(f"meta must be a float32 tensor [{bits.shape[0]}, {M}] on {env.device}")
+        bits, meta = bits.contiguous(), meta.contiguous()
+        ids, _ = self._id_array((0,), 1)
+        return self._trunk(env, bits.data_ptr(), meta.data_ptr(), bits.shape[0], 1, ids, 1)
+
+    @torch.no_grad()
+    def forward_from_env(self, agent_ids, env=None, envs=None):
+        """(value [S, 1], logits [S, 9]) fp32 for the samples of ``trunk_from_env``."""
+        return self._head(self.trunk_from_env(agent_ids, env, envs))
+
+    @torch.no_grad()
+    def forward_packed(self, bits: torch.Tensor, meta: torch.Tensor):
+        """(value [S, 1], logits [S, 9]) fp32 for packed observations ``bits`` int32 [S, wpa] and ``meta`` [S, M]."""
+        return self._head(self.trunk_packed(bits, meta))
+
+    def forward(self, agent_ids=None, bits=None, meta=None, env=None, envs=None):
+        if agent_ids is not None:
+            return self.forward_from_env(agent_ids, env=env, envs=envs)
+        if bits is None or meta is None:
+            raise ValueError("pass agent_ids (read the env in place) or bits and meta")
+        return self.forward_packed(bits, meta)
+
+    __call__ = forward
+
+    @torch.no_grad()
+    def get_action_and_value(self, use_action_mask, action=None, *, agent_ids=None, bits=None, meta=None, env=None,
+                             envs=None):
+        """``CtfPolicy.get_action_and_value``'s (action, log_prob, entropy, value) for the samples of ``forward``;
+        use_action_mask is the per-sample flag in sample order.  Masking is ``CtfPolicy.masked_logits``."""
+        value, logits = self.forward(agent_ids, bits, meta, env, envs)
+        probs = Categorical(logits=self.policy.masked_logits(logits, use_action_mask), validate_args=False)
+        if action is None:
+            action = probs.sample()
+        return action, probs.log_prob(action), probs.entropy(), value
+
+    @torch.no_grad()
+    def get_action(self, use_action_mask, *, agent_ids=None, bits=None, meta=None, env=None, envs=None):
+        _, logits = self.forward(agent_ids, bits, meta, env, envs)
+        return Categorical(logits=self.policy.masked_logits(logits, use_action_mask), validate_args=False).sample()

@@ -17,6 +17,7 @@ from collections import defaultdict
 import torch
 
 from .env import GridworldCtfGPU, metrics_dict
+from .fused_policy import FusedPolicy
 from .rollout import batched_action
 
 
@@ -28,13 +29,19 @@ def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 25
     Returns (results [P, D] int64 of +1/0/-1 from team 0's view, metrics).  metrics is None unless collect_metrics;
     then a list of P ``env.metrics``-style dicts summed over the pair's duels, or with per_duel_metrics a list of P
     lists of D dicts — one per duel, what ``utils.duel(return_result=False)`` returns (utils.py:571).
+
+    ``fused_policy.FusedPolicy`` policies read the env's packed observations in place; when every policy is one, the
+    env is created packed-only and never writes dense observations.
     """
     P, D = len(pairs), int(duels_per_pair)
+    fused = [isinstance(pol, FusedPolicy) for pair in pairs for pol in pair]
+    packed_kw = {} if not any(fused) else dict(packed_obs=True, dense_obs=not all(fused))
     env = GridworldCtfGPU(**env_config, num_envs=P * D, device=device, seed=seed, env_id_base=env_id_base,
-                          reverse_team1_actions=True, stats="counters" if collect_metrics else "none")
+                          reverse_team1_actions=True, stats="counters" if collect_metrics else "none", **packed_kw)
     B, N, dev = env.num_envs, env.N_AGENTS, env.device
     C, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
-    teams = [torch.tensor([i for i in range(N) if env.AGENT_TEAMS[i] == t], device=dev) for t in (0, 1)]
+    team_ids = [[i for i in range(N) if env.AGENT_TEAMS[i] == t] for t in (0, 1)]
+    teams = [torch.tensor(ids, device=dev) for ids in team_ids]
     obs, meta, _ = env.reset()
     actions = torch.empty((B, N), dtype=torch.uint8, device=dev)
     step_count = 0
@@ -42,14 +49,16 @@ def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 25
         step_count += 1
         for p, pair in enumerate(pairs):
             sl = slice(p * D, (p + 1) * D)
-            for idx, pol in zip(teams, pair):
+            for idx, ids, pol in zip(teams, team_ids, pair):
                 k = idx.numel()
                 if k == 0:
                     continue
-                a = batched_action(
-                    pol, obs[sl][:, idx].reshape(D * k, C, G, G).float(), meta[sl][:, idx].reshape(D * k, M),
-                    env.use_action_mask[idx].unsqueeze(0).expand(D, k).reshape(D * k),
-                )
+                flags = env.use_action_mask[idx].unsqueeze(0).expand(D, k).reshape(D * k)
+                if isinstance(pol, FusedPolicy):
+                    a = pol.get_action_and_value(flags, agent_ids=ids, env=env, envs=sl)[0]
+                else:
+                    a = batched_action(pol, obs[sl][:, idx].reshape(D * k, C, G, G).float(), meta[sl][:, idx].reshape(D * k, M),
+                                       flags)
                 actions[sl, idx] = a.reshape(D, k).to(torch.uint8)
         obs, meta, _, _, _ = env.step(actions)
         if step_count > max_steps or step_count >= env.GAME_STEPS:

@@ -4,6 +4,7 @@ Layer names and shapes match the reference's ``Agent`` (conv1, conv2, fc1, fc2, 
 so ``CtfPolicy.load_state_dict(reference_agent.state_dict())`` works.  This is stock torch/cuDNN — the
 policy is outside the hot path of this repo (SURVEY.md §2 row 6); it exists so the batched rollout / duel
 adapters and BASELINE config 5 can run where the reference tree is absent.
+For rollout / duel inference from packed observations use ``fused_policy.FusedPolicy`` (bf16, a CUDA trunk kernel).
 """
 from __future__ import annotations
 

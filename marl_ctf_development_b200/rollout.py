@@ -12,13 +12,17 @@ back by the kernel (``reverse_team1_actions=True``), as ppo.py:84-93 and utils.p
 Policies are any module with the reference ``Agent.get_action_and_value(grid, meta, use_action_mask)`` on batched
 inputs — the reference ``Agent`` itself (agent_network.py:63-81 is batch-safe) or ``policy.CtfPolicy``.  The duel
 adapters sample through the same method: ``Agent.get_action`` ends in ``action.item()`` (agent_network.py:58) and
-only takes one sample at a time.
+only takes one sample at a time.  A ``fused_policy.FusedPolicy`` on either side reads the packed observations
+``env.obs_bits`` and ``env.meta`` in place instead; an env created packed-only (``dense_obs=False, packed_obs=True``)
+is accepted when every policy on it is fused.
 """
 from __future__ import annotations
 
 from dataclasses import dataclass
 
 import torch
+
+from .fused_policy import FusedPolicy
 
 
 @dataclass
@@ -65,8 +69,9 @@ def _team_indices(env, team):
     return [i for i in range(env.N_AGENTS) if env.AGENT_TEAMS[i] == team]
 
 
-def _require_dense_obs(env):
-    if env.obs is None:
+def _require_dense_obs(env, *policies):
+    """Stock policies read env.obs; when every policy given is a FusedPolicy, a packed-only env is fine."""
+    if env.obs is None and not (policies and all(isinstance(p, FusedPolicy) for p in policies)):
         raise ValueError("this adapter feeds policies from env.obs: create the env with dense_obs=True")
 
 
@@ -88,9 +93,10 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
     stores the kernel's 1-bit-per-element copy (env created with packed_obs=True), 32x smaller than float32.
     """
     _require_folded_reversal(env)
-    _require_dense_obs(env)
     team = 0 if train_team1 else 1
     mine, theirs = _team_indices(env, team), _team_indices(env, 1 - team)
+    _require_dense_obs(env, agent, *([opponent] if theirs else []))
+    fused_agent, fused_opponent = isinstance(agent, FusedPolicy), isinstance(opponent, FusedPolicy)
     apt = len(mine)
     T = env.GAME_STEPS if num_env_steps is None else int(num_env_steps)
     B, N, dev = env.num_envs, env.N_AGENTS, env.device
@@ -102,6 +108,8 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
     packed = obs_storage_dtype == "packed"
     if packed and env.obs_bits is None:
         raise ValueError('obs_storage_dtype="packed" needs an env created with packed_obs=True')
+    if env.obs is None and not packed:
+        raise ValueError('an env created with dense_obs=False stores its rollout with obs_storage_dtype="packed"')
     out = Rollout(
         grid_states=(torch.zeros((T * apt, B, env.bits_words_per_agent), dtype=torch.int32, device=dev) if packed
                      else torch.zeros((T * apt, B, C, G, G), dtype=obs_storage_dtype, device=dev)),
@@ -119,12 +127,19 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
     for t in range(T):
         sl = slice(t * apt, (t + 1) * apt)
         # trained team: [B, apt, ...] -> [apt, B, ...] so that buffer row = step*apt + agent_offset (ppo.py:74-79)
-        g = obs[:, mine_t].transpose(0, 1).contiguous()
+        if not (fused_agent and packed):
+            g = obs[:, mine_t].transpose(0, 1).contiguous()
         m = meta[:, mine_t].transpose(0, 1).contiguous()
         flags = mask_flags[mine_t].unsqueeze(1).expand(apt, B)
-        a, logp, _, v = agent.get_action_and_value(
-            g.reshape(apt * B, C, G, G).float(), m.reshape(apt * B, M), flags.reshape(apt * B)
-        )
+        if fused_agent:
+            # samples come env-major (b * apt + j): reorder to the buffer's agent-major rows
+            fe = mask_flags[mine_t].unsqueeze(0).expand(B, apt).reshape(B * apt)
+            a, logp, _, v = agent.get_action_and_value(fe, agent_ids=mine, env=env)
+            a, logp, v = (x.reshape(B, apt).t().reshape(apt * B) for x in (a, logp, v.reshape(-1)))
+        else:
+            a, logp, _, v = agent.get_action_and_value(
+                g.reshape(apt * B, C, G, G).float(), m.reshape(apt * B, M), flags.reshape(apt * B)
+            )
         if packed:
             out.grid_states[sl] = env.obs_bits[:, mine_t].transpose(0, 1)
         else:
@@ -137,15 +152,21 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
         actions[:, mine_t] = a.reshape(apt, B).t().to(torch.uint8)
         if theirs:
             k = len(theirs)
-            go = obs[:, theirs_t].reshape(B * k, C, G, G).float()
-            mo = meta[:, theirs_t].reshape(B * k, M)
             fo = mask_flags[theirs_t].unsqueeze(0).expand(B, k).reshape(B * k)
-            ao = opponent.get_action_and_value(go, mo, fo)[0]
+            if fused_opponent:
+                ao = opponent.get_action_and_value(fo, agent_ids=theirs, env=env)[0]
+            else:
+                go = obs[:, theirs_t].reshape(B * k, C, G, G).float()
+                mo = meta[:, theirs_t].reshape(B * k, M)
+                ao = opponent.get_action_and_value(go, mo, fo)[0]
             actions[:, theirs_t] = ao.reshape(B, k).to(torch.uint8)
         obs, meta, rewards, dones, _ = env.step(actions)                          # ppo.py:98
         out.rewards[sl] = rewards[:, mine_t].t()                                  # ppo.py:106-109
     first = min(mine)
-    out.next_grid_state = obs[:, first].clone().float()                           # ppo.py:116-118
+    if obs is None:                                                               # packed-only env
+        out.next_grid_state = env.unpack_obs(env.obs_bits[:, first])
+    else:
+        out.next_grid_state = obs[:, first].clone().float()                       # ppo.py:116-118
     out.next_metadata_state = meta[:, first].clone()
     out.next_done = dones.float().clone()                                         # ppo.py:111
     return out
@@ -161,24 +182,26 @@ def batched_duel(env, agent, opponent, max_steps=256, return_result=True):
     all-reduced ``env.metrics`` dict when return_result=False (:571).
     """
     _require_folded_reversal(env)
-    _require_dense_obs(env)
+    _require_dense_obs(env, agent, opponent)
     B, N, dev = env.num_envs, env.N_AGENTS, env.device
     C, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
-    teams = [torch.tensor(_team_indices(env, t), device=dev) for t in (0, 1)]
+    team_ids = [_team_indices(env, t) for t in (0, 1)]
+    teams = [torch.tensor(ids, device=dev) for ids in team_ids]
     policies = (agent, opponent)
     obs, meta, _ = env.reset()
     actions = torch.empty((B, N), dtype=torch.uint8, device=dev)
     step_count = 0
     while True:
         step_count += 1
-        for idx, pol in zip(teams, policies):
+        for idx, ids, pol in zip(teams, team_ids, policies):
             k = idx.numel()
             if k == 0:
                 continue
-            a = batched_action(
-                pol, obs[:, idx].reshape(B * k, C, G, G).float(), meta[:, idx].reshape(B * k, M),
-                env.use_action_mask[idx].unsqueeze(0).expand(B, k).reshape(B * k),
-            )
+            flags = env.use_action_mask[idx].unsqueeze(0).expand(B, k).reshape(B * k)
+            if isinstance(pol, FusedPolicy):
+                a = pol.get_action_and_value(flags, agent_ids=ids, env=env)[0]
+            else:
+                a = batched_action(pol, obs[:, idx].reshape(B * k, C, G, G).float(), meta[:, idx].reshape(B * k, M), flags)
             actions[:, idx] = a.reshape(B, k).to(torch.uint8)
         obs, meta, _, dones, _ = env.step(actions)
         if step_count > max_steps or step_count >= env.GAME_STEPS:  # all envs finish in lock-step
