@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 5
+#define CTF_ABI_VERSION 6
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -242,24 +242,11 @@ int ctf_take_faults(ctf_handle_t h, void* stream, uint32_t* faults);
  * ([B] uint8) out, valid when the call returns.  Pinned (page-locked) buffers
  * are accessed by the kernel directly over PCIe; pageable ones are staged with
  * copies.  Observations and metadata stay on the device in `out`.
+ * One handle must not have two steps in flight on different streams: the
+ * host-step staging buffers are per handle.
  */
 int ctf_step_host(ctf_handle_t h, ctf_state_t state, const uint8_t* actions_host, ctf_outputs_t out,
                   float* rewards_host, uint8_t* dones_host, void* stream);
-
-/*
- * Which kernel ctf_step launches for this handle (no reference counterpart; for benchmarks and profiles).
- * persistent = 1: the persistent warp-specialised kernel k_step_ws (ctas CTAs of logic_warps + stream_warps warps,
- * envs handed out in order from a device counter); 0: the warp-per-env kernel k_step.  Both give identical results.
- * One handle must not have two steps in flight on different streams (the persistent kernel's env counter and the
- * host-step staging buffers are per handle).
- */
-typedef struct ctf_kernel_info {
-    int persistent, logic_warps, stream_warps, ctas;
-    int64_t min_envs_for_persistent;
-    int warp_per_env_ctas_per_sm; /* resident-CTA cap of k_step / k_reset / k_observe (0: as many as fit) */
-    int reserved;
-} ctf_kernel_info_t;
-int ctf_get_kernel_info(ctf_handle_t h, ctf_kernel_info_t* out);
 
 /*
  * Policy inference from packed observations (no reference counterpart: the reference feeds agent_network.Agent a dense

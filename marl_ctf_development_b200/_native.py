@@ -25,10 +25,9 @@ EXPORTS = (
     "ctf_stats_sum",
     "ctf_take_faults",
     "ctf_step_host",
-    "ctf_get_kernel_info",
     "ctf_policy_features",
 )
-ABI_VERSION = 5
+ABI_VERSION = 6
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
 
 
@@ -68,11 +67,6 @@ class CtfSizes(C.Structure):
             "hp_bytes",
         )
     ]
-
-
-class CtfKernelInfo(C.Structure):
-    _fields_ = [("persistent", C.c_int), ("logic_warps", C.c_int), ("stream_warps", C.c_int), ("ctas", C.c_int),
-                ("min_envs_for_persistent", C.c_int64), ("warp_per_env_ctas_per_sm", C.c_int), ("reserved", C.c_int)]
 
 
 class CtfPolicyWeights(C.Structure):
@@ -121,7 +115,6 @@ def load():
     L.ctf_unpack_obs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p]
     L.ctf_stats_sum.argtypes = [C.c_void_p, CtfState, C.c_void_p, C.c_void_p]
     L.ctf_take_faults.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
-    L.ctf_get_kernel_info.argtypes = [C.c_void_p, C.POINTER(CtfKernelInfo)]
     L.ctf_step_host.argtypes = [C.c_void_p, CtfState, C.c_void_p, CtfOutputs, C.c_void_p, C.c_void_p, C.c_void_p]
     L.ctf_policy_features.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
                                       C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]

@@ -19,7 +19,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>   // snprintf for error messages
-#include <stdlib.h>  // getenv: kernel-shape overrides for A/B runs
 #include <string.h>
 
 #include <new>
@@ -29,25 +28,7 @@
 
 namespace {
 
-#ifndef CTF_WARPS_PER_CTA
-#define CTF_WARPS_PER_CTA 4
-#endif
-#ifndef CTF_STORE_OP
-// 0: st.global.cs (streaming), 1: default write-back, 2: st.global.wt.  Measured on B200 (profiles/r01_ab_store_op.log):
-// plain write-back stores are 4 % faster than .cs for this stream (L2 merges and schedules the write-backs).
-#define CTF_STORE_OP 1
-#endif
-#ifndef CTF_STATE_HINT
-// 1: env state loads / stores carry an L2 evict_last policy (and, with CTF_STORE_OP 3, the observation stream an
-// evict_first policy) so that the 22 MB of state written by step t are still in L2 when step t+1 reads them.
-#define CTF_STATE_HINT 0
-#endif
-#ifndef CTF_DIAG
-// TIMING DIAGNOSTICS ONLY (results are wrong when non-zero): bit 0 skip the state read, 1 skip the state write-back,
-// 2 skip metadata, 3 skip rewards / dones, 4 skip the statistics reductions, 5 skip the actions read
-#define CTF_DIAG 0
-#endif
-constexpr int kWarpsPerCta = CTF_WARPS_PER_CTA;
+constexpr int kWarpsPerCta = 4;   // 2 warps per CTA tie with 4, 8 and 16 lose (see k_step)
 constexpr int kThreads = kWarpsPerCta * 32;
 constexpr int kRow = 16;       // shared/global grid row stride (cells)
 constexpr int kGridBytes = 256;
@@ -170,16 +151,6 @@ __device__ __forceinline__ uint4 expand_bits<float>(uint32_t b) {  // 4 elements
     return v;
 }
 
-template <>
-__device__ __forceinline__ uint4 expand_bits<uint8_t>(uint32_t b) {  // 16 elements
-    uint4 v;
-    v.x = ((b & 15u) * 0x00204081u) & 0x01010101u;
-    v.y = (((b >> 4) & 15u) * 0x00204081u) & 0x01010101u;
-    v.z = (((b >> 8) & 15u) * 0x00204081u) & 0x01010101u;
-    v.w = (((b >> 12) & 15u) * 0x00204081u) & 0x01010101u;
-    return v;
-}
-
 // 8 elements of a 16-bit float type whose 1.0 is ONE: word k packs bits 2k (low half) and 2k+1 (high half)
 template <uint32_t ONE>
 __device__ __forceinline__ uint4 expand_bits16(uint32_t b) {
@@ -202,67 +173,6 @@ __device__ __forceinline__ __half from_bit<__half>(uint32_t bit) { return __usho
 template <>
 __device__ __forceinline__ __nv_bfloat16 from_bit<__nv_bfloat16>(uint32_t bit) {
     return __ushort_as_bfloat16((unsigned short)(bit ? 0x3F80u : 0u));
-}
-
-#if CTF_STATE_HINT || CTF_STORE_OP == 3
-__device__ __forceinline__ uint64_t l2_evict_first() {
-    uint64_t pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-__device__ __forceinline__ uint64_t l2_evict_last() {
-    uint64_t pol;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-#endif
-
-__device__ __forceinline__ void store_vec(uint4* p, uint4 v) {
-#if CTF_STORE_OP == 0
-    __stcs(p, v);
-#elif CTF_STORE_OP == 1
-    *p = v;
-#elif CTF_STORE_OP == 2
-    __stwt(p, v);
-#else
-    asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1,%2,%3,%4}, %5;" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w),
-                 "l"(l2_evict_first()) : "memory");
-#endif
-}
-
-// env state accesses (tile map, agent records, env record)
-__device__ __forceinline__ uint4 ld_state(const uint4* p) {
-#if CTF_STATE_HINT
-    uint4 v;
-    asm volatile("ld.global.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p), "l"(l2_evict_last()));
-    return v;
-#else
-    return *p;
-#endif
-}
-__device__ __forceinline__ unsigned long long ld_state(const unsigned long long* p) {
-#if CTF_STATE_HINT
-    unsigned long long v;
-    asm volatile("ld.global.L2::cache_hint.u64 %0, [%1], %2;" : "=l"(v) : "l"(p), "l"(l2_evict_last()));
-    return v;
-#else
-    return *p;
-#endif
-}
-__device__ __forceinline__ void st_state(uint4* p, uint4 v) {
-#if CTF_STATE_HINT
-    asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1,%2,%3,%4}, %5;" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w),
-                 "l"(l2_evict_last()) : "memory");
-#else
-    *p = v;
-#endif
-}
-__device__ __forceinline__ void st_state(unsigned long long* p, unsigned long long v) {
-#if CTF_STATE_HINT
-    asm volatile("st.global.L2::cache_hint.u64 [%0], %1, %2;" ::"l"(p), "l"(v), "l"(l2_evict_last()) : "memory");
-#else
-    *p = v;
-#endif
 }
 
 // Builds the env's observation block as one bit per element in shared memory (w.bits): element
@@ -318,29 +228,29 @@ __device__ __forceinline__ void build_obs_bits(const DevPlan& P, const WarpMem& 
     __syncwarp();
 }
 
+// One 128-bit vector of the observation stream.  A plain write-back store: 4 % faster than .cs for this stream (L2 merges
+// and schedules the write-backs; profiles/r01_ab_store_op.log); evict-first hints are 5-8 % slower (r02_ab_l2_hints.log).
+__device__ __forceinline__ void store_vec(uint4* p, uint4 v) { *p = v; }
+
 // elements (= bits of the string) per 128-bit store
 template <typename T>
 constexpr int kVecElems = 16 / (int)sizeof(T);
 
-#ifndef CTF_PAD_BYTES
-// Alignment unit of the store vectors: 16 (vector), 32 (sector) or 128 (cache line).  Measured on one B200
-// (profiles/r02_ab_pad.log, ms per step 8_arena B=65536 / 7_gridlocked B=65536 / B=16384): 16 -> 1.003 / 0.618 / 0.173,
-// 32 -> 1.003 / 0.551 / 0.151, 128 -> 1.035 / 0.569 / 0.154: whole sectors matter (a sector shared by two store
-// instructions is written twice into L2), whole lines do not.
-#define CTF_PAD_BYTES 32
-#endif
-// number of elements between the previous CTF_PAD_BYTES boundary and `out`: 0 .. CTF_PAD_BYTES / sizeof(T) - 1
+// Alignment unit of the store vectors: a 32-byte sector.  Measured on one B200 (profiles/r02_ab_pad.log, ms per step
+// 8_arena B=65536 / 7_gridlocked B=65536 / B=16384): 16 B -> 1.003 / 0.618 / 0.173, 32 B -> 1.003 / 0.551 / 0.151,
+// 128 B -> 1.035 / 0.569 / 0.154: whole sectors matter (a sector shared by two store instructions is written twice
+// into L2), whole lines do not.
+constexpr int kPadBytes = 32;
+// number of elements between the previous kPadBytes boundary and `out`: 0 .. kPadBytes / sizeof(T) - 1
 template <typename T>
 __device__ __forceinline__ int obs_pad(const T* out) {
-    return (int)((reinterpret_cast<uintptr_t>(out) & (uintptr_t)(CTF_PAD_BYTES - 1)) / sizeof(T));
+    return (int)((reinterpret_cast<uintptr_t>(out) & (uintptr_t)(kPadBytes - 1)) / sizeof(T));
 }
 
-#ifndef CTF_U8_LUT
-#define CTF_U8_LUT 1   // uint8 stream: expand 8 bits -> 8 bytes with one 64-bit shared load from a 256-entry table
-#endif
-// bytes at the start of a kernel's dynamic shared memory taken by the expansion table of element type T
+// uint8 stream: expand 8 bits -> 8 bytes with one 64-bit shared load from a 256-entry table.
+// Bytes at the start of a kernel's dynamic shared memory taken by the expansion table of element type T.
 template <typename T>
-constexpr int kLutBytes = (CTF_U8_LUT && sizeof(T) == 1) ? 2048 : 0;
+constexpr int kLutBytes = sizeof(T) == 1 ? 2048 : 0;
 
 // Fills the table (all threads of the CTA, before any thread leaves the kernel); returns it, or nullptr for other types.
 template <typename T>
@@ -399,7 +309,7 @@ __device__ __forceinline__ void stream_vectors(const uint32_t* __restrict__ bits
 }
 
 // Streams `nbits` elements to `out` (any element alignment) from a bit string built with pad = obs_pad(out), i.e.
-// laid out from the CTF_PAD_BYTES boundary below `out`: store vectors are then sector-aligned whatever the block's
+// laid out from the kPadBytes boundary below `out`: store vectors are then sector-aligned whatever the block's
 // alignment (7_gridlocked's 52 728-byte env blocks start at every multiple of 8 bytes), no 32-byte sector is shared
 // by two store instructions.  Vectors that lie completely inside the block go out as 128-bit stores, the
 // fewer than VB elements before the first / after the last full vector as scalar stores (their neighbours belong
@@ -423,9 +333,9 @@ __device__ __forceinline__ void stream_env(const uint32_t* __restrict__ bits, in
 // Packed copy of the observation block for rollout storage: agent a's C*G*G bits start at word a*wpa
 // (32x smaller than float32; ctf_unpack_obs expands it again).
 __device__ __forceinline__ void store_packed(const DevPlan& P, const uint32_t* __restrict__ bits, int pad,
-                                             uint32_t* __restrict__ out_env, int wi, int nw, int lane) {
+                                             uint32_t* __restrict__ out_env, int lane) {
     const int CGG = P.C * P.GG, wpa = P.wpa, total = P.N * wpa;
-    for (int i = wi * 32 + lane; i < total; i += nw * 32) {
+    for (int i = lane; i < total; i += 32) {
         const int a = i / wpa, j = i - a * wpa;
         const int o = pad + a * CGG + 32 * j;
         uint32_t v = __funnelshift_r(bits[o >> 5], bits[(o >> 5) + 1], o & 31);
@@ -442,16 +352,10 @@ __device__ __forceinline__ void write_obs(const DevPlan& P, const Launch& L, con
     T* out = L.obs ? reinterpret_cast<T*>(L.obs) + env * (long long)P.E : nullptr;
     const int pad = out ? obs_pad(out) : 0;
     build_obs_bits(P, w, me, rev_mask, pad, lane);
-    if (L.obs_bits) store_packed(P, w.bits, pad, L.obs_bits + env * (long long)(P.N * P.wpa), 0, 1, lane);
+    if (L.obs_bits) store_packed(P, w.bits, pad, L.obs_bits + env * (long long)(P.N * P.wpa), lane);
     if (out) stream_env<T>(w.bits, P.E, out, 0, 1, lane, lut);
 }
 
-#ifndef CTF_COOP_STREAM
-#define CTF_COOP_STREAM 1   // k_step: 1 = the CTA's warps stream its env blocks together (below), 0 = every warp streams its own
-#endif
-#ifndef CTF_META_VEC
-#define CTF_META_VEC 1   // 1: whole [N][M] block as float4 stores; 0: one 4-byte store per element
-#endif
 // Element codes of the metadata block (host-built, DevPlan::meta_codes): the LANE whose value the element takes.
 // write_meta spreads the block's distinct values over the warp — lane i < 8: hp8 of agent i, lane 8 + i: has_flag of
 // agent i, lanes 16 / 17 / 18: game progress and the two capture ratios, lane 19: 1.0, lane 20: 0.0 — so that every
@@ -478,7 +382,6 @@ __device__ __forceinline__ void write_meta(const DevPlan& P, uint32_t me, double
     const int den = lane == 16 ? P.game_steps : (lane == 17 ? caps1 + 1 : caps0 + 1);
     const float quot = __half2float(__double2half((double)num / (double)den));
     const float val = lane < 8 ? hp8 : (lane < 16 ? (float)ag_flag(mine) : (lane < 19 ? quot : (lane == 19 ? 1.0f : 0.0f)));
-#if CTF_META_VEC
     // The block's layout is static, so the host compiled it into one source lane per element; lane l of pass `it`
     // produces elements 4k .. 4k+3 (k = 32 it + l) and stores them as one float4 (N*M is a multiple of 4 for every N).
     const int n4 = (N * M) >> 2;
@@ -492,15 +395,6 @@ __device__ __forceinline__ void write_meta(const DevPlan& P, uint32_t me, double
         v.w = __shfl_sync(kFull, val, (codes >> 24) & 31u);
         if (k < n4) reinterpret_cast<float4*>(meta_env)[k] = v;
     }
-#else
-    const int total = N * M;                  // one 4-byte store per element
-    for (int e0 = 0; e0 < total; e0 += 32) {
-        const int e = e0 + lane;
-        const uint32_t code = (P.meta_codes[(e >> 2) & 63] >> (8 * (e & 3))) & 31u;
-        const float x = __shfl_sync(kFull, val, code);
-        if (e < total) meta_env[e] = x;
-    }
-#endif
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -510,15 +404,15 @@ __device__ __forceinline__ void store_state(const DevPlan& P, const Launch& L, c
                                             uint32_t me, double hpd, int inv, uint4 ev, int lane) {
     if (P.hp_float && lane < P.N) L.hp[env * P.N + lane] = hpd;
     if (lane < kGridBytes / 16)
-        st_state(reinterpret_cast<uint4*>(L.grid + env * kGridBytes) + lane, reinterpret_cast<const uint4*>(w.grid)[lane]);
+        reinterpret_cast<uint4*>(L.grid + env * kGridBytes)[lane] = reinterpret_cast<const uint4*>(w.grid)[lane];
     if (lane < P.N) {
         const unsigned long long rec = (unsigned long long)ag_r(me) | ((unsigned long long)ag_c(me) << 8) |
                                        ((unsigned long long)ag_flag(me) << 16) |
                                        ((unsigned long long)(uint16_t)ag_hp(me) << 32) |
                                        ((unsigned long long)(uint16_t)inv << 48);
-        st_state(L.agents + env * P.N + lane, rec);
+        L.agents[env * P.N + lane] = rec;
     }
-    if (lane == 0) st_state(L.envs + env, ev);
+    if (lane == 0) L.envs[env] = ev;
 }
 
 // Per-step counter deltas of this lane's agent, 4 bits per metric (every per-step increment is <= 15:
@@ -591,16 +485,16 @@ __global__ void __launch_bounds__(kThreads) k_observe(const __grid_constant__ De
     if (env >= L.B) return;
     const WarpMem w = warp_mem(P, reinterpret_cast<unsigned char*>(smem_raw) + kLutBytes<T>, warp);
     if (lane < kGridBytes / 16)
-        reinterpret_cast<uint4*>(w.grid)[lane] = ld_state(reinterpret_cast<const uint4*>(L.grid + env * kGridBytes) + lane);
+        reinterpret_cast<uint4*>(w.grid)[lane] = reinterpret_cast<const uint4*>(L.grid + env * kGridBytes)[lane];
     const int li = lane & 7;
     uint32_t me = 0;
     double hpd = 0.0;
     if (lane < P.N) {
-        const unsigned long long rec = ld_state(L.agents + env * P.N + lane);
+        const unsigned long long rec = L.agents[env * P.N + lane];
         me = pack_agent((int)(rec & 0xFF), (int)((rec >> 8) & 0xFF), (int)((rec >> 16) & 1), (int)(short)(rec >> 32));
         if (P.hp_float) hpd = L.hp[env * P.N + lane];
     }
-    const uint4 ev = ld_state(L.envs + env);
+    const uint4 ev = L.envs[env];
     __syncwarp();
     const uint32_t rev_mask = (L.rev_override & 0x100u) ? (L.rev_override & 0xFFu)
                                                         : __ballot_sync(kFull, lane < P.N && P.obs_rev[li]);
@@ -627,26 +521,18 @@ __device__ __forceinline__ uint32_t step_env(const DevPlan& P, const Launch& L, 
     const int li = lane & 7;
 
     // ---- stage state: tile map -> shared memory, agent i -> lane i
-#if CTF_DIAG & 1
-    if (lane < kGridBytes / 16) reinterpret_cast<uint4*>(w.grid)[lane] = reinterpret_cast<const uint4*>(P.grid_template)[lane];
-    uint32_t me = pack_agent(P.start_r[lane & 7], P.start_c[lane & 7], 0, P.hp_max_q[P.type[lane & 7]]);
-    int inv = 0;
-    int action = (CTF_DIAG & 32) ? (int)((env + lane) % 9) : (lane < N ? L.actions[env * N + lane] : 4);
-    uint4 ev = make_uint4((uint32_t)(env & 255), 0, 0, 0);
-#else
     if (lane < kGridBytes / 16)
-        reinterpret_cast<uint4*>(w.grid)[lane] = ld_state(reinterpret_cast<const uint4*>(L.grid + env * kGridBytes) + lane);
+        reinterpret_cast<uint4*>(w.grid)[lane] = reinterpret_cast<const uint4*>(L.grid + env * kGridBytes)[lane];
     uint32_t me = 0;
     int inv = 0;
     int action = 4;
     if (lane < N) {
-        const unsigned long long rec = ld_state(L.agents + env * N + lane);
+        const unsigned long long rec = L.agents[env * N + lane];
         me = pack_agent((int)(rec & 0xFF), (int)((rec >> 8) & 0xFF), (int)((rec >> 16) & 1), (int)(short)(rec >> 32));
         inv = (int)((rec >> 48) & 0xFFFF);
-        action = (CTF_DIAG & 32) ? (int)((env + lane) % 9) : L.actions[env * N + lane];
+        action = L.actions[env * N + lane];
     }
-    uint4 ev = ld_state(L.envs + env);
-#endif
+    uint4 ev = L.envs[env];
     double hpd = 0.0;   // this lane's agent's HP (HPF only; dead code otherwise)
     if (HPF && lane < N) hpd = L.hp[env * N + lane];
     Deltas dl;
@@ -871,28 +757,22 @@ __device__ __forceinline__ uint32_t step_env(const DevPlan& P, const Launch& L, 
             if (my_team == winner) r = __dadd_rn(r, __dmul_rn(margin, P.win_margin));
             else r = __dadd_rn(r, -__dmul_rn(margin, P.loss_margin));
         }
-        if (!(CTF_DIAG & 8) && L.rewards && lane < N) L.rewards[env * N + lane] = (float)r;
+        if (L.rewards && lane < N) L.rewards[env * N + lane] = (float)r;
     }
-    if (!(CTF_DIAG & 8) && L.dones && lane == 0) L.dones[env] = done ? 1 : 0;
+    if (L.dones && lane == 0) L.dones[env] = done ? 1 : 0;
     ev.z = (uint32_t)caps0;
     ev.w = (uint32_t)caps1;
 
     // ---- write state back
     __syncwarp();
-    if (!(CTF_DIAG & 2)) store_state(P, L, w, env, me, hpd, inv, ev, lane);
-    if (STATS && !(CTF_DIAG & 16)) {
+    store_state(P, L, w, env, me, hpd, inv, ev, lane);
+    if (STATS) {
         if (lane < N) {   // fire-and-forget reductions: no load latency, nothing held in registers
             uint32_t* sp = L.stats + env * (long long)(CTF_N_METRICS * N) + lane;
 #pragma unroll
             for (int m = 0; m < CTF_N_METRICS; ++m) {
                 const uint32_t v = ((m < 8 ? dl.lo : dl.hi) >> (4 * (m & 7))) & 15u;
-                if (v) {
-#if CTF_STATE_HINT
-                    asm volatile("red.global.add.L2::cache_hint.u32 [%0], %1, %2;" ::"l"(sp + m * N), "r"(v), "l"(l2_evict_last()) : "memory");
-#else
-                    atomicAdd(sp + m * N, v);
-#endif
-                }
+                if (v) atomicAdd(sp + m * N, v);
             }
         }
         if (L.visits && lane < N) {   // update_visitation_map (:911), uint8 wrap
@@ -902,11 +782,11 @@ __device__ __forceinline__ uint32_t step_env(const DevPlan& P, const Launch& L, 
     }
 
     rev_mask_out = (L.rev_override & 0x100u) ? (L.rev_override & 0xFFu) : __ballot_sync(kFull, lane < N && P.obs_rev[li]);
-    if (!(CTF_DIAG & 4) && L.meta) write_meta<HPF>(P, me, hpd, step, caps0, caps1, L.meta + env * (long long)N * P.M, lane);
+    if (L.meta) write_meta<HPF>(P, me, hpd, step, caps0, caps1, L.meta + env * (long long)N * P.M, lane);
     return me;
 }
 
-// Warp-per-env step kernel, the default kernel of ctf_step: every warp steps its env and builds that env's observation
+// Warp-per-env step kernel of ctf_step: every warp steps its env and builds that env's observation
 // bit string in its own shared-memory buffer; after one barrier the CTA's warps write the CTA's kWarpsPerCta consecutive
 // env blocks one after the other, all warps on the same block (2 KB contiguous per pass) — a quarter as many open
 // write streams as when every warp streams its own block, and each CTA's region goes out in address order.
@@ -920,7 +800,6 @@ __global__ void __launch_bounds__(kThreads) k_step(const __grid_constant__ DevPl
     const uint2* lut = init_expand_lut<T>(smem_raw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long env = (long long)blockIdx.x * kWarpsPerCta + warp;
-#if CTF_COOP_STREAM
     unsigned char* base = reinterpret_cast<unsigned char*>(smem_raw) + kLutBytes<T>;
     if (env < L.B) {
         const WarpMem w = warp_mem(P, base, warp);
@@ -930,7 +809,7 @@ __global__ void __launch_bounds__(kThreads) k_step(const __grid_constant__ DevPl
             T* out = L.obs ? reinterpret_cast<T*>(L.obs) + env * (long long)P.E : nullptr;
             const int pad = out ? obs_pad(out) : 0;
             build_obs_bits(P, w, me, rev_mask, pad, lane);
-            if (L.obs_bits) store_packed(P, w.bits, pad, L.obs_bits + env * (long long)(P.N * P.wpa), 0, 1, lane);
+            if (L.obs_bits) store_packed(P, w.bits, pad, L.obs_bits + env * (long long)(P.N * P.wpa), lane);
         }
     }
     __syncthreads();
@@ -941,150 +820,6 @@ __global__ void __launch_bounds__(kThreads) k_step(const __grid_constant__ DevPl
             stream_env<T>(warp_mem(P, base, e).bits, P.E, reinterpret_cast<T*>(L.obs) + env_e * (long long)P.E, warp, kWarpsPerCta, lane, lut);
         }
     }
-#else
-    if (env >= L.B) return;
-    const WarpMem w = warp_mem(P, reinterpret_cast<unsigned char*>(smem_raw) + kLutBytes<T>, warp);
-    uint32_t rev_mask;
-    const uint32_t me = step_env<STATS, HPF>(P, L, w, env, lane, rev_mask);
-    write_obs<T>(P, L, w, env, me, rev_mask, lane, lut);   // observations straight into the policy's input buffers
-#endif
-}
-
-// ------------------------------------------------------------------------------------------------
-// Persistent, warp-specialised step kernel (opt-in: CTF_WS=1)
-// ------------------------------------------------------------------------------------------------
-// What bounds the step is the 100 KB-per-env observation write, and HBM takes that stream fastest when few env
-// blocks are open at a time and they are visited in address order (profiles/r02_write_span_microbench.log: 0.88 ms
-// for 65536 blocks written one per 512-thread CTA in order, 0.96 ms when every warp streams its own block).  SMs
-// also differ by up to 1.46x in store bandwidth, so work has to be handed out dynamically.  Hence:
-//   * one persistent CTA per SM (or two): n_logic "logic" warps + n_stream "stream" warps;
-//   * a logic warp takes the next env id from a global counter (in order), runs step_env, builds the env's
-//     observation bit string in its own shared-memory buffer and queues it in a shared-memory FIFO;
-//   * the stream warps take the FIFO entries in order and write ONE env block at a time, together;
-//   * a logic warp reuses its buffer when the stream group is done with it — the queue is the back-pressure.
-#ifndef CTF_WS_PROFILE
-#define CTF_WS_PROFILE 0         // 1: per-phase cycle totals of logic / stream warps (tools/ws_sweep.py --profile build)
-#endif
-#if CTF_WS_PROFILE
-#define CTF_PROF_T(var) const long long var = clock64()
-#define CTF_PROF_ADD(acc, t0, t1) acc += (t1) - (t0)
-#else
-#define CTF_PROF_T(var)
-#define CTF_PROF_ADD(acc, t0, t1)
-#endif
-#ifndef CTF_WS_SLEEP_NS
-#define CTF_WS_SLEEP_NS 32       // back-off of the FIFO / buffer polls
-#endif
-constexpr int kWsQ = 32;         // FIFO slots (>= logic warps per CTA)
-constexpr int kWsCtlBytes = 1024;
-struct WsCtl {
-    int tail;                    // next ticket
-    int producers;               // logic warps still running
-    volatile int ready[kWsQ];    // ticket + 1 once the entry is filled, 0 when free
-    int env[kWsQ];
-    int buf[kWsQ];               // logic warp whose buffer holds the bit string
-    int done[kWsQ];              // stream warps finished with the entry
-    volatile int busy[32];       // logic warp's buffer is queued / being streamed
-};
-static_assert(sizeof(WsCtl) <= kWsCtlBytes, "control block");
-
-template <typename T, bool STATS, bool HPF>
-__global__ void __launch_bounds__(1024, 1) k_step_ws(const __grid_constant__ DevPlan P, const __grid_constant__ Launch L,
-                                                     int n_logic, int n_stream, unsigned int* __restrict__ ctr) {
-    extern __shared__ uint4 smem_raw[];
-    const uint2* lut = init_expand_lut<T>(smem_raw);
-    WsCtl* c = reinterpret_cast<WsCtl*>(reinterpret_cast<unsigned char*>(smem_raw) + kLutBytes<T>);
-    unsigned char* warp_base = reinterpret_cast<unsigned char*>(smem_raw) + kLutBytes<T> + kWsCtlBytes;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) { c->tail = 0; c->producers = n_logic; }
-    if (threadIdx.x < kWsQ) { c->ready[threadIdx.x] = 0; c->done[threadIdx.x] = 0; }
-    if (threadIdx.x < 32) c->busy[threadIdx.x] = 0;
-    __syncthreads();
-    const bool any_obs = L.obs || L.obs_bits;
-#if CTF_WS_PROFILE
-    long long pf[6] = {0, 0, 0, 0, 0, 0};   // logic: fetch, step, wait, build+publish; stream: idle, stream
-    unsigned long long* prof = reinterpret_cast<unsigned long long*>(ctr + 4);
-#endif
-    if (warp < n_logic) {
-        const WarpMem w = warp_mem(P, warp_base, warp);
-        for (;;) {
-            CTF_PROF_T(t0);
-            unsigned int e = 0;
-            if (lane == 0) e = atomicAdd(ctr, 1u);
-            e = __shfl_sync(kFull, e, 0);
-            if ((long long)e >= L.B) break;
-            CTF_PROF_T(t1);
-            uint32_t rev_mask;
-            const uint32_t me = step_env<STATS, HPF>(P, L, w, (long long)e, lane, rev_mask);
-            if (!any_obs) continue;
-            CTF_PROF_T(t2);
-            if (lane == 0) while (c->busy[warp]) __nanosleep(CTF_WS_SLEEP_NS);   // previous env of this warp still being streamed
-            __syncwarp();
-            CTF_PROF_T(t3);
-            const int pad = L.obs ? obs_pad(reinterpret_cast<T*>(L.obs) + (long long)e * P.E) : 0;
-            build_obs_bits(P, w, me, rev_mask, pad, lane);
-            if (lane == 0) {
-                c->busy[warp] = 1;
-                const int t = atomicAdd(&c->tail, 1);
-                const int slot = t % kWsQ;
-                while (c->ready[slot] != 0) __nanosleep(CTF_WS_SLEEP_NS);
-                c->env[slot] = (int)e;
-                c->buf[slot] = warp;
-                __threadfence_block();
-                c->ready[slot] = t + 1;
-            }
-            __syncwarp();
-            CTF_PROF_T(t4);
-            CTF_PROF_ADD(pf[0], t0, t1); CTF_PROF_ADD(pf[1], t1, t2); CTF_PROF_ADD(pf[2], t2, t3); CTF_PROF_ADD(pf[3], t3, t4);
-        }
-        if (lane == 0) {
-#if CTF_WS_PROFILE
-            for (int i = 0; i < 4; ++i) atomicAdd(prof + i, (unsigned long long)pf[i]);
-#endif
-            atomicSub(&c->producers, 1);
-            // every logic warp of the grid fails its last fetch exactly once; the last one re-arms the counters
-            if (atomicAdd(ctr + 1, 1u) == gridDim.x * (unsigned)n_logic - 1u) { ctr[0] = 0; ctr[1] = 0; }
-        }
-    } else {
-        const int wi = warp - n_logic;
-        for (int head = 0;; ++head) {
-            const int slot = head % kWsQ;
-            int got = 0;
-            CTF_PROF_T(t0);
-            if (lane == 0) {
-                for (;;) {
-                    if (c->ready[slot] == head + 1) { got = 1; break; }
-                    if (*(volatile int*)&c->producers == 0 && *(volatile int*)&c->tail == head) break;
-                    __nanosleep(CTF_WS_SLEEP_NS);
-                }
-                __threadfence_block();
-            }
-            got = __shfl_sync(kFull, got, 0);
-            if (!got) break;
-            CTF_PROF_T(t1);
-            const long long env = c->env[slot];
-            const int buf = c->buf[slot];
-            const uint32_t* bits = warp_mem(P, warp_base, buf).bits;
-            T* out = L.obs ? reinterpret_cast<T*>(L.obs) + env * (long long)P.E : nullptr;
-            if (L.obs_bits) store_packed(P, bits, out ? obs_pad(out) : 0, L.obs_bits + env * (long long)(P.N * P.wpa), wi, n_stream, lane);
-            if (out) stream_env<T>(bits, P.E, out, wi, n_stream, lane, lut);
-            __syncwarp();
-            if (lane == 0) {
-                __threadfence_block();
-                if (atomicAdd(&c->done[slot], 1) == n_stream - 1) {   // last stream warp frees the buffer and the slot
-                    c->done[slot] = 0;
-                    c->busy[buf] = 0;
-                    __threadfence_block();
-                    c->ready[slot] = 0;
-                }
-            }
-            CTF_PROF_T(t2);
-            CTF_PROF_ADD(pf[4], t0, t1); CTF_PROF_ADD(pf[5], t1, t2);
-        }
-#if CTF_WS_PROFILE
-        if (lane == 0) { atomicAdd(prof + 4, (unsigned long long)pf[4]); atomicAdd(prof + 5, (unsigned long long)pf[5]); }
-#endif
-    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1093,10 +828,7 @@ __global__ void __launch_bounds__(1024, 1) k_step_ws(const __grid_constant__ Dev
 // The chunk's packed words (wpa per block, coalesced) are re-packed in shared memory into ONE contiguous bit string
 // (block b's nbits elements follow block b-1's directly, shifted by the output's alignment pad) and all warps stream
 // the chunk's output region together — CTAs are scheduled in address order, so few blocks are open at a time.
-#ifndef CTF_UNPACK_THREADS
-#define CTF_UNPACK_THREADS 256   // 512 measured too: profiles/r02_unpack_threads.log
-#endif
-constexpr int kUnpackThreads = CTF_UNPACK_THREADS;
+constexpr int kUnpackThreads = 256;   // 512 measured too: profiles/r02_unpack_threads.log
 template <typename T>
 __global__ void __launch_bounds__(kUnpackThreads) k_unpack(const uint32_t* __restrict__ packed, T* __restrict__ out,
                                                           long long n_blocks, int nbits, int wpa, int chunk, int bits_words) {
@@ -1342,13 +1074,6 @@ struct ctf_env {
     float* rewards_stage;    // device [B][N], used by ctf_step_host when out.rewards is NULL
     uint8_t* dones_stage;    // device [B]
     size_t smem_bytes;
-    // persistent warp-specialised step kernel (k_step_ws)
-    unsigned int* ws_ctr;    // device [2]: next env id, logic warps that have finished; re-armed by the kernel itself
-    int ws_logic, ws_stream, ws_ctas;   // logic / stream warps per CTA, CTAs in the grid
-    long long ws_min_envs;   // batches below this use the warp-per-env kernel
-    int n_sm;
-    int k_step_ctas_per_sm;  // resident-CTA cap of the warp-per-env kernels (0: whatever fits)
-    size_t ws_smem_bytes;
     size_t trunk_smem_bytes; // k_policy_trunk: dynamic shared memory for this plan
     int trunk_ctas;          // k_policy_trunk: CTAs that fit on the device at once
 };
@@ -1364,11 +1089,6 @@ struct DeviceGuard {
     }
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
-
-static int env_int(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return (v && *v) ? atoi(v) : fallback;
-}
 
 static thread_local char g_err[512] = "";
 
@@ -1530,9 +1250,7 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
     if (rc != CTF_OK) { delete h; return rc; }
     h->cfg = *cfg; h->B = num_envs; h->device = device; h->stats_level = stats_level; h->obs_dtype = obs_dtype;
     h->seed = seed; h->env_id_base = env_id_base;
-    const size_t lut_bytes = (CTF_U8_LUT && obs_dtype == CTF_OBS_U8) ? 2048 : 0;   // kLutBytes<uint8_t>
-    h->smem_bytes = lut_bytes + (size_t)h->plan.warp_smem_bytes * kWarpsPerCta;
-    h->k_step_ctas_per_sm = 0;   // decided below, once the SM count is known
+    h->smem_bytes = (obs_dtype == CTF_OBS_U8 ? kLutBytes<uint8_t> : 0) + (size_t)h->plan.warp_smem_bytes * kWarpsPerCta;
     DeviceGuard guard(device);
     cudaError_t e = guard.err;
     if (e == cudaSuccess) e = cudaMalloc(&h->faults, sizeof(uint32_t));
@@ -1540,74 +1258,36 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
     if (e == cudaSuccess) e = cudaMalloc(&h->actions_stage, (size_t)num_envs * cfg->n_agents);
     if (e == cudaSuccess) e = cudaMalloc(&h->rewards_stage, (size_t)num_envs * cfg->n_agents * sizeof(float));
     if (e == cudaSuccess) e = cudaMalloc(&h->dones_stage, (size_t)num_envs);
-    h->ws_ctr = nullptr;
-    if (e == cudaSuccess) e = cudaMalloc(&h->ws_ctr, 128);   // two 32-bit counters (+ the profiling build's cycle totals)
-    if (e == cudaSuccess) e = cudaMemset(h->ws_ctr, 0, 128);
-    // The persistent kernel is opt-in (CTF_WS=1; shape: one CTA per SM with 8 logic + 16 stream warps unless overridden,
-    // tools/ws_sweep.py).  It only ever beat the warp-per-env kernel where the observation stream dwarfs the env logic —
-    // float32 8_arena-sized blocks: 0.989 vs 1.002 ms at B = 65536 when it was written, 0.996 vs 1.001 ms after the env
-    // logic was trimmed (profiles/r02_ws_final_sweep.jsonl) — and loses everywhere else (7_gridlocked 0.73 vs 0.55 ms,
-    // uint8 / bf16 / packed-only outputs: profiles/r02_ws_matrix.log).  Half a per cent does not pay for a second hot
-    // kernel, so ctf_step launches k_step unless asked otherwise; both pass the whole parity suite.
     int n_sm = 0;
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
-    h->ws_logic = env_int("CTF_WS_LOGIC", 8);
-    h->ws_stream = env_int("CTF_WS_STREAM", 16);
-    const int ctas_per_sm = env_int("CTF_WS_CTAS_PER_SM", 1);
-    if (h->ws_logic < 1 || h->ws_logic > kWsQ || h->ws_stream < 1 || (h->ws_logic + h->ws_stream) > 32 || ctas_per_sm < 1 ||
-        ctas_per_sm > 4) {
-        cudaFree(h->faults); cudaFree(h->actions_stage); cudaFree(h->rewards_stage); cudaFree(h->dones_stage); cudaFree(h->ws_ctr);
-        delete h;
-        return fail(CTF_ERR_INVALID, "CTF_WS_LOGIC / CTF_WS_STREAM / CTF_WS_CTAS_PER_SM out of range");
-    }
-    h->n_sm = n_sm;
     // Resident CTAs per SM of the warp-per-env kernels.  Registers allow 9 (36 warps); when the step is bound by the
     // observation stream, FEWER concurrent streams write faster (8_arena float32 B = 65536: 9 -> 1.001 ms, 7 -> 0.989,
     // 5 -> 0.980, 4 -> 0.982; 7_gridlocked 0.551 -> 0.536; bf16 0.526 -> 0.516), when it is bound by the env logic they
     // are slower (uint8 0.283 -> 0.347, 0_the_split 0.174 -> 0.229): profiles/r02_ab_residency*.log.  So blocks of
     // >= 6 KB per agent run with 5 CTAs per SM when there are many waves of them, and with the cap in 5..9 that fills
     // the last wave best when there are few (B = 16384: 7).  The cap is applied by padding dynamic shared memory.
-    {
-        int cap = env_int("CTF_K_STEP_CTAS_PER_SM", -1);
-        if (cap < 0) {
-            cap = 0;
-            const size_t obs_bytes_per_agent = (size_t)h->plan.C * h->plan.GG * (obs_dtype == CTF_OBS_F32 ? 4 : (obs_dtype == CTF_OBS_U8 ? 1 : 2));
-            if (obs_bytes_per_agent >= 6000 && n_sm > 0) {
-                const double ctas_per_sm_total = (double)((num_envs + kWarpsPerCta - 1) / kWarpsPerCta) / n_sm;
-                if (ctas_per_sm_total >= 64.0) {
-                    cap = 5;
-                } else {
-                    double best = -1.0;
-                    for (int c = 5; c <= 9; ++c) {   // fill of the last wave; ties go to the smaller cap
-                        const double waves = ctas_per_sm_total / c, full = (double)(long long)(waves + 0.999999);
-                        const double fill = full > 0 ? waves / full : 0.0;
-                        if (fill > best + 1e-9) { best = fill; cap = c; }
-                    }
-                }
+    if (n_sm > 0 && (size_t)h->plan.C * h->plan.GG * (obs_dtype == CTF_OBS_F32 ? 4 : (obs_dtype == CTF_OBS_U8 ? 1 : 2)) >= 6000) {
+        const double ctas_per_sm_total = (double)((num_envs + kWarpsPerCta - 1) / kWarpsPerCta) / n_sm;
+        int cap = 5;
+        if (ctas_per_sm_total < 64.0) {
+            double best = -1.0;
+            for (int c = 5; c <= 9; ++c) {   // fill of the last wave; ties go to the smaller cap
+                const double waves = ctas_per_sm_total / c, full = (double)(long long)(waves + 0.999999);
+                const double fill = full > 0 ? waves / full : 0.0;
+                if (fill > best + 1e-9) { best = fill; cap = c; }
             }
         }
-        h->k_step_ctas_per_sm = cap;
-        if (cap > 0) {
-            const size_t want = (size_t)(227 * 1024) / (size_t)cap - 1024;
-            if (want > h->smem_bytes) h->smem_bytes = want;
-        }
+        const size_t want = (size_t)(227 * 1024) / (size_t)cap - 1024;
+        if (want > h->smem_bytes) h->smem_bytes = want;
     }
-    h->ws_ctas = n_sm * ctas_per_sm;
-    h->ws_smem_bytes = lut_bytes + (size_t)kWsCtlBytes + (size_t)h->plan.warp_smem_bytes * h->ws_logic;
-    // below ~4 envs per logic warp the persistent kernel is all ramp-up and tail: use the warp-per-env kernel
-    h->ws_min_envs = (long long)env_int("CTF_WS_MIN_ENVS", 4 * h->ws_ctas * h->ws_logic);
-    if (env_int("CTF_WS", 0) != 1 || num_envs > 0x7FFFFFFFll) h->ws_min_envs = 0x7FFFFFFFFFFFFFFFll;
     // The attribute is per kernel, not per handle: give every kernel a ceiling that covers any handle's launch (another
     // handle with a smaller footprint must not lower it under this one's), not this handle's own size.
     const int smem = h->smem_bytes > 100 * 1024 ? (int)h->smem_bytes : 100 * 1024;
-    const int ws_smem = h->ws_smem_bytes > 200 * 1024 ? (int)h->ws_smem_bytes : 200 * 1024;
 #define CTF_SET_SMEM(K, BYTES) if (e == cudaSuccess) e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES)
 #define CTF_SET_SMEM_T(T)                                                                                       \
     CTF_SET_SMEM((k_step<T, false, false>), smem); CTF_SET_SMEM((k_step<T, true, false>), smem);               \
     CTF_SET_SMEM((k_step<T, false, true>), smem); CTF_SET_SMEM((k_step<T, true, true>), smem);                 \
     CTF_SET_SMEM((k_reset<T, false>), smem); CTF_SET_SMEM((k_reset<T, true>), smem); CTF_SET_SMEM((k_observe<T>), smem); \
-    CTF_SET_SMEM((k_step_ws<T, false, false>), ws_smem); CTF_SET_SMEM((k_step_ws<T, true, false>), ws_smem);   \
-    CTF_SET_SMEM((k_step_ws<T, false, true>), ws_smem); CTF_SET_SMEM((k_step_ws<T, true, true>), ws_smem);     \
     CTF_SET_SMEM((k_unpack<T>), smem)
     CTF_SET_SMEM_T(float); CTF_SET_SMEM_T(uint8_t); CTF_SET_SMEM_T(__half); CTF_SET_SMEM_T(__nv_bfloat16);
     // k_policy_trunk needs at most 94 KB (G = 16, C = 14); the ceiling is per kernel, so it covers every plan
@@ -1624,7 +1304,7 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
 #undef CTF_SET_SMEM
     if (e != cudaSuccess) {
         fail(CTF_ERR_CUDA, "ctf_create: %s", cudaGetErrorString(e));
-        cudaFree(h->faults); cudaFree(h->actions_stage); cudaFree(h->rewards_stage); cudaFree(h->dones_stage); cudaFree(h->ws_ctr);
+        cudaFree(h->faults); cudaFree(h->actions_stage); cudaFree(h->rewards_stage); cudaFree(h->dones_stage);
         delete h;
         return CTF_ERR_CUDA;
     }
@@ -1635,7 +1315,7 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
 extern "C" int ctf_destroy(ctf_handle_t h) {
     if (!h) return CTF_OK;
     DeviceGuard guard(h->device);
-    cudaFree(h->faults); cudaFree(h->actions_stage); cudaFree(h->rewards_stage); cudaFree(h->dones_stage); cudaFree(h->ws_ctr);
+    cudaFree(h->faults); cudaFree(h->actions_stage); cudaFree(h->rewards_stage); cudaFree(h->dones_stage);
     delete h;
     return CTF_OK;
 }
@@ -1719,18 +1399,12 @@ extern "C" int ctf_reset(ctf_handle_t h, ctf_state_t st, ctf_outputs_t out, int 
 
 static int launch_step(ctf_handle_t h, const Launch& L, cudaStream_t s) {
     const bool stats = h->stats_level > 0;
-    const bool ws = h->B >= h->ws_min_envs;
     const bool hpf = h->plan.hp_float != 0;
     with_obs_type(h->obs_dtype, [&](auto tag) {
         using T = decltype(tag);
         auto launch = [&](auto stats_c, auto hpf_c) {
             constexpr bool S = decltype(stats_c)::value, F = decltype(hpf_c)::value;
-            if (ws) {
-                const unsigned threads = (unsigned)(h->ws_logic + h->ws_stream) * 32u;
-                k_step_ws<T, S, F><<<h->ws_ctas, threads, h->ws_smem_bytes, s>>>(h->plan, L, h->ws_logic, h->ws_stream, h->ws_ctr);
-            } else {
-                k_step<T, S, F><<<grid_dim(h->B), kThreads, h->smem_bytes, s>>>(h->plan, L);
-            }
+            k_step<T, S, F><<<grid_dim(h->B), kThreads, h->smem_bytes, s>>>(h->plan, L);
         };
         if (stats) { if (hpf) launch(std::true_type{}, std::true_type{}); else launch(std::true_type{}, std::false_type{}); }
         else { if (hpf) launch(std::false_type{}, std::true_type{}); else launch(std::false_type{}, std::false_type{}); }
@@ -1782,19 +1456,16 @@ extern "C" int ctf_unpack_obs(ctf_handle_t h, const uint32_t* packed, void* out,
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const int nbits = h->plan.C * h->plan.GG, wpa = h->plan.wpa;
     const int elem = out_dtype == CTF_OBS_F32 ? 4 : (out_dtype == CTF_OBS_U8 ? 1 : 2);
-    static const int chunk_kb = env_int("CTF_UNPACK_CHUNK_KB", 48);   // 12 .. 384 KB swept: profiles/r02_unpack_chunk_sweep.log
-    int chunk = (chunk_kb * 1024) / (nbits * elem);    // ~48 KB of output per CTA
+    int chunk = (48 * 1024) / (nbits * elem);    // ~48 KB of output per CTA (12 .. 384 KB swept: profiles/r02_unpack_chunk_sweep.log)
     chunk = chunk < 1 ? 1 : (chunk > 64 ? 64 : chunk);
     while (chunk > 1 && ((size_t)(chunk * nbits) / 8 + (size_t)chunk * wpa * 4) > 40 * 1024) --chunk;   // static shared-memory budget
     const int bits_words = (((chunk * nbits + 128 + 31) / 32 + 1) + 15) / 16 * 16;
     const unsigned grid = (unsigned)((n_agent_blocks + chunk - 1) / chunk);
-    size_t smem = ((size_t)bits_words + (size_t)chunk * wpa) * sizeof(uint32_t) + ((CTF_U8_LUT && out_dtype == CTF_OBS_U8) ? 2048 : 0);
+    size_t smem = ((size_t)bits_words + (size_t)chunk * wpa) * sizeof(uint32_t) + (out_dtype == CTF_OBS_U8 ? kLutBytes<uint8_t> : 0);
     // like k_step: fewer resident CTAs = fewer concurrent write streams (profiles/r02_unpack_residency.log)
     // float32 6 777 -> 6 838 GB/s and bf16 6 600 -> 6 703 at 5 CTAs per SM, uint8 (issue-bound) 6 365 -> 5 239: capped for >= 2-byte elements
-    static const int unpack_ctas_env = env_int("CTF_UNPACK_CTAS_PER_SM", -1);
-    const int unpack_ctas = unpack_ctas_env >= 0 ? unpack_ctas_env : (elem >= 2 ? 5 : 0);
-    if (unpack_ctas > 0) {
-        const size_t want = (size_t)(227 * 1024) / (size_t)unpack_ctas - 1024;
+    if (elem >= 2) {
+        const size_t want = (size_t)(227 * 1024) / 5 - 1024;
         if (want > smem) smem = want;
     }
     with_obs_type(out_dtype, [&](auto tag) {
@@ -1859,15 +1530,6 @@ extern "C" int ctf_stats_sum(ctf_handle_t h, ctf_state_t st, int64_t* stats_sum,
     return CTF_OK;
 }
 
-extern "C" int ctf_get_kernel_info(ctf_handle_t h, ctf_kernel_info_t* out) {
-    if (!h || !out) return fail(CTF_ERR_INVALID, "null argument");
-    out->persistent = h->B >= h->ws_min_envs ? 1 : 0;
-    out->logic_warps = h->ws_logic; out->stream_warps = h->ws_stream; out->ctas = h->ws_ctas;
-    out->min_envs_for_persistent = h->ws_min_envs;
-    out->warp_per_env_ctas_per_sm = h->k_step_ctas_per_sm;
-    return CTF_OK;
-}
-
 extern "C" int ctf_take_faults(ctf_handle_t h, void* stream, uint32_t* faults) {
     if (!h || !faults) return fail(CTF_ERR_INVALID, "null argument");
     DeviceGuard guard(h->device);
@@ -1922,14 +1584,3 @@ extern "C" int ctf_step_host(ctf_handle_t h, ctf_state_t st, const uint8_t* acti
     CTF_CUDA(cudaStreamSynchronize(s));
     return CTF_OK;
 }
-
-#if CTF_WS_PROFILE
-// profiling builds only (tools/ws_sweep.py --profile): cycle totals {fetch, step, wait, build, stream-idle, stream}, then cleared
-extern "C" int ctf_debug_ws_profile(ctf_handle_t h, unsigned long long* out6) {
-    DeviceGuard guard(h->device);
-    CTF_CUDA(cudaDeviceSynchronize());
-    CTF_CUDA(cudaMemcpy(out6, reinterpret_cast<unsigned char*>(h->ws_ctr) + 16, 6 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    CTF_CUDA(cudaMemset(reinterpret_cast<unsigned char*>(h->ws_ctr) + 16, 0, 6 * sizeof(unsigned long long)));
-    return CTF_OK;
-}
-#endif

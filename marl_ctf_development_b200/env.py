@@ -394,13 +394,8 @@ class GridworldCtfGPU:
 
     @property
     def uses_persistent_kernel(self) -> bool:
-        """True when step() launches the persistent warp-specialised kernel for this batch size (see ctf_get_kernel_info)."""
-        return bool(self.kernel_info().persistent)
-
-    def kernel_info(self):
-        info = _native.CtfKernelInfo()
-        _native.check(self._lib.ctf_get_kernel_info(self._handle, C.byref(info)))
-        return info
+        """Always False: step() launches the warp-per-env kernel k_step; kept for callers that name the kernel by it."""
+        return False
 
     # ------------------------------------------------------------------ reference API that does not touch the device
     def get_env_dims(self):

@@ -620,53 +620,11 @@ def test_soak_every_experiment_full_episode_with_visits(exp):
     assert np.array_equal(st["stats"], so["stats"]) and np.array_equal(st["visits"], so["visits"])
 
 
-# ---------------------------------------------------------------------------------------------------
-# the persistent warp-specialised kernel (k_step_ws): same results as the warp-per-env kernel and the oracle
-# ---------------------------------------------------------------------------------------------------
-@pytest.fixture
-def force_persistent_kernel(monkeypatch):
-    """ctf_create reads these: every batch size and output type then runs k_step_ws (default: never)."""
-    monkeypatch.setenv("CTF_WS", "1")
-    monkeypatch.setenv("CTF_WS_MIN_ENVS", "1")
-
-
-@pytest.mark.parametrize("exp,B,dtype,policy", [
-    ("8_arena", 3000, torch.float32, "seek"),          # ~2.5 envs per logic warp: buffers are reused, FIFO wraps
-    ("7_gridlocked", 2500, torch.float32, "builder"),  # 8-byte aligned env blocks: padded bit strings, scalar head / tail
-    ("0_the_split", 5000, torch.uint8, "uniform"),
-    ("8_arena", 1500, torch.bfloat16, "uniform"),
-    ("5_skittles", 7, torch.float32, "seek"),          # fewer envs than logic warps
-])
-def test_persistent_kernel_against_oracle(force_persistent_kernel, exp, B, dtype, policy):
-    env, _ = _run_against_oracle(exp, B, 40, policy, seed=21, obs_every=13, stats="full", obs_dtype=dtype)
-    assert env.uses_persistent_kernel
-    info = env.kernel_info()
-    assert info.ctas >= 1 and info.logic_warps + info.stream_warps <= 32
-
-
-def test_persistent_kernel_is_opt_in_and_gives_identical_results(monkeypatch):
-    for k in ("CTF_WS", "CTF_WS_MIN_ENVS"):
-        monkeypatch.delenv(k, raising=False)
-    plain = _env("8_arena", 20000)
-    assert not plain.uses_persistent_kernel                                    # default: the warp-per-env kernel
-    monkeypatch.setenv("CTF_WS", "1")
-    assert not _env("8_arena", 64).uses_persistent_kernel                      # under ~4 envs per logic warp: never
-    big = _env("8_arena", 20000)
-    assert big.uses_persistent_kernel
-    acts = torch.randint(0, 9, (6, 20000, 8), dtype=torch.uint8, device="cuda", generator=torch.Generator(device="cuda").manual_seed(2))
-    for t in range(6):
-        big.step(acts[t])
-        plain.step(acts[t])
-    assert torch.equal(big.obs, plain.obs) and torch.equal(big.meta, plain.meta) and torch.equal(big.rewards, plain.rewards)
-    assert torch.equal(big._grid, plain._grid) and torch.equal(big._agents, plain._agents)
-
-
-def test_persistent_kernel_packed_outputs_and_graph_replay(force_persistent_kernel):
-    """The env counter re-arms itself at the end of every launch, so captured launches replay; packed + dense outputs agree."""
+def test_step_graph_replay_with_dense_and_packed_outputs():
+    """Captured steps writing dense + packed observations replay like eager steps; the packed copy unpacks to the dense one."""
     B = 2000
     eager = _env("8_arena", B, seed=8, stats="counters", packed_obs=True)
     graphed = _env("8_arena", B, seed=8, stats="counters", packed_obs=True, validate_actions=True)
-    assert eager.uses_persistent_kernel
     acts = torch.zeros((B, 8), dtype=torch.uint8, device="cuda")
     gen = torch.Generator(device="cuda").manual_seed(9)
     graph = graphed.make_step_graph(acts, steps_per_replay=1)   # validate_actions is suspended inside the capture
@@ -685,13 +643,9 @@ def test_persistent_kernel_packed_outputs_and_graph_replay(force_persistent_kern
 # ---------------------------------------------------------------------------------------------------
 # defined behaviour where the reference raises: a lethal tag with a full spawn window (gridworld_ctf.py:771)
 # ---------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("persistent", [False, True])
-def test_respawn_into_a_full_spawn_window_sets_the_fault_bit(monkeypatch, persistent):
+def test_respawn_into_a_full_spawn_window_sets_the_fault_bit():
     from marl_ctf_development_b200 import _native
 
-    if persistent:
-        monkeypatch.setenv("CTF_WS", "1")
-        monkeypatch.setenv("CTF_WS_MIN_ENVS", "1")
     B = 6
     env = _env("0_the_split", B, seed=3, env_id_base=50, env_overrides={"AGENT_TYPE_DAMAGE": {0: 100, 1: 100, 2: 100, 3: 100}, "TAG_PROBABILITY": 1.0})
     ce = env.ce
