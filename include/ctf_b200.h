@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 6
+#define CTF_ABI_VERSION 7
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -276,6 +276,37 @@ typedef struct ctf_policy_weights {
 int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uint32_t* packed, const float* meta,
                         int64_t n_envs, int agents_per_env, const uint8_t* agent_ids, int k,
                         void* features, int64_t feature_stride, void* stream);
+
+/* fp32 gradients of the trunk's parameters in torch layout (device memory). */
+typedef struct ctf_policy_grads {
+    float* conv1_w;   /* [16][C][3][3] */
+    float* conv1_b;   /* [16] */
+    float* conv2_w;   /* [32][16][3][3] */
+    float* conv2_b;   /* [32] */
+} ctf_policy_grads_t;
+
+/* Bytes of device workspace ctf_policy_features_backward needs on this handle (fixed per handle: one row of partial
+   sums per CTA of the backward kernel, a count taken from the device's occupancy at ctf_create). */
+int ctf_policy_grad_workspace_size(ctf_handle_t h, size_t* bytes);
+
+/*
+ * Backward of ctf_policy_features for training: the gradients of conv1 / conv2 weights and biases given the
+ * gradient of the loss with respect to the feature rows.  Same sample -> block addressing as ctf_policy_features.
+ * features: the rows ctf_policy_features wrote for these samples with the weights `w` (their conv2 outputs are h2);
+ * grad_features: bf16 [n_samples][feature_stride], only columns < 32*(G-4)^2 are read (metadata and pad columns have no
+ * parameters).  conv2_w_t: bf16 [9 taps][2 k-halves][2 n-tiles][32 lanes][4], conv2.weight in the transposed
+ * mma.sync B-fragment order of fused_policy.conv2_transpose_layout_index().
+ * Per sample: h1 = bf16(tanh(conv1)) recomputed bit for bit as the forward computes it; dz2 = bf16(dF * (1 - h2^2))
+ * (fp32 operations); dW2 and db2 accumulate dz2 (x) h1 in fp32 on tensor cores; dh1 = conv2^T(dz2) on tensor cores
+ * (bf16 weights, fp32 accumulation); dz1 = dh1 * (1 - h1^2) in fp32; dW1 and db1 are exact fp32 sums of dz1 over the
+ * set input bits.  Per-CTA partial sums go to `workspace` (>= ctf_policy_grad_workspace_size bytes, 16-byte aligned)
+ * and are summed in a fixed order: reruns are bit-identical (no atomics).  The gradient buffers are overwritten, not
+ * accumulated into; n_envs = 0 writes zeros.  No allocation and no host synchronisation.
+ */
+int ctf_policy_features_backward(ctf_handle_t h, const ctf_policy_weights_t* w, const void* conv2_w_t,
+                                 const uint32_t* packed, int64_t n_envs, int agents_per_env, const uint8_t* agent_ids,
+                                 int k, const void* features, const void* grad_features, int64_t feature_stride,
+                                 void* workspace, size_t workspace_bytes, const ctf_policy_grads_t* grads, void* stream);
 
 #ifdef __cplusplus
 }

@@ -26,8 +26,10 @@ EXPORTS = (
     "ctf_take_faults",
     "ctf_step_host",
     "ctf_policy_features",
+    "ctf_policy_grad_workspace_size",
+    "ctf_policy_features_backward",
 )
-ABI_VERSION = 6
+ABI_VERSION = 7
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
 
 
@@ -70,6 +72,10 @@ class CtfSizes(C.Structure):
 
 
 class CtfPolicyWeights(C.Structure):
+    _fields_ = [("conv1_w", C.c_void_p), ("conv1_b", C.c_void_p), ("conv2_w", C.c_void_p), ("conv2_b", C.c_void_p)]
+
+
+class CtfPolicyGrads(C.Structure):
     _fields_ = [("conv1_w", C.c_void_p), ("conv1_b", C.c_void_p), ("conv2_w", C.c_void_p), ("conv2_b", C.c_void_p)]
 
 
@@ -118,6 +124,10 @@ def load():
     L.ctf_step_host.argtypes = [C.c_void_p, CtfState, C.c_void_p, CtfOutputs, C.c_void_p, C.c_void_p, C.c_void_p]
     L.ctf_policy_features.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
                                       C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]
+    L.ctf_policy_grad_workspace_size.argtypes = [C.c_void_p, C.POINTER(C.c_size_t)]
+    L.ctf_policy_features_backward.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64,
+                                               C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
+                                               C.c_void_p, C.c_size_t, C.POINTER(CtfPolicyGrads), C.c_void_p]
     if L.ctf_abi_version() != ABI_VERSION:
         raise NativeError(f"ABI version mismatch: library {L.ctf_abi_version()}, binding {ABI_VERSION}")
     if L.ctf_config_size() != C.sizeof(CtfConfig):

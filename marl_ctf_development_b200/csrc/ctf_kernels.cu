@@ -914,6 +914,54 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     return *reinterpret_cast<const uint32_t*>(&v);
 }
 
+// Channel mask of every cell, then conv1 -> tanh -> bf16 of one sample into act ([S1*S1][8] bf16x2): the part of the
+// trunk that k_policy_trunk computes and k_policy_trunk_backward recomputes bit for bit.  Cells and positions first,
+// first + step, ...: the forward's warp passes (lane, 32, __syncwarp), the backward's CTA (thread, CTA size,
+// __syncthreads).  conv1 adds, for every output position, the bias plus the weight columns of the set (cell, channel)
+// pairs of its 3x3 window in a fixed order (dy, dx, c ascending).
+template <typename Sync>
+__device__ __forceinline__ void trunk_conv1(const uint32_t* bits, uint16_t* cmask, uint32_t* act, const float* w1,
+                                            const float* b1, int C, int G, int GG, int S1, int first, int step, Sync sync) {
+    // channel mask of every cell: bit c = element c*GG + p
+    for (int p = first; p < GG; p += step) {
+        uint32_t m = 0;
+        for (int c = 0; c < C; ++c) {
+            const int el = c * GG + p;
+            m |= ((bits[el >> 5] >> (el & 31)) & 1u) << c;
+        }
+        cmask[p] = (uint16_t)m;
+    }
+    sync();
+    for (int q = first; q < S1 * S1; q += step) {
+        const int y = q / S1, x = q - y * S1;
+        float acc[16];
+#pragma unroll
+        for (int o = 0; o < 16; ++o) acc[o] = b1[o];
+        for (int dy = 0; dy < 3; ++dy) {
+            for (int dx = 0; dx < 3; ++dx) {
+                uint32_t m = cmask[(y + dy) * G + x + dx];
+                while (m) {
+                    const int c = __ffs(m) - 1;
+                    m &= m - 1;
+                    const float4* col = reinterpret_cast<const float4*>(w1 + ((c * 3 + dy) * 3 + dx) * 16);
+#pragma unroll
+                    for (int v = 0; v < 4; ++v) {
+                        const float4 wv = col[v];
+                        acc[4 * v] += wv.x; acc[4 * v + 1] += wv.y; acc[4 * v + 2] += wv.z; acc[4 * v + 3] += wv.w;
+                    }
+                }
+            }
+        }
+        uint4 lo, hi;
+        lo.x = pack_bf16x2(tanhf(acc[0]), tanhf(acc[1]));   lo.y = pack_bf16x2(tanhf(acc[2]), tanhf(acc[3]));
+        lo.z = pack_bf16x2(tanhf(acc[4]), tanhf(acc[5]));   lo.w = pack_bf16x2(tanhf(acc[6]), tanhf(acc[7]));
+        hi.x = pack_bf16x2(tanhf(acc[8]), tanhf(acc[9]));   hi.y = pack_bf16x2(tanhf(acc[10]), tanhf(acc[11]));
+        hi.z = pack_bf16x2(tanhf(acc[12]), tanhf(acc[13])); hi.w = pack_bf16x2(tanhf(acc[14]), tanhf(acc[15]));
+        reinterpret_cast<uint4*>(act)[2 * q] = lo;
+        reinterpret_cast<uint4*>(act)[2 * q + 1] = hi;
+    }
+}
+
 __global__ void __launch_bounds__(kTrunkThreads) k_policy_trunk(const __grid_constant__ TrunkArgs A) {
     extern __shared__ uint4 smem_raw[];
     float* w1 = reinterpret_cast<float*>(smem_raw);                      // [C*9][16]: column of one (c, dy, dx) tap
@@ -947,45 +995,7 @@ __global__ void __launch_bounds__(kTrunkThreads) k_policy_trunk(const __grid_con
         const uint32_t* src = A.packed + blk * A.wpa;
         for (int i = lane; i < A.wpa; i += 32) bits[i] = __ldg(src + i);
         __syncwarp();
-        // channel mask of every cell: bit c = element c*GG + p
-        for (int p = lane; p < GG; p += 32) {
-            uint32_t m = 0;
-            for (int c = 0; c < C; ++c) {
-                const int el = c * GG + p;
-                m |= ((bits[el >> 5] >> (el & 31)) & 1u) << c;
-            }
-            cmask[p] = (uint16_t)m;
-        }
-        __syncwarp();
-        // conv1: bias + the weight columns of the set (cell, channel) pairs, fixed order (dy, dx, c ascending)
-        for (int q = lane; q < S1 * S1; q += 32) {
-            const int y = q / S1, x = q - y * S1;
-            float acc[16];
-#pragma unroll
-            for (int o = 0; o < 16; ++o) acc[o] = b1[o];
-            for (int dy = 0; dy < 3; ++dy) {
-                for (int dx = 0; dx < 3; ++dx) {
-                    uint32_t m = cmask[(y + dy) * G + x + dx];
-                    while (m) {
-                        const int c = __ffs(m) - 1;
-                        m &= m - 1;
-                        const float4* col = reinterpret_cast<const float4*>(w1 + ((c * 3 + dy) * 3 + dx) * 16);
-#pragma unroll
-                        for (int v = 0; v < 4; ++v) {
-                            const float4 wv = col[v];
-                            acc[4 * v] += wv.x; acc[4 * v + 1] += wv.y; acc[4 * v + 2] += wv.z; acc[4 * v + 3] += wv.w;
-                        }
-                    }
-                }
-            }
-            uint4 lo, hi;
-            lo.x = pack_bf16x2(tanhf(acc[0]), tanhf(acc[1]));   lo.y = pack_bf16x2(tanhf(acc[2]), tanhf(acc[3]));
-            lo.z = pack_bf16x2(tanhf(acc[4]), tanhf(acc[5]));   lo.w = pack_bf16x2(tanhf(acc[6]), tanhf(acc[7]));
-            hi.x = pack_bf16x2(tanhf(acc[8]), tanhf(acc[9]));   hi.y = pack_bf16x2(tanhf(acc[10]), tanhf(acc[11]));
-            hi.z = pack_bf16x2(tanhf(acc[12]), tanhf(acc[13])); hi.w = pack_bf16x2(tanhf(acc[14]), tanhf(acc[15]));
-            reinterpret_cast<uint4*>(act)[2 * q] = lo;
-            reinterpret_cast<uint4*>(act)[2 * q + 1] = hi;
-        }
+        trunk_conv1(bits, cmask, act, w1, b1, C, G, GG, S1, lane, 32, [] { __syncwarp(); });
         __syncwarp();
         __nv_bfloat16* row = A.features + s * A.stride;
         // conv2: n-tile (8 output channels) outer, m-tile (16 positions) inner, one k-step per tap
@@ -1055,6 +1065,288 @@ static __host__ void trunk_layout(const DevPlan& P, TrunkArgs& A, size_t& smem) 
     smem = (shared_words + (size_t)kTrunkWarps * A.warp_words) * 4;
 }
 
+// ------------------------------------------------------------------------------------------------
+// backward of the policy trunk: parameter gradients of conv1 / conv2 from packed observations, saved rows and dRows
+// ------------------------------------------------------------------------------------------------
+// One CTA works on one sample at a time (samples blockIdx.x, + gridDim.x, ...) and accumulates the parameter gradients
+// of all its samples in registers; every gradient slot has exactly one owner thread, so there are no atomics.
+//   1. stage the packed words; trunk_conv1 rebuilds the channel mask and h1 = bf16(tanh(conv1)) as the forward does;
+//      dz2 = bf16(dRow * (1 - h2^2)) (fp32, h2 = the saved row) into a [position][32 channels] tile.
+//   2. dW2 (+ db2) on tensor cores: D[co][(tap, ci)] += dz2[co][m] * h1[ci][m + tap], M = 32, K = the (G-4)^2 positions,
+//      N = 144 + one column of ones whose product is db2; both operands come from [position][channel] tiles through
+//      ldmatrix.trans.  Warp w owns n-tiles w, w + 8, w + 16 of both m-tiles.
+//      dh1 = conv2^T(dz2) on tensor cores: M = (G-2)^2 positions, N = 16, K = 9 taps x 32 channels (18 k-steps), B from
+//      the transposed fragment layout (fused_policy.conv2_transpose_layout_index); dz1 = dh1 * (1 - h1^2) in fp32.
+//   3. dW1 sparsely: thread j owns column (c, tap) = j / 2 and output channels 8 (j & 1) .. + 7 and walks the set bits
+//      of channel c, adding dz1 of the output position each one feeds (exact fp32 adds, fixed order); one more column
+//      sums dz1 over every position (db1).
+// Each CTA writes its partial sums to its row of the workspace; k_policy_grad_reduce sums the rows in index order.
+constexpr int kBwdThreads = 256;
+constexpr int kBwdWarps = kBwdThreads / 32;
+constexpr int kBwdNt = 19;                      // dW2 n-tiles: 18 of (tap, 8 input channels) + the ones column (db2)
+constexpr int kBwdW2tWords = 9 * 2 * 2 * 32 * 2;   // conv2^T B fragments: [tap][k-half][n-tile][lane][2 x bf16x2]
+// partial sums of one CTA: [dW2 [32][tap*16 + ci] | db2 [32] | dW1 [c*9 + tap][16] | db1 [16]]
+constexpr int kGradW2 = 0, kGradB2 = 32 * 144, kGradW1 = kGradB2 + 32;
+__host__ __device__ constexpr int grad_count(int C) { return kGradW1 + C * 9 * 16 + 16; }
+
+struct TrunkBwdArgs {
+    const float* conv1_w;
+    const float* conv1_b;
+    const uint2* conv2_wt;
+    const uint32_t* packed;
+    const __nv_bfloat16* features;
+    const __nv_bfloat16* grad_features;
+    float* partial;           // [gridDim.x][grad_count(C)]
+    long long n_samples;
+    long long stride;
+    int ape, k;
+    int G, C, GG, wpa;
+    int S1, S2, K2;           // conv1 / conv2 output side, conv2 positions padded to a multiple of 16
+    int off_bits, off_mask, off_act, off_dz2;   // word offsets of the per-sample buffers (dz1 shares the mask's words)
+    unsigned char ids[CTF_MAX_AGENTS];
+};
+
+__device__ __forceinline__ void ldsm_x4_trans(uint32_t (&r)[4], const void* p) {
+    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];\n"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"((unsigned)__cvta_generic_to_shared(p)));
+}
+__device__ __forceinline__ void ldsm_x2_trans(uint32_t& r0, uint32_t& r1, const void* p) {
+    asm volatile("ldmatrix.sync.aligned.m8n8.x2.trans.shared.b16 {%0,%1}, [%2];\n"
+                 : "=r"(r0), "=r"(r1) : "r"((unsigned)__cvta_generic_to_shared(p)));
+}
+__device__ __forceinline__ void mma_bf16(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
+                                         uint32_t b1) {
+    asm volatile(
+        "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};\n"
+        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+        : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+}
+// d * (1 - h*h) with one rounding per operation and no contraction, as torch evaluates it in fp32
+__device__ __forceinline__ float tanh_grad(float d, float h) { return __fmul_rn(d, __fsub_rn(1.f, __fmul_rn(h, h))); }
+
+// 3 CTAs per SM: 80 registers without spills (126 unbounded = 2 CTAs; 4 CTAs = 64 registers and spills)
+__global__ void __launch_bounds__(kBwdThreads, 3) k_policy_trunk_backward(const __grid_constant__ TrunkBwdArgs A) {
+    extern __shared__ uint4 smem_raw[];
+    float* w1 = reinterpret_cast<float*>(smem_raw);                      // [C*9][16] as in k_policy_trunk
+    float* b1 = w1 + A.C * 9 * 16;                                        // [16]
+    uint32_t* ones = reinterpret_cast<uint32_t*>(b1 + 16);                // [4]: 8 bf16 ones (one ldmatrix row)
+    uint2* w2t = reinterpret_cast<uint2*>(ones + 4);                      // [9][2][2][32]
+    uint32_t* base = reinterpret_cast<uint32_t*>(smem_raw);
+    uint32_t* bits = base + A.off_bits;                                   // [wpa]
+    uint16_t* cmask = reinterpret_cast<uint16_t*>(base + A.off_mask);     // [GG]
+    float* dz1 = reinterpret_cast<float*>(base + A.off_mask);            // [S1*S1][16], after conv1 (cmask is dead)
+    uint32_t* act = base + A.off_act;                                     // [S1*S1][8] bf16x2 = h1
+    __nv_bfloat16* dz2 = reinterpret_cast<__nv_bfloat16*>(base + A.off_dz2);   // [K2][32]
+    const uint32_t* dz2w = base + A.off_dz2;
+    const int C = A.C, G = A.G, GG = A.GG, S1 = A.S1, S2 = A.S2, M2 = S2 * S2, Q = S1 * S1, K2 = A.K2;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
+    for (int i = tid; i < C * 9 * 16; i += kBwdThreads) {
+        const int o = i & 15, tap = i >> 4;
+        w1[i] = A.conv1_w[o * C * 9 + tap];
+    }
+    if (tid < 16) b1[tid] = A.conv1_b[tid];
+    if (tid < 4) ones[tid] = 0x3F803F80u;                                  // bf16 1.0 twice
+    for (int i = tid; i < kBwdW2tWords / 2; i += kBwdThreads) w2t[i] = A.conv2_wt[i];
+
+    float accw2[3][2][4];                                                  // [n-tile w + 8i][m-tile][mma D]
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+            for (int r = 0; r < 4; ++r) accw2[i][mt][r] = 0.f;
+    const int col = tid >> 1, half = tid & 1;                              // dW1 column (c*9 + tap, or C*9: db1)
+    const bool has_col = col <= C * 9;
+    const int cc = col / 9, ctap = col - cc * 9, cdy = ctap / 3, cdx = ctap - cdy * 3;
+    float accw1[8];
+#pragma unroll
+    for (int o = 0; o < 8; ++o) accw1[o] = 0.f;
+    const int n_mt1 = (Q + 15) >> 4;                                        // dh1 m-tiles
+    const unsigned div_g = 65536u / (unsigned)G + 1u;                       // p / G = (p * div_g) >> 16 for p < 256
+
+    for (long long s = blockIdx.x; s < A.n_samples; s += gridDim.x) {
+        const long long e = s / A.k;
+        const int j = (int)(s - e * A.k);
+        const long long blk = e * A.ape + A.ids[j];
+        const uint32_t* src = A.packed + blk * A.wpa;
+        for (int i = tid; i < A.wpa; i += kBwdThreads) bits[i] = __ldg(src + i);
+        __syncthreads();                                                   // also orders the weights on the first pass
+        trunk_conv1(bits, cmask, act, w1, b1, C, G, GG, S1, tid, kBwdThreads, [] { __syncthreads(); });
+        // dz2 = dRow * (1 - h2^2), 8 row elements per 16-byte load; element co*M2 + m goes to dz2[m][co]
+        const uint4* hrow = reinterpret_cast<const uint4*>(A.features + s * A.stride);
+        const uint4* drow = reinterpret_cast<const uint4*>(A.grad_features + s * A.stride);
+        for (int i = tid; i < 4 * M2; i += kBwdThreads) {
+            const uint4 hv = __ldg(hrow + i), dv = __ldg(drow + i);
+            const __nv_bfloat16* h8 = reinterpret_cast<const __nv_bfloat16*>(&hv);
+            const __nv_bfloat16* d8 = reinterpret_cast<const __nv_bfloat16*>(&dv);
+            int co = (8 * i) / M2, m = 8 * i - co * M2;
+#pragma unroll
+            for (int u = 0; u < 8; ++u) {
+                dz2[m * 32 + co] = __float2bfloat16_rn(tanh_grad(__bfloat162float(d8[u]), __bfloat162float(h8[u])));
+                if (++m == M2) { m = 0; ++co; }
+            }
+        }
+        for (int i = M2 * 16 + tid; i < K2 * 16; i += kBwdThreads) base[A.off_dz2 + i] = 0u;   // K padding rows
+        __syncthreads();
+
+        // dW2 and db2: A = dz2 (rows co), B = h1 at position m + tap (columns (tap, ci)) or ones
+        for (int k0 = 0; k0 < K2; k0 += 16) {
+            uint32_t a[2][4];
+            {
+                const int mat = lane >> 3, m = k0 + (mat >> 1) * 8 + (lane & 7);
+#pragma unroll
+                for (int mt = 0; mt < 2; ++mt) ldsm_x4_trans(a[mt], dz2 + m * 32 + 16 * mt + (mat & 1) * 8);
+            }
+            const int mb = min(k0 + (lane & 15), M2 - 1);                   // pad rows: A is zero there
+            const int yb = mb / S2, pb = yb * S1 + (mb - yb * S2);
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+                const int nt = warp + 8 * i;
+                if (nt < kBwdNt) {
+                    const int tap = nt >> 1;
+                    const void* bp = nt == 18 ? static_cast<const void*>(ones)
+                                              : static_cast<const void*>(act + (pb + (tap / 3) * S1 + tap % 3) * 8 + (nt & 1) * 4);
+                    uint32_t b0, b1r;
+                    ldsm_x2_trans(b0, b1r, bp);
+#pragma unroll
+                    for (int mt = 0; mt < 2; ++mt) mma_bf16(accw2[i][mt], a[mt][0], a[mt][1], a[mt][2], a[mt][3], b0, b1r);
+                }
+            }
+        }
+        // dh1 = conv2^T(dz2) per (m-tile of conv1 positions, n-tile of 8 input channels); dz1 = dh1 * (1 - h1^2)
+        for (int job = (warp + 5) & 7; job < 2 * n_mt1; job += kBwdWarps) {
+            const int mt = job >> 1, nt = job & 1;
+            const int q0 = mt * 16 + g, q1 = q0 + 8;
+            const int y0 = q0 / S1, x0 = q0 - y0 * S1, y1 = q1 / S1, x1 = q1 - y1 * S1;
+            float d[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+            for (int tap = 0; tap < 9; ++tap) {
+                const int dy = tap / 3, dx = tap % 3;
+                const int r0y = y0 - dy, r0x = x0 - dx, r1y = y1 - dy, r1x = x1 - dx;
+                const bool v0 = q0 < Q && (unsigned)r0y < (unsigned)S2 && (unsigned)r0x < (unsigned)S2;
+                const bool v1 = q1 < Q && (unsigned)r1y < (unsigned)S2 && (unsigned)r1x < (unsigned)S2;
+                const int m0 = v0 ? r0y * S2 + r0x : 0, m1 = v1 ? r1y * S2 + r1x : 0;
+#pragma unroll
+                for (int kh = 0; kh < 2; ++kh) {
+                    const uint32_t a0 = v0 ? dz2w[m0 * 16 + kh * 8 + t] : 0u, a2 = v0 ? dz2w[m0 * 16 + kh * 8 + 4 + t] : 0u;
+                    const uint32_t a1 = v1 ? dz2w[m1 * 16 + kh * 8 + t] : 0u, a3 = v1 ? dz2w[m1 * 16 + kh * 8 + 4 + t] : 0u;
+                    const uint2 b = w2t[((tap * 2 + kh) * 2 + nt) * 32 + lane];
+                    mma_bf16(d, a0, a1, a2, a3, b.x, b.y);
+                }
+            }
+            const int ci = nt * 8 + 2 * t;
+            if (q0 < Q) {
+                const __nv_bfloat162 h = *reinterpret_cast<const __nv_bfloat162*>(act + q0 * 8 + (ci >> 1));
+                *reinterpret_cast<float2*>(dz1 + q0 * 16 + ci) =
+                    make_float2(tanh_grad(d[0], __low2float(h)), tanh_grad(d[1], __high2float(h)));
+            }
+            if (q1 < Q) {
+                const __nv_bfloat162 h = *reinterpret_cast<const __nv_bfloat162*>(act + q1 * 8 + (ci >> 1));
+                *reinterpret_cast<float2*>(dz1 + q1 * 16 + ci) =
+                    make_float2(tanh_grad(d[2], __low2float(h)), tanh_grad(d[3], __high2float(h)));
+            }
+        }
+        __syncthreads();
+
+        // dW1: the set bits of channel cc feed output position (cell - tap) when it is inside the conv1 output
+        if (has_col) {
+            const float4* z = reinterpret_cast<const float4*>(dz1) + half * 2;
+            if (col < C * 9) {
+                const int el0 = cc * GG, el1 = el0 + GG;
+                for (int w = el0 >> 5; w <= (el1 - 1) >> 5; ++w) {
+                    uint32_t m = bits[w];
+                    if (32 * w < el0) m &= ~0u << (el0 - 32 * w);
+                    if (32 * w + 32 > el1) m &= ~0u >> (32 * w + 32 - el1);
+                    while (m) {
+                        const int p = 32 * w + __ffs(m) - 1 - el0;
+                        m &= m - 1;
+                        const int py = (int)(((unsigned)p * div_g) >> 16), px = p - py * G;
+                        const int qy = py - cdy, qx = px - cdx;
+                        if ((unsigned)qy < (unsigned)S1 && (unsigned)qx < (unsigned)S1) {
+                            const float4 u = z[(qy * S1 + qx) * 4], v = z[(qy * S1 + qx) * 4 + 1];
+                            accw1[0] += u.x; accw1[1] += u.y; accw1[2] += u.z; accw1[3] += u.w;
+                            accw1[4] += v.x; accw1[5] += v.y; accw1[6] += v.z; accw1[7] += v.w;
+                        }
+                    }
+                }
+            } else {
+                for (int q = 0; q < Q; ++q) {
+                    const float4 u = z[q * 4], v = z[q * 4 + 1];
+                    accw1[0] += u.x; accw1[1] += u.y; accw1[2] += u.z; accw1[3] += u.w;
+                    accw1[4] += v.x; accw1[5] += v.y; accw1[6] += v.z; accw1[7] += v.w;
+                }
+            }
+        }
+        __syncthreads();
+    }
+
+    // partial sums of this CTA (zeros when it had no sample)
+    float* out = A.partial + (size_t)blockIdx.x * grad_count(C);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        const int nt = warp + 8 * i;
+        if (nt < kBwdNt) {
+#pragma unroll
+            for (int mt = 0; mt < 2; ++mt) {
+                const int co = mt * 16 + g;
+                if (nt < 18) {
+                    const int n = nt * 8 + 2 * t;
+                    *reinterpret_cast<float2*>(out + kGradW2 + co * 144 + n) = make_float2(accw2[i][mt][0], accw2[i][mt][1]);
+                    *reinterpret_cast<float2*>(out + kGradW2 + (co + 8) * 144 + n) = make_float2(accw2[i][mt][2], accw2[i][mt][3]);
+                } else if (t == 0) {                                                         // column 0 of the ones tile
+                    out[kGradB2 + co] = accw2[i][mt][0];
+                    out[kGradB2 + co + 8] = accw2[i][mt][2];
+                }
+            }
+        }
+    }
+    if (has_col) {
+        float4* o = reinterpret_cast<float4*>(out + kGradW1 + col * 16 + half * 8);
+        o[0] = make_float4(accw1[0], accw1[1], accw1[2], accw1[3]);
+        o[1] = make_float4(accw1[4], accw1[5], accw1[6], accw1[7]);
+    }
+}
+
+// Sums the n_parts partial rows in row order (fixed, so reruns are bit-identical) and writes the gradients in torch
+// layout: thread i produces element i of [conv1.weight [16][C][3][3] | conv1.bias | conv2.weight [32][16][3][3] | conv2.bias].
+__global__ void k_policy_grad_reduce(const float* __restrict__ partial, int n_parts, int C, float* __restrict__ g_c1w,
+                                     float* __restrict__ g_c1b, float* __restrict__ g_c2w, float* __restrict__ g_c2b) {
+    const int n_c1w = 16 * C * 9, n = grad_count(C);
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    int src;
+    float* dst;
+    if (i < n_c1w) {
+        const int o = i / (C * 9), col = i - o * C * 9;                  // col = c*9 + tap
+        src = kGradW1 + col * 16 + o; dst = g_c1w + i;
+    } else if ((i -= n_c1w) < 16) {
+        src = kGradW1 + C * 9 * 16 + i; dst = g_c1b + i;
+    } else if ((i -= 16) < 32 * 144) {
+        const int co = i / 144, r = i - co * 144, ci = r / 9, tap = r - ci * 9;
+        src = kGradW2 + co * 144 + tap * 16 + ci; dst = g_c2w + i;
+    } else if ((i -= 32 * 144) < 32) {
+        src = kGradB2 + i; dst = g_c2b + i;
+    } else {
+        return;
+    }
+    float acc = 0.f;
+#pragma unroll 8
+    for (int p = 0; p < n_parts; ++p) acc += __ldg(partial + (size_t)p * n + src);
+    *dst = acc;
+}
+
+// shared-memory layout of k_policy_trunk_backward for a plan
+static __host__ void trunk_bwd_layout(const DevPlan& P, TrunkBwdArgs& A, size_t& smem) {
+    const int S1 = P.G - 2, S2 = P.G - 4;
+    const auto up4 = [](int w) { return (w + 3) & ~3; };
+    A.G = P.G; A.C = P.C; A.GG = P.GG; A.wpa = P.wpa; A.S1 = S1; A.S2 = S2; A.K2 = (S2 * S2 + 15) & ~15;
+    A.off_bits = P.C * 9 * 16 + 16 + 4 + kBwdW2tWords;                 // after w1, b1, ones, w2t (all 16-byte multiples)
+    A.off_mask = A.off_bits + up4(P.wpa);
+    const int mask_words = up4((P.GG + 1) / 2), dz1_words = S1 * S1 * 16;
+    A.off_act = A.off_mask + (mask_words > dz1_words ? mask_words : dz1_words);
+    A.off_dz2 = A.off_act + S1 * S1 * 8;
+    smem = (size_t)(A.off_dz2 + A.K2 * 16) * 4;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -1076,6 +1368,8 @@ struct ctf_env {
     size_t smem_bytes;
     size_t trunk_smem_bytes; // k_policy_trunk: dynamic shared memory for this plan
     int trunk_ctas;          // k_policy_trunk: CTAs that fit on the device at once
+    size_t bwd_smem_bytes;   // k_policy_trunk_backward: dynamic shared memory for this plan
+    int bwd_ctas;            // k_policy_trunk_backward: CTAs (= workspace rows) of every launch with >= bwd_ctas samples
 };
 
 // cudaSetDevice for the duration of an entry point; the caller's current device is restored on return
@@ -1300,6 +1594,16 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
             e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk, kTrunkThreads, h->trunk_smem_bytes);
         h->trunk_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
     }
+    // k_policy_trunk_backward needs at most 46 KB (G = 16, C = 14)
+    CTF_SET_SMEM(k_policy_trunk_backward, 64 * 1024);
+    {
+        TrunkBwdArgs ba;
+        trunk_bwd_layout(h->plan, ba, h->bwd_smem_bytes);
+        int per_sm = 0;
+        if (e == cudaSuccess && h->plan.G >= 5)
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk_backward, kBwdThreads, h->bwd_smem_bytes);
+        h->bwd_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
+    }
 #undef CTF_SET_SMEM_T
 #undef CTF_SET_SMEM
     if (e != cudaSuccess) {
@@ -1511,6 +1815,72 @@ extern "C" int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w
     const long long want = (n + kTrunkWarps - 1) / kTrunkWarps;
     const unsigned grid = (unsigned)(want < h->trunk_ctas ? want : h->trunk_ctas);
     k_policy_trunk<<<grid, kTrunkThreads, smem, static_cast<cudaStream_t>(stream)>>>(A);
+    CTF_CUDA(cudaGetLastError());
+    return CTF_OK;
+}
+
+extern "C" int ctf_policy_grad_workspace_size(ctf_handle_t h, size_t* bytes) {
+    if (!h || !bytes) return fail(CTF_ERR_INVALID, "ctf_policy_grad_workspace_size: null argument");
+    if (h->plan.G < 5)
+        return fail(CTF_ERR_INVALID, "ctf_policy_grad_workspace_size: the policy needs grid_size >= 5 (two valid 3x3 convolutions)");
+    *bytes = (size_t)h->bwd_ctas * grad_count(h->plan.C) * sizeof(float);
+    return CTF_OK;
+}
+
+extern "C" int ctf_policy_features_backward(ctf_handle_t h, const ctf_policy_weights_t* w, const void* conv2_w_t,
+                                            const uint32_t* packed, int64_t n_envs, int agents_per_env,
+                                            const uint8_t* agent_ids, int k, const void* features,
+                                            const void* grad_features, int64_t feature_stride, void* workspace,
+                                            size_t workspace_bytes, const ctf_policy_grads_t* grads, void* stream) {
+    if (!h || !w || !conv2_w_t || !packed || !agent_ids || !features || !grad_features || !workspace || !grads)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: null argument");
+    if (!w->conv1_w || !w->conv1_b || !w->conv2_w || !w->conv2_b)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: null weight pointer");
+    if (!grads->conv1_w || !grads->conv1_b || !grads->conv2_w || !grads->conv2_b)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: null gradient pointer");
+    const DevPlan& P = h->plan;
+    if (P.G < 5) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: the policy needs grid_size >= 5 (two valid 3x3 convolutions)");
+    if (k < 1 || k > CTF_MAX_AGENTS) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: k must be in 1..8");
+    if (agents_per_env < 1) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: agents_per_env must be >= 1");
+    if (n_envs < 0) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: negative n_envs");
+    for (int j = 0; j < k; ++j)
+        if (agent_ids[j] >= agents_per_env)
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: an agent id is >= agents_per_env");
+    const long long k1 = 32LL * (P.G - 4) * (P.G - 4) + P.M;
+    if (feature_stride < k1 || (feature_stride & 7))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: feature_stride must be a multiple of 8 and >= 32*(G-4)^2 + M");
+    if ((reinterpret_cast<uintptr_t>(features) & 15) || (reinterpret_cast<uintptr_t>(grad_features) & 15))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: features and grad_features must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(w->conv1_w) & 15) || (reinterpret_cast<uintptr_t>(conv2_w_t) & 7) ||
+        (reinterpret_cast<uintptr_t>(w->conv1_b) & 3) || (reinterpret_cast<uintptr_t>(packed) & 3) ||
+        (reinterpret_cast<uintptr_t>(workspace) & 15) || (reinterpret_cast<uintptr_t>(grads->conv1_w) & 3) ||
+        (reinterpret_cast<uintptr_t>(grads->conv1_b) & 3) || (reinterpret_cast<uintptr_t>(grads->conv2_w) & 3) ||
+        (reinterpret_cast<uintptr_t>(grads->conv2_b) & 3))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: misaligned weights, inputs, workspace or gradients");
+    const int n_grad = grad_count(P.C);
+    if (workspace_bytes < (size_t)h->bwd_ctas * n_grad * sizeof(float))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: workspace smaller than ctf_policy_grad_workspace_size");
+    const long long n = (long long)n_envs * k;
+    TrunkBwdArgs A;
+    memset(&A, 0, sizeof(A));
+    size_t smem = 0;
+    trunk_bwd_layout(P, A, smem);
+    A.conv1_w = w->conv1_w; A.conv1_b = w->conv1_b; A.conv2_wt = static_cast<const uint2*>(conv2_w_t);
+    A.packed = packed;
+    A.features = static_cast<const __nv_bfloat16*>(features);
+    A.grad_features = static_cast<const __nv_bfloat16*>(grad_features);
+    A.partial = static_cast<float*>(workspace);
+    A.n_samples = n; A.stride = feature_stride; A.ape = agents_per_env; A.k = k;
+    for (int j = 0; j < k; ++j) A.ids[j] = agent_ids[j];
+    DeviceGuard guard(h->device);
+    CTF_CUDA(guard.err);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    // one CTA per sample up to bwd_ctas: the partition of samples into rows, and so every sum, depends on n alone
+    const int parts = (int)(n < h->bwd_ctas ? n : h->bwd_ctas);
+    if (parts > 0) k_policy_trunk_backward<<<parts, kBwdThreads, smem, s>>>(A);
+    const int total = 16 * P.C * 9 + 16 + 32 * 144 + 32;
+    k_policy_grad_reduce<<<(total + 255) / 256, 256, 0, s>>>(A.partial, parts, P.C, grads->conv1_w, grads->conv1_b,
+                                                             grads->conv2_w, grads->conv2_b);
     CTF_CUDA(cudaGetLastError());
     return CTF_OK;
 }

@@ -11,7 +11,13 @@ to it (the pad columns of the rows are exact zeros), which keeps K a multiple of
 
 Precision: this is a bf16 path, like running ``CtfPolicy`` under ``torch.autocast(dtype=torch.bfloat16)``; it is not
 bit-equal to fp32 ``CtfPolicy``.  ``reference_features`` states in torch exactly what the kernel computes.
-Inference only: the PPO update keeps using ``CtfPolicy`` on ``env.unpack_obs`` output.
+
+Training: ``FusedPolicy.evaluate_actions`` is the differentiable counterpart of ``CtfPolicy.get_action_and_value`` with
+a given action, for the PPO update on a packed minibatch.  Its trunk runs ``ctf_policy_features`` forward and
+``ctf_policy_features_backward`` (``k_policy_trunk_backward``) for the conv1 / conv2 gradients; fc1 ... heads run in
+bf16 through autograd.  ``reference_trunk_grads`` states in torch what the backward kernel computes.  Each sample keeps
+2 x stride bf16 values alive between forward and backward (its rows and their gradient: 15.6 KB at 8_arena), so a
+caller splits a large minibatch into chunks and lets the gradients accumulate.
 """
 from __future__ import annotations
 
@@ -44,6 +50,20 @@ def conv2_kernel_layout_index(device=None) -> torch.Tensor:
     g, t = lane // 4, lane % 4
     ci = 2 * t + torch.tensor([0, 1, 8, 9]).view(1, 1, 1, 4)
     return ((8 * nt + g) * 144 + ci * 9 + tap).reshape(-1).to(device)
+
+
+def conv2_transpose_layout_index(device=None) -> torch.Tensor:
+    """Index into ``conv2.weight.reshape(-1)`` that gives the backward kernel's bf16 layout of conv2 transposed,
+    [tap 9][k-half 2][n-tile 2][lane 32][4]: the mma.sync m16n8k16 B registers of dh1 = conv2^T(dz2), whose K is the
+    32 output channels of a tap (two k-steps) and N the 16 input channels.  Lane 4*g + t of n-tile j in k-half h holds,
+    for input channel 8*j + g, output channels 16*h + (2t, 2t+1, 2t+8, 2t+9) of the tap."""
+    tap = torch.arange(9).view(9, 1, 1, 1, 1)
+    kh = torch.arange(2).view(1, 2, 1, 1, 1)
+    nt = torch.arange(2).view(1, 1, 2, 1, 1)
+    lane = torch.arange(32).view(1, 1, 1, 32, 1)
+    g, t = lane // 4, lane % 4
+    co = 16 * kh + 2 * t + torch.tensor([0, 1, 8, 9]).view(1, 1, 1, 1, 4)
+    return (co * 144 + (8 * nt + g) * 9 + tap).reshape(-1).to(device)
 
 
 @torch.no_grad()
@@ -80,6 +100,69 @@ def reference_features(policy, dense_obs: torch.Tensor, meta: torch.Tensor, roun
     h2 = F.conv2d(h1.double(), w2).float() + policy.conv2.bias.float().view(1, -1, 1, 1)
     h2 = bf(torch.tanh(h2))
     return torch.cat((h2.reshape(h2.shape[0], -1), bf(meta.float())), dim=1)
+
+
+def reference_trunk_grads(policy, dense_obs: torch.Tensor, grad_rows: torch.Tensor, round_bf16: bool = True,
+                          features: torch.Tensor | None = None):
+    """What ``k_policy_trunk_backward`` computes, in torch: the gradients (conv1.weight, conv1.bias, conv2.weight,
+    conv2.bias) of sum(rows[:, :32*(G-4)^2] * grad_rows[:, :32*(G-4)^2]), float32.
+
+    h1 is ``reference_conv1`` (bf16 values); h2 is the conv2 part of ``features`` (the rows the forward kernel wrote)
+    or, when None, of ``reference_features``; dz2 = bf16(dF * (1 - h2^2)) in fp32 operations; db2 and dW2 = dz2 (x) h1
+    are summed exactly (float64) and rounded to fp32 once; dh1 = conv2^T(dz2) with bf16 weights, summed exactly and
+    rounded to fp32; dz1 = dh1 * (1 - h1^2) in fp32; dW1 and db1 are exact sums of dz1 over the set input bits, rounded
+    once.  The kernel's sums are fp32 (tensor cores for dW2, db2 and dh1, ordered adds for dW1 and db1), which is the
+    whole difference.  With round_bf16=False nothing is rounded: everything runs in float64 from the float64
+    parameters (``features`` is ignored) and the result, float64, is autograd of the ``CtfPolicy`` trunk.
+    """
+    from torch.nn.grad import conv2d_input, conv2d_weight
+
+    S, Cn, G, _ = dense_obs.shape
+    S2 = G - 4
+    n2 = 32 * S2 * S2
+    x = dense_obs.double()
+    w1, b1 = policy.conv1.weight.detach(), policy.conv1.bias.detach()
+    w2, b2 = policy.conv2.weight.detach(), policy.conv2.bias.detach()
+    with torch.no_grad():
+        if round_bf16:
+            h1 = reference_conv1(policy, dense_obs)
+            if features is None:
+                h2 = F.conv2d(h1.double(), w2.float().bfloat16().double()).float() + b2.float().view(1, -1, 1, 1)
+                h2 = torch.tanh(h2).bfloat16().float()
+            else:
+                h2 = features[:, :n2].float().reshape(S, 32, S2, S2)
+            d = grad_rows[:, :n2].float().reshape(S, 32, S2, S2)
+            dz2 = (d * (1 - h2 * h2)).bfloat16().float()
+            dh1 = conv2d_input(h1.shape, w2.float().bfloat16().double(), dz2.double()).float()
+            dz1 = dh1 * (1 - h1 * h1)
+            out = (conv2d_weight(x, w1.shape, dz1.double()), dz1.double().sum((0, 2, 3)),
+                   conv2d_weight(h1.double(), w2.shape, dz2.double()), dz2.double().sum((0, 2, 3)))
+            return tuple(t.float() for t in out)
+        w1, b1, w2, b2 = w1.double(), b1.double(), w2.double(), b2.double()
+        h1 = torch.tanh(F.conv2d(x, w1, b1))
+        h2 = torch.tanh(F.conv2d(h1, w2, b2))
+        dz2 = grad_rows[:, :n2].double().reshape(S, 32, S2, S2) * (1 - h2 * h2)
+        dz1 = conv2d_input(h1.shape, w2, dz2) * (1 - h1 * h1)
+        return (conv2d_weight(x, w1.shape, dz1), dz1.sum((0, 2, 3)), conv2d_weight(h1, w2.shape, dz2),
+                dz2.sum((0, 2, 3)))
+
+
+class _PackedTrunk(torch.autograd.Function):
+    """rows = trunk(bits, meta; conv1, conv2) through ctf_policy_features, with ctf_policy_features_backward as its
+    backward.  The rows are saved (a tensor of their own) and the backward re-reads the parameters it was given."""
+
+    @staticmethod
+    def forward(ctx, bits, w1, b1, w2, b2, fused, meta):
+        rows = fused._train_forward(bits, meta, w1, b1, w2, b2)
+        ctx.fused = fused
+        ctx.save_for_backward(bits, rows, w1, b1, w2, b2)
+        return rows
+
+    @staticmethod
+    def backward(ctx, grad_rows):
+        bits, rows, w1, b1, w2, b2 = ctx.saved_tensors
+        g = ctx.fused._train_backward(bits, rows, grad_rows, w1, b1, w2, b2)
+        return (None, *g, None, None)
 
 
 class FusedPolicy:
@@ -122,6 +205,7 @@ class FusedPolicy:
                                                  self._c2b.data_ptr())
         self._features = None   # bf16 [S_max, stride] rows, reused by every call (see features())
         self._ids = {}
+        self._train = None      # training-only weight buffers and workspace, created by the first evaluate_actions
         self.refresh()
 
     @torch.no_grad()
@@ -247,3 +331,105 @@ class FusedPolicy:
     def get_action(self, use_action_mask, *, agent_ids=None, bits=None, meta=None, env=None, envs=None):
         _, logits = self.forward(agent_ids, bits, meta, env, envs)
         return Categorical(logits=self.policy.masked_logits(logits, use_action_mask), validate_args=False).sample()
+
+    # ------------------------------------------------------------------ training
+    def evaluate_actions(self, bits: torch.Tensor, meta: torch.Tensor, use_action_mask, action):
+        """(log_prob [S], entropy [S], value [S, 1]) of ``action`` for packed observations ``bits`` int32 [S, wpa] and
+        ``meta`` [S, M], differentiable into every parameter of ``self.policy``: what ``CtfPolicy.get_action_and_value``
+        with a given action gives the PPO loss, from packed observations.
+
+        The trunk runs the CUDA kernels (``ctf_policy_features`` forward, ``ctf_policy_features_backward`` backward)
+        with the live conv parameters, copied into training-only buffers: the inference buffers of ``refresh()`` (and
+        CUDA graphs captured around them) do not change.  fc1 -> tanh -> fc2 -> tanh run in bf16 on cuBLAS from the
+        fp32 parameters (fc1.weight zero-padded to the row stride as in inference); the small heads run in fp32
+        (``train_head``).  Between forward and backward each sample holds 2 x stride bf16 values (rows and their
+        gradient); split large minibatches into chunks and accumulate gradients over them."""
+        self._check_packed(bits, meta)
+        p = self.policy
+        rows = _PackedTrunk.apply(bits.contiguous(), p.conv1.weight, p.conv1.bias, p.conv2.weight, p.conv2.bias, self,
+                                  meta.contiguous())
+        value, logits = self.train_head(rows)
+        probs = Categorical(logits=p.masked_logits(logits, use_action_mask), validate_args=False)
+        return probs.log_prob(action), probs.entropy(), value
+
+    def train_head(self, rows: torch.Tensor):
+        """(value [S, 1], logits [S, 9]) fp32 from feature rows [S, stride], differentiable into fc1, fc2 and the heads:
+        the part of ``evaluate_actions`` after the trunk.  fc1 -> tanh -> fc2 -> tanh in bf16 on cuBLAS, fc1.weight
+        zero-padded to the stride.  The heads (128 -> 10, 0.1 % of the FLOPs) run in fp32, so value and logits enter
+        the loss unrounded: a bf16 output adds a per-sample rounding that dominates the error of the value-head bias
+        gradient."""
+        p, bf = self.policy, torch.bfloat16
+        x = torch.tanh(F.linear(rows, F.pad(p.fc1.weight, (0, self.stride - self.k1)).to(bf), p.fc1.bias.to(bf)))
+        x = torch.tanh(F.linear(x, p.fc2.weight.to(bf), p.fc2.bias.to(bf)))
+        hw = torch.cat((p.value_head.weight, p.action_head.weight))
+        out = F.linear(x.float(), hw, torch.cat((p.value_head.bias, p.action_head.bias)))
+        return out[:, :1], out[:, 1:]
+
+    def _check_packed(self, bits, meta):
+        env = self.env
+        wpa, M = env.bits_words_per_agent, env.meta_size
+        if bits.dtype != torch.int32 or bits.dim() != 2 or bits.shape[1] != wpa or bits.device != env.device:
+            raise ValueError(f"bits must be an int32 tensor [S, {wpa}] on {env.device}")
+        if meta.dtype != torch.float32 or tuple(meta.shape) != (bits.shape[0], M) or meta.device != env.device:
+            raise ValueError(f"meta must be a float32 tensor [{bits.shape[0]}, {M}] on {env.device}")
+
+    def _train_state(self):
+        if self._train is None:
+            env, dev = self.env, self.env.device
+            Cn = env.n_channels
+            tr = dict(
+                c1w=torch.empty((16, Cn, 3, 3), dtype=torch.float32, device=dev),
+                c1b=torch.empty(16, dtype=torch.float32, device=dev),
+                c2w=torch.empty(9 * 4 * 32 * 4, dtype=torch.bfloat16, device=dev),
+                c2wt=torch.empty(9 * 2 * 2 * 32 * 4, dtype=torch.bfloat16, device=dev),
+                c2b=torch.empty(32, dtype=torch.float32, device=dev),
+                c2t_index=conv2_transpose_layout_index(dev),
+            )
+            tr["weights"] = _native.CtfPolicyWeights(tr["c1w"].data_ptr(), tr["c1b"].data_ptr(), tr["c2w"].data_ptr(),
+                                                     tr["c2b"].data_ptr())
+            n = C.c_size_t()
+            _native.check(env._lib.ctf_policy_grad_workspace_size(env._handle, C.byref(n)))
+            tr["workspace"] = torch.empty(max(n.value // 4, 4), dtype=torch.float32, device=dev)
+            self._train = tr
+        return self._train
+
+    @torch.no_grad()
+    def _load_train_weights(self, w1, b1, w2, b2):
+        tr = self._train_state()
+        tr["c1w"].copy_(w1)
+        tr["c1b"].copy_(b1)
+        tr["c2w"].copy_(w2.reshape(-1)[self._c2_index])
+        tr["c2wt"].copy_(w2.reshape(-1)[tr["c2t_index"]])
+        tr["c2b"].copy_(b2)
+        return tr
+
+    def _train_forward(self, bits, meta, w1, b1, w2, b2):
+        env = self.env
+        tr = self._load_train_weights(w1, b1, w2, b2)
+        rows = torch.empty((bits.shape[0], self.stride), dtype=torch.bfloat16, device=env.device)
+        if bits.shape[0] == 0:
+            return rows
+        ids, _ = self._id_array((0,), 1)
+        stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
+        _native.check(env._lib.ctf_policy_features(
+            env._handle, C.byref(tr["weights"]), C.c_void_p(bits.data_ptr()), C.c_void_p(meta.data_ptr()),
+            bits.shape[0], 1, ids, 1, C.c_void_p(rows.data_ptr()), self.stride, stream))
+        return rows
+
+    def _train_backward(self, bits, rows, grad_rows, w1, b1, w2, b2):
+        env = self.env
+        tr = self._load_train_weights(w1, b1, w2, b2)
+        grad_rows = grad_rows.to(torch.bfloat16).contiguous()
+        grads = [torch.empty_like(t, dtype=torch.float32) for t in (w1, b1, w2, b2)]
+        gs = _native.CtfPolicyGrads(*(g.data_ptr() for g in grads))
+        ids, _ = self._id_array((0,), 1)
+        ws = tr["workspace"]
+        # no samples: the kernel reads no input and writes zero gradients; empty tensors have no address, so the
+        # workspace stands in for the three input pointers
+        ptrs = [t.data_ptr() if bits.shape[0] else ws.data_ptr() for t in (bits, rows, grad_rows)]
+        stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
+        _native.check(env._lib.ctf_policy_features_backward(
+            env._handle, C.byref(tr["weights"]), C.c_void_p(tr["c2wt"].data_ptr()), C.c_void_p(ptrs[0]),
+            bits.shape[0], 1, ids, 1, C.c_void_p(ptrs[1]), C.c_void_p(ptrs[2]), self.stride,
+            C.c_void_p(ws.data_ptr()), ws.numel() * 4, C.byref(gs), stream))
+        return [g.to(t.dtype) for g, t in zip(grads, (w1, b1, w2, b2))]
