@@ -23,12 +23,13 @@
 
 #include <stddef.h>
 #include <stdint.h>
+#include <sys/types.h> /* ssize_t */
 
 #ifdef __cplusplus
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 7
+#define CTF_ABI_VERSION 8
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -307,6 +308,30 @@ int ctf_policy_features_backward(ctf_handle_t h, const ctf_policy_weights_t* w, 
                                  const uint32_t* packed, int64_t n_envs, int agents_per_env, const uint8_t* agent_ids,
                                  int k, const void* features, const void* grad_features, int64_t feature_stride,
                                  void* workspace, size_t workspace_bytes, const ctf_policy_grads_t* grads, void* stream);
+
+/*
+ * Compressible device memory for the dense observation buffer.  On devices with Compute Data Compression the memory
+ * is compressed between L2 and DRAM, invisibly to every kernel and reader: the bytes read back are the bytes written.
+ * The observations are mostly zero sectors, so their store stream moves far fewer DRAM bytes (DESIGN §4).
+ * The two allocation entry points have the signatures torch.cuda.memory.CUDAPluggableAllocator expects (the stream
+ * is unused).  ctf_compressible_alloc maps `size` bytes, rounded up to the allocation granularity, with
+ * cuMemCreate / cuMemAddressReserve / cuMemMap / cuMemSetAccess (read-write for `device`).  It asks for
+ * CU_MEM_ALLOCATION_COMP_GENERIC when the device reports support and compression is enabled, and otherwise, or when
+ * the driver does not grant it, maps ordinary memory on the same path, so ctf_compressible_free releases either kind.
+ * Returns NULL on failure (ctf_last_error has the reason).  The driver entry points are resolved through the CUDA
+ * runtime: the library does not link libcuda.
+ */
+void* ctf_compressible_alloc(ssize_t size, int device, void* stream);
+/* Unmaps and releases a pointer ctf_compressible_alloc returned; `size` is the size it was asked for. */
+void ctf_compressible_free(void* p, ssize_t size, int device, void* stream);
+/* *out = 1 when `device` reports CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, else 0. */
+int ctf_compression_supported(int device, int* out);
+/* *out = 1 when `p` lies in a cuMemMap'ed allocation whose properties say CU_MEM_ALLOCATION_COMP_GENERIC, else 0
+   (also for memory from cudaMalloc or the host). */
+int ctf_mem_is_compressed(const void* p, int* out);
+/* enabled = 0 makes later ctf_compressible_alloc calls map ordinary memory, the path of devices without compression
+   (tests of that path and A/B measurements); 1 (the default) restores compression.  Returns the previous setting. */
+int ctf_compressible_set_enabled(int enabled);
 
 #ifdef __cplusplus
 }

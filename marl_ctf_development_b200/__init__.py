@@ -4,6 +4,7 @@ Public surface:
     GridworldCtfGPU   batched env (B envs per GPU), device tensors in / out
     GridworldCtf      single-env view with the reference's exact methods (drop-in for ppo.py / utils.py)
     FusedPolicy       CtfPolicy inference from packed observations (fused_policy.py)
+    compressible_empty  torch.empty in compressible device memory, for caller-bound observation buffers
     compile_config    (AGENT_CONFIG, SCENARIO, kwargs) -> ctf_config_t
     experiment_env_config / experiment_names   the reference's nine experiment configs as data
 """
@@ -17,6 +18,10 @@ def __getattr__(name):
         from . import env
 
         return getattr(env, name)
+    if name == "compressible_empty":
+        from .compressible import compressible_empty
+
+        return compressible_empty
     if name == "FusedPolicy":
         from .fused_policy import FusedPolicy
 

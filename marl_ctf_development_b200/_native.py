@@ -28,8 +28,13 @@ EXPORTS = (
     "ctf_policy_features",
     "ctf_policy_grad_workspace_size",
     "ctf_policy_features_backward",
+    "ctf_compressible_alloc",
+    "ctf_compressible_free",
+    "ctf_compression_supported",
+    "ctf_mem_is_compressed",
+    "ctf_compressible_set_enabled",
 )
-ABI_VERSION = 7
+ABI_VERSION = 8
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
 
 
@@ -128,6 +133,13 @@ def load():
     L.ctf_policy_features_backward.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64,
                                                C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
                                                C.c_void_p, C.c_size_t, C.POINTER(CtfPolicyGrads), C.c_void_p]
+    L.ctf_compressible_alloc.restype = C.c_void_p
+    L.ctf_compressible_alloc.argtypes = [C.c_ssize_t, C.c_int, C.c_void_p]
+    L.ctf_compressible_free.restype = None
+    L.ctf_compressible_free.argtypes = [C.c_void_p, C.c_ssize_t, C.c_int, C.c_void_p]
+    L.ctf_compression_supported.argtypes = [C.c_int, C.POINTER(C.c_int)]
+    L.ctf_mem_is_compressed.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
+    L.ctf_compressible_set_enabled.argtypes = [C.c_int]
     if L.ctf_abi_version() != ABI_VERSION:
         raise NativeError(f"ABI version mismatch: library {L.ctf_abi_version()}, binding {ABI_VERSION}")
     if L.ctf_config_size() != C.sizeof(CtfConfig):

@@ -14,6 +14,8 @@
 // Randomness is Philox4x32-10 addressed by (seed, global env id, episode, step,
 // site); see marl_ctf_development_b200/draws.py for the site map.  Lane l of the
 // warp generates site l.
+#include <cuda.h>           // driver API types of the compressible allocator (entry points come through the runtime)
+#include <cudaTypedefs.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -21,8 +23,11 @@
 #include <stdio.h>   // snprintf for error messages
 #include <string.h>
 
+#include <atomic>
+#include <mutex>
 #include <new>
 #include <type_traits>
+#include <unordered_map>
 
 #include "../../include/ctf_b200.h"
 
@@ -1365,7 +1370,10 @@ struct ctf_env {
     uint8_t* actions_stage;  // device [B][N], for ctf_step_host
     float* rewards_stage;    // device [B][N], used by ctf_step_host when out.rewards is NULL
     uint8_t* dones_stage;    // device [B]
-    size_t smem_bytes;
+    size_t smem_bytes;       // warp-per-env kernels writing a plain observation buffer (padded to the residency cap)
+    size_t smem_bytes_comp;  // the same kernels writing a compressed one (a different cap, see ctf_create)
+    const void* obs_seen;    // the last outputs.obs launched on, and whether it lies in compressed memory
+    bool obs_seen_comp;
     size_t trunk_smem_bytes; // k_policy_trunk: dynamic shared memory for this plan
     int trunk_ctas;          // k_policy_trunk: CTAs that fit on the device at once
     size_t bwd_smem_bytes;   // k_policy_trunk_backward: dynamic shared memory for this plan
@@ -1400,6 +1408,177 @@ static int fail(int code, const char* fmt, const char* a = "", const char* b = "
 extern "C" const char* ctf_last_error(void) { return g_err; }
 extern "C" int ctf_abi_version(void) { return CTF_ABI_VERSION; }
 extern "C" size_t ctf_config_size(void) { return sizeof(ctf_config_t); }
+
+// ------------------------------------------------------------------ compressible device memory (DESIGN §4)
+// The driver's virtual-memory entry points, resolved through the runtime so that the library does not link libcuda.
+struct VmmApi {
+    PFN_cuGetErrorString err_str = nullptr;
+    PFN_cuDeviceGetAttribute dev_attr = nullptr;
+    PFN_cuMemGetAllocationGranularity granularity = nullptr;
+    PFN_cuMemCreate create = nullptr;
+    PFN_cuMemRelease release = nullptr;
+    PFN_cuMemAddressReserve reserve = nullptr;
+    PFN_cuMemAddressFree addr_free = nullptr;
+    PFN_cuMemMap map = nullptr;
+    PFN_cuMemUnmap unmap = nullptr;
+    PFN_cuMemSetAccess set_access = nullptr;
+    PFN_cuMemRetainAllocationHandle retain = nullptr;
+    PFN_cuMemGetAllocationPropertiesFromHandle props = nullptr;
+    const char* missing = nullptr;   // the first entry point the driver did not provide
+};
+
+static const VmmApi& vmm_api() {
+    static VmmApi api;
+    static std::once_flag once;
+    std::call_once(once, [] {
+        auto get = [](const char* sym, auto& fn) {
+            void* p = nullptr;
+            cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+            if (cudaGetDriverEntryPointByVersion(sym, &p, 12000, cudaEnableDefault, &q) != cudaSuccess ||
+                q != cudaDriverEntryPointSuccess || !p) {
+                if (!api.missing) api.missing = sym;
+                return;
+            }
+            fn = reinterpret_cast<std::remove_reference_t<decltype(fn)>>(p);
+        };
+        get("cuGetErrorString", api.err_str);
+        get("cuDeviceGetAttribute", api.dev_attr);
+        get("cuMemGetAllocationGranularity", api.granularity);
+        get("cuMemCreate", api.create);
+        get("cuMemRelease", api.release);
+        get("cuMemAddressReserve", api.reserve);
+        get("cuMemAddressFree", api.addr_free);
+        get("cuMemMap", api.map);
+        get("cuMemUnmap", api.unmap);
+        get("cuMemSetAccess", api.set_access);
+        get("cuMemRetainAllocationHandle", api.retain);
+        get("cuMemGetAllocationPropertiesFromHandle", api.props);
+    });
+    return api;
+}
+
+static int cu_fail(const VmmApi& api, const char* what, CUresult r) {
+    const char* msg = nullptr;
+    if (api.err_str) api.err_str(r, &msg);
+    return fail(CTF_ERR_CUDA, "%s: %s", what, msg ? msg : "unknown CUDA driver error");
+}
+
+struct VmmBlock {
+    CUmemGenericAllocationHandle handle;
+    size_t bytes;   // mapped size (the request rounded up to the granularity)
+};
+// never destroyed: torch may free its cached blocks after this library's static destructors have run
+static std::mutex* const g_vmm_mu = new std::mutex;
+static std::unordered_map<uintptr_t, VmmBlock>* const g_vmm_blocks = new std::unordered_map<uintptr_t, VmmBlock>;
+static std::atomic<int> g_compression_enabled{1};
+
+static int compression_supported(const VmmApi& api, int device, int* out) {
+    if (api.missing) return fail(CTF_ERR_CUDA, "the CUDA driver does not provide %s", api.missing);
+    int v = 0;
+    CUresult r = api.dev_attr(&v, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, (CUdevice)device);
+    if (r != CUDA_SUCCESS) return cu_fail(api, "cuDeviceGetAttribute(GENERIC_COMPRESSION_SUPPORTED)", r);
+    *out = v ? 1 : 0;
+    return CTF_OK;
+}
+
+static int vmm_alloc(int device, size_t size, void** out) {
+    const VmmApi& api = vmm_api();
+    DeviceGuard guard(device);   // the runtime's primary context is current for the driver calls
+    CTF_CUDA(guard.err);
+    int supported = 0;
+    int rc = compression_supported(api, device, &supported);
+    if (rc != CTF_OK) return rc;
+    CUmemAllocationProp prop;
+    memset(&prop, 0, sizeof(prop));
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = device;
+    prop.allocFlags.compressionType =
+        supported && g_compression_enabled.load() ? CU_MEM_ALLOCATION_COMP_GENERIC : CU_MEM_ALLOCATION_COMP_NONE;
+    CUmemGenericAllocationHandle handle;
+    size_t gran = 0, bytes = 0;
+    for (;;) {
+        CUresult r = api.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED);
+        if (r != CUDA_SUCCESS) return cu_fail(api, "cuMemGetAllocationGranularity", r);
+        bytes = ((size > 0 ? size : 1) + gran - 1) / gran * gran;
+        r = api.create(&handle, bytes, &prop, 0);
+        if (r == CUDA_SUCCESS) break;
+        if (prop.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_NONE) return cu_fail(api, "cuMemCreate", r);
+        prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_NONE;   // compression refused: ordinary memory instead
+    }
+    CUdeviceptr ptr = 0;
+    CUresult r = api.reserve(&ptr, bytes, gran, 0, 0);
+    if (r != CUDA_SUCCESS) { api.release(handle); return cu_fail(api, "cuMemAddressReserve", r); }
+    r = api.map(ptr, bytes, 0, handle, 0);
+    if (r != CUDA_SUCCESS) { api.addr_free(ptr, bytes); api.release(handle); return cu_fail(api, "cuMemMap", r); }
+    CUmemAccessDesc access;
+    memset(&access, 0, sizeof(access));
+    access.location = prop.location;
+    access.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    r = api.set_access(ptr, bytes, &access, 1);
+    if (r != CUDA_SUCCESS) {
+        api.unmap(ptr, bytes); api.release(handle); api.addr_free(ptr, bytes);
+        return cu_fail(api, "cuMemSetAccess", r);
+    }
+    {
+        std::lock_guard<std::mutex> lock(*g_vmm_mu);
+        (*g_vmm_blocks)[(uintptr_t)ptr] = VmmBlock{handle, bytes};
+    }
+    *out = reinterpret_cast<void*>(ptr);
+    return CTF_OK;
+}
+
+extern "C" void* ctf_compressible_alloc(ssize_t size, int device, void* /*stream*/) {
+    if (size < 0) { fail(CTF_ERR_INVALID, "ctf_compressible_alloc: negative size"); return nullptr; }
+    void* p = nullptr;
+    return vmm_alloc(device, (size_t)size, &p) == CTF_OK ? p : nullptr;
+}
+
+extern "C" void ctf_compressible_free(void* p, ssize_t /*size*/, int device, void* /*stream*/) {
+    if (!p) return;
+    VmmBlock b;
+    {
+        std::lock_guard<std::mutex> lock(*g_vmm_mu);
+        auto it = g_vmm_blocks->find((uintptr_t)p);
+        if (it == g_vmm_blocks->end()) { fail(CTF_ERR_INVALID, "ctf_compressible_free: not a ctf_compressible_alloc pointer"); return; }
+        b = it->second;
+        g_vmm_blocks->erase(it);
+    }
+    const VmmApi& api = vmm_api();
+    DeviceGuard guard(device);
+    const CUdeviceptr ptr = (CUdeviceptr)(uintptr_t)p;
+    api.unmap(ptr, b.bytes);
+    api.release(b.handle);
+    api.addr_free(ptr, b.bytes);
+}
+
+extern "C" int ctf_compression_supported(int device, int* out) {
+    if (!out) return fail(CTF_ERR_INVALID, "null argument");
+    *out = 0;
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) return fail(CTF_ERR_NO_DEVICE, "no CUDA device");
+    if (device < 0 || device >= n_dev) return fail(CTF_ERR_INVALID, "device index out of range");
+    return compression_supported(vmm_api(), device, out);
+}
+
+extern "C" int ctf_mem_is_compressed(const void* p, int* out) {
+    if (!out) return fail(CTF_ERR_INVALID, "null argument");
+    *out = 0;
+    if (!p) return CTF_OK;
+    const VmmApi& api = vmm_api();
+    if (api.missing) return fail(CTF_ERR_CUDA, "the CUDA driver does not provide %s", api.missing);
+    CUmemGenericAllocationHandle h;
+    if (api.retain(&h, const_cast<void*>(p)) != CUDA_SUCCESS) return CTF_OK;   // not in a cuMemMap'ed range
+    CUmemAllocationProp prop;
+    memset(&prop, 0, sizeof(prop));
+    CUresult r = api.props(&prop, h);
+    api.release(h);   // the reference cuMemRetainAllocationHandle took
+    if (r != CUDA_SUCCESS) return cu_fail(api, "cuMemGetAllocationPropertiesFromHandle", r);
+    *out = prop.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC ? 1 : 0;
+    return CTF_OK;
+}
+
+extern "C" int ctf_compressible_set_enabled(int enabled) { return g_compression_enabled.exchange(enabled ? 1 : 0); }
 
 static int build_plan(const ctf_config_t& c, int stats_level, int obs_dtype, DevPlan& P) {
     memset(&P, 0, sizeof(P));
@@ -1560,7 +1739,17 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
     // are slower (uint8 0.283 -> 0.347, 0_the_split 0.174 -> 0.229): profiles/r02_ab_residency*.log.  So blocks of
     // >= 6 KB per agent run with 5 CTAs per SM when there are many waves of them, and with the cap in 5..9 that fills
     // the last wave best when there are few (B = 16384: 7).  The cap is applied by padding dynamic shared memory.
-    if (n_sm > 0 && (size_t)h->plan.C * h->plan.GG * (obs_dtype == CTF_OBS_F32 ? 4 : (obs_dtype == CTF_OBS_U8 ? 1 : 2)) >= 6000) {
+    //
+    // Into compressed memory (ctf_compressible_alloc, DESIGN §4) the mostly-zero stream moves far fewer DRAM bytes and
+    // the env logic weighs more, so more resident CTAs win there (profiles/r05_residency_compressed.log, ms per step by
+    // cap 5 / 7 / 9): 8_arena bf16 B = 65536 0.471 / 0.428 / 0.416, 7_gridlocked float32 0.507 / 0.492 / 0.484, at
+    // B = 16384 bf16 0.135 / 0.123 / 0.119 and 7_gridlocked 0.151 / 0.136 / 0.132.  Only the 12.6 KB float32 blocks of
+    // 8_arena stay write-bound enough to prefer 7 (0.832 / 0.822 / 0.831; B = 16384 0.242 / 0.226 / 0.230).  So on a
+    // compressed buffer the cap is 7 for blocks of >= 12 KB per agent and 9 (what registers allow) below.  The launch picks the
+    // padding from where outputs.obs lies (obs_in_compressed_memory).
+    const size_t block_bytes = (size_t)h->plan.C * h->plan.GG * (obs_dtype == CTF_OBS_F32 ? 4 : (obs_dtype == CTF_OBS_U8 ? 1 : 2));
+    h->smem_bytes_comp = h->smem_bytes;
+    if (n_sm > 0 && block_bytes >= 6000) {
         const double ctas_per_sm_total = (double)((num_envs + kWarpsPerCta - 1) / kWarpsPerCta) / n_sm;
         int cap = 5;
         if (ctas_per_sm_total < 64.0) {
@@ -1573,6 +1762,8 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
         }
         const size_t want = (size_t)(227 * 1024) / (size_t)cap - 1024;
         if (want > h->smem_bytes) h->smem_bytes = want;
+        const size_t want_comp = (size_t)(227 * 1024) / (block_bytes >= 12 * 1024 ? 7 : 9) - 1024;
+        if (want_comp > h->smem_bytes_comp) h->smem_bytes_comp = want_comp;
     }
     // The attribute is per kernel, not per handle: give every kernel a ceiling that covers any handle's launch (another
     // handle with a smaller footprint must not lower it under this one's), not this handle's own size.
@@ -1671,6 +1862,20 @@ static int make_launch(ctf_handle_t h, const ctf_state_t& st, const ctf_outputs_
 
 static unsigned grid_dim(long long B) { return (unsigned)((B + kWarpsPerCta - 1) / kWarpsPerCta); }
 
+// Dynamic shared memory of a warp-per-env launch that writes `obs`: the residency cap depends on whether the buffer
+// lies in compressed memory (ctf_create).  The answer is cached per pointer, so a step with the same buffer costs one
+// comparison.
+static size_t launch_smem(ctf_handle_t h, const void* obs) {
+    if (!obs) return h->smem_bytes;
+    if (obs != h->obs_seen) {
+        int comp = 0;
+        if (ctf_mem_is_compressed(obs, &comp) != CTF_OK) comp = 0;
+        h->obs_seen = obs;
+        h->obs_seen_comp = comp != 0;
+    }
+    return h->obs_seen_comp ? h->smem_bytes_comp : h->smem_bytes;
+}
+
 // calls f(T{}) with the observation element type of the handle
 template <typename F>
 static void with_obs_type(int obs_dtype, F&& f) {
@@ -1692,10 +1897,11 @@ extern "C" int ctf_reset(ctf_handle_t h, ctf_state_t st, ctf_outputs_t out, int 
     CTF_CUDA(guard.err);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const bool stats = h->stats_level > 0;
+    const size_t smem = launch_smem(h, out.obs);
     with_obs_type(h->obs_dtype, [&](auto tag) {
         using T = decltype(tag);
-        if (stats) k_reset<T, true><<<grid_dim(h->B), kThreads, h->smem_bytes, s>>>(h->plan, L);
-        else k_reset<T, false><<<grid_dim(h->B), kThreads, h->smem_bytes, s>>>(h->plan, L);
+        if (stats) k_reset<T, true><<<grid_dim(h->B), kThreads, smem, s>>>(h->plan, L);
+        else k_reset<T, false><<<grid_dim(h->B), kThreads, smem, s>>>(h->plan, L);
     });
     CTF_CUDA(cudaGetLastError());
     return CTF_OK;
@@ -1704,11 +1910,12 @@ extern "C" int ctf_reset(ctf_handle_t h, ctf_state_t st, ctf_outputs_t out, int 
 static int launch_step(ctf_handle_t h, const Launch& L, cudaStream_t s) {
     const bool stats = h->stats_level > 0;
     const bool hpf = h->plan.hp_float != 0;
+    const size_t smem = launch_smem(h, L.obs);
     with_obs_type(h->obs_dtype, [&](auto tag) {
         using T = decltype(tag);
         auto launch = [&](auto stats_c, auto hpf_c) {
             constexpr bool S = decltype(stats_c)::value, F = decltype(hpf_c)::value;
-            k_step<T, S, F><<<grid_dim(h->B), kThreads, h->smem_bytes, s>>>(h->plan, L);
+            k_step<T, S, F><<<grid_dim(h->B), kThreads, smem, s>>>(h->plan, L);
         };
         if (stats) { if (hpf) launch(std::true_type{}, std::true_type{}); else launch(std::true_type{}, std::false_type{}); }
         else { if (hpf) launch(std::false_type{}, std::true_type{}); else launch(std::false_type{}, std::false_type{}); }
@@ -1742,8 +1949,9 @@ extern "C" int ctf_observe(ctf_handle_t h, ctf_state_t st, const uint8_t* revers
     DeviceGuard guard(h->device);
     CTF_CUDA(guard.err);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const size_t smem = launch_smem(h, out.obs);
     with_obs_type(h->obs_dtype, [&](auto tag) {
-        k_observe<decltype(tag)><<<grid_dim(h->B), kThreads, h->smem_bytes, s>>>(h->plan, L);
+        k_observe<decltype(tag)><<<grid_dim(h->B), kThreads, smem, s>>>(h->plan, L);
     });
     CTF_CUDA(cudaGetLastError());
     return CTF_OK;

@@ -21,6 +21,7 @@ import numpy as np
 import torch
 
 from . import _native
+from .compressible import compressible_empty, is_compressed
 from .config import METRIC_NAMES, N_METRICS, compile_config, env_dims
 from .sharding import all_reduce_stats
 
@@ -147,10 +148,12 @@ class GridworldCtfGPU:
         self._stats = torch.zeros((B, N_METRICS, N), dtype=torch.int32, device=dev) if self.stats_level > 0 else None
         self._visits = torch.zeros((B, N, G, G), dtype=torch.uint8, device=dev) if self.stats_level > 1 else None
         # ---- outputs (the policy's input buffers unless the caller binds its own)
-        # dense_obs=False skips the [B,N,C,G,G] buffer (storage-only use: packed_obs=True + unpack_obs on demand)
+        # dense_obs=False skips the [B,N,C,G,G] buffer (storage-only use: packed_obs=True + unpack_obs on demand).
+        # The env's own buffer is compressible memory where the device has it: the observations are ~90 % zero
+        # sectors, so the step's store stream, which bounds it, moves far fewer DRAM bytes (DESIGN §4).
         self.obs = None
         if dense_obs:
-            self.obs = torch.empty((B, N, Cn, G, G), dtype=obs_dtype, device=dev) if obs_out is None else obs_out
+            self.obs = compressible_empty((B, N, Cn, G, G), obs_dtype, dev) if obs_out is None else obs_out
             self._check_out(self.obs, (B, N, Cn, G, G), obs_dtype, "obs_out")
         elif not packed_obs:
             raise ValueError("dense_obs=False needs packed_obs=True")
@@ -391,6 +394,11 @@ class GridworldCtfGPU:
         if f & _native.FAULT_RESPAWN_BLOCKED:
             raise ValueError("respawn found no open cell in a 3x3 spawn window (np.random.randint(0) raises ValueError in "
                              "the reference, gridworld_ctf.py:771); the victim was left in place with HP <= 0")
+
+    @property
+    def obs_compressed(self) -> bool:
+        """Whether the bound observation buffer lies in memory the driver compresses (see ``compressible_empty``)."""
+        return self.obs is not None and is_compressed(self.obs)
 
     @property
     def uses_persistent_kernel(self) -> bool:
