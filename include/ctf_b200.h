@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 8
+#define CTF_ABI_VERSION 9
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -277,6 +277,49 @@ typedef struct ctf_policy_weights {
 int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uint32_t* packed, const float* meta,
                         int64_t n_envs, int agents_per_env, const uint8_t* agent_ids, int k,
                         void* features, int64_t feature_stride, void* stream);
+
+/*
+ * Grouped trunk: ctf_policy_features for many segments, each with its own policy, in one launch (league evaluation
+ * and every other workload that runs several policies on one env batch).  A segment names a policy (an index into
+ * the weights table), an env range, k agent ids and the feature row of its sample 0.  Its sample s = e*k + j
+ * (e < n_envs, j < k) reads packed block (env_begin + e)*agents_per_env + agent_ids[j] and the metadata row with the
+ * same index, as ctf_policy_features does, and writes feature row out_row + s.  Every row is bit-identical to what
+ * ctf_policy_features writes with that segment's weights for the same sample (the kernels share the per-sample code).
+ * Rows outside every segment are not written.
+ * Scheduling: the samples are cut into tiles of 8 consecutive samples of one segment, in table order; every CTA takes
+ * a contiguous range of tiles and restages conv weights in shared memory only where the policy changes, so put the
+ * segments of one policy next to each other.  Deterministic (no atomics), no allocation and no host synchronisation:
+ * capturable in a CUDA graph; the tables are validated on the host and passed by value as kernel parameters, so a
+ * captured graph keeps its own copy.
+ * Limits: 1..CTF_GROUPED_MAX_POLICIES policies and 1..CTF_GROUPED_MAX_SEGMENTS segments per call (the tables fill
+ * about 26 KB of the 32 764 bytes of kernel parameters).
+ * Rejected with CTF_ERR_INVALID: a policy index out of range; k outside 1..8 or an id >= agents_per_env; an env range
+ * outside [0, n_envs); output rows outside [0, n_rows) or two segments whose rows overlap; feature_stride or features
+ * as ctf_policy_features requires them; null or misaligned weights or inputs; too many policies or segments.
+ * Segments with n_envs = 0 are allowed; when every segment is empty nothing is launched.
+ */
+#define CTF_GROUPED_MAX_POLICIES 64
+#define CTF_GROUPED_MAX_SEGMENTS 512
+
+typedef struct ctf_policy_segment {
+    int64_t env_begin;   /* first env of the segment */
+    int64_t n_envs;      /* envs of the segment (>= 0) */
+    int64_t out_row;     /* feature row of the segment's sample 0 */
+    int32_t policy;      /* index into the weights table */
+    int32_t k;           /* 1..8 agents per env */
+    uint8_t agent_ids[CTF_MAX_AGENTS];   /* the first k are read */
+} ctf_policy_segment_t;
+
+/* weights: host table of n_policies ctf_policy_weights_t (device pointers); segments: host table of n_segments;
+   n_envs: envs in the packed / meta buffers; n_rows: rows of the feature buffer. */
+int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weights_t* weights, int n_policies,
+                                const ctf_policy_segment_t* segments, int n_segments, const uint32_t* packed,
+                                const float* meta, int64_t n_envs, int agents_per_env, void* features,
+                                int64_t feature_stride, int64_t n_rows, void* stream);
+
+/* CTAs the trunk kernels run at most per launch on this handle (the device's SMs times the CTAs resident per SM for
+   this plan, counted at ctf_create): k_policy_trunk (ctf_policy_features) and k_policy_trunk_grouped. */
+int ctf_policy_trunk_ctas(ctf_handle_t h, int* trunk_ctas, int* grouped_ctas);
 
 /* fp32 gradients of the trunk's parameters in torch layout (device memory). */
 typedef struct ctf_policy_grads {

@@ -4,6 +4,7 @@ Public surface:
     GridworldCtfGPU   batched env (B envs per GPU), device tensors in / out
     GridworldCtf      single-env view with the reference's exact methods (drop-in for ppo.py / utils.py)
     FusedPolicy       CtfPolicy inference from packed observations (fused_policy.py)
+    PolicyPool        several policies' inference on one env batch: one grouped trunk launch per forward (fused_policy.py)
     compressible_empty  torch.empty in compressible device memory, for caller-bound observation buffers
     compile_config    (AGENT_CONFIG, SCENARIO, kwargs) -> ctf_config_t
     experiment_env_config / experiment_names   the reference's nine experiment configs as data
@@ -22,8 +23,8 @@ def __getattr__(name):
         from .compressible import compressible_empty
 
         return compressible_empty
-    if name == "FusedPolicy":
-        from .fused_policy import FusedPolicy
+    if name in ("FusedPolicy", "PolicyPool"):
+        from . import fused_policy
 
-        return FusedPolicy
+        return getattr(fused_policy, name)
     raise AttributeError(name)

@@ -28,13 +28,15 @@ EXPORTS = (
     "ctf_policy_features",
     "ctf_policy_grad_workspace_size",
     "ctf_policy_features_backward",
+    "ctf_policy_features_grouped",
+    "ctf_policy_trunk_ctas",
     "ctf_compressible_alloc",
     "ctf_compressible_free",
     "ctf_compression_supported",
     "ctf_mem_is_compressed",
     "ctf_compressible_set_enabled",
 )
-ABI_VERSION = 8
+ABI_VERSION = 9
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
 
 
@@ -78,6 +80,14 @@ class CtfSizes(C.Structure):
 
 class CtfPolicyWeights(C.Structure):
     _fields_ = [("conv1_w", C.c_void_p), ("conv1_b", C.c_void_p), ("conv2_w", C.c_void_p), ("conv2_b", C.c_void_p)]
+
+
+GROUPED_MAX_POLICIES, GROUPED_MAX_SEGMENTS = 64, 512
+
+
+class CtfPolicySegment(C.Structure):
+    _fields_ = [("env_begin", C.c_int64), ("n_envs", C.c_int64), ("out_row", C.c_int64), ("policy", C.c_int32),
+                ("k", C.c_int32), ("agent_ids", C.c_uint8 * 8)]
 
 
 class CtfPolicyGrads(C.Structure):
@@ -129,6 +139,10 @@ def load():
     L.ctf_step_host.argtypes = [C.c_void_p, CtfState, C.c_void_p, CtfOutputs, C.c_void_p, C.c_void_p, C.c_void_p]
     L.ctf_policy_features.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
                                       C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]
+    L.ctf_policy_features_grouped.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_int, C.POINTER(CtfPolicySegment),
+                                              C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
+                                              C.c_int64, C.c_void_p]
+    L.ctf_policy_trunk_ctas.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]
     L.ctf_policy_grad_workspace_size.argtypes = [C.c_void_p, C.POINTER(C.c_size_t)]
     L.ctf_policy_features_backward.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64,
                                                C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,

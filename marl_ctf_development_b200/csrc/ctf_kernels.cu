@@ -23,6 +23,7 @@
 #include <stdio.h>   // snprintf for error messages
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <new>
@@ -967,6 +968,87 @@ __device__ __forceinline__ void trunk_conv1(const uint32_t* bits, uint16_t* cmas
     }
 }
 
+// Copies one policy's conv weights into the CTA's shared memory for k_policy_trunk_grouped: conv1 as [C*9][16] columns,
+// the biases, the conv2 B fragments; the same copy k_policy_trunk makes at its start (which keeps its own inline
+// statement of it: calling this helper there changes that kernel's instruction schedule).  The caller synchronises the
+// CTA after it, and before it when other warps may still read the previous policy's weights.
+__device__ __forceinline__ void trunk_stage_weights(const float* conv1_w, const float* conv1_b, const uint2* conv2_w,
+                                                    const float* conv2_b, int C, float* w1, float* b1, float* b2, uint2* w2) {
+    for (int i = threadIdx.x; i < C * 9 * 16; i += kTrunkThreads) {
+        const int o = i & 15, tap = i >> 4;                              // tap = c*9 + dy*3 + dx
+        w1[i] = conv1_w[o * C * 9 + tap];
+    }
+    if (threadIdx.x < 16) b1[threadIdx.x] = conv1_b[threadIdx.x];
+    if (threadIdx.x < 32) b2[threadIdx.x] = conv2_b[threadIdx.x];
+    for (int i = threadIdx.x; i < kTrunkW2Words / 2; i += kTrunkThreads) w2[i] = conv2_w[i];
+}
+
+// One sample of the trunk, computed by one warp with the weights staged in shared memory: stages packed block `blk`
+// (A.packed, A.wpa words), conv1 (trunk_conv1), conv2 on tensor cores, tanh, bf16, then the metadata row `blk` and
+// zeros up to A.stride, into feature row `r` of A.features.  k_policy_trunk and k_policy_trunk_grouped both run exactly this code.
+__device__ __forceinline__ void trunk_sample(const TrunkArgs& A, long long blk, long long r, const float* w1,
+                                             const float* b1, const float* b2, const uint2* w2, uint32_t* bits,
+                                             uint16_t* cmask, uint32_t* act, __nv_bfloat16* stage, int lane, int C, int G,
+                                             int GG, int S1, int S2, int M2, int g, int t, int n_mt, long long conv_elems) {
+    const uint32_t* src = A.packed + blk * A.wpa;
+    for (int i = lane; i < A.wpa; i += 32) bits[i] = __ldg(src + i);
+    __syncwarp();
+    trunk_conv1(bits, cmask, act, w1, b1, C, G, GG, S1, lane, 32, [] { __syncwarp(); });
+    __syncwarp();
+    __nv_bfloat16* row = A.features + r * A.stride;
+    // conv2: n-tile (8 output channels) outer, m-tile (16 positions) inner, one k-step per tap
+    for (int nt = 0; nt < 4; ++nt) {
+        const float bias0 = b2[8 * nt + 2 * t], bias1 = b2[8 * nt + 2 * t + 1];
+        for (int mt = 0; mt < n_mt; ++mt) {
+            const int m0 = min(mt * 16 + g, M2 - 1), m1 = min(mt * 16 + g + 8, M2 - 1);   // pad rows: any valid position
+            const int y0 = m0 / S2, y1 = m1 / S2;
+            const int p0 = y0 * S1 + (m0 - y0 * S2), p1 = y1 * S1 + (m1 - y1 * S2);
+            float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f;
+#pragma unroll
+            for (int tap = 0; tap < 9; ++tap) {
+                const int off = (tap / 3) * S1 + (tap % 3);
+                const uint32_t a0 = act[(p0 + off) * 8 + t], a1 = act[(p1 + off) * 8 + t];
+                const uint32_t a2 = act[(p0 + off) * 8 + t + 4], a3 = act[(p1 + off) * 8 + t + 4];
+                const uint2 b = w2[(tap * 4 + nt) * 32 + lane];
+                asm volatile(
+                    "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
+                    "{%0,%1,%2,%3};\n"
+                    : "+f"(d0), "+f"(d1), "+f"(d2), "+f"(d3)
+                    : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b.x), "r"(b.y));
+            }
+            const int r0 = mt * 16 + g, r1 = r0 + 8;
+            if (r0 < M2) {
+                stage[(2 * t) * M2 + r0] = __float2bfloat16_rn(tanhf(d0 + bias0));
+                stage[(2 * t + 1) * M2 + r0] = __float2bfloat16_rn(tanhf(d1 + bias1));
+            }
+            if (r1 < M2) {
+                stage[(2 * t) * M2 + r1] = __float2bfloat16_rn(tanhf(d2 + bias0));
+                stage[(2 * t + 1) * M2 + r1] = __float2bfloat16_rn(tanhf(d3 + bias1));
+            }
+        }
+        __syncwarp();
+        // channels 8nt .. 8nt+7 are elements [8nt*M2, 8(nt+1)*M2) of the row: 16*M2 bytes, 16-byte aligned
+        uint4* dst = reinterpret_cast<uint4*>(row + (long long)8 * nt * M2);
+        const uint4* sv = reinterpret_cast<const uint4*>(stage);
+        for (int i = lane; i < M2; i += 32) dst[i] = sv[i];
+        __syncwarp();
+    }
+    // metadata as bf16, then zeros up to the stride (8 elements per 16-byte store)
+    const float* mrow = A.meta + blk * A.M;
+    const int tail = (int)((A.stride - conv_elems) >> 3);
+    uint4* dst = reinterpret_cast<uint4*>(row + conv_elems);
+    for (int i = lane; i < tail; i += 32) {
+        float v[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+            const int c = 8 * i + u;
+            v[u] = c < A.M ? __ldg(mrow + c) : 0.f;
+        }
+        dst[i] = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+    }
+    __syncwarp();
+}
+
 __global__ void __launch_bounds__(kTrunkThreads) k_policy_trunk(const __grid_constant__ TrunkArgs A) {
     extern __shared__ uint4 smem_raw[];
     float* w1 = reinterpret_cast<float*>(smem_raw);                      // [C*9][16]: column of one (c, dy, dx) tap
@@ -997,63 +1079,8 @@ __global__ void __launch_bounds__(kTrunkThreads) k_policy_trunk(const __grid_con
         const long long e = s / A.k;
         const int j = (int)(s - e * A.k);
         const long long blk = e * A.ape + A.ids[j];
-        const uint32_t* src = A.packed + blk * A.wpa;
-        for (int i = lane; i < A.wpa; i += 32) bits[i] = __ldg(src + i);
-        __syncwarp();
-        trunk_conv1(bits, cmask, act, w1, b1, C, G, GG, S1, lane, 32, [] { __syncwarp(); });
-        __syncwarp();
-        __nv_bfloat16* row = A.features + s * A.stride;
-        // conv2: n-tile (8 output channels) outer, m-tile (16 positions) inner, one k-step per tap
-        for (int nt = 0; nt < 4; ++nt) {
-            const float bias0 = b2[8 * nt + 2 * t], bias1 = b2[8 * nt + 2 * t + 1];
-            for (int mt = 0; mt < n_mt; ++mt) {
-                const int m0 = min(mt * 16 + g, M2 - 1), m1 = min(mt * 16 + g + 8, M2 - 1);   // pad rows: any valid position
-                const int y0 = m0 / S2, y1 = m1 / S2;
-                const int p0 = y0 * S1 + (m0 - y0 * S2), p1 = y1 * S1 + (m1 - y1 * S2);
-                float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f;
-#pragma unroll
-                for (int tap = 0; tap < 9; ++tap) {
-                    const int off = (tap / 3) * S1 + (tap % 3);
-                    const uint32_t a0 = act[(p0 + off) * 8 + t], a1 = act[(p1 + off) * 8 + t];
-                    const uint32_t a2 = act[(p0 + off) * 8 + t + 4], a3 = act[(p1 + off) * 8 + t + 4];
-                    const uint2 b = w2[(tap * 4 + nt) * 32 + lane];
-                    asm volatile(
-                        "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
-                        "{%0,%1,%2,%3};\n"
-                        : "+f"(d0), "+f"(d1), "+f"(d2), "+f"(d3)
-                        : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b.x), "r"(b.y));
-                }
-                const int r0 = mt * 16 + g, r1 = r0 + 8;
-                if (r0 < M2) {
-                    stage[(2 * t) * M2 + r0] = __float2bfloat16_rn(tanhf(d0 + bias0));
-                    stage[(2 * t + 1) * M2 + r0] = __float2bfloat16_rn(tanhf(d1 + bias1));
-                }
-                if (r1 < M2) {
-                    stage[(2 * t) * M2 + r1] = __float2bfloat16_rn(tanhf(d2 + bias0));
-                    stage[(2 * t + 1) * M2 + r1] = __float2bfloat16_rn(tanhf(d3 + bias1));
-                }
-            }
-            __syncwarp();
-            // channels 8nt .. 8nt+7 are elements [8nt*M2, 8(nt+1)*M2) of the row: 16*M2 bytes, 16-byte aligned
-            uint4* dst = reinterpret_cast<uint4*>(row + (long long)8 * nt * M2);
-            const uint4* sv = reinterpret_cast<const uint4*>(stage);
-            for (int i = lane; i < M2; i += 32) dst[i] = sv[i];
-            __syncwarp();
-        }
-        // metadata as bf16, then zeros up to the stride (8 elements per 16-byte store)
-        const float* mrow = A.meta + blk * A.M;
-        const int tail = (int)((A.stride - conv_elems) >> 3);
-        uint4* dst = reinterpret_cast<uint4*>(row + conv_elems);
-        for (int i = lane; i < tail; i += 32) {
-            float v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int c = 8 * i + u;
-                v[u] = c < A.M ? __ldg(mrow + c) : 0.f;
-            }
-            dst[i] = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
-        }
-        __syncwarp();
+        trunk_sample(A, blk, s, w1, b1, b2, w2, bits, cmask, act, stage, lane, C, G, GG, S1, S2,
+                     M2, g, t, n_mt, conv_elems);
     }
 }
 
@@ -1068,6 +1095,89 @@ static __host__ void trunk_layout(const DevPlan& P, TrunkArgs& A, size_t& smem) 
     A.warp_words = A.off_stage + up4(4 * S2 * S2);                       // 8 channels x S2^2 bf16
     const size_t shared_words = (size_t)P.C * 9 * 16 + 16 + 32 + kTrunkW2Words;
     smem = (shared_words + (size_t)kTrunkWarps * A.warp_words) * 4;
+}
+
+// ------------------------------------------------------------------------------------------------
+// grouped policy trunk: the samples of many (policy, env range, agent ids) segments in one launch
+// ------------------------------------------------------------------------------------------------
+// The segments' samples are cut into tiles of kTrunkWarps consecutive samples of one segment (a segment's last tile may
+// be shorter); the host numbers the tiles in table order (TrunkSegment::tile_begin).  CTA b takes the contiguous tile
+// range [n_tiles*b/grid, n_tiles*(b+1)/grid) and warp w computes sample w of each tile with k_policy_trunk's own
+// per-sample code (trunk_sample).  The CTA stages a policy's conv weights only when its next tile belongs to a different
+// policy than the one staged, between two __syncthreads(): with the segments of a policy adjacent in the table, a CTA
+// restages at most once per policy boundary inside its range.  Warps sync with each other only there.
+struct TrunkSegment {
+    long long blk_begin;     // env_begin * agents_per_env: the packed block of env 0 of the segment, agent 0
+    long long row_begin;     // feature row of sample 0
+    long long n_samples;     // n_envs * k
+    long long tile_begin;    // first tile of the segment (tiles of all earlier segments before it)
+    int policy, k;
+    unsigned char ids[CTF_MAX_AGENTS];
+};
+
+struct TrunkPolicyWeights {
+    const float* conv1_w;
+    const float* conv1_b;
+    const uint2* conv2_w;
+    const float* conv2_b;
+};
+
+struct TrunkGroupedArgs {
+    TrunkArgs geo;           // shapes, shared-memory layout, packed / meta / features / stride / ape (conv*_w, n_samples,
+                             // k and ids unused)
+    long long n_tiles;
+    int n_segments, pad;
+    TrunkPolicyWeights w[CTF_GROUPED_MAX_POLICIES];
+    TrunkSegment seg[CTF_GROUPED_MAX_SEGMENTS];
+};
+static_assert(sizeof(TrunkGroupedArgs) <= 32764, "kernel parameters are limited to 32 764 bytes");
+
+// The register cap (5 CTAs of 256 threads per SM) holds it to k_policy_trunk's 48 registers, no spills: unbounded, the
+// compiler keeps segment fields live and takes 126, which would cap residency below k_policy_trunk's on small maps.
+__global__ void __launch_bounds__(kTrunkThreads, 5) k_policy_trunk_grouped(const __grid_constant__ TrunkGroupedArgs A) {
+    extern __shared__ uint4 smem_raw[];
+    const TrunkArgs& T = A.geo;
+    float* w1 = reinterpret_cast<float*>(smem_raw);                      // the layout of k_policy_trunk
+    float* b1 = w1 + T.C * 9 * 16;
+    float* b2 = b1 + 16;
+    uint2* w2 = reinterpret_cast<uint2*>(b2 + 32);
+    uint32_t* warp_base = reinterpret_cast<uint32_t*>(w2 + kTrunkW2Words / 2);
+    const int C = T.C, G = T.G, GG = T.GG, S1 = T.S1, S2 = T.S2, M2 = S2 * S2;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t* bits = warp_base + (size_t)warp * T.warp_words;
+    uint16_t* cmask = reinterpret_cast<uint16_t*>(bits + T.off_mask);
+    uint32_t* act = bits + T.off_act;
+    __nv_bfloat16* stage = reinterpret_cast<__nv_bfloat16*>(bits + T.off_stage);
+    const int g = lane >> 2, t = lane & 3;
+    const int n_mt = (M2 + 15) >> 4;
+    const long long conv_elems = 32LL * M2;
+
+    const long long t0 = A.n_tiles * blockIdx.x / gridDim.x, t1 = A.n_tiles * (blockIdx.x + 1) / gridDim.x;
+    // the segment of tile t0: the last one whose first tile is <= t0 (empty segments share their successor's tile_begin)
+    int lo = 0, hi = A.n_segments - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (A.seg[mid].tile_begin <= t0) lo = mid; else hi = mid - 1;
+    }
+    int si = lo, staged = -1;
+    for (long long tile = t0; tile < t1; ++tile) {
+        while (si + 1 < A.n_segments && A.seg[si + 1].tile_begin <= tile) ++si;
+        const TrunkSegment& S = A.seg[si];
+        if (S.policy != staged) {
+            __syncthreads();
+            const TrunkPolicyWeights& W = A.w[S.policy];
+            trunk_stage_weights(W.conv1_w, W.conv1_b, W.conv2_w, W.conv2_b, C, w1, b1, b2, w2);
+            __syncthreads();
+            staged = S.policy;
+        }
+        const long long s = (tile - S.tile_begin) * kTrunkWarps + warp;
+        if (s < S.n_samples) {
+            const long long e = s / S.k;
+            const int j = (int)(s - e * S.k);
+            trunk_sample(T, S.blk_begin + e * T.ape + S.ids[j], S.row_begin + s, w1, b1, b2, w2, bits, cmask, act, stage,
+                         lane, C, G, GG, S1, S2, M2, g, t, n_mt, conv_elems);
+        }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1376,6 +1486,7 @@ struct ctf_env {
     bool obs_seen_comp;
     size_t trunk_smem_bytes; // k_policy_trunk: dynamic shared memory for this plan
     int trunk_ctas;          // k_policy_trunk: CTAs that fit on the device at once
+    int grouped_ctas;        // k_policy_trunk_grouped: CTAs that fit on the device at once
     size_t bwd_smem_bytes;   // k_policy_trunk_backward: dynamic shared memory for this plan
     int bwd_ctas;            // k_policy_trunk_backward: CTAs (= workspace rows) of every launch with >= bwd_ctas samples
 };
@@ -1785,6 +1896,14 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
             e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk, kTrunkThreads, h->trunk_smem_bytes);
         h->trunk_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
     }
+    // k_policy_trunk_grouped: k_policy_trunk's shared-memory layout
+    CTF_SET_SMEM(k_policy_trunk_grouped, 100 * 1024);
+    {
+        int per_sm = 0;
+        if (e == cudaSuccess && h->plan.G >= 5)
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk_grouped, kTrunkThreads, h->trunk_smem_bytes);
+        h->grouped_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
+    }
     // k_policy_trunk_backward needs at most 46 KB (G = 16, C = 14)
     CTF_SET_SMEM(k_policy_trunk_backward, 64 * 1024);
     {
@@ -2024,6 +2143,95 @@ extern "C" int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w
     const unsigned grid = (unsigned)(want < h->trunk_ctas ? want : h->trunk_ctas);
     k_policy_trunk<<<grid, kTrunkThreads, smem, static_cast<cudaStream_t>(stream)>>>(A);
     CTF_CUDA(cudaGetLastError());
+    return CTF_OK;
+}
+
+extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weights_t* weights, int n_policies,
+                                           const ctf_policy_segment_t* segments, int n_segments, const uint32_t* packed,
+                                           const float* meta, int64_t n_envs, int agents_per_env, void* features,
+                                           int64_t feature_stride, int64_t n_rows, void* stream) {
+    if (!h || !weights || !segments || !packed || !meta || !features)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: null argument");
+    const DevPlan& P = h->plan;
+    if (P.G < 5) return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: the policy needs grid_size >= 5 (two valid 3x3 convolutions)");
+    if (n_policies < 1 || n_policies > CTF_GROUPED_MAX_POLICIES)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: n_policies must be in 1..CTF_GROUPED_MAX_POLICIES (64)");
+    if (n_segments < 1 || n_segments > CTF_GROUPED_MAX_SEGMENTS)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: n_segments must be in 1..CTF_GROUPED_MAX_SEGMENTS (512)");
+    if (agents_per_env < 1) return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: agents_per_env must be >= 1");
+    if (n_envs < 0 || n_rows < 0) return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: negative n_envs or n_rows");
+    const long long k1 = 32LL * (P.G - 4) * (P.G - 4) + P.M;
+    if (feature_stride < k1 || (feature_stride & 7))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: feature_stride must be a multiple of 8 and >= 32*(G-4)^2 + M");
+    if (reinterpret_cast<uintptr_t>(features) & 15)
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: features must be 16-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(packed) & 3) || (reinterpret_cast<uintptr_t>(meta) & 3))
+        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: misaligned inputs");
+    // the argument block is large (about 26 KB): keep it off the caller's stack
+    static thread_local TrunkGroupedArgs A;
+    memset(&A, 0, sizeof(A));
+    size_t smem = 0;
+    trunk_layout(P, A.geo, smem);
+    for (int p = 0; p < n_policies; ++p) {
+        const ctf_policy_weights_t& w = weights[p];
+        if (!w.conv1_w || !w.conv1_b || !w.conv2_w || !w.conv2_b)
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: null weight pointer");
+        if ((reinterpret_cast<uintptr_t>(w.conv1_w) & 15) || (reinterpret_cast<uintptr_t>(w.conv2_w) & 7) ||
+            (reinterpret_cast<uintptr_t>(w.conv1_b) & 3) || (reinterpret_cast<uintptr_t>(w.conv2_b) & 3))
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: misaligned weights");
+        A.w[p].conv1_w = w.conv1_w; A.w[p].conv1_b = w.conv1_b;
+        A.w[p].conv2_w = static_cast<const uint2*>(w.conv2_w); A.w[p].conv2_b = w.conv2_b;
+    }
+    long long tiles = 0;
+    int order[CTF_GROUPED_MAX_SEGMENTS];
+    int n_busy = 0;
+    for (int i = 0; i < n_segments; ++i) {
+        const ctf_policy_segment_t& g = segments[i];
+        if (g.policy < 0 || g.policy >= n_policies)
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's policy index is out of range");
+        if (g.k < 1 || g.k > CTF_MAX_AGENTS)
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's k must be in 1..8");
+        for (int j = 0; j < g.k; ++j)
+            if (g.agent_ids[j] >= agents_per_env)
+                return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: an agent id is >= agents_per_env");
+        if (g.env_begin < 0 || g.n_envs < 0 || g.env_begin > n_envs || g.n_envs > n_envs - g.env_begin)
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's env range is outside [0, n_envs)");
+        const long long ns = g.n_envs * g.k;
+        if (g.out_row < 0 || g.out_row > n_rows || ns > n_rows - g.out_row)
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's output rows are outside [0, n_rows)");
+        TrunkSegment& S = A.seg[i];
+        S.blk_begin = g.env_begin * agents_per_env;
+        S.row_begin = g.out_row;
+        S.n_samples = ns;
+        S.tile_begin = tiles;
+        S.policy = g.policy;
+        S.k = g.k;
+        for (int j = 0; j < g.k; ++j) S.ids[j] = g.agent_ids[j];
+        tiles += (ns + kTrunkWarps - 1) / kTrunkWarps;
+        if (ns > 0) order[n_busy++] = i;
+    }
+    // no two segments may write the same row (the result would depend on the schedule)
+    std::sort(order, order + n_busy, [&](int a, int b) { return A.seg[a].row_begin < A.seg[b].row_begin; });
+    for (int i = 1; i < n_busy; ++i)
+        if (A.seg[order[i - 1]].row_begin + A.seg[order[i - 1]].n_samples > A.seg[order[i]].row_begin)
+            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: the output rows of two segments overlap");
+    if (tiles == 0) return CTF_OK;
+    A.geo.packed = packed; A.geo.meta = meta; A.geo.features = static_cast<__nv_bfloat16*>(features);
+    A.geo.stride = feature_stride; A.geo.ape = agents_per_env;
+    A.n_tiles = tiles;
+    A.n_segments = n_segments;
+    DeviceGuard guard(h->device);
+    CTF_CUDA(guard.err);
+    const unsigned grid = (unsigned)(tiles < h->grouped_ctas ? tiles : h->grouped_ctas);
+    k_policy_trunk_grouped<<<grid, kTrunkThreads, smem, static_cast<cudaStream_t>(stream)>>>(A);
+    CTF_CUDA(cudaGetLastError());
+    return CTF_OK;
+}
+
+extern "C" int ctf_policy_trunk_ctas(ctf_handle_t h, int* trunk_ctas, int* grouped_ctas) {
+    if (!h || !trunk_ctas || !grouped_ctas) return fail(CTF_ERR_INVALID, "ctf_policy_trunk_ctas: null argument");
+    *trunk_ctas = h->trunk_ctas;
+    *grouped_ctas = h->grouped_ctas;
     return CTF_OK;
 }
 

@@ -18,6 +18,11 @@ a given action, for the PPO update on a packed minibatch.  Its trunk runs ``ctf_
 bf16 through autograd.  ``reference_trunk_grads`` states in torch what the backward kernel computes.  Each sample keeps
 2 x stride bf16 values alive between forward and backward (its rows and their gradient: 15.6 KB at 8_arena), so a
 caller splits a large minibatch into chunks and lets the gradients accumulate.
+
+Several policies on one env batch: ``PolicyPool(env, policies)`` runs any number of (policy, env slice, agent ids)
+segments with one ``ctf_policy_features_grouped`` launch (``k_policy_trunk_grouped``, the same per-sample code as
+``k_policy_trunk``, so every row is bit-identical to ``FusedPolicy``'s) and one bf16 ``torch.baddbmm`` head chain over
+all policies; league evaluation uses it (``league.duel_pairs(grouped=True)``).
 """
 from __future__ import annotations
 
@@ -147,6 +152,24 @@ def reference_trunk_grads(policy, dense_obs: torch.Tensor, grad_rows: torch.Tens
                 dz2.sum((0, 2, 3)))
 
 
+def _check_policy(env, policy):
+    """Raises ValueError unless ``policy`` has the layer shapes of a CtfPolicy for ``env`` and lives on its device."""
+    Cn, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
+    k1 = trunk_dims(Cn, G, M)[0]
+    want = {
+        "conv1.weight": (16, Cn, 3, 3), "conv2.weight": (32, 16, 3, 3), "fc1.weight": (256, k1),
+        "fc2.weight": (128, 256), "action_head.weight": (N_ACTIONS, 128), "value_head.weight": (1, 128),
+    }
+    for name, shape in want.items():
+        mod, attr = name.split(".")
+        got = tuple(getattr(getattr(policy, mod, None), attr, torch.empty(0)).shape)
+        if got != shape:
+            raise ValueError(f"policy {name} has shape {got}; this env (C={Cn}, G={G}, M={M}, {N_ACTIONS} actions) "
+                             f"needs {shape}")
+    if policy.conv1.weight.device != env.device:
+        raise ValueError(f"policy is on {policy.conv1.weight.device}, env on {env.device}")
+
+
 class _PackedTrunk(torch.autograd.Function):
     """rows = trunk(bits, meta; conv1, conv2) through ctf_policy_features, with ctf_policy_features_backward as its
     backward.  The rows are saved (a tensor of their own) and the backward re-reads the parameters it was given."""
@@ -178,18 +201,7 @@ class FusedPolicy:
         if G < 5:
             raise ValueError(f"the policy needs GRID_SIZE >= 5 (two valid 3x3 convolutions), env has {G}")
         self.k1, self.stride = trunk_dims(Cn, G, M)
-        want = {
-            "conv1.weight": (16, Cn, 3, 3), "conv2.weight": (32, 16, 3, 3), "fc1.weight": (256, self.k1),
-            "fc2.weight": (128, 256), "action_head.weight": (N_ACTIONS, 128), "value_head.weight": (1, 128),
-        }
-        for name, shape in want.items():
-            mod, attr = name.split(".")
-            got = tuple(getattr(getattr(policy, mod, None), attr, torch.empty(0)).shape)
-            if got != shape:
-                raise ValueError(f"policy {name} has shape {got}; this env (C={Cn}, G={G}, M={M}, {N_ACTIONS} actions) "
-                                 f"needs {shape}")
-        if policy.conv1.weight.device != env.device:
-            raise ValueError(f"policy is on {policy.conv1.weight.device}, env on {env.device}")
+        _check_policy(env, policy)
         dev = env.device
         bf = dict(dtype=torch.bfloat16, device=dev)
         self._c1w = torch.empty((16, Cn, 3, 3), dtype=torch.float32, device=dev)
@@ -433,3 +445,223 @@ class FusedPolicy:
             bits.shape[0], 1, ids, 1, C.c_void_p(ptrs[1]), C.c_void_p(ptrs[2]), self.stride,
             C.c_void_p(ws.data_ptr()), ws.numel() * 4, C.byref(gs), stream))
         return [g.to(t.dtype) for g, t in zip(grads, (w1, b1, w2, b2))]
+
+
+# ---------------------------------------------------------------------------------------------------- policy pools
+class PoolPlan:
+    """The launch plan ``PolicyPool.plan`` builds once on the host for a fixed list of segments.
+
+    Policy p owns the feature rows [p*s_max, p*s_max + n_samples[p]); s_max is the largest policy's sample count, and
+    the rest of each block (the pad rows) stays zero and is never scattered.  The forward's outputs are in plan order:
+    segment after segment as given, sample s = e*k + j of a segment (agent ids[j] of its e-th env).
+
+    * ``seg_rows[i]``: (start, stop) of segment i in the outputs;
+    * ``row_index`` [S]: the feature row of every output row; ``policy_of_row`` [S]: its policy;
+    * ``flat_index`` [S]: env * N + agent of every output row (where ``act`` writes its action in ``actions[B, N]``);
+    * ``mask_add`` [S, 9] float32: the additive action mask, ``(mask - 1) * 1e9`` of ``CtfPolicy.masked_logits`` for
+      rows whose policy masks and whose agent type is masked, zeros elsewhere;
+    * ``features`` bf16 [L * s_max, stride]: the trunk's output buffer.
+    """
+
+    def __init__(self, segments, n_samples, s_max, seg_rows, row_index, flat_index, mask_add, features, tables):
+        self.segments, self.n_samples, self.s_max, self.seg_rows = segments, n_samples, s_max, seg_rows
+        self.row_index, self.flat_index, self.mask_add, self.features = row_index, flat_index, mask_add, features
+        self.policy_of_row = row_index // s_max
+        self.n_rows = features.shape[0]
+        self._tables = tables   # [(ctypes segment array, count)], policy-major, at most GROUPED_MAX_SEGMENTS each
+
+    @property
+    def n_outputs(self) -> int:
+        return int(self.row_index.numel())
+
+
+class PolicyPool:
+    """Inference for several policies on one env batch: one grouped trunk launch (``ctf_policy_features_grouped``,
+    ``k_policy_trunk_grouped``) and one bf16 ``torch.baddbmm`` chain for the heads of all policies per forward.
+
+    ``policies``: ``CtfPolicy`` modules or ``FusedPolicy`` views of them (their ``policy`` is used), each policy once,
+    at most ``GROUPED_MAX_POLICIES`` (64).  Every weight lives in stacked persistent buffers: conv1 / conv2 in the
+    kernel's layouts, fc1 bf16 [L, 256, stride] zero-padded as in ``FusedPolicy``, fc2 [L, 128, 256], the value | action
+    heads [L, 10, 128].  ``refresh()`` copies the modules' current weights into them in place, so a CUDA graph captured
+    around ``forward`` / ``act`` follows optimiser steps.
+
+    Precision: each policy's rows are exactly what ``FusedPolicy.trunk_from_env`` writes for it (the kernels share the
+    per-sample code); the heads are the same bf16 computation as ``FusedPolicy`` run as a batched GEMM, within the same
+    contract against fp32 ``CtfPolicy``.
+    """
+
+    def __init__(self, env, policies):
+        Cn, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
+        if G < 5:
+            raise ValueError(f"the policy needs GRID_SIZE >= 5 (two valid 3x3 convolutions), env has {G}")
+        mods = [p.policy if isinstance(p, FusedPolicy) else p for p in policies]
+        if not mods:
+            raise ValueError("a PolicyPool needs at least one policy")
+        if len(mods) > _native.GROUPED_MAX_POLICIES:
+            raise ValueError(f"a PolicyPool holds at most {_native.GROUPED_MAX_POLICIES} policies, got {len(mods)}")
+        if len({id(m) for m in mods}) != len(mods):
+            raise ValueError("every policy may appear only once in a PolicyPool")
+        for m in mods:
+            _check_policy(env, m)
+        self.env, self.policies = env, mods
+        self.k1, self.stride = trunk_dims(Cn, G, M)
+        L, dev = len(mods), env.device
+        bf = dict(dtype=torch.bfloat16, device=dev)
+        self._c1w = torch.empty((L, 16, Cn, 3, 3), dtype=torch.float32, device=dev)
+        self._c1b = torch.empty((L, 16), dtype=torch.float32, device=dev)
+        self._c2w = torch.empty((L, 9 * 4 * 32 * 4), **bf)
+        self._c2b = torch.empty((L, 32), dtype=torch.float32, device=dev)
+        self._c2_index = conv2_kernel_layout_index(dev)
+        self._fc1w, self._fc1b = torch.zeros((L, 256, self.stride), **bf), torch.empty((L, 256), **bf)
+        self._fc2w, self._fc2b = torch.empty((L, 128, 256), **bf), torch.empty((L, 128), **bf)
+        self._hw, self._hb = torch.empty((L, 1 + N_ACTIONS, 128), **bf), torch.empty((L, 1 + N_ACTIONS), **bf)
+        self._weights = (_native.CtfPolicyWeights * L)(*(
+            _native.CtfPolicyWeights(self._c1w[p].data_ptr(), self._c1b[p].data_ptr(), self._c2w[p].data_ptr(),
+                                     self._c2b[p].data_ptr()) for p in range(L)))
+        self.refresh()
+
+    def __len__(self):
+        return len(self.policies)
+
+    @torch.no_grad()
+    def refresh(self):
+        """Copies every policy's current weights into the stacked buffers, on the device (no host round trip)."""
+        for p, m in enumerate(self.policies):
+            self._c1w[p].copy_(m.conv1.weight)
+            self._c1b[p].copy_(m.conv1.bias)
+            self._c2w[p].copy_(m.conv2.weight.reshape(-1)[self._c2_index])
+            self._c2b[p].copy_(m.conv2.bias)
+            self._fc1w[p, :, : self.k1].copy_(m.fc1.weight)
+            self._fc1b[p].copy_(m.fc1.bias)
+            self._fc2w[p].copy_(m.fc2.weight)
+            self._fc2b[p].copy_(m.fc2.bias)
+            self._hw[p, :1].copy_(m.value_head.weight)
+            self._hw[p, 1:].copy_(m.action_head.weight)
+            self._hb[p, :1].copy_(m.value_head.bias)
+            self._hb[p, 1:].copy_(m.action_head.bias)
+
+    def _env_for(self, env):
+        if env is None:
+            return self.env
+        mine = (self.env.n_channels, self.env.GRID_SIZE, self.env.meta_size, self.env.N_AGENTS, self.env.device)
+        if (env.n_channels, env.GRID_SIZE, env.meta_size, env.N_AGENTS, env.device) != mine:
+            raise ValueError("env does not have the shapes (C, G, M, N) or the device this PolicyPool was built for")
+        return env
+
+    # ------------------------------------------------------------------ plan
+    def plan(self, segments) -> PoolPlan:
+        """Builds the launch plan for ``segments``, a list of (policy index, env slice, agent ids): the agents ``ids``
+        (1..8 of them) of the envs ``slice`` (contiguous, step 1) of the pool's env, run by policy ``index``.  Runs on
+        the host once; ``forward`` and ``act`` with the plan are then a fixed sequence of launches."""
+        env = self.env
+        B, N, L = env.num_envs, env.N_AGENTS, len(self.policies)
+        norm = []
+        for i, seg in enumerate(segments):
+            pol, sl, ids = seg
+            pol = int(pol)
+            if not 0 <= pol < L:
+                raise ValueError(f"segment {i}: policy index {pol} out of range for {L} policies")
+            if isinstance(sl, tuple):
+                sl = slice(*sl)
+            e0, e1, step = sl.indices(B)
+            if step != 1 or e1 < e0:
+                raise ValueError(f"segment {i}: envs must be a contiguous slice of env indices")
+            ids = tuple(int(a) for a in (ids.tolist() if isinstance(ids, torch.Tensor) else ids))
+            if not 1 <= len(ids) <= MAX_IDS:
+                raise ValueError(f"segment {i}: agent ids must name 1..{MAX_IDS} agents, got {len(ids)}")
+            if any(a < 0 or a >= N for a in ids):
+                raise ValueError(f"segment {i}: agent ids {ids} out of range for {N} agents per env")
+            norm.append((pol, e0, e1, ids))
+        n_samples = [0] * L
+        seg_first_row = []
+        for pol, e0, e1, ids in norm:            # rows of a policy: its segments in the order given
+            seg_first_row.append(n_samples[pol])
+            n_samples[pol] += (e1 - e0) * len(ids)
+        s_max = max(max(n_samples), 1)
+        # per agent, the additive mask CtfPolicy.masked_logits applies: (mask_5 - 1) * 1e9 for masked agent types
+        masked_type = env.use_action_mask.detach().cpu().reshape(N, 1) == 1
+        mask5 = torch.tensor([0.0] * 5 + [-1e9] * (N_ACTIONS - 5))
+        agent_mask = torch.where(masked_type, mask5, torch.zeros(N_ACTIONS))
+        seg_rows, row_index, flat_index, mask_add = [], [], [], []
+        out = 0
+        for (pol, e0, e1, ids), first in zip(norm, seg_first_row):
+            k = len(ids)
+            n = (e1 - e0) * k
+            seg_rows.append((out, out + n))
+            out += n
+            s = torch.arange(n)
+            agent = torch.tensor(ids, dtype=torch.int64)[s % k]
+            row_index.append(pol * s_max + first + s)
+            flat_index.append((e0 + s // k) * N + agent)
+            mask_add.append(agent_mask[agent] if self.policies[pol].use_masking else torch.zeros((n, N_ACTIONS)))
+        dev = env.device
+        # the kernel's tables, policy-major (a CTA restages weights only where the policy changes)
+        order = sorted(range(len(norm)), key=lambda i: norm[i][0])
+        tables = []
+        for c in range(0, len(order), _native.GROUPED_MAX_SEGMENTS):
+            chunk = order[c : c + _native.GROUPED_MAX_SEGMENTS]
+            arr = (_native.CtfPolicySegment * len(chunk))()
+            for slot, i in enumerate(chunk):
+                pol, e0, e1, ids = norm[i]
+                arr[slot].env_begin, arr[slot].n_envs = e0, e1 - e0
+                arr[slot].out_row, arr[slot].policy, arr[slot].k = pol * s_max + seg_first_row[i], pol, len(ids)
+                for j, a in enumerate(ids):
+                    arr[slot].agent_ids[j] = a
+            tables.append((arr, len(chunk)))
+        def cat(ts, shape):
+            return (torch.cat(ts) if ts else torch.zeros(shape)).to(dev)
+
+        return PoolPlan(
+            norm, n_samples, s_max, seg_rows,
+            cat(row_index, (0,)).long(), cat(flat_index, (0,)).long(), cat(mask_add, (0, N_ACTIONS)).float(),
+            torch.zeros((L * s_max, self.stride), dtype=torch.bfloat16, device=dev),
+            tables,
+        )
+
+    # ------------------------------------------------------------------ launches
+    def trunk(self, plan: PoolPlan, env=None) -> torch.Tensor:
+        """Runs the grouped trunk for ``plan`` on ``env`` (default: the pool's env) and returns ``plan.features``:
+        bf16 [L * s_max, stride], policy p's rows at [p*s_max, p*s_max + plan.n_samples[p]), pad rows untouched."""
+        env = self._env_for(env)
+        if env.obs_bits is None:
+            raise ValueError("PolicyPool reads env.obs_bits: create the env with packed_obs=True")
+        stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
+        feat = plan.features
+        for arr, n in plan._tables:
+            _native.check(env._lib.ctf_policy_features_grouped(
+                env._handle, self._weights, len(self.policies), arr, n, C.c_void_p(env.obs_bits.data_ptr()),
+                C.c_void_p(env.meta.data_ptr()), env.num_envs, env.N_AGENTS, C.c_void_p(feat.data_ptr()), self.stride,
+                feat.shape[0], stream))
+        return feat
+
+    def head(self, plan: PoolPlan, feat: torch.Tensor | None = None):
+        """(value [S, 1], logits [S, 9]) fp32 in plan order from the feature rows: fc1 -> tanh -> fc2 -> tanh -> heads
+        as one bf16 ``torch.baddbmm`` chain over [L, s_max, .], then the plan's rows gathered."""
+        L = len(self.policies)
+        x = (plan.features if feat is None else feat).view(L, plan.s_max, self.stride)
+        x = torch.tanh(torch.baddbmm(self._fc1b.unsqueeze(1), x, self._fc1w.transpose(1, 2)))
+        x = torch.tanh(torch.baddbmm(self._fc2b.unsqueeze(1), x, self._fc2w.transpose(1, 2)))
+        out = torch.baddbmm(self._hb.unsqueeze(1), x, self._hw.transpose(1, 2)).view(L * plan.s_max, 1 + N_ACTIONS)
+        out = out.index_select(0, plan.row_index).float()
+        return out[:, :1], out[:, 1:]
+
+    @torch.no_grad()
+    def forward(self, plan: PoolPlan, env=None):
+        """(value [S, 1], logits [S, 9]) fp32 of every sample of ``plan``, in plan order."""
+        return self.head(plan, self.trunk(plan, env))
+
+    __call__ = forward
+
+    @torch.no_grad()
+    def act(self, plan: PoolPlan, actions: torch.Tensor, env=None) -> torch.Tensor:
+        """Samples one action per row of ``plan`` (one ``Categorical`` over all rows, each masked by its own policy's
+        ``use_masking`` as ``CtfPolicy.masked_logits`` does) and writes it into ``actions`` (uint8 [B, N], contiguous)
+        at the row's (env, agent).  Returns the sampled actions [S] int64 in plan order."""
+        env = self._env_for(env)
+        if actions.dtype != torch.uint8 or tuple(actions.shape) != (env.num_envs, env.N_AGENTS) \
+                or not actions.is_contiguous():
+            raise ValueError(f"actions must be a contiguous uint8 tensor [{env.num_envs}, {env.N_AGENTS}]")
+        _, logits = self.forward(plan, env)
+        a = Categorical(logits=logits + plan.mask_add, validate_args=False).sample()
+        actions.view(-1).index_copy_(0, plan.flat_index, a.to(torch.uint8))
+        return a

@@ -2,8 +2,9 @@
 
 The reference evaluates a league by submitting ``number_of_duels`` Ray tasks per (agent, opponent) pair, each a
 full ``utils.duel`` on a pickled env copy (league_training.py:368-459, 573-648).  Here every duel is one env of a
-batch: pair p owns the envs [p*D, (p+1)*D) and all pairs advance with one step-kernel launch per step; only the
-policy forwards are per pair.  Results come back in the reference's formats:
+batch: pair p owns the envs [p*D, (p+1)*D) and all pairs advance with one step-kernel launch per step.  By default the
+policy forwards are per pair; with ``grouped=True`` one ``PolicyPool`` runs every policy of every pair per step (one
+grouped trunk launch and one batched head, whatever the number of pairs).  Results come back in the reference's formats:
 
 * ``winrate_matrix_symmetric / non_symmetric``  ==  ``LeagueTrainer.calculate_winrate_matrix_*`` (:368-400, :427-455)
 * ``generate_metrics_symmetric / non_symmetric`` ==  ``LeagueTrainer.generate_metrics_*`` (:573-648): every duel's
@@ -17,13 +18,37 @@ from collections import defaultdict
 import torch
 
 from .env import GridworldCtfGPU, metrics_dict
-from .fused_policy import FusedPolicy
+from .fused_policy import FusedPolicy, PolicyPool
+from .policy import CtfPolicy
 from .rollout import batched_action
+
+
+def pool_segments(pairs, duels_per_pair: int, team_ids):
+    """(policies, segments) of a ``PolicyPool`` that plays ``pairs`` as ``duel_pairs`` lays them out: the distinct
+    ``CtfPolicy`` modules (a ``FusedPolicy`` stands for its ``policy``, so a module and its views count once) by
+    identity, in order of first appearance, and one segment (policy index, envs of the pair, team ids) per (pair, team)
+    with agents, pair p owning the envs [p*D, (p+1)*D)."""
+    D = int(duels_per_pair)
+    uniq, index = [], {}
+
+    def module(pol):
+        return pol.policy if isinstance(pol, FusedPolicy) else pol
+
+    for pair in pairs:
+        for pol in pair:
+            m = module(pol)
+            if id(m) not in index:
+                index[id(m)] = len(uniq)
+                uniq.append(m)
+    segments = [(index[id(module(pol))], slice(p * D, (p + 1) * D), tuple(ids))
+                for p, pair in enumerate(pairs) for ids, pol in zip(team_ids, pair) if ids]
+    return uniq, segments
 
 
 @torch.no_grad()
 def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 256, device=None, seed: int = 0,
-               env_id_base: int = 0, collect_metrics: bool = False, per_duel_metrics: bool = False):
+               env_id_base: int = 0, collect_metrics: bool = False, per_duel_metrics: bool = False,
+               grouped: bool = False):
     """Plays ``duels_per_pair`` duels (utils.py:500-573) for every (agent, opponent) in ``pairs`` at once.
 
     Returns (results [P, D] int64 of +1/0/-1 from team 0's view, metrics).  metrics is None unless collect_metrics;
@@ -32,34 +57,51 @@ def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 25
 
     ``fused_policy.FusedPolicy`` policies read the env's packed observations in place; when every policy is one, the
     env is created packed-only and never writes dense observations.
+
+    ``grouped=True``: every policy must be a ``FusedPolicy`` or a ``CtfPolicy``; the distinct modules go into
+    one ``fused_policy.PolicyPool`` on a packed-only env, with one plan segment per (pair, team), and each step is
+    ``pool.act`` followed by ``env.step``.  The results and metrics have the same structure as the per-pair path's;
+    the draws differ (one ``Categorical`` over all rows consumes torch's random stream differently).
     """
     P, D = len(pairs), int(duels_per_pair)
-    fused = [isinstance(pol, FusedPolicy) for pair in pairs for pol in pair]
-    packed_kw = {} if not any(fused) else dict(packed_obs=True, dense_obs=not all(fused))
+    if grouped:
+        if any(not isinstance(pol, (FusedPolicy, CtfPolicy)) for pair in pairs for pol in pair):
+            raise ValueError("grouped=True needs every policy to be a FusedPolicy or a CtfPolicy")
+        packed_kw = dict(packed_obs=True, dense_obs=False)
+    else:
+        fused = [isinstance(pol, FusedPolicy) for pair in pairs for pol in pair]
+        packed_kw = {} if not any(fused) else dict(packed_obs=True, dense_obs=not all(fused))
     env = GridworldCtfGPU(**env_config, num_envs=P * D, device=device, seed=seed, env_id_base=env_id_base,
                           reverse_team1_actions=True, stats="counters" if collect_metrics else "none", **packed_kw)
     B, N, dev = env.num_envs, env.N_AGENTS, env.device
     C, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
     team_ids = [[i for i in range(N) if env.AGENT_TEAMS[i] == t] for t in (0, 1)]
     teams = [torch.tensor(ids, device=dev) for ids in team_ids]
+    if grouped:
+        uniq, segments = pool_segments(pairs, D, team_ids)
+        pool = PolicyPool(env, uniq)
+        plan = pool.plan(segments)
     obs, meta, _ = env.reset()
     actions = torch.empty((B, N), dtype=torch.uint8, device=dev)
     step_count = 0
     while True:
         step_count += 1
-        for p, pair in enumerate(pairs):
-            sl = slice(p * D, (p + 1) * D)
-            for idx, ids, pol in zip(teams, team_ids, pair):
-                k = idx.numel()
-                if k == 0:
-                    continue
-                flags = env.use_action_mask[idx].unsqueeze(0).expand(D, k).reshape(D * k)
-                if isinstance(pol, FusedPolicy):
-                    a = pol.get_action_and_value(flags, agent_ids=ids, env=env, envs=sl)[0]
-                else:
-                    a = batched_action(pol, obs[sl][:, idx].reshape(D * k, C, G, G).float(), meta[sl][:, idx].reshape(D * k, M),
-                                       flags)
-                actions[sl, idx] = a.reshape(D, k).to(torch.uint8)
+        if grouped:
+            pool.act(plan, actions)
+        else:
+            for p, pair in enumerate(pairs):
+                sl = slice(p * D, (p + 1) * D)
+                for idx, ids, pol in zip(teams, team_ids, pair):
+                    k = idx.numel()
+                    if k == 0:
+                        continue
+                    flags = env.use_action_mask[idx].unsqueeze(0).expand(D, k).reshape(D * k)
+                    if isinstance(pol, FusedPolicy):
+                        a = pol.get_action_and_value(flags, agent_ids=ids, env=env, envs=sl)[0]
+                    else:
+                        a = batched_action(pol, obs[sl][:, idx].reshape(D * k, C, G, G).float(),
+                                           meta[sl][:, idx].reshape(D * k, M), flags)
+                    actions[sl, idx] = a.reshape(D, k).to(torch.uint8)
         obs, meta, _, _, _ = env.step(actions)
         if step_count > max_steps or step_count >= env.GAME_STEPS:
             break
