@@ -7,9 +7,12 @@ from helpers import compiled
 from marl_ctf_development_b200.fused_policy import conv2_kernel_layout_index, reference_features, trunk_dims
 from marl_ctf_development_b200.policy import CtfPolicy
 
+# (C, G, M) of three shipped maps and of the rows of test_gpu_trunk_geometry.GEOMETRY: every G from 5 to 16, C = 5 and 14
+GEOMETRY_SHAPES = [(5, 5, 10), (14, 5, 22), (11, 6, 16), (5, 6, 12), (9, 7, 16), (5, 8, 10), (14, 8, 22), (14, 9, 20),
+                   (11, 10, 16), (7, 12, 14), (14, 12, 22), (11, 14, 18), (5, 16, 10), (11, 16, 16), (14, 16, 22)]
 SHAPES = [(4, 6, 10)] + [
     (ce.n_channels, ce.GRID_SIZE, ce.meta_size) for ce in (compiled(e) for e in ("0_the_split", "7_gridlocked", "8_arena"))
-]
+] + GEOMETRY_SHAPES
 
 
 def _inputs(C, G, M, S, seed):

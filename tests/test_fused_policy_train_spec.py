@@ -5,13 +5,14 @@ import pytest
 import torch
 
 from helpers import compiled
+from test_fused_policy_spec import GEOMETRY_SHAPES
 from marl_ctf_development_b200.fused_policy import (conv2_kernel_layout_index, conv2_transpose_layout_index,
                                                     reference_features, reference_trunk_grads, trunk_dims)
 from marl_ctf_development_b200.policy import CtfPolicy
 
-SHAPES = [(4, 6, 10), (14, 16, 22)] + [
+SHAPES = [(4, 6, 10)] + [
     (ce.n_channels, ce.GRID_SIZE, ce.meta_size) for ce in (compiled(e) for e in ("0_the_split", "7_gridlocked", "8_arena"))
-]
+] + GEOMETRY_SHAPES
 
 
 def _case(C, G, M, S, seed):

@@ -114,7 +114,8 @@ def test_trunk_grads_match_reference(name, steps):
 
 
 def test_trunk_grads_for_any_binary_input():
-    """Every bit pattern, not only one-hot cells (G = 16, C = 14 is the largest plan)."""
+    """Every bit pattern, not only one-hot cells (G = 16, C = 10; the largest plan, G = 16, C = 14, is a row of
+    test_gpu_trunk_geometry)."""
     env = _stepped_env(SCENARIOS["random-4-G16"](), 8, 0)
     fp = FusedPolicy(env, _policy(env, 2))
     g = torch.Generator(device=DEV).manual_seed(0)
@@ -245,7 +246,7 @@ def test_many_samples_per_cta_match_reference_and_are_deterministic_in_place_and
 
 
 def test_many_samples_per_cta_for_any_binary_input():
-    """Random non-one-hot words on the largest plan (G = 16, C = 14), 3 n_ctas + 37 samples."""
+    """Random non-one-hot words at G = 16, C = 10, 3 n_ctas + 37 samples."""
     env = _stepped_env(SCENARIOS["random-4-G16"](), 8, 0)
     fp = FusedPolicy(env, _policy(env, 2))
     n = _n_ctas(fp)
