@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 9
+#define CTF_ABI_VERSION 10
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -351,6 +351,26 @@ int ctf_policy_features_backward(ctf_handle_t h, const ctf_policy_weights_t* w, 
                                  const uint32_t* packed, int64_t n_envs, int agents_per_env, const uint8_t* agent_ids,
                                  int k, const void* features, const void* grad_features, int64_t feature_stride,
                                  void* workspace, size_t workspace_bytes, const ctf_policy_grads_t* grads, void* stream);
+
+/*
+ * Generalised advantage estimation (GAE) over a rollout, on the device.  Layout of a collect_rollout buffer:
+ * rewards, values, advantages and returns are fp32 [n_steps * agents_per_step][n_envs], row t*agents_per_step + j =
+ * trained agent j at step t; next_value is fp32 [agents_per_step][n_envs], the bootstrap V(s_T) of every (agent, env)
+ * (0 when the rollout ended the episode).  Each (agent, env) column is its own sequence over t; there is no done
+ * input, because the envs of a rollout end only together at its last step.  Backwards over t, with nv = next_value at
+ * t = n_steps - 1 and values[t + 1] below it:
+ *     delta = (rewards[t] + gamma*nv) - values[t];  last = delta + gamma_lambda*last (last = 0 before the first row);
+ *     advantages[t] = last;  returns[t] = last + values[t]
+ * Every operation is rounded on its own (no fused multiply-add), so the result is bit for bit what eager torch computes
+ * for the same statements on fp32 tensors with Python scalars gamma and gamma*lambda: pass gamma = (float)gamma and
+ * gamma_lambda = (float)(gamma * lambda computed in double).
+ * Rejected with CTF_ERR_INVALID: a null pointer; n_steps < 1; agents_per_step outside 1..CTF_MAX_AGENTS; n_envs < 1;
+ * gamma or gamma_lambda not finite or outside [0, 1]; a buffer not 4-byte aligned; an output that overlaps an input
+ * or the other output.  No allocation and no host synchronisation (can be captured in a CUDA graph).
+ */
+int ctf_gae(ctf_handle_t h, const float* rewards, const float* values, const float* next_value, float* advantages,
+            float* returns, int64_t n_steps, int64_t agents_per_step, int64_t n_envs, float gamma, float gamma_lambda,
+            void* stream);
 
 /*
  * Compressible device memory for the dense observation buffer.  On devices with Compute Data Compression the memory

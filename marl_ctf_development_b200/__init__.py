@@ -5,6 +5,7 @@ Public surface:
     GridworldCtf      single-env view with the reference's exact methods (drop-in for ppo.py / utils.py)
     FusedPolicy       CtfPolicy inference from packed observations (fused_policy.py)
     PolicyPool        several policies' inference on one env batch: one grouped trunk launch per forward (fused_policy.py)
+    PackedPPO         PPO for a CtfPolicy from packed rollouts, advantages by the ctf_gae kernel (ppo.py)
     compressible_empty  torch.empty in compressible device memory, for caller-bound observation buffers
     compile_config    (AGENT_CONFIG, SCENARIO, kwargs) -> ctf_config_t
     experiment_env_config / experiment_names   the reference's nine experiment configs as data
@@ -27,4 +28,8 @@ def __getattr__(name):
         from . import fused_policy
 
         return getattr(fused_policy, name)
+    if name == "PackedPPO":
+        from .ppo import PackedPPO
+
+        return PackedPPO
     raise AttributeError(name)

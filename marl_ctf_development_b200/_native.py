@@ -30,13 +30,14 @@ EXPORTS = (
     "ctf_policy_features_backward",
     "ctf_policy_features_grouped",
     "ctf_policy_trunk_ctas",
+    "ctf_gae",
     "ctf_compressible_alloc",
     "ctf_compressible_free",
     "ctf_compression_supported",
     "ctf_mem_is_compressed",
     "ctf_compressible_set_enabled",
 )
-ABI_VERSION = 9
+ABI_VERSION = 10
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
 
 
@@ -147,6 +148,8 @@ def load():
     L.ctf_policy_features_backward.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64,
                                                C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
                                                C.c_void_p, C.c_size_t, C.POINTER(CtfPolicyGrads), C.c_void_p]
+    L.ctf_gae.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
+                          C.c_int64, C.c_float, C.c_float, C.c_void_p]
     L.ctf_compressible_alloc.restype = C.c_void_p
     L.ctf_compressible_alloc.argtypes = [C.c_ssize_t, C.c_int, C.c_void_p]
     L.ctf_compressible_free.restype = None

@@ -41,6 +41,7 @@ class Rollout:
     next_metadata_state: torch.Tensor  # [B, M]
     next_done: torch.Tensor        # [B]
     packed: bool = False
+    next_value: torch.Tensor | None = None  # [apt, B] bootstrap V(s_T) per (agent, env), set by ppo.PackedPPO.collect
 
     def as_reference_arrays(self):
         """The eleven values ``train_ppo`` keeps per update (ppo.py:298-305, 362-376), in the reference's order.
