@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 10
+#define CTF_ABI_VERSION 11
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -357,8 +357,8 @@ int ctf_policy_features_backward(ctf_handle_t h, const ctf_policy_weights_t* w, 
  * rewards, values, advantages and returns are fp32 [n_steps * agents_per_step][n_envs], row t*agents_per_step + j =
  * trained agent j at step t; next_value is fp32 [agents_per_step][n_envs], the bootstrap V(s_T) of every (agent, env)
  * (0 when the rollout ended the episode).  Each (agent, env) column is its own sequence over t; there is no done
- * input, because the envs of a rollout end only together at its last step.  Backwards over t, with nv = next_value at
- * t = n_steps - 1 and values[t + 1] below it:
+ * input, for rollouts whose envs end only together at their last step (ctf_gae_dones takes one).  Backwards over t,
+ * with nv = next_value at t = n_steps - 1 and values[t + 1] below it:
  *     delta = (rewards[t] + gamma*nv) - values[t];  last = delta + gamma_lambda*last (last = 0 before the first row);
  *     advantages[t] = last;  returns[t] = last + values[t]
  * Every operation is rounded on its own (no fused multiply-add), so the result is bit for bit what eager torch computes
@@ -371,6 +371,23 @@ int ctf_policy_features_backward(ctf_handle_t h, const ctf_policy_weights_t* w, 
 int ctf_gae(ctf_handle_t h, const float* rewards, const float* values, const float* next_value, float* advantages,
             float* returns, int64_t n_steps, int64_t agents_per_step, int64_t n_envs, float gamma, float gamma_lambda,
             void* stream);
+
+/*
+ * ctf_gae for rollouts that cross episode boundaries (ABI 11).  dones is fp32 [n_steps * agents_per_step][n_envs],
+ * the layout of rewards; a nonzero dones[t*agents_per_step + j][b] means that observation t of (agent j, env b)
+ * starts a new episode (CleanRL's convention).  The recurrence is ctf_gae's, except that after row t, when dones[t]
+ * is nonzero, nv and last both become exactly 0 (a select, not a multiply by 1 - dones) before row t - 1:
+ *     delta = (rewards[t] + gamma*nv) - values[t];  last = delta + gamma_lambda*last;
+ *     advantages[t] = last;  returns[t] = last + values[t];  nv = values[t];
+ *     if (dones[t] != 0) nv = last = 0
+ * next_value is the bootstrap of the last row, so pass 0 where the last step ended the episode.  dones[0] changes
+ * nothing in this rollout.  With all dones zero the result is bit for bit ctf_gae's, which reads 4 fewer bytes per
+ * element.  Rejected as ctf_gae rejects, and also: a null dones, a dones not 4-byte aligned, an output that overlaps
+ * dones.  No allocation and no host synchronisation.
+ */
+int ctf_gae_dones(ctf_handle_t h, const float* rewards, const float* values, const float* dones, const float* next_value,
+                  float* advantages, float* returns, int64_t n_steps, int64_t agents_per_step, int64_t n_envs,
+                  float gamma, float gamma_lambda, void* stream);
 
 /*
  * Compressible device memory for the dense observation buffer.  On devices with Compute Data Compression the memory

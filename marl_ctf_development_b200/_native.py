@@ -31,13 +31,14 @@ EXPORTS = (
     "ctf_policy_features_grouped",
     "ctf_policy_trunk_ctas",
     "ctf_gae",
+    "ctf_gae_dones",
     "ctf_compressible_alloc",
     "ctf_compressible_free",
     "ctf_compression_supported",
     "ctf_mem_is_compressed",
     "ctf_compressible_set_enabled",
 )
-ABI_VERSION = 10
+ABI_VERSION = 11
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
 
 
@@ -150,6 +151,8 @@ def load():
                                                C.c_void_p, C.c_size_t, C.POINTER(CtfPolicyGrads), C.c_void_p]
     L.ctf_gae.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                           C.c_int64, C.c_float, C.c_float, C.c_void_p]
+    L.ctf_gae_dones.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_float, C.c_void_p]
     L.ctf_compressible_alloc.restype = C.c_void_p
     L.ctf_compressible_alloc.argtypes = [C.c_ssize_t, C.c_int, C.c_void_p]
     L.ctf_compressible_free.restype = None

@@ -1467,28 +1467,34 @@ static __host__ void trunk_bwd_layout(const DevPlan& P, TrunkBwdArgs& A, size_t&
 // ================================================================================================
 constexpr int kGaeThreads = 256;
 constexpr int kGaeUnroll = 8;   // rows whose loads are issued before the recurrence consumes the first of them
-// 6 CTAs per SM leave 40 registers, enough for the 16 loads in flight without spills (8 CTAs spill)
+// 6 CTAs per SM leave 40 registers, enough for the 16 loads in flight without spills (8 CTAs spill); the 24 loads of
+// k_gae<true> spill at 40 registers, so it runs 5 CTAs per SM (48 registers)
 
 // Rows are [T*apt][B] fp32 with row t*apt + j = agent j at step t, so column c = j*B + b of a row is contiguous over
 // the threads of a warp: every load and store is coalesced.  The recurrence runs backwards over t with one explicit
 // rounding per operation (no FMA contraction), which is bit for bit the eager torch statement ppo.reference_advantages:
 //   delta = (r[t] + gamma*nv) - v[t];  last = delta + gamma_lambda*last;  adv[t] = last;  ret[t] = last + v[t]
 // with nv = next_value for t = T-1 and v[t+1] below it.
-__global__ void __launch_bounds__(kGaeThreads, 6) k_gae(const float* __restrict__ rewards, const float* __restrict__ values,
+// kDones (ctf_gae_dones): a nonzero dones[t] means observation t starts a new episode (CleanRL's convention), so after
+// row t both nv and last are selected to exactly 0 before row t-1: no bootstrap and no advantage crosses the boundary.
+// dones is the last parameter so that the other parameters keep their offsets and k_gae<false> its code.
+template <bool kDones>
+__global__ void __launch_bounds__(kGaeThreads, kDones ? 5 : 6) k_gae(const float* __restrict__ rewards, const float* __restrict__ values,
                                                      const float* __restrict__ next_value, float* __restrict__ adv,
                                                      float* __restrict__ ret, long long T, long long cols, float gamma,
-                                                     float gamma_lambda) {
+                                                     float gamma_lambda, const float* __restrict__ dones) {
     const long long c = (long long)blockIdx.x * kGaeThreads + threadIdx.x;
     if (c >= cols) return;
     float nv = __ldg(next_value + c), last = 0.f;
     long long t = T - 1;
     for (; t >= kGaeUnroll - 1; t -= kGaeUnroll) {
-        float r[kGaeUnroll], v[kGaeUnroll];
+        float r[kGaeUnroll], v[kGaeUnroll], d[kGaeUnroll];
 #pragma unroll
         for (int u = 0; u < kGaeUnroll; ++u) {
             const size_t i = (size_t)(t - u) * cols + c;
             r[u] = __ldcs(rewards + i);
             v[u] = __ldcs(values + i);
+            if (kDones) d[u] = __ldcs(dones + i);
         }
 #pragma unroll
         for (int u = 0; u < kGaeUnroll; ++u) {
@@ -1498,16 +1504,19 @@ __global__ void __launch_bounds__(kGaeThreads, 6) k_gae(const float* __restrict_
             __stcs(adv + i, last);
             __stcs(ret + i, __fadd_rn(last, v[u]));
             nv = v[u];
+            if (kDones && d[u] != 0.f) nv = last = 0.f;
         }
     }
     for (; t >= 0; --t) {
         const size_t i = (size_t)t * cols + c;
         const float r = __ldcs(rewards + i), v = __ldcs(values + i);
+        const bool start = kDones && __ldcs(dones + i) != 0.f;
         const float delta = __fsub_rn(__fadd_rn(r, __fmul_rn(gamma, nv)), v);
         last = __fadd_rn(delta, __fmul_rn(gamma_lambda, last));
         __stcs(adv + i, last);
         __stcs(ret + i, __fadd_rn(last, v));
         nv = v;
+        if (start) nv = last = 0.f;
     }
 }
 
@@ -2426,38 +2435,60 @@ static bool overlaps(const void* a, size_t a_bytes, const void* b, size_t b_byte
     return x < y + b_bytes && y < x + a_bytes;
 }
 
-extern "C" int ctf_gae(ctf_handle_t h, const float* rewards, const float* values, const float* next_value,
-                       float* advantages, float* returns, int64_t n_steps, int64_t agents_per_step, int64_t n_envs,
-                       float gamma, float gamma_lambda, void* stream) {
+// ctf_gae and ctf_gae_dones: checks every argument, then launches k_gae<dones != nullptr>.  `fn` names the entry point
+// in the error messages.
+static int launch_gae(const char* fn, ctf_handle_t h, const float* rewards, const float* values, const float* dones,
+                      const float* next_value, float* advantages, float* returns, int64_t n_steps,
+                      int64_t agents_per_step, int64_t n_envs, float gamma, float gamma_lambda, void* stream) {
     if (!h || !rewards || !values || !next_value || !advantages || !returns)
-        return fail(CTF_ERR_INVALID, "ctf_gae: null argument");
-    if (n_steps < 1) return fail(CTF_ERR_INVALID, "ctf_gae: n_steps must be >= 1");
+        return fail(CTF_ERR_INVALID, "%s: null argument", fn);
+    if (n_steps < 1) return fail(CTF_ERR_INVALID, "%s: n_steps must be >= 1", fn);
     if (agents_per_step < 1 || agents_per_step > CTF_MAX_AGENTS)
-        return fail(CTF_ERR_INVALID, "ctf_gae: agents_per_step must be in 1..CTF_MAX_AGENTS (8)");
-    if (n_envs < 1) return fail(CTF_ERR_INVALID, "ctf_gae: n_envs must be >= 1");
+        return fail(CTF_ERR_INVALID, "%s: agents_per_step must be in 1..CTF_MAX_AGENTS (8)", fn);
+    if (n_envs < 1) return fail(CTF_ERR_INVALID, "%s: n_envs must be >= 1", fn);
     // the comparisons are false for NaN, so a NaN is rejected too
-    if (!(gamma >= 0.f && gamma <= 1.f)) return fail(CTF_ERR_INVALID, "ctf_gae: gamma must be finite and in [0, 1]");
+    if (!(gamma >= 0.f && gamma <= 1.f)) return fail(CTF_ERR_INVALID, "%s: gamma must be finite and in [0, 1]", fn);
     if (!(gamma_lambda >= 0.f && gamma_lambda <= 1.f))
-        return fail(CTF_ERR_INVALID, "ctf_gae: gamma_lambda must be finite and in [0, 1]");
+        return fail(CTF_ERR_INVALID, "%s: gamma_lambda must be finite and in [0, 1]", fn);
     const long long cols = (long long)agents_per_step * n_envs;
     // one thread per column: the grid must stay below 2^31 CTAs, and the byte sizes must fit 64 bits
     if (n_envs > (1LL << 35) || n_steps > (1LL << 60) / cols)
-        return fail(CTF_ERR_INVALID, "ctf_gae: n_steps * agents_per_step * n_envs is too large");
+        return fail(CTF_ERR_INVALID, "%s: n_steps * agents_per_step * n_envs is too large", fn);
     if ((reinterpret_cast<uintptr_t>(rewards) | reinterpret_cast<uintptr_t>(values) |
-         reinterpret_cast<uintptr_t>(next_value) | reinterpret_cast<uintptr_t>(advantages) |
-         reinterpret_cast<uintptr_t>(returns)) & 3)
-        return fail(CTF_ERR_INVALID, "ctf_gae: every buffer must be 4-byte aligned");
+         reinterpret_cast<uintptr_t>(dones) | reinterpret_cast<uintptr_t>(next_value) |
+         reinterpret_cast<uintptr_t>(advantages) | reinterpret_cast<uintptr_t>(returns)) & 3)
+        return fail(CTF_ERR_INVALID, "%s: every buffer must be 4-byte aligned", fn);
     const size_t bytes = (size_t)(n_steps * cols) * sizeof(float), nv_bytes = (size_t)cols * sizeof(float);
     for (const float* out : {advantages, returns})
         if (overlaps(out, bytes, rewards, bytes) || overlaps(out, bytes, values, bytes) ||
-            overlaps(out, bytes, next_value, nv_bytes))
-            return fail(CTF_ERR_INVALID, "ctf_gae: an output overlaps an input");
-    if (overlaps(advantages, bytes, returns, bytes)) return fail(CTF_ERR_INVALID, "ctf_gae: advantages overlaps returns");
+            overlaps(out, bytes, next_value, nv_bytes) || (dones && overlaps(out, bytes, dones, bytes)))
+            return fail(CTF_ERR_INVALID, "%s: an output overlaps an input", fn);
+    if (overlaps(advantages, bytes, returns, bytes)) return fail(CTF_ERR_INVALID, "%s: advantages overlaps returns", fn);
     DeviceGuard guard(h->device);
     CTF_CUDA(guard.err);
     const unsigned grid = (unsigned)((cols + kGaeThreads - 1) / kGaeThreads);
-    k_gae<<<grid, kGaeThreads, 0, static_cast<cudaStream_t>(stream)>>>(rewards, values, next_value, advantages, returns,
-                                                                        n_steps, cols, gamma, gamma_lambda);
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (dones)
+        k_gae<true><<<grid, kGaeThreads, 0, s>>>(rewards, values, next_value, advantages, returns, n_steps, cols, gamma,
+                                                 gamma_lambda, dones);
+    else
+        k_gae<false><<<grid, kGaeThreads, 0, s>>>(rewards, values, next_value, advantages, returns, n_steps, cols, gamma,
+                                                  gamma_lambda, nullptr);
     CTF_CUDA(cudaGetLastError());
     return CTF_OK;
+}
+
+extern "C" int ctf_gae(ctf_handle_t h, const float* rewards, const float* values, const float* next_value,
+                       float* advantages, float* returns, int64_t n_steps, int64_t agents_per_step, int64_t n_envs,
+                       float gamma, float gamma_lambda, void* stream) {
+    return launch_gae("ctf_gae", h, rewards, values, nullptr, next_value, advantages, returns, n_steps, agents_per_step,
+                      n_envs, gamma, gamma_lambda, stream);
+}
+
+extern "C" int ctf_gae_dones(ctf_handle_t h, const float* rewards, const float* values, const float* dones,
+                             const float* next_value, float* advantages, float* returns, int64_t n_steps,
+                             int64_t agents_per_step, int64_t n_envs, float gamma, float gamma_lambda, void* stream) {
+    if (!dones) return fail(CTF_ERR_INVALID, "ctf_gae_dones: null argument");
+    return launch_gae("ctf_gae_dones", h, rewards, values, dones, next_value, advantages, returns, n_steps,
+                      agents_per_step, n_envs, gamma, gamma_lambda, stream);
 }

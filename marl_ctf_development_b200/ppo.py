@@ -12,6 +12,10 @@ Two deliberate differences from the reference's ``PPOTrainer`` (ppo.py): every (
 sequence over the T steps, where the reference chains the apt agents' rows of an env into one sequence of T*apt rows;
 and every (agent, env) bootstraps from its own V(s_T), where the reference bootstraps every env from the last env's
 state.  The reference's exact update stays available through ``Rollout.as_reference_arrays``.
+
+``PackedPPO(..., rollout_steps=T)`` trains on rollouts of T <= GAME_STEPS steps that continue the env's episodes
+across updates (CleanRL's and Isaac Gym's scheme), where the reference resets the envs at every rollout: the env is reset
+when its episodes end, and GAE (``ctf_gae_dones``) stops at every episode boundary.
 """
 from __future__ import annotations
 
@@ -28,15 +32,19 @@ from .rollout import Rollout, _team_indices, collect_rollout
 # ---------------------------------------------------------------------------------------------------- advantages
 @torch.no_grad()
 def reference_advantages(rewards: torch.Tensor, values: torch.Tensor, next_value: torch.Tensor, gamma: float,
-                         lam: float):
-    """What ``ctf_gae`` computes, in eager torch: (advantages, returns), fp32 [T*apt, B].
+                         lam: float, dones: torch.Tensor | None = None):
+    """What ``ctf_gae`` (``ctf_gae_dones`` with ``dones``) computes, in eager torch: (advantages, returns), fp32
+    [T*apt, B].
 
     ``rewards`` / ``values`` fp32 [T*apt, B] (row t*apt + j = trained agent j at step t), ``next_value`` fp32 [apt, B].
     Each (agent, env) column is one sequence over t; one rounding per operation, in the kernel's order, with the
-    Python scalars ``gamma`` and ``gamma * lam``."""
+    Python scalars ``gamma`` and ``gamma * lam``.  ``dones`` fp32 [T*apt, B]: a nonzero ``dones[t*apt + j, b]`` means
+    observation t starts a new episode (CleanRL's convention), so below row t the bootstrap and the running advantage
+    are both exactly 0.  ``dones=None`` or all zeros give the same bits."""
     apt, B = next_value.shape
     T = rewards.shape[0] // apt
     r, v = rewards.reshape(T, apt, B), values.reshape(T, apt, B)
+    start = None if dones is None else dones.reshape(T, apt, B) != 0
     adv = torch.empty_like(r)
     gl = gamma * lam
     nv, last = next_value, torch.zeros_like(next_value)
@@ -45,26 +53,37 @@ def reference_advantages(rewards: torch.Tensor, values: torch.Tensor, next_value
         last = delta + gl * last
         adv[t] = last
         nv = v[t]
+        if start is not None:
+            nv = torch.where(start[t], 0.0, nv)
+            last = torch.where(start[t], 0.0, last)
     return adv.reshape(T * apt, B), (adv + v).reshape(T * apt, B)
 
 
-def advantages(env, rollout: Rollout, next_value: torch.Tensor, gamma: float, lam: float):
+def advantages(env, rollout: Rollout, next_value: torch.Tensor, gamma: float, lam: float,
+               dones: torch.Tensor | None = None):
     """(advantages, returns) fp32 [T*apt, B] of ``rollout`` with the bootstrap ``next_value`` [apt, B], from one
-    ``ctf_gae`` launch on the current stream; bit for bit ``reference_advantages``."""
+    ``ctf_gae`` launch on the current stream, or one ``ctf_gae_dones`` launch when ``dones`` [T*apt, B] is given (a
+    rollout that crosses episode boundaries); bit for bit ``reference_advantages``."""
     rew, val = rollout.rewards, rollout.values
     if next_value.dim() != 2 or next_value.shape[1] != rew.shape[1] or rew.shape[0] % next_value.shape[0]:
         raise ValueError(f"next_value must be [apt, B] with B = {rew.shape[1]} and apt dividing {rew.shape[0]}")
-    for name, x in (("rewards", rew), ("values", val), ("next_value", next_value)):
-        if x.dtype != torch.float32 or x.device != env.device:
+    if dones is not None and dones.shape != rew.shape:
+        raise ValueError(f"dones must have the rewards' shape {tuple(rew.shape)}")
+    for name, x in (("rewards", rew), ("values", val), ("next_value", next_value), ("dones", dones)):
+        if x is not None and (x.dtype != torch.float32 or x.device != env.device):
             raise ValueError(f"{name} must be a float32 tensor on {env.device}")
     rew, val, nv = rew.contiguous(), val.contiguous(), next_value.contiguous()
     adv, ret = torch.empty_like(rew), torch.empty_like(rew)
     apt, B = nv.shape
-    stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
-    _native.check(env._lib.ctf_gae(
-        env._handle, C.c_void_p(rew.data_ptr()), C.c_void_p(val.data_ptr()), C.c_void_p(nv.data_ptr()),
-        C.c_void_p(adv.data_ptr()), C.c_void_p(ret.data_ptr()), rew.shape[0] // apt, apt, B, float(gamma),
-        float(gamma * lam), stream))
+    ptr = lambda x: C.c_void_p(x.data_ptr())
+    sizes = (rew.shape[0] // apt, apt, B, float(gamma), float(gamma * lam),
+             C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream))
+    if dones is None:
+        rc = env._lib.ctf_gae(env._handle, ptr(rew), ptr(val), ptr(nv), ptr(adv), ptr(ret), *sizes)
+    else:
+        d = dones.contiguous()
+        rc = env._lib.ctf_gae_dones(env._handle, ptr(rew), ptr(val), ptr(d), ptr(nv), ptr(adv), ptr(ret), *sizes)
+    _native.check(rc)
     return adv, ret
 
 
@@ -117,9 +136,16 @@ class PackedPPO:
     (``dense_obs=False``) saves its dense observation writes.  ``agent`` is a ``CtfPolicy`` (load a reference ``Agent``
     into one with ``load_state_dict``); ``self.fused`` is its ``FusedPolicy``, which collects the rollouts and computes
     the training forward and backward.  ``chunk`` bounds the samples of one forward / backward: each holds about
-    2 x stride bf16 values between them (15.6 KB at 8_arena)."""
+    2 x stride bf16 values between them (15.6 KB at 8_arena).
 
-    def __init__(self, env, agent, args, optimizer=None, chunk=262144):
+    ``rollout_steps=None`` collects one fresh episode of every env per update.  An int T in 1..GAME_STEPS selects
+    continuing mode: every ``collect`` runs T steps, the first one from ``env.reset()`` and every later one from where
+    the env is (``collect_rollout(reset=False)``), resetting the env when its episodes end; GAE then stops at each
+    episode boundary.  The opponent may change between updates; ``train_team1`` may change only between episodes
+    (ValueError while one is in progress).  The env belongs to the trainer in this mode: stepping or resetting it
+    elsewhere breaks the episodes the trainer continues."""
+
+    def __init__(self, env, agent, args, optimizer=None, chunk=262144, rollout_steps=None):
         if env.obs_bits is None:
             raise ValueError("PackedPPO trains from packed observations: create the env with packed_obs=True")
         if not env.ce.cfg.reverse_team1_actions:
@@ -130,30 +156,57 @@ class PackedPPO:
             raise ValueError("PackedPPO estimates advantages with GAE only: args.gae must be True")
         if int(chunk) < 1:
             raise ValueError("chunk must be >= 1")
+        if rollout_steps is not None and not 1 <= int(rollout_steps) <= env.GAME_STEPS:
+            raise ValueError(f"rollout_steps must be None or in 1..GAME_STEPS ({env.GAME_STEPS})")
+        self.rollout_steps = None if rollout_steps is None else int(rollout_steps)
         self.env, self.agent, self.args, self.chunk = env, agent, args, int(chunk)
         self.fused = FusedPolicy(env, agent)
         self.optimizer = optimizer if optimizer is not None else torch.optim.Adam(
             agent.parameters(), lr=args.learning_rate, eps=1e-5)
         self.rollout = None
+        self._train_team1 = None     # continuing mode: the team of the episode in progress (None before the first collect)
+        self._running_return = None  # continuing mode: fp32 [apt, B] return of every trained (agent, env) so far
 
     def collect(self, opponent, train_team1=True, num_env_steps=None) -> Rollout:
         """One packed rollout of every env (``collect_rollout``) with the trained agent's ``FusedPolicy`` against
         ``opponent`` (a ``FusedPolicy``, or a ``CtfPolicy`` run through one), and its bootstrap ``next_value`` [apt, B]:
         0 when the rollout reached ``GAME_STEPS`` (every env ended), else the trained agents' V(s_T) from
         ``forward_from_env``.  The previous rollout is released first, so one rollout is alive at a time (as long as
-        the caller keeps no reference to the old one)."""
+        the caller keeps no reference to the old one).
+
+        In continuing mode ``num_env_steps`` defaults to ``rollout_steps``, the rollout continues the env's episodes
+        (its ``dones`` mark where new ones start), the bootstrap is 0 exactly where the last step ended the episode,
+        and ``rollout.episode_stats`` holds the device tensors that ``optimise`` reports (see there)."""
         env = self.env
-        T = env.GAME_STEPS if num_env_steps is None else int(num_env_steps)
+        continuing = self.rollout_steps is not None
+        T = (self.rollout_steps if continuing else env.GAME_STEPS) if num_env_steps is None else int(num_env_steps)
         if not 1 <= T <= env.GAME_STEPS:
-            raise ValueError(f"num_env_steps must be in 1..GAME_STEPS ({env.GAME_STEPS}): envs may not end inside a rollout")
+            raise ValueError(f"num_env_steps must be in 1..GAME_STEPS ({env.GAME_STEPS})"
+                             + ("" if continuing else ": envs may not end inside a rollout"))
+        train_team1 = bool(train_team1)
+        if continuing and self._train_team1 is not None and train_team1 != self._train_team1:
+            step = int(env.step_counts()[0])
+            if 0 < step < env.GAME_STEPS:
+                raise ValueError(f"train_team1 may change only between episodes: the envs are at step {step} of "
+                                 f"{env.GAME_STEPS}")
         if not isinstance(opponent, FusedPolicy):
             opponent = FusedPolicy(env, opponent)
         self.rollout = None
+        if continuing and self._train_team1 is None:
+            # the first episode starts here; collecting with reset=False records its end wherever it falls, even on
+            # the last step of this rollout
+            env.reset()
+            self._running_return = None
         ro = collect_rollout(env, self.fused, opponent, train_team1=train_team1, num_env_steps=T,
-                             obs_storage_dtype="packed")
+                             obs_storage_dtype="packed", reset=not continuing)
         mine = _team_indices(env, 0 if train_team1 else 1)
         apt, B = len(mine), env.num_envs
-        if T == env.GAME_STEPS:
+        if continuing:
+            v, _ = self.fused.forward_from_env(mine)          # env-major samples b*apt + j
+            ro.next_value = torch.where(ro.next_done.bool().unsqueeze(0), 0.0, v.reshape(B, apt).t()).contiguous()
+            ro.episode_stats = self._episode_stats(ro, train_team1)
+            self._train_team1 = train_team1
+        elif T == env.GAME_STEPS:
             ro.next_value = torch.zeros((apt, B), device=env.device)
         else:
             v, _ = self.fused.forward_from_env(mine)          # env-major samples b*apt + j
@@ -161,9 +214,33 @@ class PackedPPO:
         self.rollout = ro
         return ro
 
+    def _episode_stats(self, ro: Rollout, train_team1: bool) -> dict:
+        """Device tensors of the episodes that ended in ``ro``, with the return of every trained (agent, env) carried
+        from rollout to rollout in ``self._running_return`` (an episode spans several rollouts)."""
+        apt, B = ro.next_value.shape
+        r = ro.rewards.reshape(-1, apt, B)
+        run = self._running_return
+        if run is None or run.shape != (apt, B):   # the first rollout, or a team switch at an episode boundary
+            run = torch.zeros((apt, B), device=r.device)
+        me = 0 if train_team1 else 1
+        returns, outcomes, t0 = [], [], 0
+        for t, caps in ro.episode_ends:
+            returns.append(run + r[t0 : t + 1].sum(0))
+            outcomes.append(torch.sign(caps[:, me] - caps[:, 1 - me]))
+            run, t0 = torch.zeros_like(run), t + 1
+        self._running_return = run + r[t0:].sum(0)
+        nan = torch.tensor(float("nan"), device=r.device)
+        res = torch.stack(outcomes) if outcomes else None
+        return dict(episodes_completed=apt * B * len(returns),
+                    episode_return=torch.stack(returns).mean() if returns else nan,
+                    win_fraction=(res == 1).float().mean() if outcomes else nan,
+                    draw_fraction=(res == 0).float().mean() if outcomes else nan)
+
     def advantages(self, rollout: Rollout):
-        """(advantages, returns) fp32 [T*apt, B] of a rollout from ``collect``, with ``args.gamma`` / ``gae_lambda``."""
-        return advantages(self.env, rollout, rollout.next_value, self.args.gamma, self.args.gae_lambda)
+        """(advantages, returns) fp32 [T*apt, B] of a rollout from ``collect``, with ``args.gamma`` / ``gae_lambda``:
+        ``ctf_gae``, or in continuing mode ``ctf_gae_dones`` with the rollout's ``dones``."""
+        dones = rollout.dones if self.rollout_steps is not None else None
+        return advantages(self.env, rollout, rollout.next_value, self.args.gamma, self.args.gae_lambda, dones)
 
     def optimise(self, rollout: Rollout, adv: torch.Tensor, ret: torch.Tensor, generator=None) -> dict:
         """``update_epochs`` epochs over the rollout's T*apt*B samples, each a ``torch.randperm`` (drawn with
@@ -177,7 +254,11 @@ class PackedPPO:
         Returns floats: ``v_loss``, ``pg_loss``, ``entropy`` and ``approx_kl`` of the last minibatch, ``clipfrac``
         averaged over every minibatch, ``epochs_run``, and ``first_approx_kl`` / ``first_clipfrac`` of the first
         minibatch, taken before any step (the rollout's log-probs come from the bf16 inference head, the update's from
-        the fp32 heads of ``train_head``, so these are not exactly 0)."""
+        the fp32 heads of ``train_head``, so these are not exactly 0).  A rollout collected in continuing mode adds
+        ``episodes_completed`` (episodes ended inside it, counted per trained (agent, env)), ``episode_return`` (the
+        mean return of those episodes, including the rewards of earlier rollouts) and ``win_fraction`` /
+        ``draw_fraction`` of the trained team over those episodes' envs (from ``env.flag_captures()`` at the last
+        step); the last three are NaN when no episode ended."""
         args, env, fp = self.args, self.env, self.fused
         dev = env.device
         bits = rollout.grid_states.reshape(-1, env.bits_words_per_agent)
@@ -214,12 +295,17 @@ class PackedPPO:
             if args.target_kl is not None and out["approx_kl"] > args.target_kl:
                 break
         fp.refresh()
-        return dict(v_loss=out["v_loss"], pg_loss=out["pg_loss"], entropy=out["entropy"], approx_kl=out["approx_kl"],
-                    clipfrac=sum(clipfracs) / len(clipfracs), epochs_run=epochs_run,
-                    first_approx_kl=first["approx_kl"], first_clipfrac=first["clipfrac"])
+        res = dict(v_loss=out["v_loss"], pg_loss=out["pg_loss"], entropy=out["entropy"], approx_kl=out["approx_kl"],
+                   clipfrac=sum(clipfracs) / len(clipfracs), epochs_run=epochs_run,
+                   first_approx_kl=first["approx_kl"], first_clipfrac=first["clipfrac"])
+        stats = getattr(rollout, "episode_stats", None)
+        if stats is not None:
+            res.update({k: x if isinstance(x, int) else float(x) for k, x in stats.items()})
+        return res
 
     def update(self, opponent, train_team1=True) -> dict:
-        """One PPO update: ``collect`` (one episode of every env) -> ``advantages`` -> ``optimise``."""
+        """One PPO update: ``collect`` (one episode of every env, or ``rollout_steps`` steps in continuing mode) ->
+        ``advantages`` -> ``optimise``."""
         ro = self.collect(opponent, train_team1)
         adv, ret = self.advantages(ro)
         return self.optimise(ro, adv, ret)

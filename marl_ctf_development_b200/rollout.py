@@ -18,7 +18,7 @@ is accepted when every policy on it is fused.
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 
 import torch
 
@@ -35,13 +35,17 @@ class Rollout:
     use_action_mask: torch.Tensor  # [T*apt, B]
     logprobs: torch.Tensor         # [T*apt, B]
     rewards: torch.Tensor          # [T*apt, B]
-    dones: torch.Tensor            # [T*apt, B]  (never written by the reference, ppo.py:53 — kept zero)
+    dones: torch.Tensor            # [T*apt, B]  (never written by the reference, ppo.py:53 — zero unless reset=False:
+                                   # 1 on the rows of an observation that starts a new episode, CleanRL's convention)
     values: torch.Tensor           # [T*apt, B]
     next_grid_state: torch.Tensor  # [B, C, G, G]
     next_metadata_state: torch.Tensor  # [B, M]
     next_done: torch.Tensor        # [B]
     packed: bool = False
     next_value: torch.Tensor | None = None  # [apt, B] bootstrap V(s_T) per (agent, env), set by ppo.PackedPPO.collect
+    # reset=False: (t, env.flag_captures() [B, 2] read after step t) for every step t at which the episodes ended
+    episode_ends: list = field(default_factory=list)
+    episode_stats: dict | None = None  # episodes ended in this rollout, set by ppo.PackedPPO.collect in continuing mode
 
     def as_reference_arrays(self):
         """The eleven values ``train_ppo`` keeps per update (ppo.py:298-305, 362-376), in the reference's order.
@@ -86,12 +90,21 @@ def batched_action(policy, grid, meta, use_action_mask) -> torch.Tensor:
 
 
 @torch.no_grad()
-def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, obs_storage_dtype=torch.float32) -> Rollout:
+def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, obs_storage_dtype=torch.float32,
+                    reset=True) -> Rollout:
     """One rollout of every env (ppo.py:31-131).  ``train_team1=True`` trains team 0 (ppo.py:274-279).
 
     num_env_steps defaults to GAME_STEPS (one episode per rollout, as num_steps == GAME_STEPS in every
     experiment).  obs_storage_dtype=torch.uint8 stores the {0,1} observations 4x smaller; obs_storage_dtype="packed"
     stores the kernel's 1-bit-per-element copy (env created with packed_obs=True), 32x smaller than float32.
+
+    ``reset=True`` starts every env from ``env.reset()`` (ppo.py:57) and leaves ``dones`` zero.  ``reset=False``
+    continues from the env's current state, so a rollout may be shorter than an episode or cross one: the envs must be
+    in lock-step (one ``env.step_counts()`` read on entry; unequal counts raise ValueError).  When a step reaches
+    ``GAME_STEPS`` its rewards are recorded as usual, ``episode_ends`` gets (t, ``env.flag_captures()``), and
+    ``env.reset()`` runs before the next policy call, whose rows get ``dones = 1``.  An env already at ``GAME_STEPS`` on
+    entry (the previous rollout ended the episode) is reset first and row 0 gets ``dones = 1``; an env never reset is
+    reset first.  ``next_done`` marks a last step that ended the episode.
     """
     _require_folded_reversal(env)
     team = 0 if train_team1 else 1
@@ -123,7 +136,20 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
         values=torch.zeros((T * apt, B), device=dev),
         next_grid_state=torch.empty(0), next_metadata_state=torch.empty(0), next_done=torch.empty(0), packed=packed,
     )
-    obs, meta, _ = env.reset()                                                    # ppo.py:57
+    step = 0
+    if reset or env._first:
+        obs, meta, _ = env.reset()                                                # ppo.py:57
+    else:
+        lo, hi = torch.aminmax(env.step_counts())
+        step, hi = int(lo), int(hi)
+        if step != hi:
+            raise ValueError(f"reset=False continues envs in lock-step, but their step counts range from {step} to {hi}")
+        if step >= env.GAME_STEPS:
+            obs, meta, _ = env.reset()
+            out.dones[:apt] = 1
+            step = 0
+        else:
+            obs, meta = env.obs, env.meta
     actions = torch.empty((B, N), dtype=torch.uint8, device=dev)
     for t in range(T):
         sl = slice(t * apt, (t + 1) * apt)
@@ -163,6 +189,13 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
             actions[:, theirs_t] = ao.reshape(B, k).to(torch.uint8)
         obs, meta, rewards, dones, _ = env.step(actions)                          # ppo.py:98
         out.rewards[sl] = rewards[:, mine_t].t()                                  # ppo.py:106-109
+        step += 1
+        if not reset and step >= env.GAME_STEPS:
+            out.episode_ends.append((t, env.flag_captures().clone()))
+            if t + 1 < T:
+                obs, meta, _ = env.reset()
+                out.dones[(t + 1) * apt : (t + 2) * apt] = 1
+                step = 0
     first = min(mine)
     if obs is None:                                                               # packed-only env
         out.next_grid_state = env.unpack_obs(env.obs_bits[:, first])
