@@ -251,7 +251,8 @@ int ctf_step_host(ctf_handle_t h, ctf_state_t state, const uint8_t* actions_host
 
 /*
  * Policy inference from packed observations (no reference counterpart: the reference feeds agent_network.Agent a dense
- * float32 grid).  Weights of the convolutional trunk of policy.CtfPolicy; all pointers are device memory.
+ * float32 grid).  Weights of the convolutional trunk of policy.CtfPolicy; all pointers are device memory, none null,
+ * conv1_w 16-byte, conv2_w 8-byte and the biases 4-byte aligned.
  */
 typedef struct ctf_policy_weights {
     const float* conv1_w;   /* [16][C][3][3] fp32 (conv1.weight as stored by torch) */

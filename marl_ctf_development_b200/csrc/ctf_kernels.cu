@@ -1944,34 +1944,24 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
     CTF_SET_SMEM((k_reset<T, false>), smem); CTF_SET_SMEM((k_reset<T, true>), smem); CTF_SET_SMEM((k_observe<T>), smem); \
     CTF_SET_SMEM((k_unpack<T>), smem)
     CTF_SET_SMEM_T(float); CTF_SET_SMEM_T(uint8_t); CTF_SET_SMEM_T(__half); CTF_SET_SMEM_T(__nv_bfloat16);
-    // k_policy_trunk needs at most 94 KB (G = 16, C = 14); the ceiling is per kernel, so it covers every plan
-    CTF_SET_SMEM(k_policy_trunk, 100 * 1024);
-    {
-        TrunkArgs ta;
-        trunk_layout(h->plan, ta, h->trunk_smem_bytes);
+    // A trunk kernel's dynamic shared memory ceiling (per kernel, so it covers every plan), then how many of its CTAs
+    // this plan's launch fits on the device at once (at least one per SM; no query without a trunk, G < 5)
+    auto trunk_ctas = [&](auto kernel, int threads, int ceiling, size_t smem_bytes) {
+        CTF_SET_SMEM(kernel, ceiling);
         int per_sm = 0;
         if (e == cudaSuccess && h->plan.G >= 5)
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk, kTrunkThreads, h->trunk_smem_bytes);
-        h->trunk_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
-    }
-    // k_policy_trunk_grouped: k_policy_trunk's shared-memory layout
-    CTF_SET_SMEM(k_policy_trunk_grouped, 100 * 1024);
-    {
-        int per_sm = 0;
-        if (e == cudaSuccess && h->plan.G >= 5)
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk_grouped, kTrunkThreads, h->trunk_smem_bytes);
-        h->grouped_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
-    }
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem_bytes);
+        return (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
+    };
+    TrunkArgs ta;
+    trunk_layout(h->plan, ta, h->trunk_smem_bytes);
+    TrunkBwdArgs ba;
+    trunk_bwd_layout(h->plan, ba, h->bwd_smem_bytes);
+    // k_policy_trunk needs at most 94 KB (G = 16, C = 14); k_policy_trunk_grouped has its shared-memory layout
+    h->trunk_ctas = trunk_ctas(k_policy_trunk, kTrunkThreads, 100 * 1024, h->trunk_smem_bytes);
+    h->grouped_ctas = trunk_ctas(k_policy_trunk_grouped, kTrunkThreads, 100 * 1024, h->trunk_smem_bytes);
     // k_policy_trunk_backward needs at most 46 KB (G = 16, C = 14)
-    CTF_SET_SMEM(k_policy_trunk_backward, 64 * 1024);
-    {
-        TrunkBwdArgs ba;
-        trunk_bwd_layout(h->plan, ba, h->bwd_smem_bytes);
-        int per_sm = 0;
-        if (e == cudaSuccess && h->plan.G >= 5)
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_trunk_backward, kBwdThreads, h->bwd_smem_bytes);
-        h->bwd_ctas = (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
-    }
+    h->bwd_ctas = trunk_ctas(k_policy_trunk_backward, kBwdThreads, 64 * 1024, h->bwd_smem_bytes);
 #undef CTF_SET_SMEM_T
 #undef CTF_SET_SMEM
     if (e != cudaSuccess) {
@@ -2165,26 +2155,53 @@ extern "C" int ctf_unpack_obs(ctf_handle_t h, const uint32_t* packed, void* out,
     return CTF_OK;
 }
 
+// The checks the three trunk entry points share.  `fn` names the entry point in the error messages.
+//
+// The plan has a trunk (G >= 5), the packed blocks are addressed with agents_per_env >= 1 and n_envs >= 0, and a
+// feature row holds 32*(G-4)^2 + M values with a stride that keeps its 16-byte stores aligned.
+static int check_trunk_geometry(const char* fn, const DevPlan& P, int64_t n_envs, int agents_per_env,
+                                int64_t feature_stride) {
+    if (P.G < 5) return fail(CTF_ERR_INVALID, "%s: the policy needs grid_size >= 5 (two valid 3x3 convolutions)", fn);
+    if (agents_per_env < 1) return fail(CTF_ERR_INVALID, "%s: agents_per_env must be >= 1", fn);
+    if (n_envs < 0) return fail(CTF_ERR_INVALID, "%s: negative n_envs", fn);
+    const long long k1 = 32LL * (P.G - 4) * (P.G - 4) + P.M;
+    if (feature_stride < k1 || (feature_stride & 7))
+        return fail(CTF_ERR_INVALID, "%s: feature_stride must be a multiple of 8 and >= 32*(G-4)^2 + M", fn);
+    return CTF_OK;
+}
+
+// 1..8 agent ids, each < agents_per_env; `k_name` is how the entry point calls k
+static int check_agent_ids(const char* fn, const char* k_name, const uint8_t* agent_ids, int k, int agents_per_env) {
+    if (k < 1 || k > CTF_MAX_AGENTS) return fail(CTF_ERR_INVALID, "%s: %s must be in 1..8", fn, k_name);
+    for (int j = 0; j < k; ++j)
+        if (agent_ids[j] >= agents_per_env) return fail(CTF_ERR_INVALID, "%s: an agent id is >= agents_per_env", fn);
+    return CTF_OK;
+}
+
+// No weight pointer is null, and the ones the kernel reads are aligned for its loads: conv1_w 16 bytes, the fp32
+// biases 4.  The forward kernels read conv2_w (8 bytes) and conv2_b; the backward reads conv1 only from `w` (its conv2
+// comes transposed, in a buffer of its own).
+static int check_trunk_weights(const char* fn, const ctf_policy_weights_t& w, bool reads_conv2) {
+    if (!w.conv1_w || !w.conv1_b || !w.conv2_w || !w.conv2_b) return fail(CTF_ERR_INVALID, "%s: null weight pointer", fn);
+    if ((reinterpret_cast<uintptr_t>(w.conv1_w) & 15) || (reinterpret_cast<uintptr_t>(w.conv1_b) & 3) ||
+        (reads_conv2 && ((reinterpret_cast<uintptr_t>(w.conv2_w) & 7) || (reinterpret_cast<uintptr_t>(w.conv2_b) & 3))))
+        return fail(CTF_ERR_INVALID, "%s: misaligned weights", fn);
+    return CTF_OK;
+}
+
 extern "C" int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uint32_t* packed, const float* meta,
                                    int64_t n_envs, int agents_per_env, const uint8_t* agent_ids, int k, void* features,
                                    int64_t feature_stride, void* stream) {
-    if (!h || !w || !packed || !meta || !agent_ids || !features) return fail(CTF_ERR_INVALID, "ctf_policy_features: null argument");
-    if (!w->conv1_w || !w->conv1_b || !w->conv2_w || !w->conv2_b)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features: null weight pointer");
+    const char* fn = "ctf_policy_features";
+    if (!h || !w || !packed || !meta || !agent_ids || !features) return fail(CTF_ERR_INVALID, "%s: null argument", fn);
     const DevPlan& P = h->plan;
-    if (P.G < 5) return fail(CTF_ERR_INVALID, "ctf_policy_features: the policy needs grid_size >= 5 (two valid 3x3 convolutions)");
-    if (k < 1 || k > CTF_MAX_AGENTS) return fail(CTF_ERR_INVALID, "ctf_policy_features: k must be in 1..8");
-    if (agents_per_env < 1) return fail(CTF_ERR_INVALID, "ctf_policy_features: agents_per_env must be >= 1");
-    if (n_envs < 0) return fail(CTF_ERR_INVALID, "ctf_policy_features: negative n_envs");
-    for (int j = 0; j < k; ++j)
-        if (agent_ids[j] >= agents_per_env) return fail(CTF_ERR_INVALID, "ctf_policy_features: an agent id is >= agents_per_env");
-    const long long k1 = 32LL * (P.G - 4) * (P.G - 4) + P.M;
-    if (feature_stride < k1 || (feature_stride & 7))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features: feature_stride must be a multiple of 8 and >= 32*(G-4)^2 + M");
-    if (reinterpret_cast<uintptr_t>(features) & 15) return fail(CTF_ERR_INVALID, "ctf_policy_features: features must be 16-byte aligned");
-    if ((reinterpret_cast<uintptr_t>(w->conv1_w) & 15) || (reinterpret_cast<uintptr_t>(w->conv2_w) & 7) ||
-        (reinterpret_cast<uintptr_t>(packed) & 3) || (reinterpret_cast<uintptr_t>(meta) & 3))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features: misaligned weights or inputs");
+    int rc = check_trunk_geometry(fn, P, n_envs, agents_per_env, feature_stride);
+    if (rc == CTF_OK) rc = check_agent_ids(fn, "k", agent_ids, k, agents_per_env);
+    if (rc == CTF_OK) rc = check_trunk_weights(fn, *w, true);
+    if (rc != CTF_OK) return rc;
+    if (reinterpret_cast<uintptr_t>(features) & 15) return fail(CTF_ERR_INVALID, "%s: features must be 16-byte aligned", fn);
+    if ((reinterpret_cast<uintptr_t>(packed) & 3) || (reinterpret_cast<uintptr_t>(meta) & 3))
+        return fail(CTF_ERR_INVALID, "%s: misaligned inputs", fn);
     const long long n = (long long)n_envs * k;
     if (n == 0) return CTF_OK;
     TrunkArgs A;
@@ -2208,23 +2225,19 @@ extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weig
                                            const ctf_policy_segment_t* segments, int n_segments, const uint32_t* packed,
                                            const float* meta, int64_t n_envs, int agents_per_env, void* features,
                                            int64_t feature_stride, int64_t n_rows, void* stream) {
-    if (!h || !weights || !segments || !packed || !meta || !features)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: null argument");
+    const char* fn = "ctf_policy_features_grouped";
+    if (!h || !weights || !segments || !packed || !meta || !features) return fail(CTF_ERR_INVALID, "%s: null argument", fn);
     const DevPlan& P = h->plan;
-    if (P.G < 5) return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: the policy needs grid_size >= 5 (two valid 3x3 convolutions)");
+    int rc = check_trunk_geometry(fn, P, n_envs, agents_per_env, feature_stride);
+    if (rc != CTF_OK) return rc;
     if (n_policies < 1 || n_policies > CTF_GROUPED_MAX_POLICIES)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: n_policies must be in 1..CTF_GROUPED_MAX_POLICIES (64)");
+        return fail(CTF_ERR_INVALID, "%s: n_policies must be in 1..CTF_GROUPED_MAX_POLICIES (64)", fn);
     if (n_segments < 1 || n_segments > CTF_GROUPED_MAX_SEGMENTS)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: n_segments must be in 1..CTF_GROUPED_MAX_SEGMENTS (512)");
-    if (agents_per_env < 1) return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: agents_per_env must be >= 1");
-    if (n_envs < 0 || n_rows < 0) return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: negative n_envs or n_rows");
-    const long long k1 = 32LL * (P.G - 4) * (P.G - 4) + P.M;
-    if (feature_stride < k1 || (feature_stride & 7))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: feature_stride must be a multiple of 8 and >= 32*(G-4)^2 + M");
-    if (reinterpret_cast<uintptr_t>(features) & 15)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: features must be 16-byte aligned");
+        return fail(CTF_ERR_INVALID, "%s: n_segments must be in 1..CTF_GROUPED_MAX_SEGMENTS (512)", fn);
+    if (n_rows < 0) return fail(CTF_ERR_INVALID, "%s: negative n_rows", fn);
+    if (reinterpret_cast<uintptr_t>(features) & 15) return fail(CTF_ERR_INVALID, "%s: features must be 16-byte aligned", fn);
     if ((reinterpret_cast<uintptr_t>(packed) & 3) || (reinterpret_cast<uintptr_t>(meta) & 3))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: misaligned inputs");
+        return fail(CTF_ERR_INVALID, "%s: misaligned inputs", fn);
     // the argument block is large (about 26 KB): keep it off the caller's stack
     static thread_local TrunkGroupedArgs A;
     memset(&A, 0, sizeof(A));
@@ -2232,11 +2245,7 @@ extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weig
     trunk_layout(P, A.geo, smem);
     for (int p = 0; p < n_policies; ++p) {
         const ctf_policy_weights_t& w = weights[p];
-        if (!w.conv1_w || !w.conv1_b || !w.conv2_w || !w.conv2_b)
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: null weight pointer");
-        if ((reinterpret_cast<uintptr_t>(w.conv1_w) & 15) || (reinterpret_cast<uintptr_t>(w.conv2_w) & 7) ||
-            (reinterpret_cast<uintptr_t>(w.conv1_b) & 3) || (reinterpret_cast<uintptr_t>(w.conv2_b) & 3))
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: misaligned weights");
+        if ((rc = check_trunk_weights(fn, w, true)) != CTF_OK) return rc;
         A.w[p].conv1_w = w.conv1_w; A.w[p].conv1_b = w.conv1_b;
         A.w[p].conv2_w = static_cast<const uint2*>(w.conv2_w); A.w[p].conv2_b = w.conv2_b;
     }
@@ -2246,17 +2255,13 @@ extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weig
     for (int i = 0; i < n_segments; ++i) {
         const ctf_policy_segment_t& g = segments[i];
         if (g.policy < 0 || g.policy >= n_policies)
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's policy index is out of range");
-        if (g.k < 1 || g.k > CTF_MAX_AGENTS)
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's k must be in 1..8");
-        for (int j = 0; j < g.k; ++j)
-            if (g.agent_ids[j] >= agents_per_env)
-                return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: an agent id is >= agents_per_env");
+            return fail(CTF_ERR_INVALID, "%s: a segment's policy index is out of range", fn);
+        if ((rc = check_agent_ids(fn, "a segment's k", g.agent_ids, g.k, agents_per_env)) != CTF_OK) return rc;
         if (g.env_begin < 0 || g.n_envs < 0 || g.env_begin > n_envs || g.n_envs > n_envs - g.env_begin)
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's env range is outside [0, n_envs)");
+            return fail(CTF_ERR_INVALID, "%s: a segment's env range is outside [0, n_envs)", fn);
         const long long ns = g.n_envs * g.k;
         if (g.out_row < 0 || g.out_row > n_rows || ns > n_rows - g.out_row)
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: a segment's output rows are outside [0, n_rows)");
+            return fail(CTF_ERR_INVALID, "%s: a segment's output rows are outside [0, n_rows)", fn);
         TrunkSegment& S = A.seg[i];
         S.blk_begin = g.env_begin * agents_per_env;
         S.row_begin = g.out_row;
@@ -2272,7 +2277,7 @@ extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weig
     std::sort(order, order + n_busy, [&](int a, int b) { return A.seg[a].row_begin < A.seg[b].row_begin; });
     for (int i = 1; i < n_busy; ++i)
         if (A.seg[order[i - 1]].row_begin + A.seg[order[i - 1]].n_samples > A.seg[order[i]].row_begin)
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_grouped: the output rows of two segments overlap");
+            return fail(CTF_ERR_INVALID, "%s: the output rows of two segments overlap", fn);
     if (tiles == 0) return CTF_OK;
     A.geo.packed = packed; A.geo.meta = meta; A.geo.features = static_cast<__nv_bfloat16*>(features);
     A.geo.stride = feature_stride; A.geo.ape = agents_per_env;
@@ -2306,34 +2311,26 @@ extern "C" int ctf_policy_features_backward(ctf_handle_t h, const ctf_policy_wei
                                             const uint8_t* agent_ids, int k, const void* features,
                                             const void* grad_features, int64_t feature_stride, void* workspace,
                                             size_t workspace_bytes, const ctf_policy_grads_t* grads, void* stream) {
+    const char* fn = "ctf_policy_features_backward";
     if (!h || !w || !conv2_w_t || !packed || !agent_ids || !features || !grad_features || !workspace || !grads)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: null argument");
-    if (!w->conv1_w || !w->conv1_b || !w->conv2_w || !w->conv2_b)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: null weight pointer");
+        return fail(CTF_ERR_INVALID, "%s: null argument", fn);
     if (!grads->conv1_w || !grads->conv1_b || !grads->conv2_w || !grads->conv2_b)
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: null gradient pointer");
+        return fail(CTF_ERR_INVALID, "%s: null gradient pointer", fn);
     const DevPlan& P = h->plan;
-    if (P.G < 5) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: the policy needs grid_size >= 5 (two valid 3x3 convolutions)");
-    if (k < 1 || k > CTF_MAX_AGENTS) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: k must be in 1..8");
-    if (agents_per_env < 1) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: agents_per_env must be >= 1");
-    if (n_envs < 0) return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: negative n_envs");
-    for (int j = 0; j < k; ++j)
-        if (agent_ids[j] >= agents_per_env)
-            return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: an agent id is >= agents_per_env");
-    const long long k1 = 32LL * (P.G - 4) * (P.G - 4) + P.M;
-    if (feature_stride < k1 || (feature_stride & 7))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: feature_stride must be a multiple of 8 and >= 32*(G-4)^2 + M");
+    int rc = check_trunk_geometry(fn, P, n_envs, agents_per_env, feature_stride);
+    if (rc == CTF_OK) rc = check_agent_ids(fn, "k", agent_ids, k, agents_per_env);
+    if (rc == CTF_OK) rc = check_trunk_weights(fn, *w, false);
+    if (rc != CTF_OK) return rc;
     if ((reinterpret_cast<uintptr_t>(features) & 15) || (reinterpret_cast<uintptr_t>(grad_features) & 15))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: features and grad_features must be 16-byte aligned");
-    if ((reinterpret_cast<uintptr_t>(w->conv1_w) & 15) || (reinterpret_cast<uintptr_t>(conv2_w_t) & 7) ||
-        (reinterpret_cast<uintptr_t>(w->conv1_b) & 3) || (reinterpret_cast<uintptr_t>(packed) & 3) ||
+        return fail(CTF_ERR_INVALID, "%s: features and grad_features must be 16-byte aligned", fn);
+    if ((reinterpret_cast<uintptr_t>(conv2_w_t) & 7) || (reinterpret_cast<uintptr_t>(packed) & 3) ||
         (reinterpret_cast<uintptr_t>(workspace) & 15) || (reinterpret_cast<uintptr_t>(grads->conv1_w) & 3) ||
         (reinterpret_cast<uintptr_t>(grads->conv1_b) & 3) || (reinterpret_cast<uintptr_t>(grads->conv2_w) & 3) ||
         (reinterpret_cast<uintptr_t>(grads->conv2_b) & 3))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: misaligned weights, inputs, workspace or gradients");
+        return fail(CTF_ERR_INVALID, "%s: misaligned conv2_w_t, inputs, workspace or gradients", fn);
     const int n_grad = grad_count(P.C);
     if (workspace_bytes < (size_t)h->bwd_ctas * n_grad * sizeof(float))
-        return fail(CTF_ERR_INVALID, "ctf_policy_features_backward: workspace smaller than ctf_policy_grad_workspace_size");
+        return fail(CTF_ERR_INVALID, "%s: workspace smaller than ctf_policy_grad_workspace_size", fn);
     const long long n = (long long)n_envs * k;
     TrunkBwdArgs A;
     memset(&A, 0, sizeof(A));

@@ -152,22 +152,111 @@ def reference_trunk_grads(policy, dense_obs: torch.Tensor, grad_rows: torch.Tens
                 dz2.sum((0, 2, 3)))
 
 
-def _check_policy(env, policy):
-    """Raises ValueError unless ``policy`` has the layer shapes of a CtfPolicy for ``env`` and lives on its device."""
+def _check_policies(env, policies):
+    """(K1, stride) of ``env``'s trunk (``trunk_dims``).  Raises ValueError unless the env has G >= 5 and every policy
+    has the layer shapes of a CtfPolicy for ``env`` and lives on its device."""
     Cn, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
-    k1 = trunk_dims(Cn, G, M)[0]
+    if G < 5:
+        raise ValueError(f"the policy needs GRID_SIZE >= 5 (two valid 3x3 convolutions), env has {G}")
+    k1, stride = trunk_dims(Cn, G, M)
     want = {
         "conv1.weight": (16, Cn, 3, 3), "conv2.weight": (32, 16, 3, 3), "fc1.weight": (256, k1),
         "fc2.weight": (128, 256), "action_head.weight": (N_ACTIONS, 128), "value_head.weight": (1, 128),
     }
-    for name, shape in want.items():
-        mod, attr = name.split(".")
-        got = tuple(getattr(getattr(policy, mod, None), attr, torch.empty(0)).shape)
-        if got != shape:
-            raise ValueError(f"policy {name} has shape {got}; this env (C={Cn}, G={G}, M={M}, {N_ACTIONS} actions) "
-                             f"needs {shape}")
-    if policy.conv1.weight.device != env.device:
-        raise ValueError(f"policy is on {policy.conv1.weight.device}, env on {env.device}")
+    for policy in policies:
+        for name, shape in want.items():
+            mod, attr = name.split(".")
+            got = tuple(getattr(getattr(policy, mod, None), attr, torch.empty(0)).shape)
+            if got != shape:
+                raise ValueError(f"policy {name} has shape {got}; this env (C={Cn}, G={G}, M={M}, {N_ACTIONS} actions) "
+                                 f"needs {shape}")
+        if policy.conv1.weight.device != env.device:
+            raise ValueError(f"policy is on {policy.conv1.weight.device}, env on {env.device}")
+    return k1, stride
+
+
+def _check_agent_ids(agent_ids, n_per_env, where=""):
+    """``agent_ids`` (a sequence or tensor) as a tuple of ints; raises ValueError (message prefixed by ``where``) unless
+    it names 1..MAX_IDS agents, each in [0, n_per_env)."""
+    ids = tuple(int(i) for i in (agent_ids.tolist() if isinstance(agent_ids, torch.Tensor) else agent_ids))
+    if not 1 <= len(ids) <= MAX_IDS:
+        raise ValueError(f"{where}agent ids must name 1..{MAX_IDS} agents, got {len(ids)}")
+    if any(i < 0 or i >= n_per_env for i in ids):
+        raise ValueError(f"{where}agent ids {ids} out of range for {n_per_env} agents per env")
+    return ids
+
+
+def _check_packed(env, bits, meta):
+    """Raises ValueError unless ``bits`` is int32 [S, wpa] and ``meta`` float32 [S, M] on ``env``'s device."""
+    wpa, M = env.bits_words_per_agent, env.meta_size
+    if bits.dtype != torch.int32 or bits.dim() != 2 or bits.shape[1] != wpa or bits.device != env.device:
+        raise ValueError(f"bits must be an int32 tensor [S, {wpa}] on {env.device}")
+    if meta.dtype != torch.float32 or tuple(meta.shape) != (bits.shape[0], M) or meta.device != env.device:
+        raise ValueError(f"meta must be a float32 tensor [{bits.shape[0]}, {M}] on {env.device}")
+
+
+def _trunk_forward(env, weights, packed_ptr, meta_ptr, n_envs, agents_per_env, ids, k, out, stride):
+    """Runs ``ctf_policy_features`` on the current stream with ``weights`` (``C.byref`` of a ``CtfPolicyWeights``) into
+    ``out``, bf16 [n_envs * k, stride]; returns ``out``."""
+    stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
+    _native.check(env._lib.ctf_policy_features(
+        env._handle, weights, C.c_void_p(packed_ptr), C.c_void_p(meta_ptr), n_envs, agents_per_env, ids, k,
+        C.c_void_p(out.data_ptr()), stride, stream))
+    return out
+
+
+class _TrunkWeights:
+    """The conv weights of L policies in the layouts the trunk kernels read, one slot per policy: conv1.weight and the
+    biases fp32, conv2.weight bf16 gathered by ``conv2_kernel_layout_index`` and, with ``transposed`` (the backward),
+    also by ``conv2_transpose_layout_index`` into ``c2wt``.  ``native`` is the ``CtfPolicyWeights`` array over the
+    slots.  ``load`` copies into the buffers in place, so the pointers (and CUDA graphs captured around them) stay."""
+
+    def __init__(self, L, n_channels, device, transposed=False):
+        f32, bf = dict(dtype=torch.float32, device=device), dict(dtype=torch.bfloat16, device=device)
+        self.c1w = torch.empty((L, 16, n_channels, 3, 3), **f32)
+        self.c1b = torch.empty((L, 16), **f32)
+        self.c2w = torch.empty((L, 9 * 4 * 32 * 4), **bf)
+        self.c2b = torch.empty((L, 32), **f32)
+        self._c2_index = conv2_kernel_layout_index(device)
+        self.c2wt = torch.empty((L, 9 * 2 * 2 * 32 * 4), **bf) if transposed else None
+        self._c2t_index = conv2_transpose_layout_index(device) if transposed else None
+        self.native = (_native.CtfPolicyWeights * L)(*(
+            _native.CtfPolicyWeights(self.c1w[p].data_ptr(), self.c1b[p].data_ptr(), self.c2w[p].data_ptr(),
+                                     self.c2b[p].data_ptr()) for p in range(L)))
+
+    @torch.no_grad()
+    def load(self, slot, w1, b1, w2, b2):
+        self.c1w[slot].copy_(w1)
+        self.c1b[slot].copy_(b1)
+        w2 = w2.reshape(-1)
+        self.c2w[slot].copy_(w2[self._c2_index])
+        if self.c2wt is not None:
+            self.c2wt[slot].copy_(w2[self._c2t_index])
+        self.c2b[slot].copy_(b2)
+
+
+class _HeadWeights:
+    """bf16 copies of the fc1, fc2 and value | action head layers of L policies, one slot per policy: fc1.weight in
+    columns :K1 of [256, stride], zeros after (a K that is a multiple of 8 keeps cuBLAS on its aligned kernel; the pad
+    columns of the feature rows are zeros too), fc2 [128, 256], the value and action heads stacked as [1 + 9, 128]."""
+
+    def __init__(self, L, k1, stride, device):
+        bf = dict(dtype=torch.bfloat16, device=device)
+        self.k1 = k1
+        self.fc1w, self.fc1b = torch.zeros((L, 256, stride), **bf), torch.empty((L, 256), **bf)
+        self.fc2w, self.fc2b = torch.empty((L, 128, 256), **bf), torch.empty((L, 128), **bf)
+        self.hw, self.hb = torch.empty((L, 1 + N_ACTIONS, 128), **bf), torch.empty((L, 1 + N_ACTIONS), **bf)
+
+    @torch.no_grad()
+    def load(self, slot, policy):
+        self.fc1w[slot, :, : self.k1].copy_(policy.fc1.weight)
+        self.fc1b[slot].copy_(policy.fc1.bias)
+        self.fc2w[slot].copy_(policy.fc2.weight)
+        self.fc2b[slot].copy_(policy.fc2.bias)
+        self.hw[slot, :1].copy_(policy.value_head.weight)
+        self.hw[slot, 1:].copy_(policy.action_head.weight)
+        self.hb[slot, :1].copy_(policy.value_head.bias)
+        self.hb[slot, 1:].copy_(policy.action_head.bias)
 
 
 class _PackedTrunk(torch.autograd.Function):
@@ -197,45 +286,24 @@ class FusedPolicy:
 
     def __init__(self, env, policy):
         self.env, self.policy = env, policy
-        Cn, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
-        if G < 5:
-            raise ValueError(f"the policy needs GRID_SIZE >= 5 (two valid 3x3 convolutions), env has {G}")
-        self.k1, self.stride = trunk_dims(Cn, G, M)
-        _check_policy(env, policy)
-        dev = env.device
-        bf = dict(dtype=torch.bfloat16, device=dev)
-        self._c1w = torch.empty((16, Cn, 3, 3), dtype=torch.float32, device=dev)
-        self._c1b = torch.empty(16, dtype=torch.float32, device=dev)
-        self._c2w = torch.empty(9 * 4 * 32 * 4, **bf)
-        self._c2b = torch.empty(32, dtype=torch.float32, device=dev)
-        self._c2_index = conv2_kernel_layout_index(dev)
-        # fc1.weight in columns :K1, zeros up to the row stride
-        self._fc1w, self._fc1b = torch.zeros((256, self.stride), **bf), torch.empty(256, **bf)
-        self._fc2w, self._fc2b = torch.empty((128, 256), **bf), torch.empty(128, **bf)
-        self._hw, self._hb = torch.empty((1 + N_ACTIONS, 128), **bf), torch.empty(1 + N_ACTIONS, **bf)  # value | logits
-        self._weights = _native.CtfPolicyWeights(self._c1w.data_ptr(), self._c1b.data_ptr(), self._c2w.data_ptr(),
-                                                 self._c2b.data_ptr())
+        self.k1, self.stride = _check_policies(env, [policy])
+        self._trunk_w = _TrunkWeights(1, env.n_channels, env.device)
+        self._weights = self._trunk_w.native[0]     # the CtfPolicyWeights of the one slot, what the trunk reads
+        self._head_w = _HeadWeights(1, self.k1, self.stride, env.device)
+        # the one slot's 2-D views, what _head passes to F.linear (value | logits heads stacked)
+        hw = self._head_w
+        self._fc1w, self._fc1b, self._fc2w, self._fc2b, self._hw, self._hb = (
+            t[0] for t in (hw.fc1w, hw.fc1b, hw.fc2w, hw.fc2b, hw.hw, hw.hb))
         self._features = None   # bf16 [S_max, stride] rows, reused by every call (see features())
         self._ids = {}
         self._train = None      # training-only weight buffers and workspace, created by the first evaluate_actions
         self.refresh()
 
-    @torch.no_grad()
     def refresh(self):
         """Copies the policy's current weights into the persistent buffers, on the device (no host round trip)."""
         p = self.policy
-        self._c1w.copy_(p.conv1.weight)
-        self._c1b.copy_(p.conv1.bias)
-        self._c2w.copy_(p.conv2.weight.reshape(-1)[self._c2_index])
-        self._c2b.copy_(p.conv2.bias)
-        self._fc1w[:, : self.k1].copy_(p.fc1.weight)
-        self._fc1b.copy_(p.fc1.bias)
-        self._fc2w.copy_(p.fc2.weight)
-        self._fc2b.copy_(p.fc2.bias)
-        self._hw[:1].copy_(p.value_head.weight)
-        self._hw[1:].copy_(p.action_head.weight)
-        self._hb[:1].copy_(p.value_head.bias)
-        self._hb[1:].copy_(p.action_head.bias)
+        self._trunk_w.load(0, p.conv1.weight, p.conv1.bias, p.conv2.weight, p.conv2.bias)
+        self._head_w.load(0, p)
 
     # ------------------------------------------------------------------ plumbing
     def _env_for(self, env):
@@ -247,11 +315,7 @@ class FusedPolicy:
         return env
 
     def _id_array(self, agent_ids, n_per_env):
-        ids = tuple(int(i) for i in (agent_ids.tolist() if isinstance(agent_ids, torch.Tensor) else agent_ids))
-        if not 1 <= len(ids) <= MAX_IDS:
-            raise ValueError(f"agent_ids must name 1..{MAX_IDS} agents, got {len(ids)}")
-        if any(i < 0 or i >= n_per_env for i in ids):
-            raise ValueError(f"agent_ids {ids} out of range for {n_per_env} agents per env")
+        ids = _check_agent_ids(agent_ids, n_per_env)
         arr = self._ids.get(ids)
         if arr is None:
             arr = self._ids[ids] = (C.c_uint8 * len(ids))(*ids)
@@ -265,14 +329,6 @@ class FusedPolicy:
             self._features = None   # release the old rows before allocating the larger ones
             self._features = torch.empty((n_samples, self.stride), dtype=torch.bfloat16, device=self.env.device)
         return self._features[:n_samples]
-
-    def _trunk(self, env, packed_ptr, meta_ptr, n_envs, agents_per_env, ids, k):
-        feat = self.features(n_envs * k)
-        stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
-        _native.check(env._lib.ctf_policy_features(
-            env._handle, C.byref(self._weights), C.c_void_p(packed_ptr), C.c_void_p(meta_ptr), n_envs, agents_per_env,
-            ids, k, C.c_void_p(feat.data_ptr()), self.stride, stream))
-        return feat
 
     def _head(self, feat):
         x = torch.tanh(F.linear(feat, self._fc1w, self._fc1b))
@@ -294,20 +350,17 @@ class FusedPolicy:
         if step != 1 or e1 < e0:
             raise ValueError("envs must be a contiguous slice of env indices")
         ids, k = self._id_array(agent_ids, N)
-        return self._trunk(env, env.obs_bits.data_ptr() + e0 * N * wpa * 4, env.meta.data_ptr() + e0 * N * M * 4,
-                           e1 - e0, N, ids, k)
+        return _trunk_forward(env, C.byref(self._weights), env.obs_bits.data_ptr() + e0 * N * wpa * 4,
+                              env.meta.data_ptr() + e0 * N * M * 4, e1 - e0, N, ids, k, self.features((e1 - e0) * k),
+                              self.stride)
 
     def trunk_packed(self, bits: torch.Tensor, meta: torch.Tensor) -> torch.Tensor:
         """Feature rows (as ``trunk_from_env``) for packed observations ``bits`` int32 [S, wpa] and ``meta`` [S, M]."""
-        env = self.env
-        wpa, M = env.bits_words_per_agent, env.meta_size
-        if bits.dtype != torch.int32 or bits.dim() != 2 or bits.shape[1] != wpa or bits.device != env.device:
-            raise ValueError(f"bits must be an int32 tensor [S, {wpa}] on {env.device}")
-        if meta.dtype != torch.float32 or tuple(meta.shape) != (bits.shape[0], M) or meta.device != env.device:
-            raise ValueError(f"meta must be a float32 tensor [{bits.shape[0]}, {M}] on {env.device}")
+        _check_packed(self.env, bits, meta)
         bits, meta = bits.contiguous(), meta.contiguous()
         ids, _ = self._id_array((0,), 1)
-        return self._trunk(env, bits.data_ptr(), meta.data_ptr(), bits.shape[0], 1, ids, 1)
+        return _trunk_forward(self.env, C.byref(self._weights), bits.data_ptr(), meta.data_ptr(), bits.shape[0], 1, ids,
+                              1, self.features(bits.shape[0]), self.stride)
 
     @torch.no_grad()
     def forward_from_env(self, agent_ids, env=None, envs=None):
@@ -356,7 +409,7 @@ class FusedPolicy:
         fp32 parameters (fc1.weight zero-padded to the row stride as in inference); the small heads run in fp32
         (``train_head``).  Between forward and backward each sample holds 2 x stride bf16 values (rows and their
         gradient); split large minibatches into chunks and accumulate gradients over them."""
-        self._check_packed(bits, meta)
+        _check_packed(self.env, bits, meta)
         p = self.policy
         rows = _PackedTrunk.apply(bits.contiguous(), p.conv1.weight, p.conv1.bias, p.conv2.weight, p.conv2.bias, self,
                                   meta.contiguous())
@@ -377,60 +430,34 @@ class FusedPolicy:
         out = F.linear(x.float(), hw, torch.cat((p.value_head.bias, p.action_head.bias)))
         return out[:, :1], out[:, 1:]
 
-    def _check_packed(self, bits, meta):
-        env = self.env
-        wpa, M = env.bits_words_per_agent, env.meta_size
-        if bits.dtype != torch.int32 or bits.dim() != 2 or bits.shape[1] != wpa or bits.device != env.device:
-            raise ValueError(f"bits must be an int32 tensor [S, {wpa}] on {env.device}")
-        if meta.dtype != torch.float32 or tuple(meta.shape) != (bits.shape[0], M) or meta.device != env.device:
-            raise ValueError(f"meta must be a float32 tensor [{bits.shape[0]}, {M}] on {env.device}")
-
     def _train_state(self):
+        """The training-only buffers, created by the first call and separate from the inference buffers, which only
+        ``refresh()`` changes: ``trunk``, a one-slot ``_TrunkWeights`` with the transposed conv2; ``weights`` and
+        ``c2wt``, its slot's ``CtfPolicyWeights`` and transposed conv2 as the trunk kernels read them; ``workspace``,
+        the backward's partial gradient sums."""
         if self._train is None:
-            env, dev = self.env, self.env.device
-            Cn = env.n_channels
-            tr = dict(
-                c1w=torch.empty((16, Cn, 3, 3), dtype=torch.float32, device=dev),
-                c1b=torch.empty(16, dtype=torch.float32, device=dev),
-                c2w=torch.empty(9 * 4 * 32 * 4, dtype=torch.bfloat16, device=dev),
-                c2wt=torch.empty(9 * 2 * 2 * 32 * 4, dtype=torch.bfloat16, device=dev),
-                c2b=torch.empty(32, dtype=torch.float32, device=dev),
-                c2t_index=conv2_transpose_layout_index(dev),
-            )
-            tr["weights"] = _native.CtfPolicyWeights(tr["c1w"].data_ptr(), tr["c1b"].data_ptr(), tr["c2w"].data_ptr(),
-                                                     tr["c2b"].data_ptr())
+            env = self.env
             n = C.c_size_t()
             _native.check(env._lib.ctf_policy_grad_workspace_size(env._handle, C.byref(n)))
-            tr["workspace"] = torch.empty(max(n.value // 4, 4), dtype=torch.float32, device=dev)
-            self._train = tr
+            tw = _TrunkWeights(1, env.n_channels, env.device, transposed=True)
+            self._train = dict(trunk=tw, weights=tw.native[0], c2wt=tw.c2wt[0],
+                               workspace=torch.empty(max(n.value // 4, 4), dtype=torch.float32, device=env.device))
         return self._train
 
-    @torch.no_grad()
-    def _load_train_weights(self, w1, b1, w2, b2):
-        tr = self._train_state()
-        tr["c1w"].copy_(w1)
-        tr["c1b"].copy_(b1)
-        tr["c2w"].copy_(w2.reshape(-1)[self._c2_index])
-        tr["c2wt"].copy_(w2.reshape(-1)[tr["c2t_index"]])
-        tr["c2b"].copy_(b2)
-        return tr
-
     def _train_forward(self, bits, meta, w1, b1, w2, b2):
-        env = self.env
-        tr = self._load_train_weights(w1, b1, w2, b2)
-        rows = torch.empty((bits.shape[0], self.stride), dtype=torch.bfloat16, device=env.device)
+        tr = self._train_state()
+        tr["trunk"].load(0, w1, b1, w2, b2)
+        rows = torch.empty((bits.shape[0], self.stride), dtype=torch.bfloat16, device=self.env.device)
         if bits.shape[0] == 0:
             return rows
         ids, _ = self._id_array((0,), 1)
-        stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
-        _native.check(env._lib.ctf_policy_features(
-            env._handle, C.byref(tr["weights"]), C.c_void_p(bits.data_ptr()), C.c_void_p(meta.data_ptr()),
-            bits.shape[0], 1, ids, 1, C.c_void_p(rows.data_ptr()), self.stride, stream))
-        return rows
+        return _trunk_forward(self.env, C.byref(tr["weights"]), bits.data_ptr(), meta.data_ptr(), bits.shape[0], 1, ids,
+                              1, rows, self.stride)
 
     def _train_backward(self, bits, rows, grad_rows, w1, b1, w2, b2):
         env = self.env
-        tr = self._load_train_weights(w1, b1, w2, b2)
+        tr = self._train_state()
+        tr["trunk"].load(0, w1, b1, w2, b2)
         grad_rows = grad_rows.to(torch.bfloat16).contiguous()
         grads = [torch.empty_like(t, dtype=torch.float32) for t in (w1, b1, w2, b2)]
         gs = _native.CtfPolicyGrads(*(g.data_ptr() for g in grads))
@@ -491,9 +518,6 @@ class PolicyPool:
     """
 
     def __init__(self, env, policies):
-        Cn, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
-        if G < 5:
-            raise ValueError(f"the policy needs GRID_SIZE >= 5 (two valid 3x3 convolutions), env has {G}")
         mods = [p.policy if isinstance(p, FusedPolicy) else p for p in policies]
         if not mods:
             raise ValueError("a PolicyPool needs at least one policy")
@@ -501,44 +525,21 @@ class PolicyPool:
             raise ValueError(f"a PolicyPool holds at most {_native.GROUPED_MAX_POLICIES} policies, got {len(mods)}")
         if len({id(m) for m in mods}) != len(mods):
             raise ValueError("every policy may appear only once in a PolicyPool")
-        for m in mods:
-            _check_policy(env, m)
+        self.k1, self.stride = _check_policies(env, mods)
         self.env, self.policies = env, mods
-        self.k1, self.stride = trunk_dims(Cn, G, M)
-        L, dev = len(mods), env.device
-        bf = dict(dtype=torch.bfloat16, device=dev)
-        self._c1w = torch.empty((L, 16, Cn, 3, 3), dtype=torch.float32, device=dev)
-        self._c1b = torch.empty((L, 16), dtype=torch.float32, device=dev)
-        self._c2w = torch.empty((L, 9 * 4 * 32 * 4), **bf)
-        self._c2b = torch.empty((L, 32), dtype=torch.float32, device=dev)
-        self._c2_index = conv2_kernel_layout_index(dev)
-        self._fc1w, self._fc1b = torch.zeros((L, 256, self.stride), **bf), torch.empty((L, 256), **bf)
-        self._fc2w, self._fc2b = torch.empty((L, 128, 256), **bf), torch.empty((L, 128), **bf)
-        self._hw, self._hb = torch.empty((L, 1 + N_ACTIONS, 128), **bf), torch.empty((L, 1 + N_ACTIONS), **bf)
-        self._weights = (_native.CtfPolicyWeights * L)(*(
-            _native.CtfPolicyWeights(self._c1w[p].data_ptr(), self._c1b[p].data_ptr(), self._c2w[p].data_ptr(),
-                                     self._c2b[p].data_ptr()) for p in range(L)))
+        self._trunk_w = _TrunkWeights(len(mods), env.n_channels, env.device)
+        self._weights = self._trunk_w.native        # the grouped kernel's weight table, one entry per policy
+        self._head_w = _HeadWeights(len(mods), self.k1, self.stride, env.device)
         self.refresh()
 
     def __len__(self):
         return len(self.policies)
 
-    @torch.no_grad()
     def refresh(self):
         """Copies every policy's current weights into the stacked buffers, on the device (no host round trip)."""
         for p, m in enumerate(self.policies):
-            self._c1w[p].copy_(m.conv1.weight)
-            self._c1b[p].copy_(m.conv1.bias)
-            self._c2w[p].copy_(m.conv2.weight.reshape(-1)[self._c2_index])
-            self._c2b[p].copy_(m.conv2.bias)
-            self._fc1w[p, :, : self.k1].copy_(m.fc1.weight)
-            self._fc1b[p].copy_(m.fc1.bias)
-            self._fc2w[p].copy_(m.fc2.weight)
-            self._fc2b[p].copy_(m.fc2.bias)
-            self._hw[p, :1].copy_(m.value_head.weight)
-            self._hw[p, 1:].copy_(m.action_head.weight)
-            self._hb[p, :1].copy_(m.value_head.bias)
-            self._hb[p, 1:].copy_(m.action_head.bias)
+            self._trunk_w.load(p, m.conv1.weight, m.conv1.bias, m.conv2.weight, m.conv2.bias)
+            self._head_w.load(p, m)
 
     def _env_for(self, env):
         if env is None:
@@ -566,12 +567,7 @@ class PolicyPool:
             e0, e1, step = sl.indices(B)
             if step != 1 or e1 < e0:
                 raise ValueError(f"segment {i}: envs must be a contiguous slice of env indices")
-            ids = tuple(int(a) for a in (ids.tolist() if isinstance(ids, torch.Tensor) else ids))
-            if not 1 <= len(ids) <= MAX_IDS:
-                raise ValueError(f"segment {i}: agent ids must name 1..{MAX_IDS} agents, got {len(ids)}")
-            if any(a < 0 or a >= N for a in ids):
-                raise ValueError(f"segment {i}: agent ids {ids} out of range for {N} agents per env")
-            norm.append((pol, e0, e1, ids))
+            norm.append((pol, e0, e1, _check_agent_ids(ids, N, f"segment {i}: ")))
         n_samples = [0] * L
         seg_first_row = []
         for pol, e0, e1, ids in norm:            # rows of a policy: its segments in the order given
@@ -637,11 +633,11 @@ class PolicyPool:
     def head(self, plan: PoolPlan, feat: torch.Tensor | None = None):
         """(value [S, 1], logits [S, 9]) fp32 in plan order from the feature rows: fc1 -> tanh -> fc2 -> tanh -> heads
         as one bf16 ``torch.baddbmm`` chain over [L, s_max, .], then the plan's rows gathered."""
-        L = len(self.policies)
+        L, w = len(self.policies), self._head_w
         x = (plan.features if feat is None else feat).view(L, plan.s_max, self.stride)
-        x = torch.tanh(torch.baddbmm(self._fc1b.unsqueeze(1), x, self._fc1w.transpose(1, 2)))
-        x = torch.tanh(torch.baddbmm(self._fc2b.unsqueeze(1), x, self._fc2w.transpose(1, 2)))
-        out = torch.baddbmm(self._hb.unsqueeze(1), x, self._hw.transpose(1, 2)).view(L * plan.s_max, 1 + N_ACTIONS)
+        x = torch.tanh(torch.baddbmm(w.fc1b.unsqueeze(1), x, w.fc1w.transpose(1, 2)))
+        x = torch.tanh(torch.baddbmm(w.fc2b.unsqueeze(1), x, w.fc2w.transpose(1, 2)))
+        out = torch.baddbmm(w.hb.unsqueeze(1), x, w.hw.transpose(1, 2)).view(L * plan.s_max, 1 + N_ACTIONS)
         out = out.index_select(0, plan.row_index).float()
         return out[:, :1], out[:, 1:]
 

@@ -387,6 +387,8 @@ def test_bad_arguments_are_rejected():
     bad = [
         dict(k=0), dict(k=9), dict(ape=2), dict(st=k1), dict(st=stride - 8), dict(out=feat.data_ptr() + 2),
         dict(packed=0), dict(meta=0), dict(out=0), dict(ids=None), dict(weights=None),
+        dict(weights=C.byref(_native.CtfPolicyWeights(w.conv1_w, w.conv1_b + 2, w.conv2_w, w.conv2_b))),
+        dict(weights=C.byref(_native.CtfPolicyWeights(w.conv1_w, w.conv1_b, w.conv2_w, w.conv2_b + 2))),
     ]
     for kw in bad:
         assert call(**kw) == -1, kw
