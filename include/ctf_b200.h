@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 11
+#define CTF_ABI_VERSION 12
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -62,6 +62,8 @@ enum ctf_metric {
 #define CTF_FAULT_RESPAWN_BLOCKED 2u /* a lethal tag found no open cell in the victim's 3x3 spawn window: the
                                         reference raises ValueError from np.random.randint(0) (gridworld_ctf.py:771);
                                         here the victim stays where it is with HP <= 0 and the bit is set */
+#define CTF_FAULT_BAD_INDEX 4u       /* a row of ctf_sample_actions named a flat_index outside [0, B*N); the row
+                                        wrote nothing */
 
 enum ctf_error {
     CTF_OK = 0,
@@ -389,6 +391,34 @@ int ctf_gae(ctf_handle_t h, const float* rewards, const float* values, const flo
 int ctf_gae_dones(ctf_handle_t h, const float* rewards, const float* values, const float* dones, const float* next_value,
                   float* advantages, float* returns, int64_t n_steps, int64_t agents_per_step, int64_t n_envs,
                   float gamma, float gamma_lambda, void* stream);
+
+/*
+ * Seeded action sampling for policy rows (ABI 12): one categorical draw per row from the value | logits head output,
+ * with counter-based randomness like the env's, so that a rollout or duel is a function of its seeds alone.
+ * head: fp32 [n_rows][head_stride], column 0 the value (not read), columns 1..9 the logits.  masked: uint8 [n_rows] or
+ * NULL; a nonzero flag applies CtfPolicy.masked_logits (x_i += -1e9f for i >= 5, one fp32 add).  flat_index: int64
+ * [n_rows], env * N + agent of every row (env b = flat_index / N, agent a = flat_index % N, env b of this handle).
+ * Per row, with x the (masked) logits:
+ *   u = (w0 >> 8) * 2^-24, w0 = word 0 of Philox4x32-10 with key (seed & 0xffffffff, seed >> 32) and counter
+ *       (env_id_base + b, episode[b], env_step_count[b], 0x80000000 | a), the counts read from state.envs on the device
+ *       at launch (a captured CUDA graph draws fresh words at every replay; the site's top bit keeps these counters apart
+ *       from the env's sites 0..31 even when seed is the env's seed);
+ *   m = max x;  e_i = expf(x_i - m);  c_i = e_0 + ... + e_i in fp32, ascending;  Z = c_8;
+ *   action = the smallest i with u*Z < c_i; if none (rounding), the largest i with e_i > 0; if none (NaN or infinite
+ *            logits), the no-op 4.  So the action is always in 0..8, and a masked row with finite logits takes 0..4;
+ *   logprob = (x_action - m) - logf(Z);  entropy = logf(Z) - (sum over e_i > 0 of e_i * (x_i - m)) / Z.
+ * Every add and multiply is rounded on its own (no FMA).  Outputs, each optional (NULL skips it): actions uint8
+ * [B][N], written at flat_index; action_out int64, logprob and entropy fp32, [n_rows] each.  A row's outputs depend only
+ * on its logits, its mask flag and (seed, global env id, episode, step, agent): not on n_rows, the row order or the
+ * other rows, and reruns are bit-identical.  No allocation and no host synchronisation (capturable in a CUDA graph).
+ * A flat_index outside [0, B*N) is a device-side error: that row writes nothing and sets CTF_FAULT_BAD_INDEX.
+ * Rejected with CTF_ERR_INVALID: a null handle, state.envs, head or flat_index; n_rows < 0; head_stride < 10;
+ * state.envs not 16-byte, flat_index or action_out not 8-byte, head, logprob or entropy not 4-byte aligned; an output
+ * that overlaps an input (head, masked, flat_index) or another output.  n_rows = 0 launches nothing.
+ */
+int ctf_sample_actions(ctf_handle_t h, ctf_state_t state, const float* head, int64_t head_stride, const uint8_t* masked,
+                       const int64_t* flat_index, int64_t n_rows, uint64_t seed, uint8_t* actions, int64_t* action_out,
+                       float* logprob, float* entropy, void* stream);
 
 /*
  * Compressible device memory for the dense observation buffer.  On devices with Compute Data Compression the memory

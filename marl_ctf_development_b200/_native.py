@@ -32,14 +32,15 @@ EXPORTS = (
     "ctf_policy_trunk_ctas",
     "ctf_gae",
     "ctf_gae_dones",
+    "ctf_sample_actions",
     "ctf_compressible_alloc",
     "ctf_compressible_free",
     "ctf_compression_supported",
     "ctf_mem_is_compressed",
     "ctf_compressible_set_enabled",
 )
-ABI_VERSION = 11
-FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED = 1, 2
+ABI_VERSION = 12
+FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED, FAULT_BAD_INDEX = 1, 2, 4
 
 
 class CtfState(C.Structure):
@@ -153,6 +154,8 @@ def load():
                           C.c_int64, C.c_float, C.c_float, C.c_void_p]
     L.ctf_gae_dones.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_float, C.c_void_p]
+    L.ctf_sample_actions.argtypes = [C.c_void_p, CtfState, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+                                     C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.ctf_compressible_alloc.restype = C.c_void_p
     L.ctf_compressible_alloc.argtypes = [C.c_ssize_t, C.c_int, C.c_void_p]
     L.ctf_compressible_free.restype = None

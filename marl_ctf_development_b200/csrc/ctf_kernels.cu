@@ -1520,6 +1520,80 @@ __global__ void __launch_bounds__(kGaeThreads, kDones ? 5 : 6) k_gae(const float
     }
 }
 
+// ================================================================================================
+// k_sample_actions — one seeded categorical draw per policy row (ctf_sample_actions), one thread per row
+// ================================================================================================
+constexpr int kSampleThreads = 256;
+constexpr uint32_t kPolicySite = 0x80000000u;   // top bit of the counter's site word: disjoint from the env's sites 0..31
+constexpr int kNoOpAction = 4;
+
+// Row r is agent a = flat_index[r] % N of env b = flat_index[r] / N.  Its draw is word 0 of Philox4x32-10 at counter
+// (env_id_base + b, episode[b], step_count[b], kPolicySite | a), read from the env state at launch, so the result of a
+// row depends on nothing but its logits, its mask flag and (seed, global env id, episode, step, agent).  Every add and
+// multiply is rounded on its own, so the action does not depend on the compiler contracting anything into an FMA
+// (marl_ctf_development_b200/draws.py: sample_action states it in float64).  The action is in 0..8 whatever the logits:
+// with no positive mass at all (NaN or infinite logits) it is the no-op 4.  A flat_index outside [0, B*N) writes
+// nothing and sets CTF_FAULT_BAD_INDEX, the only atomic (an idempotent OR into the fault word, as k_step reports its
+// faults): the outputs themselves are plain stores, bit-identical from run to run.
+__global__ void __launch_bounds__(kSampleThreads) k_sample_actions(
+    const float* __restrict__ head, long long head_stride, const uint8_t* __restrict__ masked,
+    const long long* __restrict__ flat_index, long long n_rows, const uint4* __restrict__ envs, long long n_flat,
+    int n_agents, uint32_t env_id_base, uint32_t seed_lo, uint32_t seed_hi, uint8_t* __restrict__ actions,
+    long long* __restrict__ action_out, float* __restrict__ logprob, float* __restrict__ entropy,
+    uint32_t* __restrict__ faults) {
+    const long long r = (long long)blockIdx.x * kSampleThreads + threadIdx.x;
+    if (r >= n_rows) return;
+    const long long f = __ldg(flat_index + r);
+    if (f < 0 || f >= n_flat) {
+        atomicOr(faults, CTF_FAULT_BAD_INDEX);
+        return;
+    }
+    const long long b = f / n_agents;
+    const uint32_t a = (uint32_t)(f - b * n_agents);
+    const uint4 ev = envs[b];   // x = env_step_count, y = episode
+    uint32_t w[4];
+    philox4x32_10(env_id_base + (uint32_t)b, ev.y, ev.x, kPolicySite | a, seed_lo, seed_hi, w);
+    const float u = __fmul_rn((float)(w[0] >> 8), 0x1p-24f);
+
+    const float* row = head + r * head_stride + 1;
+    const bool mask = masked != nullptr && __ldg(masked + r) != 0;
+    float x[CTF_N_ACTIONS];
+    float m = -INFINITY;
+#pragma unroll
+    for (int i = 0; i < CTF_N_ACTIONS; ++i) {
+        x[i] = __ldg(row + i);
+        if (mask && i >= 5) x[i] = __fadd_rn(x[i], -1e9f);   // CtfPolicy.masked_logits
+        m = fmaxf(m, x[i]);
+    }
+    float e[CTF_N_ACTIONS], z = 0.f;
+#pragma unroll
+    for (int i = 0; i < CTF_N_ACTIONS; ++i) {
+        e[i] = expf(__fsub_rn(x[i], m));
+        z = __fadd_rn(z, e[i]);
+    }
+    const float t = __fmul_rn(u, z);
+    int act = -1, last_pos = kNoOpAction;
+    float c = 0.f, s = 0.f;
+#pragma unroll
+    for (int i = 0; i < CTF_N_ACTIONS; ++i) {
+        c = __fadd_rn(c, e[i]);
+        if (act < 0 && t < c) act = i;
+        if (e[i] > 0.f) {
+            last_pos = i;
+            s = __fadd_rn(s, __fmul_rn(e[i], __fsub_rn(x[i], m)));
+        }
+    }
+    if (act < 0) act = last_pos;
+    float x_act = x[0];
+#pragma unroll
+    for (int i = 1; i < CTF_N_ACTIONS; ++i) x_act = i == act ? x[i] : x_act;   // a select: x stays in registers
+    const float log_z = logf(z);
+    if (actions) actions[f] = (uint8_t)act;
+    if (action_out) action_out[r] = act;
+    if (logprob) logprob[r] = __fsub_rn(__fsub_rn(x_act, m), log_z);
+    if (entropy) entropy[r] = __fsub_rn(log_z, __fdiv_rn(s, z));
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -2488,4 +2562,45 @@ extern "C" int ctf_gae_dones(ctf_handle_t h, const float* rewards, const float* 
     if (!dones) return fail(CTF_ERR_INVALID, "ctf_gae_dones: null argument");
     return launch_gae("ctf_gae_dones", h, rewards, values, dones, next_value, advantages, returns, n_steps,
                       agents_per_step, n_envs, gamma, gamma_lambda, stream);
+}
+
+extern "C" int ctf_sample_actions(ctf_handle_t h, ctf_state_t state, const float* head, int64_t head_stride,
+                                  const uint8_t* masked, const int64_t* flat_index, int64_t n_rows, uint64_t seed,
+                                  uint8_t* actions, int64_t* action_out, float* logprob, float* entropy,
+                                  void* stream) {
+    if (!h || !state.envs || !head || !flat_index) return fail(CTF_ERR_INVALID, "ctf_sample_actions: null argument");
+    if (n_rows < 0) return fail(CTF_ERR_INVALID, "ctf_sample_actions: n_rows must be >= 0");
+    if (head_stride < 1 + CTF_N_ACTIONS)
+        return fail(CTF_ERR_INVALID, "ctf_sample_actions: head_stride must be >= 10 (value, then 9 logits)");
+    // one thread per row: the grid must stay below 2^31 CTAs, and the head's byte size must fit 64 bits
+    if (n_rows > (1LL << 38) || (n_rows > 0 && head_stride > (1LL << 58) / n_rows))
+        return fail(CTF_ERR_INVALID, "ctf_sample_actions: n_rows * head_stride is too large");
+    if ((reinterpret_cast<uintptr_t>(state.envs) & 15) || (reinterpret_cast<uintptr_t>(head) & 3) ||
+        (reinterpret_cast<uintptr_t>(flat_index) & 7) || (reinterpret_cast<uintptr_t>(action_out) & 7) ||
+        (reinterpret_cast<uintptr_t>(logprob) & 3) || (reinterpret_cast<uintptr_t>(entropy) & 3))
+        return fail(CTF_ERR_INVALID, "ctf_sample_actions: misaligned buffer (state.envs 16-byte, flat_index and "
+                                     "action_out 8-byte, head, logprob and entropy 4-byte)");
+    const size_t n = (size_t)n_rows, n_flat = (size_t)h->B * h->plan.N;
+    // [pointer, bytes]: the inputs, then the outputs (absent ones have no bytes)
+    const void* ptr[7] = {head, masked, flat_index, actions, action_out, logprob, entropy};
+    const size_t bytes[7] = {n ? ((n - 1) * (size_t)head_stride + 1 + CTF_N_ACTIONS) * sizeof(float) : 0,
+                             masked ? n : 0, n * sizeof(int64_t), actions ? n_flat : 0,
+                             action_out ? n * sizeof(int64_t) : 0, logprob ? n * sizeof(float) : 0,
+                             entropy ? n * sizeof(float) : 0};
+    for (int o = 3; o < 7; ++o)
+        for (int i = 0; i < o; ++i)
+            if (bytes[o] && bytes[i] && overlaps(ptr[o], bytes[o], ptr[i], bytes[i]))
+                return fail(CTF_ERR_INVALID, i < 3 ? "ctf_sample_actions: an output overlaps an input"
+                                                   : "ctf_sample_actions: two outputs overlap");
+    if (n_rows == 0) return CTF_OK;
+    DeviceGuard guard(h->device);
+    CTF_CUDA(guard.err);
+    const unsigned grid = (unsigned)((n_rows + kSampleThreads - 1) / kSampleThreads);
+    k_sample_actions<<<grid, kSampleThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        head, head_stride, masked, reinterpret_cast<const long long*>(flat_index), n_rows,
+        reinterpret_cast<const uint4*>(state.envs), (long long)n_flat, h->plan.N, (uint32_t)h->env_id_base,
+        (uint32_t)(seed & 0xFFFFFFFFu), (uint32_t)(seed >> 32), actions, reinterpret_cast<long long*>(action_out),
+        logprob, entropy, h->faults);
+    CTF_CUDA(cudaGetLastError());
+    return CTF_OK;
 }

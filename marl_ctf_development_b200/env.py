@@ -382,7 +382,8 @@ class GridworldCtfGPU:
 
     def take_faults(self) -> int:
         """Reads and clears the device fault word (synchronises): bit 0 = action outside 0..8, bit 1 = a lethal tag
-        found the victim's 3x3 spawn window full (the reference raises there, gridworld_ctf.py:771)."""
+        found the victim's 3x3 spawn window full (the reference raises there, gridworld_ctf.py:771), bit 2 = a row of
+        ``ctf_sample_actions`` named a flat index outside [0, B*N)."""
         f = C.c_uint32(0)
         _native.check(self._lib.ctf_take_faults(self._handle, self._stream(), C.byref(f)))
         return int(f.value)
@@ -394,6 +395,8 @@ class GridworldCtfGPU:
         if f & _native.FAULT_RESPAWN_BLOCKED:
             raise ValueError("respawn found no open cell in a 3x3 spawn window (np.random.randint(0) raises ValueError in "
                              "the reference, gridworld_ctf.py:771); the victim was left in place with HP <= 0")
+        if f & _native.FAULT_BAD_INDEX:
+            raise IndexError("ctf_sample_actions was given a flat index outside [0, B*N); that row wrote nothing")
 
     @property
     def obs_compressed(self) -> bool:

@@ -19,6 +19,12 @@ bf16 through autograd.  ``reference_trunk_grads`` states in torch what the backw
 2 x stride bf16 values alive between forward and backward (its rows and their gradient: 15.6 KB at 8_arena), so a
 caller splits a large minibatch into chunks and lets the gradients accumulate.
 
+Seeded sampling: with ``seed=`` (``FusedPolicy.get_action_and_value`` / ``get_action``, ``PolicyPool.act``) the head's
+output rows go straight to ``ctf_sample_actions`` (``k_sample_actions``), one kernel that masks, samples and writes the
+log-prob, the entropy and the env's action buffer.  Each draw is a Philox word keyed by (seed, global env id, episode,
+step, agent), like the env's own draws (draws.py), so the actions do not depend on torch's random state or on how the
+envs are batched.  ``seed=None`` keeps torch's ``Categorical``.
+
 Several policies on one env batch: ``PolicyPool(env, policies)`` runs any number of (policy, env slice, agent ids)
 segments with one ``ctf_policy_features_grouped`` launch (``k_policy_trunk_grouped``, the same per-sample code as
 ``k_policy_trunk``, so every row is bit-identical to ``FusedPolicy``'s) and one bf16 ``torch.baddbmm`` head chain over
@@ -195,6 +201,39 @@ def _check_packed(env, bits, meta):
         raise ValueError(f"meta must be a float32 tensor [{bits.shape[0]}, {M}] on {env.device}")
 
 
+def _check_seed(seed) -> int:
+    seed = int(seed)
+    if not 0 <= seed < 1 << 64:
+        raise ValueError(f"a policy seed must be in [0, 2**64), got {seed}")
+    return seed
+
+
+def sample_actions(env, head_out: torch.Tensor, masked, flat_index: torch.Tensor, seed: int, actions=None):
+    """One ``ctf_sample_actions`` launch on the current stream: (action int64 [S], logprob [S], entropy [S]) of the rows
+    of ``head_out`` (fp32 [S, 10], value then the 9 logits, unit column stride), drawn with ``seed`` for the agents
+    ``flat_index`` (int64 [S], env * N + agent of ``env``) at the env's current episode and step.  ``masked``: uint8
+    [S] (nonzero: ``CtfPolicy.masked_logits`` applies) or None.  ``actions`` (uint8 [B, N], contiguous) also receives
+    every action at its flat index when given."""
+    seed = _check_seed(seed)
+    S, dev = head_out.shape[0], env.device
+    a = torch.empty(S, dtype=torch.int64, device=dev)
+    logp, ent = torch.empty(S, dtype=torch.float32, device=dev), torch.empty(S, dtype=torch.float32, device=dev)
+    if S == 0:
+        return a, logp, ent
+    ptr = lambda t: C.c_void_p(None if t is None else t.data_ptr())
+    stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    _native.check(env._lib.ctf_sample_actions(
+        env._handle, env._state_struct, ptr(head_out), head_out.stride(0), ptr(masked), ptr(flat_index), S, seed,
+        ptr(actions), ptr(a), ptr(logp), ptr(ent), stream))
+    return a, logp, ent
+
+
+def _check_actions(env, actions):
+    if actions.dtype != torch.uint8 or tuple(actions.shape) != (env.num_envs, env.N_AGENTS) \
+            or not actions.is_contiguous() or actions.device != env.device:
+        raise ValueError(f"actions must be a contiguous uint8 tensor [{env.num_envs}, {env.N_AGENTS}] on {env.device}")
+
+
 def _trunk_forward(env, weights, packed_ptr, meta_ptr, n_envs, agents_per_env, ids, k, out, stride):
     """Runs ``ctf_policy_features`` on the current stream with ``weights`` (``C.byref`` of a ``CtfPolicyWeights``) into
     ``out``, bf16 [n_envs * k, stride]; returns ``out``."""
@@ -296,6 +335,7 @@ class FusedPolicy:
             t[0] for t in (hw.fc1w, hw.fc1b, hw.fc2w, hw.fc2b, hw.hw, hw.hb))
         self._features = None   # bf16 [S_max, stride] rows, reused by every call (see features())
         self._ids = {}
+        self._flat = {}         # (ids, e0, e1, N) -> int64 [S] device flat indices env * N + agent of the samples
         self._train = None      # training-only weight buffers and workspace, created by the first evaluate_actions
         self.refresh()
 
@@ -330,11 +370,41 @@ class FusedPolicy:
             self._features = torch.empty((n_samples, self.stride), dtype=torch.bfloat16, device=self.env.device)
         return self._features[:n_samples]
 
-    def _head(self, feat):
+    def _head_out(self, feat):
+        """fp32 [S, 10]: the value, then the 9 logits, of every feature row."""
         x = torch.tanh(F.linear(feat, self._fc1w, self._fc1b))
         x = torch.tanh(F.linear(x, self._fc2w, self._fc2b))
-        out = F.linear(x, self._hw, self._hb).float()
+        return F.linear(x, self._hw, self._hb).float()
+
+    def _head(self, feat):
+        out = self._head_out(feat)
         return out[:, :1], out[:, 1:]
+
+    def _flat_index(self, agent_ids, env, envs):
+        """int64 [S] on the device: env * N + agent of every sample of ``trunk_from_env(agent_ids, env, envs)``."""
+        N = env.N_AGENTS
+        ids = _check_agent_ids(agent_ids, N)
+        e0, e1, _ = (envs if envs is not None else slice(None)).indices(env.num_envs)
+        key = (ids, e0, max(e1, e0), N)
+        flat = self._flat.get(key)
+        if flat is None:
+            k = len(ids)
+            s = torch.arange((key[2] - e0) * k)
+            flat = self._flat[key] = ((e0 + s // k) * N + torch.tensor(ids)[s % k]).to(env.device)
+        return flat
+
+    def _seeded(self, use_action_mask, agent_ids, bits, env, envs, seed, actions):
+        """(action, logprob, entropy, value) of ``get_action_and_value`` with ``seed``: one ``ctf_sample_actions``."""
+        if agent_ids is None or bits is not None:
+            raise ValueError("a seeded draw is keyed by (env, episode, step, agent): pass agent_ids (read the env in "
+                             "place), not bits / meta")
+        env = self._env_for(env)
+        if actions is not None:
+            _check_actions(env, actions)
+        out = self._head_out(self.trunk_from_env(agent_ids, env, envs))
+        masked = (use_action_mask.reshape(-1) == 1).to(torch.uint8) if self.policy.use_masking else None
+        a, logp, ent = sample_actions(env, out, masked, self._flat_index(agent_ids, env, envs), seed, actions)
+        return a, logp, ent, out[:, :1]
 
     # ------------------------------------------------------------------ trunk and forwards
     def trunk_from_env(self, agent_ids, env=None, envs=None) -> torch.Tensor:
@@ -383,9 +453,20 @@ class FusedPolicy:
 
     @torch.no_grad()
     def get_action_and_value(self, use_action_mask, action=None, *, agent_ids=None, bits=None, meta=None, env=None,
-                             envs=None):
+                             envs=None, seed=None, actions=None):
         """``CtfPolicy.get_action_and_value``'s (action, log_prob, entropy, value) for the samples of ``forward``;
-        use_action_mask is the per-sample flag in sample order.  Masking is ``CtfPolicy.masked_logits``."""
+        use_action_mask is the per-sample flag in sample order.  Masking is ``CtfPolicy.masked_logits``.
+
+        ``seed`` (an int in [0, 2**64)) samples with ``ctf_sample_actions`` instead of torch's generator: each action
+        is a function of the logits, the mask flag and (seed, global env id, episode, step, agent), so it needs
+        ``agent_ids`` (ValueError with ``bits`` / ``meta`` or a given ``action``).  ``actions`` (uint8 [B, N]) then
+        also receives every action at its (env, agent), in the same launch."""
+        if seed is not None:
+            if action is not None:
+                raise ValueError("seed draws the action: pass a seed or an action, not both")
+            return self._seeded(use_action_mask, agent_ids, bits, env, envs, seed, actions)
+        if actions is not None:
+            raise ValueError("actions is written by the seeded draw only: pass a seed with it")
         value, logits = self.forward(agent_ids, bits, meta, env, envs)
         probs = Categorical(logits=self.policy.masked_logits(logits, use_action_mask), validate_args=False)
         if action is None:
@@ -393,7 +474,10 @@ class FusedPolicy:
         return action, probs.log_prob(action), probs.entropy(), value
 
     @torch.no_grad()
-    def get_action(self, use_action_mask, *, agent_ids=None, bits=None, meta=None, env=None, envs=None):
+    def get_action(self, use_action_mask, *, agent_ids=None, bits=None, meta=None, env=None, envs=None, seed=None):
+        """The action of ``get_action_and_value`` (with ``seed``, drawn by ``ctf_sample_actions``)."""
+        if seed is not None:
+            return self._seeded(use_action_mask, agent_ids, bits, env, envs, seed, None)[0]
         _, logits = self.forward(agent_ids, bits, meta, env, envs)
         return Categorical(logits=self.policy.masked_logits(logits, use_action_mask), validate_args=False).sample()
 
@@ -487,12 +571,14 @@ class PoolPlan:
     * ``flat_index`` [S]: env * N + agent of every output row (where ``act`` writes its action in ``actions[B, N]``);
     * ``mask_add`` [S, 9] float32: the additive action mask, ``(mask - 1) * 1e9`` of ``CtfPolicy.masked_logits`` for
       rows whose policy masks and whose agent type is masked, zeros elsewhere;
+    * ``masked`` [S] uint8: 1 on exactly those rows (what ``ctf_sample_actions`` reads for a seeded ``act``);
     * ``features`` bf16 [L * s_max, stride]: the trunk's output buffer.
     """
 
     def __init__(self, segments, n_samples, s_max, seg_rows, row_index, flat_index, mask_add, features, tables):
         self.segments, self.n_samples, self.s_max, self.seg_rows = segments, n_samples, s_max, seg_rows
         self.row_index, self.flat_index, self.mask_add, self.features = row_index, flat_index, mask_add, features
+        self.masked = (mask_add[:, 5:] != 0).any(1).to(torch.uint8)
         self.policy_of_row = row_index // s_max
         self.n_rows = features.shape[0]
         self._tables = tables   # [(ctypes segment array, count)], policy-major, at most GROUPED_MAX_SEGMENTS each
@@ -630,15 +716,19 @@ class PolicyPool:
                 feat.shape[0], stream))
         return feat
 
-    def head(self, plan: PoolPlan, feat: torch.Tensor | None = None):
-        """(value [S, 1], logits [S, 9]) fp32 in plan order from the feature rows: fc1 -> tanh -> fc2 -> tanh -> heads
-        as one bf16 ``torch.baddbmm`` chain over [L, s_max, .], then the plan's rows gathered."""
+    def _head_out(self, plan: PoolPlan, feat: torch.Tensor | None = None):
+        """fp32 [S, 10] in plan order: the value, then the 9 logits, of every row (see ``head``)."""
         L, w = len(self.policies), self._head_w
         x = (plan.features if feat is None else feat).view(L, plan.s_max, self.stride)
         x = torch.tanh(torch.baddbmm(w.fc1b.unsqueeze(1), x, w.fc1w.transpose(1, 2)))
         x = torch.tanh(torch.baddbmm(w.fc2b.unsqueeze(1), x, w.fc2w.transpose(1, 2)))
         out = torch.baddbmm(w.hb.unsqueeze(1), x, w.hw.transpose(1, 2)).view(L * plan.s_max, 1 + N_ACTIONS)
-        out = out.index_select(0, plan.row_index).float()
+        return out.index_select(0, plan.row_index).float()
+
+    def head(self, plan: PoolPlan, feat: torch.Tensor | None = None):
+        """(value [S, 1], logits [S, 9]) fp32 in plan order from the feature rows: fc1 -> tanh -> fc2 -> tanh -> heads
+        as one bf16 ``torch.baddbmm`` chain over [L, s_max, .], then the plan's rows gathered."""
+        out = self._head_out(plan, feat)
         return out[:, :1], out[:, 1:]
 
     @torch.no_grad()
@@ -649,14 +739,20 @@ class PolicyPool:
     __call__ = forward
 
     @torch.no_grad()
-    def act(self, plan: PoolPlan, actions: torch.Tensor, env=None) -> torch.Tensor:
+    def act(self, plan: PoolPlan, actions: torch.Tensor, env=None, seed=None) -> torch.Tensor:
         """Samples one action per row of ``plan`` (one ``Categorical`` over all rows, each masked by its own policy's
         ``use_masking`` as ``CtfPolicy.masked_logits`` does) and writes it into ``actions`` (uint8 [B, N], contiguous)
-        at the row's (env, agent).  Returns the sampled actions [S] int64 in plan order."""
+        at the row's (env, agent).  Returns the sampled actions [S] int64 in plan order.
+
+        With ``seed`` one ``ctf_sample_actions`` launch draws and writes them instead: each row's action is keyed by
+        (seed, global env id, episode, step, agent), as ``FusedPolicy.get_action_and_value(seed=...)`` draws it."""
         env = self._env_for(env)
         if actions.dtype != torch.uint8 or tuple(actions.shape) != (env.num_envs, env.N_AGENTS) \
                 or not actions.is_contiguous():
             raise ValueError(f"actions must be a contiguous uint8 tensor [{env.num_envs}, {env.N_AGENTS}]")
+        if seed is not None:
+            out = self._head_out(plan, self.trunk(plan, env))
+            return sample_actions(env, out, plan.masked, plan.flat_index, seed, actions)[0]
         _, logits = self.forward(plan, env)
         a = Categorical(logits=logits + plan.mask_add, validate_args=False).sample()
         actions.view(-1).index_copy_(0, plan.flat_index, a.to(torch.uint8))

@@ -48,7 +48,7 @@ def pool_segments(pairs, duels_per_pair: int, team_ids):
 @torch.no_grad()
 def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 256, device=None, seed: int = 0,
                env_id_base: int = 0, collect_metrics: bool = False, per_duel_metrics: bool = False,
-               grouped: bool = False):
+               grouped: bool = False, policy_seed: int | None = None):
     """Plays ``duels_per_pair`` duels (utils.py:500-573) for every (agent, opponent) in ``pairs`` at once.
 
     Returns (results [P, D] int64 of +1/0/-1 from team 0's view, metrics).  metrics is None unless collect_metrics;
@@ -62,8 +62,17 @@ def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 25
     one ``fused_policy.PolicyPool`` on a packed-only env, with one plan segment per (pair, team), and each step is
     ``pool.act`` followed by ``env.step``.  The results and metrics have the same structure as the per-pair path's;
     the draws differ (one ``Categorical`` over all rows consumes torch's random stream differently).
+
+    ``policy_seed``: every action is drawn by ``ctf_sample_actions``, keyed by (policy_seed, global env id, episode,
+    step, agent), on both paths, so the results are a function of (seed, env_id_base, policy_seed) and the policies,
+    whatever else uses torch's random generator.  The two paths then draw the same action wherever their logits are
+    equal (the head's cuBLAS calls differ between them, so the logits may differ in the last bits).  The per-pair
+    path needs every policy to be a ``FusedPolicy``.
     """
     P, D = len(pairs), int(duels_per_pair)
+    if policy_seed is not None and not grouped and not all(isinstance(pol, FusedPolicy) for pair in pairs for pol in pair):
+        raise ValueError("policy_seed draws actions from the logits of a FusedPolicy: every policy must be one "
+                         "(or pass grouped=True, which also runs CtfPolicy modules)")
     if grouped:
         if any(not isinstance(pol, (FusedPolicy, CtfPolicy)) for pair in pairs for pol in pair):
             raise ValueError("grouped=True needs every policy to be a FusedPolicy or a CtfPolicy")
@@ -87,7 +96,8 @@ def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 25
     while True:
         step_count += 1
         if grouped:
-            pool.act(plan, actions)
+            # without a seed, act is called as before, so PolicyPool subclasses that override act(plan, actions) work
+            pool.act(plan, actions, **({} if policy_seed is None else {"seed": policy_seed}))
         else:
             for p, pair in enumerate(pairs):
                 sl = slice(p * D, (p + 1) * D)
@@ -96,6 +106,10 @@ def duel_pairs(env_config: dict, pairs, duels_per_pair: int, max_steps: int = 25
                     if k == 0:
                         continue
                     flags = env.use_action_mask[idx].unsqueeze(0).expand(D, k).reshape(D * k)
+                    if policy_seed is not None:
+                        pol.get_action_and_value(flags, agent_ids=ids, env=env, envs=sl, seed=policy_seed,
+                                                 actions=actions)
+                        continue
                     if isinstance(pol, FusedPolicy):
                         a = pol.get_action_and_value(flags, agent_ids=ids, env=env, envs=sl)[0]
                     else:

@@ -24,7 +24,7 @@ import ctypes as C
 import torch
 
 from . import _native
-from .fused_policy import FusedPolicy
+from .fused_policy import FusedPolicy, _check_seed
 from .policy import CtfPolicy
 from .rollout import Rollout, _team_indices, collect_rollout
 
@@ -143,9 +143,13 @@ class PackedPPO:
     the env is (``collect_rollout(reset=False)``), resetting the env when its episodes end; GAE then stops at each
     episode boundary.  The opponent may change between updates; ``train_team1`` may change only between episodes
     (ValueError while one is in progress).  The env belongs to the trainer in this mode: stepping or resetting it
-    elsewhere breaks the episodes the trainer continues."""
+    elsewhere breaks the episodes the trainer continues.
 
-    def __init__(self, env, agent, args, optimizer=None, chunk=262144, rollout_steps=None):
+    ``policy_seed`` (an int): every ``collect`` draws both sides' actions with ``ctf_sample_actions``
+    (``collect_rollout(policy_seed=...)``), so the rollouts do not depend on torch's random state, which ``optimise``
+    advances with its ``randperm``."""
+
+    def __init__(self, env, agent, args, optimizer=None, chunk=262144, rollout_steps=None, policy_seed=None):
         if env.obs_bits is None:
             raise ValueError("PackedPPO trains from packed observations: create the env with packed_obs=True")
         if not env.ce.cfg.reverse_team1_actions:
@@ -159,6 +163,7 @@ class PackedPPO:
         if rollout_steps is not None and not 1 <= int(rollout_steps) <= env.GAME_STEPS:
             raise ValueError(f"rollout_steps must be None or in 1..GAME_STEPS ({env.GAME_STEPS})")
         self.rollout_steps = None if rollout_steps is None else int(rollout_steps)
+        self.policy_seed = None if policy_seed is None else _check_seed(policy_seed)
         self.env, self.agent, self.args, self.chunk = env, agent, args, int(chunk)
         self.fused = FusedPolicy(env, agent)
         self.optimizer = optimizer if optimizer is not None else torch.optim.Adam(
@@ -198,7 +203,7 @@ class PackedPPO:
             env.reset()
             self._running_return = None
         ro = collect_rollout(env, self.fused, opponent, train_team1=train_team1, num_env_steps=T,
-                             obs_storage_dtype="packed", reset=not continuing)
+                             obs_storage_dtype="packed", reset=not continuing, policy_seed=self.policy_seed)
         mine = _team_indices(env, 0 if train_team1 else 1)
         apt, B = len(mine), env.num_envs
         if continuing:

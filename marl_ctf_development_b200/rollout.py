@@ -15,6 +15,12 @@ adapters sample through the same method: ``Agent.get_action`` ends in ``action.i
 only takes one sample at a time.  A ``fused_policy.FusedPolicy`` on either side reads the packed observations
 ``env.obs_bits`` and ``env.meta`` in place instead; an env created packed-only (``dense_obs=False, packed_obs=True``)
 is accepted when every policy on it is fused.
+
+``policy_seed`` (an int) makes both adapters reproducible: every action of both sides is drawn by
+``ctf_sample_actions`` from a Philox word keyed by (policy_seed, global env id, episode, step, agent), so the result
+is a function of the env seed and the policy seed alone, whatever else uses torch's random generator and however the
+envs are batched.  It needs a ``FusedPolicy`` on every side that acts (the stock dense path hands out actions, not
+logits).  ``policy_seed=None`` samples with torch's ``Categorical`` as before.
 """
 from __future__ import annotations
 
@@ -80,6 +86,11 @@ def _require_dense_obs(env, *policies):
         raise ValueError("this adapter feeds policies from env.obs: create the env with dense_obs=True")
 
 
+def _require_fused_for_seed(policy_seed, *policies):
+    if policy_seed is not None and not all(isinstance(p, FusedPolicy) for p in policies):
+        raise ValueError("policy_seed draws actions from the logits of a FusedPolicy: every policy that acts must be one")
+
+
 def batched_action(policy, grid, meta, use_action_mask) -> torch.Tensor:
     """Actions for a batch of samples from a reference-style policy: ``get_action_batch`` when the policy has one,
     else ``get_action_and_value(...)[0]`` (same Categorical sample as ``Agent.get_action``, which is scalar-only)."""
@@ -91,7 +102,7 @@ def batched_action(policy, grid, meta, use_action_mask) -> torch.Tensor:
 
 @torch.no_grad()
 def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, obs_storage_dtype=torch.float32,
-                    reset=True) -> Rollout:
+                    reset=True, policy_seed=None) -> Rollout:
     """One rollout of every env (ppo.py:31-131).  ``train_team1=True`` trains team 0 (ppo.py:274-279).
 
     num_env_steps defaults to GAME_STEPS (one episode per rollout, as num_steps == GAME_STEPS in every
@@ -105,11 +116,15 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
     ``env.reset()`` runs before the next policy call, whose rows get ``dones = 1``.  An env already at ``GAME_STEPS`` on
     entry (the previous rollout ended the episode) is reset first and row 0 gets ``dones = 1``; an env never reset is
     reset first.  ``next_done`` marks a last step that ended the episode.
+
+    ``policy_seed``: both sides draw with ``ctf_sample_actions`` (see the module docstring); the rollout's ``actions``
+    and ``logprobs`` come from it.
     """
     _require_folded_reversal(env)
     team = 0 if train_team1 else 1
     mine, theirs = _team_indices(env, team), _team_indices(env, 1 - team)
     _require_dense_obs(env, agent, *([opponent] if theirs else []))
+    _require_fused_for_seed(policy_seed, agent, *([opponent] if theirs else []))
     fused_agent, fused_opponent = isinstance(agent, FusedPolicy), isinstance(opponent, FusedPolicy)
     apt = len(mine)
     T = env.GAME_STEPS if num_env_steps is None else int(num_env_steps)
@@ -161,7 +176,9 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
         if fused_agent:
             # samples come env-major (b * apt + j): reorder to the buffer's agent-major rows
             fe = mask_flags[mine_t].unsqueeze(0).expand(B, apt).reshape(B * apt)
-            a, logp, _, v = agent.get_action_and_value(fe, agent_ids=mine, env=env)
+            # seeded: the kernel also writes the actions into the env's action buffer
+            seeded = dict(seed=policy_seed, actions=actions) if policy_seed is not None else {}
+            a, logp, _, v = agent.get_action_and_value(fe, agent_ids=mine, env=env, **seeded)
             a, logp, v = (x.reshape(B, apt).t().reshape(apt * B) for x in (a, logp, v.reshape(-1)))
         else:
             a, logp, _, v = agent.get_action_and_value(
@@ -176,17 +193,21 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
         out.actions[sl] = a.reshape(apt, B).float()
         out.use_action_mask[sl] = flags
         out.logprobs[sl] = logp.reshape(apt, B)
-        actions[:, mine_t] = a.reshape(apt, B).t().to(torch.uint8)
+        if policy_seed is None:
+            actions[:, mine_t] = a.reshape(apt, B).t().to(torch.uint8)
         if theirs:
             k = len(theirs)
             fo = mask_flags[theirs_t].unsqueeze(0).expand(B, k).reshape(B * k)
-            if fused_opponent:
-                ao = opponent.get_action_and_value(fo, agent_ids=theirs, env=env)[0]
+            if policy_seed is not None:
+                opponent.get_action_and_value(fo, agent_ids=theirs, env=env, seed=policy_seed, actions=actions)
             else:
-                go = obs[:, theirs_t].reshape(B * k, C, G, G).float()
-                mo = meta[:, theirs_t].reshape(B * k, M)
-                ao = opponent.get_action_and_value(go, mo, fo)[0]
-            actions[:, theirs_t] = ao.reshape(B, k).to(torch.uint8)
+                if fused_opponent:
+                    ao = opponent.get_action_and_value(fo, agent_ids=theirs, env=env)[0]
+                else:
+                    go = obs[:, theirs_t].reshape(B * k, C, G, G).float()
+                    mo = meta[:, theirs_t].reshape(B * k, M)
+                    ao = opponent.get_action_and_value(go, mo, fo)[0]
+                actions[:, theirs_t] = ao.reshape(B, k).to(torch.uint8)
         obs, meta, rewards, dones, _ = env.step(actions)                          # ppo.py:98
         out.rewards[sl] = rewards[:, mine_t].t()                                  # ppo.py:106-109
         step += 1
@@ -207,19 +228,21 @@ def collect_rollout(env, agent, opponent, train_team1=True, num_env_steps=None, 
 
 
 @torch.no_grad()
-def batched_duel(env, agent, opponent, max_steps=256, return_result=True):
+def batched_duel(env, agent, opponent, max_steps=256, return_result=True, policy_seed=None):
     """utils.duel (utils.py:500-573) for every env of the batch.
 
     Team 0 acts with ``agent``, team 1 with ``opponent``.  Stops when the envs are done or after
     max_steps + 1 steps (the reference's ``step_count > max_steps`` check runs after the step, :559-560).
     Returns int tensor [B] of +1 / 0 / -1 (team-0 win / draw / loss by flag captures, :562-569), or the
-    all-reduced ``env.metrics`` dict when return_result=False (:571).
+    all-reduced ``env.metrics`` dict when return_result=False (:571).  ``policy_seed``: both sides draw with
+    ``ctf_sample_actions`` (see the module docstring).
     """
     _require_folded_reversal(env)
     _require_dense_obs(env, agent, opponent)
     B, N, dev = env.num_envs, env.N_AGENTS, env.device
     C, G, M = env.n_channels, env.GRID_SIZE, env.meta_size
     team_ids = [_team_indices(env, t) for t in (0, 1)]
+    _require_fused_for_seed(policy_seed, *(p for p, ids in zip((agent, opponent), team_ids) if ids))
     teams = [torch.tensor(ids, device=dev) for ids in team_ids]
     policies = (agent, opponent)
     obs, meta, _ = env.reset()
@@ -232,6 +255,9 @@ def batched_duel(env, agent, opponent, max_steps=256, return_result=True):
             if k == 0:
                 continue
             flags = env.use_action_mask[idx].unsqueeze(0).expand(B, k).reshape(B * k)
+            if policy_seed is not None:
+                pol.get_action_and_value(flags, agent_ids=ids, env=env, seed=policy_seed, actions=actions)
+                continue
             if isinstance(pol, FusedPolicy):
                 a = pol.get_action_and_value(flags, agent_ids=ids, env=env)[0]
             else:
