@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CTF_ABI_VERSION 12
+#define CTF_ABI_VERSION 13
 
 #define CTF_MAX_AGENTS 8    /* largest AGENT_STARTING_POSITIONS in scenarios.py has 8 entries */
 #define CTF_MAX_GRID 16     /* GRID_SIZE <= 16 (shipped maps: 11, 13, 15) */
@@ -250,6 +250,28 @@ int ctf_take_faults(ctf_handle_t h, void* stream, uint32_t* faults);
  */
 int ctf_step_host(ctf_handle_t h, ctf_state_t state, const uint8_t* actions_host, ctf_outputs_t out,
                   float* rewards_host, uint8_t* dones_host, void* stream);
+
+/*
+ * Observation record (ABI 13): lets ctf_step store only the 32-byte sectors of `obs` that changed since the last
+ * write, which are about 1 % of them.  The caller keeps, for one observation buffer it owns:
+ *   record        device [B][ctf_obs_record_size / (4 B)] uint32, 16-byte aligned: per env, the padded bit string
+ *                 the last launch wrote into obs (contents need no initialisation);
+ *   record_epoch  device [B] uint32: the epoch in which each env's record was written;
+ *   epoch         device uint32: the current epoch.
+ * An env's record is valid when record_epoch[env] == *epoch.  A launch whose outputs.obs equals the bound `obs`
+ * (ctf_step, ctf_step_host, ctf_reset, ctf_observe) writes an env with a valid record as a delta (ctf_step and
+ * ctf_step_host) and any other env in full (all four), then refreshes the record and stamps record_epoch.  Every
+ * launch into another buffer writes exactly as without a record.  The contract: between two such launches nothing
+ * else may write `obs` unless *epoch is changed first (in stream order, e.g. by adding 1 on the device, which a CUDA
+ * graph can capture); otherwise the next delta leaves the foreign bytes in place.
+ * obs = NULL unbinds (record, record_epoch, epoch are then ignored).  Rejected with CTF_ERR_INVALID: a null handle; a
+ * non-null obs with a null record, record_epoch or epoch; record not 16-byte, record_epoch or epoch not 4-byte aligned;
+ * any two of obs (the handle's dense size), record, record_epoch and epoch overlapping.  The handle keeps the pointers,
+ * not the memory: unbind before freeing it.
+ */
+int ctf_bind_obs_record(ctf_handle_t h, const void* obs, uint32_t* record, uint32_t* record_epoch, const uint32_t* epoch);
+/* Bytes of the record ctf_bind_obs_record needs for this handle: B * (padded bit-string words per env) * 4. */
+int ctf_obs_record_size(ctf_handle_t h, size_t* record_bytes);
 
 /*
  * Policy inference from packed observations (no reference counterpart: the reference feeds agent_network.Agent a dense

@@ -25,6 +25,8 @@ EXPORTS = (
     "ctf_stats_sum",
     "ctf_take_faults",
     "ctf_step_host",
+    "ctf_bind_obs_record",
+    "ctf_obs_record_size",
     "ctf_policy_features",
     "ctf_policy_grad_workspace_size",
     "ctf_policy_features_backward",
@@ -39,7 +41,7 @@ EXPORTS = (
     "ctf_mem_is_compressed",
     "ctf_compressible_set_enabled",
 )
-ABI_VERSION = 12
+ABI_VERSION = 13
 FAULT_BAD_ACTION, FAULT_RESPAWN_BLOCKED, FAULT_BAD_INDEX = 1, 2, 4
 
 
@@ -140,6 +142,8 @@ def load():
     L.ctf_stats_sum.argtypes = [C.c_void_p, CtfState, C.c_void_p, C.c_void_p]
     L.ctf_take_faults.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
     L.ctf_step_host.argtypes = [C.c_void_p, CtfState, C.c_void_p, CtfOutputs, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.ctf_bind_obs_record.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.ctf_obs_record_size.argtypes = [C.c_void_p, C.POINTER(C.c_size_t)]
     L.ctf_policy_features.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
                                       C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]
     L.ctf_policy_features_grouped.argtypes = [C.c_void_p, C.POINTER(CtfPolicyWeights), C.c_int, C.POINTER(CtfPolicySegment),

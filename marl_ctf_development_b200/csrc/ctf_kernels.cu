@@ -32,6 +32,12 @@
 
 #include "../../include/ctf_b200.h"
 
+// Resident CTAs per SM of k_step when it writes observation deltas (ctf_bind_obs_record; see ctf_create).  Set on the
+// nvcc command line only to build the libraries of a residency sweep (tools/obs_delta_bench.py --cap-lib).
+#ifndef CTF_DELTA_CTAS_PER_SM
+#define CTF_DELTA_CTAS_PER_SM 9
+#endif
+
 namespace {
 
 constexpr int kWarpsPerCta = 4;   // 2 warps per CTA tie with 4, 8 and 16 lose (see k_step)
@@ -86,6 +92,11 @@ struct Launch {
     uint8_t* dones;
     const uint8_t* actions;
     uint32_t* faults;
+    // record of `obs` (ctf_bind_obs_record; all null unless outputs.obs is the bound buffer): the padded bit string
+    // each env's last launch wrote into obs ([B][bits_words]), the epoch it was written in ([B]) and the current epoch
+    uint32_t* record;
+    uint32_t* record_epoch;
+    const uint32_t* epoch;
     long long B;
     uint32_t seed_lo, seed_hi;
     uint32_t env_id_base;
@@ -272,6 +283,33 @@ __device__ __forceinline__ const uint2* init_expand_lut(uint4* smem_raw) {
     }
 }
 
+// Store vector v of a padded bit string (elements = bits VB*v .. VB*v + VB - 1).
+template <typename T>
+__device__ __forceinline__ uint4 vector_value(const uint32_t* __restrict__ bits, int v, const uint2* __restrict__ lut) {
+    if constexpr (kLutBytes<T> > 0) {
+        // uint8: the vector's 16 bits are two table lookups (8 bits -> 8 bytes each) instead of sixteen ALU operations
+        const uint32_t h = bits[v >> 1] >> ((v & 1) * 16);
+        const uint2 lo = lut[h & 0xFFu], hi = lut[(h >> 8) & 0xFFu];
+        return make_uint4(lo.x, lo.y, hi.x, hi.y);
+    } else {
+        constexpr int VB = kVecElems<T>, VW = 32 / VB;
+        return expand_bits<T>(bits[v / VW] >> ((v % VW) * VB));
+    }
+}
+
+// The fewer than VB elements of a block before its first full vector and after its last one, as scalar stores
+// (one warp).
+template <typename T>
+__device__ __forceinline__ void stream_edges(const uint32_t* __restrict__ bits, int nbits, T* __restrict__ out, int v_begin,
+                                             int v_end, int lane) {
+    constexpr int VB = kVecElems<T>;
+    const int pad = obs_pad(out), total = pad + nbits;
+    const int head_n = min(v_begin * VB - pad, nbits);          // < VB elements before the first full vector
+    if (lane < head_n) out[lane] = from_bit<T>((bits[(pad + lane) >> 5] >> ((pad + lane) & 31)) & 1u);
+    const int t = max(v_end * VB, pad + head_n) + lane;         // first bit covered by neither head nor full vectors
+    if (t < total) out[t - pad] = from_bit<T>((bits[t >> 5] >> (t & 31)) & 1u);
+}
+
 // Stores the full vectors [v_begin, v_end) of a padded bit string (vector v = bits VB*v .. VB*v + VB - 1) at vp[v];
 // warp `wi` of `nw` cooperating warps.  `bits` must be 16-byte aligned and readable up to a multiple of 16 words.
 template <typename T>
@@ -295,22 +333,9 @@ __device__ __forceinline__ void stream_vectors(const uint32_t* __restrict__ bits
             if (v0 + 24 < v_end) store_vec(vp + v0 + 24, expand_bits<T>(wd.w >> sh));
         }
     } else {
-        constexpr int VB = kVecElems<T>, VW = 32 / VB;
-        if constexpr (kLutBytes<T> > 0) {
-            // uint8: the vector's 16 bits are two table lookups (8 bits -> 8 bytes each) instead of sixteen ALU operations
 #pragma unroll 4
-            for (int v = wi * 32 + lane; v < v_end; v += nw * 32) {
-                if (v >= v_begin) {
-                    const uint32_t h = bits[v >> 1] >> ((v & 1) * 16);
-                    const uint2 lo = lut[h & 0xFFu], hi = lut[(h >> 8) & 0xFFu];
-                    store_vec(vp + v, make_uint4(lo.x, lo.y, hi.x, hi.y));
-                }
-            }
-        } else {
-#pragma unroll 4
-            for (int v = wi * 32 + lane; v < v_end; v += nw * 32)
-                if (v >= v_begin) store_vec(vp + v, expand_bits<T>(bits[v / VW] >> ((v % VW) * VB)));
-        }
+        for (int v = wi * 32 + lane; v < v_end; v += nw * 32)
+            if (v >= v_begin) store_vec(vp + v, vector_value<T>(bits, v, lut));
     }
 }
 
@@ -327,13 +352,67 @@ __device__ __forceinline__ void stream_env(const uint32_t* __restrict__ bits, in
     const int pad = obs_pad(out);
     const int total = pad + nbits;
     const int v_begin = (pad + VB - 1) / VB, v_end = total / VB;   // vectors counted from the alignment boundary
-    if (wi == 0) {
-        const int head_n = min(v_begin * VB - pad, nbits);          // < VB elements before the first full vector
-        if (lane < head_n) out[lane] = from_bit<T>((bits[(pad + lane) >> 5] >> ((pad + lane) & 31)) & 1u);
-        const int t = max(v_end * VB, pad + head_n) + lane;         // first bit covered by neither head nor full vectors
-        if (t < total) out[t - pad] = from_bit<T>((bits[t >> 5] >> (t & 31)) & 1u);
-    }
+    if (wi == 0) stream_edges<T>(bits, nbits, out, v_begin, v_end, lane);
     stream_vectors<T>(bits, reinterpret_cast<uint4*>(out - pad), v_begin, v_end, wi, nw, lane, lut);
+}
+
+// Delta form of stream_env for a block whose previous bit string (same pad) is `rec`: only the 32-byte sectors whose
+// bits differ from `rec` are stored, and only the 16-byte pieces of `rec` that differ are written back.  The string is
+// taken in chunks of 128 words (a 16-byte piece per lane, 4 KB of float32 output); the lanes' changed sectors are
+// compacted over the warp into `list` (this warp's scratch, 512 entries), then stored 16 sectors per instruction, two
+// adjacent lanes per sector, so that each sector is written whole by one store instruction like in stream_vectors.
+// The head / tail elements outside the full vectors may share a sector with a neighbouring env: they are written as
+// in stream_env, whether they changed or not.
+template <typename T>
+__device__ __forceinline__ void delta_env(const uint32_t* __restrict__ bits, uint32_t* __restrict__ rec, int bits_words,
+                                          int nbits, T* __restrict__ out, int wi, int nw, int lane,
+                                          const uint2* __restrict__ lut, uint16_t* __restrict__ list) {
+    constexpr int VB = kVecElems<T>, SB = 2 * VB;                     // bits per store vector, per 32-byte sector
+    constexpr uint32_t kSectorMask = SB == 32 ? 0xFFFFFFFFu : (1u << SB) - 1u;
+    const int pad = obs_pad(out);
+    const int total = pad + nbits;
+    const int v_begin = (pad + VB - 1) / VB, v_end = total / VB;
+    if (wi == 0) stream_edges<T>(bits, nbits, out, v_begin, v_end, lane);
+    uint4* vp = reinterpret_cast<uint4*>(out - pad);
+    for (int c = wi; 128 * c < bits_words; c += nw) {
+        const int wd = 128 * c + 4 * lane;
+        uint32_t changed = 0;   // bit j: sector j of this lane's 128 bits differs
+        if (wd < bits_words) {
+            const uint4 nv = *reinterpret_cast<const uint4*>(bits + wd);
+            const uint4 ov = *reinterpret_cast<const uint4*>(rec + wd);
+            const uint32_t d[4] = {nv.x ^ ov.x, nv.y ^ ov.y, nv.z ^ ov.z, nv.w ^ ov.w};
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 32 / SB; ++j)
+                    if ((d[i] >> (j * SB)) & kSectorMask) changed |= 1u << (i * (32 / SB) + j);
+            if (changed) *reinterpret_cast<uint4*>(rec + wd) = nv;
+        }
+        const int n = __popc(changed);
+        int incl = n;   // inclusive prefix sum of n over the warp
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(kFull, incl, o);
+            if (lane >= o) incl += t;
+        }
+        const int n_warp = __shfl_sync(kFull, incl, 31);
+        if (n_warp == 0) continue;
+        const int s0 = wd * 32 / SB;
+        for (int pos = incl - n; changed; changed &= changed - 1u) list[pos++] = (uint16_t)(s0 + __ffs(changed) - 1);
+        __syncwarp();
+        for (int i = lane >> 1; i < n_warp; i += 16) {
+            const int v = 2 * list[i] + (lane & 1);
+            if (v >= v_begin && v < v_end) store_vec(vp + v, vector_value<T>(bits, v, lut));
+        }
+        __syncwarp();
+    }
+}
+
+// Copies a block's padded bit string into its record (after a full write); warp `wi` of `nw`.
+__device__ __forceinline__ void refresh_record(const uint32_t* __restrict__ bits, uint32_t* __restrict__ rec, int bits_words,
+                                               int wi, int nw, int lane) {
+    for (int i = wi * 32 + lane; i < bits_words / 4; i += nw * 32)
+        reinterpret_cast<uint4*>(rec)[i] = reinterpret_cast<const uint4*>(bits)[i];
 }
 
 // Packed copy of the observation block for rollout storage: agent a's C*G*G bits start at word a*wpa
@@ -360,6 +439,10 @@ __device__ __forceinline__ void write_obs(const DevPlan& P, const Launch& L, con
     build_obs_bits(P, w, me, rev_mask, pad, lane);
     if (L.obs_bits) store_packed(P, w.bits, pad, L.obs_bits + env * (long long)(P.N * P.wpa), lane);
     if (out) stream_env<T>(w.bits, P.E, out, 0, 1, lane, lut);
+    if (out && L.record) {   // a full write into the bound buffer: the record follows it
+        refresh_record(w.bits, L.record + env * (long long)P.bits_words, P.bits_words, 0, 1, lane);
+        if (lane == 0) L.record_epoch[env] = *L.epoch;
+    }
 }
 
 // Element codes of the metadata block (host-built, DevPlan::meta_codes): the LANE whose value the element takes.
@@ -800,15 +883,26 @@ __device__ __forceinline__ uint32_t step_env(const DevPlan& P, const Launch& L, 
 // 4 warps x 5 resident CTAs and 2 x 9 tie, 8 x 3 (0.987) and 16 x 1 (1.18) lose: the barrier idles too much of the SM.
 // Per-env ready flags instead of the barrier (a block is written by whichever warps are ready) are SLOWER, 0.9825 vs 0.9786 ms,
 // uint8 0.295 vs 0.2835 (profiles/r02_coop_flag.log): the aligned passes are what helps.
-template <typename T, bool STATS, bool HPF>
+//
+// With a record bound to L.obs (ctf_bind_obs_record) an env whose record is valid (its epoch is the current one) is
+// written as a delta (delta_env): only the ~1.3 % of sectors that changed since the last write.  An env whose record
+// is not valid is written in full by stream_env, its record copied from the string and stamped.  Each warp decides for
+// its own env before the barrier, so that no warp of the CTA reads an epoch another warp has already stamped.
+// DELTA (L.record set) is a template parameter: the launches without a record run the code they ran before the record
+// existed (uint8, packed-only and the step logic itself lost 11-15 % when one kernel carried both paths).
+template <typename T, bool STATS, bool HPF, bool DELTA>
 __global__ void __launch_bounds__(kThreads) k_step(const __grid_constant__ DevPlan P, const __grid_constant__ Launch L) {
     extern __shared__ uint4 smem_raw[];
+    __shared__ int s_full[DELTA ? kWarpsPerCta : 1];   // env e of the CTA is written in full
     const uint2* lut = init_expand_lut<T>(smem_raw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long env = (long long)blockIdx.x * kWarpsPerCta + warp;
     unsigned char* base = reinterpret_cast<unsigned char*>(smem_raw) + kLutBytes<T>;
     if (env < L.B) {
         const WarpMem w = warp_mem(P, base, warp);
+        uint32_t* rec = DELTA ? L.record + env * (long long)P.bits_words : nullptr;
+        // the old record is read after the barrier: start moving it into L2 while the env steps
+        if (DELTA && lane * 32 < P.bits_words) asm volatile("prefetch.global.L2 [%0];" ::"l"(rec + lane * 32));
         uint32_t rev_mask;
         const uint32_t me = step_env<STATS, HPF>(P, L, w, env, lane, rev_mask);
         if (L.obs || L.obs_bits) {
@@ -817,13 +911,32 @@ __global__ void __launch_bounds__(kThreads) k_step(const __grid_constant__ DevPl
             build_obs_bits(P, w, me, rev_mask, pad, lane);
             if (L.obs_bits) store_packed(P, w.bits, pad, L.obs_bits + env * (long long)(P.N * P.wpa), lane);
         }
+        if (DELTA && lane == 0) {
+            const uint32_t ep = *L.epoch;
+            const bool full = L.record_epoch[env] != ep;
+            if (full) L.record_epoch[env] = ep;
+            s_full[warp] = full;
+        }
     }
     __syncthreads();
     if (L.obs) {
         for (int e = 0; e < kWarpsPerCta; ++e) {
             const long long env_e = (long long)blockIdx.x * kWarpsPerCta + e;
             if (env_e >= L.B) break;
-            stream_env<T>(warp_mem(P, base, e).bits, P.E, reinterpret_cast<T*>(L.obs) + env_e * (long long)P.E, warp, kWarpsPerCta, lane, lut);
+            const uint32_t* bits = warp_mem(P, base, e).bits;
+            T* out = reinterpret_cast<T*>(L.obs) + env_e * (long long)P.E;
+            if (DELTA) {
+                uint32_t* rec = L.record + env_e * (long long)P.bits_words;
+                if (!s_full[e]) {
+                    delta_env<T>(bits, rec, P.bits_words, P.E, out, warp, kWarpsPerCta, lane, lut,
+                                 reinterpret_cast<uint16_t*>(warp_mem(P, base, warp).list));
+                } else {
+                    stream_env<T>(bits, P.E, out, warp, kWarpsPerCta, lane, lut);
+                    refresh_record(bits, rec, P.bits_words, warp, kWarpsPerCta, lane);
+                }
+            } else {
+                stream_env<T>(bits, P.E, out, warp, kWarpsPerCta, lane, lut);
+            }
         }
     }
 }
@@ -1614,8 +1727,13 @@ struct ctf_env {
     uint8_t* dones_stage;    // device [B]
     size_t smem_bytes;       // warp-per-env kernels writing a plain observation buffer (padded to the residency cap)
     size_t smem_bytes_comp;  // the same kernels writing a compressed one (a different cap, see ctf_create)
+    size_t smem_bytes_delta; // k_step writing the buffer that has a record (delta writes, logic-bound)
     const void* obs_seen;    // the last outputs.obs launched on, and whether it lies in compressed memory
     bool obs_seen_comp;
+    const void* rec_obs;     // ctf_bind_obs_record: the buffer whose record is kept, and the record (device)
+    uint32_t* record;
+    uint32_t* record_epoch;
+    const uint32_t* epoch;
     size_t trunk_smem_bytes; // k_policy_trunk: dynamic shared memory for this plan
     int trunk_ctas;          // k_policy_trunk: CTAs that fit on the device at once
     int grouped_ctas;        // k_policy_trunk_grouped: CTAs that fit on the device at once
@@ -1966,7 +2084,8 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
     if (rc != CTF_OK) { delete h; return rc; }
     h->cfg = *cfg; h->B = num_envs; h->device = device; h->stats_level = stats_level; h->obs_dtype = obs_dtype;
     h->seed = seed; h->env_id_base = env_id_base;
-    h->smem_bytes = (obs_dtype == CTF_OBS_U8 ? kLutBytes<uint8_t> : 0) + (size_t)h->plan.warp_smem_bytes * kWarpsPerCta;
+    const size_t smem_unpadded = (obs_dtype == CTF_OBS_U8 ? kLutBytes<uint8_t> : 0) + (size_t)h->plan.warp_smem_bytes * kWarpsPerCta;
+    h->smem_bytes = smem_unpadded;
     DeviceGuard guard(device);
     cudaError_t e = guard.err;
     if (e == cudaSuccess) e = cudaMalloc(&h->faults, sizeof(uint32_t));
@@ -2008,13 +2127,19 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
         const size_t want_comp = (size_t)(227 * 1024) / (block_bytes >= 12 * 1024 ? 7 : 9) - 1024;
         if (want_comp > h->smem_bytes_comp) h->smem_bytes_comp = want_comp;
     }
+    // Delta writes (ctf_bind_obs_record) store ~1.3 % of the sectors, so the step is bound by the env logic and the
+    // record stream, not by the store stream: the cap is CTF_DELTA_CTAS_PER_SM on plain and compressed memory alike
+    // (the sweep of tools/obs_delta_bench.py, profiles/r10_obs_delta.log).
+    h->smem_bytes_delta = std::max(smem_unpadded, (size_t)(227 * 1024) / CTF_DELTA_CTAS_PER_SM - 1024);
     // The attribute is per kernel, not per handle: give every kernel a ceiling that covers any handle's launch (another
     // handle with a smaller footprint must not lower it under this one's), not this handle's own size.
     const int smem = h->smem_bytes > 100 * 1024 ? (int)h->smem_bytes : 100 * 1024;
 #define CTF_SET_SMEM(K, BYTES) if (e == cudaSuccess) e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES)
 #define CTF_SET_SMEM_T(T)                                                                                       \
-    CTF_SET_SMEM((k_step<T, false, false>), smem); CTF_SET_SMEM((k_step<T, true, false>), smem);               \
-    CTF_SET_SMEM((k_step<T, false, true>), smem); CTF_SET_SMEM((k_step<T, true, true>), smem);                 \
+    CTF_SET_SMEM((k_step<T, false, false, false>), smem); CTF_SET_SMEM((k_step<T, true, false, false>), smem); \
+    CTF_SET_SMEM((k_step<T, false, true, false>), smem); CTF_SET_SMEM((k_step<T, true, true, false>), smem);   \
+    CTF_SET_SMEM((k_step<T, false, false, true>), smem); CTF_SET_SMEM((k_step<T, true, false, true>), smem);   \
+    CTF_SET_SMEM((k_step<T, false, true, true>), smem); CTF_SET_SMEM((k_step<T, true, true, true>), smem);     \
     CTF_SET_SMEM((k_reset<T, false>), smem); CTF_SET_SMEM((k_reset<T, true>), smem); CTF_SET_SMEM((k_observe<T>), smem); \
     CTF_SET_SMEM((k_unpack<T>), smem)
     CTF_SET_SMEM_T(float); CTF_SET_SMEM_T(uint8_t); CTF_SET_SMEM_T(__half); CTF_SET_SMEM_T(__nv_bfloat16);
@@ -2078,6 +2203,41 @@ extern "C" int ctf_get_sizes(ctf_handle_t h, ctf_sizes_t* s) {
     return CTF_OK;
 }
 
+// [a, a + a_bytes) and [b, b + b_bytes) share a byte
+static bool overlaps(const void* a, size_t a_bytes, const void* b, size_t b_bytes) {
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+    return x < y + b_bytes && y < x + a_bytes;
+}
+
+extern "C" int ctf_obs_record_size(ctf_handle_t h, size_t* record_bytes) {
+    if (!h || !record_bytes) return fail(CTF_ERR_INVALID, "null argument");
+    *record_bytes = (size_t)h->B * h->plan.bits_words * sizeof(uint32_t);
+    return CTF_OK;
+}
+
+extern "C" int ctf_bind_obs_record(ctf_handle_t h, const void* obs, uint32_t* record, uint32_t* record_epoch,
+                                   const uint32_t* epoch) {
+    if (!h) return fail(CTF_ERR_INVALID, "null handle");
+    if (!obs) {
+        h->rec_obs = nullptr; h->record = nullptr; h->record_epoch = nullptr; h->epoch = nullptr;
+        return CTF_OK;
+    }
+    if (!record || !record_epoch || !epoch)
+        return fail(CTF_ERR_INVALID, "ctf_bind_obs_record: record, record_epoch and epoch must not be null");
+    if ((reinterpret_cast<uintptr_t>(record) & 15) || (reinterpret_cast<uintptr_t>(record_epoch) & 3) ||
+        (reinterpret_cast<uintptr_t>(epoch) & 3))
+        return fail(CTF_ERR_INVALID, "ctf_bind_obs_record: record must be 16-byte, record_epoch and epoch 4-byte aligned");
+    const size_t elem = h->obs_dtype == CTF_OBS_F32 ? 4 : (h->obs_dtype == CTF_OBS_U8 ? 1 : 2);
+    const size_t obs_bytes = (size_t)h->B * h->plan.E * elem, rec_bytes = (size_t)h->B * h->plan.bits_words * 4;
+    const size_t ep_bytes = (size_t)h->B * 4;
+    if (overlaps(obs, obs_bytes, record, rec_bytes) || overlaps(obs, obs_bytes, record_epoch, ep_bytes) ||
+        overlaps(obs, obs_bytes, epoch, 4) || overlaps(record, rec_bytes, record_epoch, ep_bytes) ||
+        overlaps(record, rec_bytes, epoch, 4) || overlaps(record_epoch, ep_bytes, epoch, 4))
+        return fail(CTF_ERR_INVALID, "ctf_bind_obs_record: obs, record, record_epoch and epoch must not overlap");
+    h->rec_obs = obs; h->record = record; h->record_epoch = record_epoch; h->epoch = epoch;
+    return CTF_OK;
+}
+
 static int make_launch(ctf_handle_t h, const ctf_state_t& st, const ctf_outputs_t& out, Launch& L) {
     if (!st.grid || !st.agents || !st.envs) return fail(CTF_ERR_INVALID, "state.grid/agents/envs must not be null");
     if (h->stats_level > 0 && !st.stats) return fail(CTF_ERR_INVALID, "state.stats is null but the handle was created with stats");
@@ -2095,6 +2255,9 @@ static int make_launch(ctf_handle_t h, const ctf_state_t& st, const ctf_outputs_
     L.visits = h->stats_level > 1 ? st.visits : nullptr;
     L.obs = out.obs; L.obs_bits = out.obs_bits; L.meta = out.meta; L.rewards = out.rewards; L.dones = out.dones;
     L.faults = h->faults;
+    if (out.obs && out.obs == h->rec_obs) {
+        L.record = h->record; L.record_epoch = h->record_epoch; L.epoch = h->epoch;
+    }
     L.B = h->B;
     L.seed_lo = (uint32_t)(h->seed & 0xFFFFFFFFu); L.seed_hi = (uint32_t)(h->seed >> 32);
     L.env_id_base = (uint32_t)h->env_id_base;
@@ -2151,12 +2314,13 @@ extern "C" int ctf_reset(ctf_handle_t h, ctf_state_t st, ctf_outputs_t out, int 
 static int launch_step(ctf_handle_t h, const Launch& L, cudaStream_t s) {
     const bool stats = h->stats_level > 0;
     const bool hpf = h->plan.hp_float != 0;
-    const size_t smem = launch_smem(h, L.obs);
+    const size_t smem = L.record ? h->smem_bytes_delta : launch_smem(h, L.obs);
     with_obs_type(h->obs_dtype, [&](auto tag) {
         using T = decltype(tag);
         auto launch = [&](auto stats_c, auto hpf_c) {
             constexpr bool S = decltype(stats_c)::value, F = decltype(hpf_c)::value;
-            k_step<T, S, F><<<grid_dim(h->B), kThreads, smem, s>>>(h->plan, L);
+            if (L.record) k_step<T, S, F, true><<<grid_dim(h->B), kThreads, smem, s>>>(h->plan, L);
+            else k_step<T, S, F, false><<<grid_dim(h->B), kThreads, smem, s>>>(h->plan, L);
         };
         if (stats) { if (hpf) launch(std::true_type{}, std::true_type{}); else launch(std::true_type{}, std::false_type{}); }
         else { if (hpf) launch(std::false_type{}, std::true_type{}); else launch(std::false_type{}, std::false_type{}); }
@@ -2498,12 +2662,6 @@ extern "C" int ctf_step_host(ctf_handle_t h, ctf_state_t st, const uint8_t* acti
     if (d_copy) CTF_CUDA(cudaMemcpyAsync(dones_host, out.dones, (size_t)h->B, cudaMemcpyDeviceToHost, s));
     CTF_CUDA(cudaStreamSynchronize(s));
     return CTF_OK;
-}
-
-// [a, a + a_bytes) and [b, b + b_bytes) share a byte
-static bool overlaps(const void* a, size_t a_bytes, const void* b, size_t b_bytes) {
-    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
-    return x < y + b_bytes && y < x + a_bytes;
 }
 
 // ctf_gae and ctf_gae_dones: checks every argument, then launches k_gae<dones != nullptr>.  `fn` names the entry point
