@@ -309,7 +309,7 @@ int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uin
  * the weights table), an env range, k agent ids and the feature row of its sample 0.  Its sample s = e*k + j
  * (e < n_envs, j < k) reads packed block (env_begin + e)*agents_per_env + agent_ids[j] and the metadata row with the
  * same index, as ctf_policy_features does, and writes feature row out_row + s.  Every row is bit-identical to what
- * ctf_policy_features writes with that segment's weights for the same sample (the kernels share the per-sample code).
+ * ctf_policy_features writes with that segment's weights for the same sample (both entry points run the same kernel).
  * Rows outside every segment are not written.
  * Scheduling: the samples are cut into tiles of 8 consecutive samples of one segment, in table order; every CTA takes
  * a contiguous range of tiles and restages conv weights in shared memory only where the policy changes, so put the
@@ -342,8 +342,9 @@ int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weights_t* weig
                                 const float* meta, int64_t n_envs, int agents_per_env, void* features,
                                 int64_t feature_stride, int64_t n_rows, void* stream);
 
-/* CTAs the trunk kernels run at most per launch on this handle (the device's SMs times the CTAs resident per SM for
-   this plan, counted at ctf_create): k_policy_trunk (ctf_policy_features) and k_policy_trunk_grouped. */
+/* CTAs the trunk kernel runs at most per launch on this handle (the device's SMs times the CTAs resident per SM for
+   this plan, counted at ctf_create), for each of its two instantiations: trunk_ctas for launches with one policy and
+   one segment (every ctf_policy_features call), grouped_ctas for every other ctf_policy_features_grouped call. */
 int ctf_policy_trunk_ctas(ctf_handle_t h, int* trunk_ctas, int* grouped_ctas);
 
 /* fp32 gradients of the trunk's parameters in torch layout (device memory). */

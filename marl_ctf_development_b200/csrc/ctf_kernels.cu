@@ -999,7 +999,7 @@ __global__ void k_stats_sum(const uint32_t* __restrict__ stats, long long B, int
 // ------------------------------------------------------------------------------------------------
 // policy trunk from packed observations: conv1 (sparse, fp32) -> tanh -> conv2 (mma.sync bf16) -> tanh -> fc1 input rows
 // ------------------------------------------------------------------------------------------------
-// One warp owns one sample at a time (grid-stride over samples); the CTA's warps share the conv weights in shared memory.
+// One warp owns one sample at a time; the CTA's warps share the conv weights in shared memory.
 // Per sample: the wpa packed words are staged, a per-cell channel mask is built from them, conv1 accumulates for every
 // output position the bias plus the weight columns of the set (cell, channel) pairs of its 3x3 window (exact for any
 // {0,1} input; cost grows with the number of set bits), and stores tanh as bf16 in a [position][16 channels] tile.
@@ -1010,22 +1010,17 @@ constexpr int kTrunkWarps = 8;
 constexpr int kTrunkThreads = kTrunkWarps * 32;
 constexpr int kTrunkW2Words = 9 * 4 * 32 * 2;   // conv2 B fragments: [tap][n-tile][lane][2 x bf16x2]
 
-struct TrunkArgs {
-    const float* conv1_w;
-    const float* conv1_b;
-    const uint2* conv2_w;
-    const float* conv2_b;
+// what every trunk launch reads, whatever its policies and segments: shapes, shared-memory layout, inputs and output
+struct TrunkGeometry {
     const uint32_t* packed;
     const float* meta;
     __nv_bfloat16* features;
-    long long n_samples;
     long long stride;
-    int ape, k;
+    int ape;
     int G, C, GG, wpa, M;
     int S1, S2;              // conv1 / conv2 output side
     int warp_words;          // shared-memory words per warp
     int off_mask, off_act, off_stage;   // word offsets inside a warp's region
-    unsigned char ids[CTF_MAX_AGENTS];
 };
 
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
@@ -1081,10 +1076,9 @@ __device__ __forceinline__ void trunk_conv1(const uint32_t* bits, uint16_t* cmas
     }
 }
 
-// Copies one policy's conv weights into the CTA's shared memory for k_policy_trunk_grouped: conv1 as [C*9][16] columns,
-// the biases, the conv2 B fragments; the same copy k_policy_trunk makes at its start (which keeps its own inline
-// statement of it: calling this helper there changes that kernel's instruction schedule).  The caller synchronises the
-// CTA after it, and before it when other warps may still read the previous policy's weights.
+// Copies one policy's conv weights into the CTA's shared memory for k_policy_trunk: conv1 as [C*9][16] columns, the
+// biases, the conv2 B fragments.  The caller synchronises the CTA after it, and before it when other warps may still
+// read the previous policy's weights.
 __device__ __forceinline__ void trunk_stage_weights(const float* conv1_w, const float* conv1_b, const uint2* conv2_w,
                                                     const float* conv2_b, int C, float* w1, float* b1, float* b2, uint2* w2) {
     for (int i = threadIdx.x; i < C * 9 * 16; i += kTrunkThreads) {
@@ -1098,8 +1092,8 @@ __device__ __forceinline__ void trunk_stage_weights(const float* conv1_w, const 
 
 // One sample of the trunk, computed by one warp with the weights staged in shared memory: stages packed block `blk`
 // (A.packed, A.wpa words), conv1 (trunk_conv1), conv2 on tensor cores, tanh, bf16, then the metadata row `blk` and
-// zeros up to A.stride, into feature row `r` of A.features.  k_policy_trunk and k_policy_trunk_grouped both run exactly this code.
-__device__ __forceinline__ void trunk_sample(const TrunkArgs& A, long long blk, long long r, const float* w1,
+// zeros up to A.stride, into feature row `r` of A.features.
+__device__ __forceinline__ void trunk_sample(const TrunkGeometry& A, long long blk, long long r, const float* w1,
                                              const float* b1, const float* b2, const uint2* w2, uint32_t* bits,
                                              uint16_t* cmask, uint32_t* act, __nv_bfloat16* stage, int lane, int C, int G,
                                              int GG, int S1, int S2, int M2, int g, int t, int n_mt, long long conv_elems) {
@@ -1162,43 +1156,8 @@ __device__ __forceinline__ void trunk_sample(const TrunkArgs& A, long long blk, 
     __syncwarp();
 }
 
-__global__ void __launch_bounds__(kTrunkThreads) k_policy_trunk(const __grid_constant__ TrunkArgs A) {
-    extern __shared__ uint4 smem_raw[];
-    float* w1 = reinterpret_cast<float*>(smem_raw);                      // [C*9][16]: column of one (c, dy, dx) tap
-    float* b1 = w1 + A.C * 9 * 16;                                        // [16]
-    float* b2 = b1 + 16;                                                  // [32]
-    uint2* w2 = reinterpret_cast<uint2*>(b2 + 32);                        // [9][4][32]
-    uint32_t* warp_base = reinterpret_cast<uint32_t*>(w2 + kTrunkW2Words / 2);
-    const int C = A.C, G = A.G, GG = A.GG, S1 = A.S1, S2 = A.S2, M2 = S2 * S2;
-    for (int i = threadIdx.x; i < C * 9 * 16; i += kTrunkThreads) {
-        const int o = i & 15, tap = i >> 4;                              // tap = c*9 + dy*3 + dx
-        w1[i] = A.conv1_w[o * C * 9 + tap];
-    }
-    if (threadIdx.x < 16) b1[threadIdx.x] = A.conv1_b[threadIdx.x];
-    if (threadIdx.x < 32) b2[threadIdx.x] = A.conv2_b[threadIdx.x];
-    for (int i = threadIdx.x; i < kTrunkW2Words / 2; i += kTrunkThreads) w2[i] = A.conv2_w[i];
-    __syncthreads();
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t* bits = warp_base + (size_t)warp * A.warp_words;                           // [wpa]
-    uint16_t* cmask = reinterpret_cast<uint16_t*>(bits + A.off_mask);                   // [GG] channel mask per cell
-    uint32_t* act = bits + A.off_act;                                                    // [S1*S1][8] bf16x2
-    __nv_bfloat16* stage = reinterpret_cast<__nv_bfloat16*>(bits + A.off_stage);        // [8][M2]
-    const int g = lane >> 2, t = lane & 3;
-    const int n_mt = (M2 + 15) >> 4;
-    const long long conv_elems = 32LL * M2;
-
-    for (long long s = (long long)blockIdx.x * kTrunkWarps + warp; s < A.n_samples; s += (long long)gridDim.x * kTrunkWarps) {
-        const long long e = s / A.k;
-        const int j = (int)(s - e * A.k);
-        const long long blk = e * A.ape + A.ids[j];
-        trunk_sample(A, blk, s, w1, b1, b2, w2, bits, cmask, act, stage, lane, C, G, GG, S1, S2,
-                     M2, g, t, n_mt, conv_elems);
-    }
-}
-
 // shared-memory layout of k_policy_trunk for a plan: bytes of the CTA-wide weights, words per warp and the offsets
-static __host__ void trunk_layout(const DevPlan& P, TrunkArgs& A, size_t& smem) {
+static __host__ void trunk_layout(const DevPlan& P, TrunkGeometry& A, size_t& smem) {
     const int S1 = P.G - 2, S2 = P.G - 4;
     const auto up4 = [](int w) { return (w + 3) & ~3; };                 // 16-byte alignment in words
     A.G = P.G; A.C = P.C; A.GG = P.GG; A.wpa = P.wpa; A.M = P.M; A.S1 = S1; A.S2 = S2;
@@ -1210,15 +1169,13 @@ static __host__ void trunk_layout(const DevPlan& P, TrunkArgs& A, size_t& smem) 
     smem = (shared_words + (size_t)kTrunkWarps * A.warp_words) * 4;
 }
 
-// ------------------------------------------------------------------------------------------------
-// grouped policy trunk: the samples of many (policy, env range, agent ids) segments in one launch
-// ------------------------------------------------------------------------------------------------
-// The segments' samples are cut into tiles of kTrunkWarps consecutive samples of one segment (a segment's last tile may
-// be shorter); the host numbers the tiles in table order (TrunkSegment::tile_begin).  CTA b takes the contiguous tile
-// range [n_tiles*b/grid, n_tiles*(b+1)/grid) and warp w computes sample w of each tile with k_policy_trunk's own
-// per-sample code (trunk_sample).  The CTA stages a policy's conv weights only when its next tile belongs to a different
-// policy than the one staged, between two __syncthreads(): with the segments of a policy adjacent in the table, a CTA
-// restages at most once per policy boundary inside its range.  Warps sync with each other only there.
+// One launch computes the samples of one or more (policy, env range, agent ids) segments.  The segments' samples are
+// cut into tiles of kTrunkWarps consecutive samples of one segment (a segment's last tile may be shorter); the host
+// numbers the tiles in table order (TrunkSegment::tile_begin).  CTA b takes the contiguous tile range
+// [n_tiles*b/grid, n_tiles*(b+1)/grid) and warp w computes sample w of each tile (trunk_sample).  The CTA stages a
+// policy's conv weights only when its next tile belongs to a different policy than the one staged, between two
+// __syncthreads(): with the segments of a policy adjacent in the table, a CTA restages at most once per policy
+// boundary inside its range.  Warps sync with each other only there.
 struct TrunkSegment {
     long long blk_begin;     // env_begin * agents_per_env: the packed block of env 0 of the segment, agent 0
     long long row_begin;     // feature row of sample 0
@@ -1235,60 +1192,84 @@ struct TrunkPolicyWeights {
     const float* conv2_b;
 };
 
-struct TrunkGroupedArgs {
-    TrunkArgs geo;           // shapes, shared-memory layout, packed / meta / features / stride / ape (conv*_w, n_samples,
-                             // k and ids unused)
+// The argument block of one launch, passed by value.  Two sizes are instantiated: <1, 1> for a launch with one policy
+// and one segment (every ctf_policy_features call), so that the per-pair league path, which is bound by the host,
+// does not ship the grouped tables; <CTF_GROUPED_MAX_POLICIES, CTF_GROUPED_MAX_SEGMENTS> for every other launch.
+template <int kMaxPolicies, int kMaxSegments>
+struct TrunkLaunch {
+    TrunkGeometry geo;
     long long n_tiles;
     int n_segments, pad;
-    TrunkPolicyWeights w[CTF_GROUPED_MAX_POLICIES];
-    TrunkSegment seg[CTF_GROUPED_MAX_SEGMENTS];
+    TrunkPolicyWeights w[kMaxPolicies];
+    TrunkSegment seg[kMaxSegments];
 };
-static_assert(sizeof(TrunkGroupedArgs) <= 32764, "kernel parameters are limited to 32 764 bytes");
+using TrunkLaunchOne = TrunkLaunch<1, 1>;
+using TrunkLaunchGrouped = TrunkLaunch<CTF_GROUPED_MAX_POLICIES, CTF_GROUPED_MAX_SEGMENTS>;
+static_assert(sizeof(TrunkLaunchOne) <= 256, "a single-policy launch keeps a parameter block of a few hundred bytes");
+static_assert(sizeof(TrunkLaunchGrouped) <= 32764, "kernel parameters are limited to 32 764 bytes");
 
-// The register cap (5 CTAs of 256 threads per SM) holds it to k_policy_trunk's 48 registers, no spills: unbounded, the
-// compiler keeps segment fields live and takes 126, which would cap residency below k_policy_trunk's on small maps.
-__global__ void __launch_bounds__(kTrunkThreads, 5) k_policy_trunk_grouped(const __grid_constant__ TrunkGroupedArgs A) {
+// Both instantiations run one schedule; <1, 1> compiles out the segment search, walk and policy compare and stages its
+// one policy's weights before its tiles.  The register cap (5 CTAs of 256 threads per SM) holds both to 48 registers,
+// no spills; unbounded they take 126 (grouped) and 111 (<1, 1>), which would cap their residency on small maps.
+template <int kMaxPolicies, int kMaxSegments>
+__global__ void __launch_bounds__(kTrunkThreads, 5)
+k_policy_trunk(const __grid_constant__ TrunkLaunch<kMaxPolicies, kMaxSegments> A) {
     extern __shared__ uint4 smem_raw[];
-    const TrunkArgs& T = A.geo;
-    float* w1 = reinterpret_cast<float*>(smem_raw);                      // the layout of k_policy_trunk
-    float* b1 = w1 + T.C * 9 * 16;
-    float* b2 = b1 + 16;
-    uint2* w2 = reinterpret_cast<uint2*>(b2 + 32);
+    const TrunkGeometry& T = A.geo;
+    float* w1 = reinterpret_cast<float*>(smem_raw);                      // [C*9][16]: column of one (c, dy, dx) tap
+    float* b1 = w1 + T.C * 9 * 16;                                        // [16]
+    float* b2 = b1 + 16;                                                  // [32]
+    uint2* w2 = reinterpret_cast<uint2*>(b2 + 32);                        // [9][4][32]
     uint32_t* warp_base = reinterpret_cast<uint32_t*>(w2 + kTrunkW2Words / 2);
     const int C = T.C, G = T.G, GG = T.GG, S1 = T.S1, S2 = T.S2, M2 = S2 * S2;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t* bits = warp_base + (size_t)warp * T.warp_words;
-    uint16_t* cmask = reinterpret_cast<uint16_t*>(bits + T.off_mask);
-    uint32_t* act = bits + T.off_act;
-    __nv_bfloat16* stage = reinterpret_cast<__nv_bfloat16*>(bits + T.off_stage);
+    uint32_t* bits = warp_base + (size_t)warp * T.warp_words;                           // [wpa]
+    uint16_t* cmask = reinterpret_cast<uint16_t*>(bits + T.off_mask);                   // [GG] channel mask per cell
+    uint32_t* act = bits + T.off_act;                                                    // [S1*S1][8] bf16x2
+    __nv_bfloat16* stage = reinterpret_cast<__nv_bfloat16*>(bits + T.off_stage);        // [8][M2]
     const int g = lane >> 2, t = lane & 3;
     const int n_mt = (M2 + 15) >> 4;
     const long long conv_elems = 32LL * M2;
 
     const long long t0 = A.n_tiles * blockIdx.x / gridDim.x, t1 = A.n_tiles * (blockIdx.x + 1) / gridDim.x;
-    // the segment of tile t0: the last one whose first tile is <= t0 (empty segments share their successor's tile_begin)
-    int lo = 0, hi = A.n_segments - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (A.seg[mid].tile_begin <= t0) lo = mid; else hi = mid - 1;
-    }
-    int si = lo, staged = -1;
-    for (long long tile = t0; tile < t1; ++tile) {
-        while (si + 1 < A.n_segments && A.seg[si + 1].tile_begin <= tile) ++si;
-        const TrunkSegment& S = A.seg[si];
-        if (S.policy != staged) {
-            __syncthreads();
-            const TrunkPolicyWeights& W = A.w[S.policy];
-            trunk_stage_weights(W.conv1_w, W.conv1_b, W.conv2_w, W.conv2_b, C, w1, b1, b2, w2);
-            __syncthreads();
-            staged = S.policy;
-        }
-        const long long s = (tile - S.tile_begin) * kTrunkWarps + warp;
-        if (s < S.n_samples) {
+    if constexpr (kMaxSegments == 1) {
+        // one segment of one policy: its weights are staged once, and the CTA's tiles are its samples in order
+        const TrunkSegment& S = A.seg[0];
+        const TrunkPolicyWeights& W = A.w[0];
+        trunk_stage_weights(W.conv1_w, W.conv1_b, W.conv2_w, W.conv2_b, C, w1, b1, b2, w2);
+        __syncthreads();
+        const long long s1 = min(t1 * kTrunkWarps, S.n_samples);
+        for (long long s = t0 * kTrunkWarps + warp; s < s1; s += kTrunkWarps) {
             const long long e = s / S.k;
             const int j = (int)(s - e * S.k);
             trunk_sample(T, S.blk_begin + e * T.ape + S.ids[j], S.row_begin + s, w1, b1, b2, w2, bits, cmask, act, stage,
                          lane, C, G, GG, S1, S2, M2, g, t, n_mt, conv_elems);
+        }
+    } else {
+        // the segment of tile t0: the last whose first tile is <= t0 (empty segments share their successor's tile_begin)
+        int lo = 0, hi = A.n_segments - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (A.seg[mid].tile_begin <= t0) lo = mid; else hi = mid - 1;
+        }
+        int si = lo, staged = -1;
+        for (long long tile = t0; tile < t1; ++tile) {
+            while (si + 1 < A.n_segments && A.seg[si + 1].tile_begin <= tile) ++si;
+            const TrunkSegment& S = A.seg[si];
+            if (S.policy != staged) {
+                __syncthreads();
+                const TrunkPolicyWeights& W = A.w[S.policy];
+                trunk_stage_weights(W.conv1_w, W.conv1_b, W.conv2_w, W.conv2_b, C, w1, b1, b2, w2);
+                __syncthreads();
+                staged = S.policy;
+            }
+            const long long s = (tile - S.tile_begin) * kTrunkWarps + warp;
+            if (s < S.n_samples) {
+                const long long e = s / S.k;
+                const int j = (int)(s - e * S.k);
+                trunk_sample(T, S.blk_begin + e * T.ape + S.ids[j], S.row_begin + s, w1, b1, b2, w2, bits, cmask, act,
+                             stage, lane, C, G, GG, S1, S2, M2, g, t, n_mt, conv_elems);
+            }
         }
     }
 }
@@ -1735,8 +1716,8 @@ struct ctf_env {
     uint32_t* record_epoch;
     const uint32_t* epoch;
     size_t trunk_smem_bytes; // k_policy_trunk: dynamic shared memory for this plan
-    int trunk_ctas;          // k_policy_trunk: CTAs that fit on the device at once
-    int grouped_ctas;        // k_policy_trunk_grouped: CTAs that fit on the device at once
+    int trunk_ctas;          // k_policy_trunk<1, 1>: CTAs that fit on the device at once
+    int grouped_ctas;        // k_policy_trunk<CTF_GROUPED_MAX_POLICIES, CTF_GROUPED_MAX_SEGMENTS>: the same
     size_t bwd_smem_bytes;   // k_policy_trunk_backward: dynamic shared memory for this plan
     int bwd_ctas;            // k_policy_trunk_backward: CTAs (= workspace rows) of every launch with >= bwd_ctas samples
 };
@@ -2152,13 +2133,14 @@ extern "C" int ctf_create(const ctf_config_t* cfg, int64_t num_envs, int device,
             e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem_bytes);
         return (per_sm > 0 ? per_sm : 1) * (n_sm > 0 ? n_sm : 1);
     };
-    TrunkArgs ta;
-    trunk_layout(h->plan, ta, h->trunk_smem_bytes);
+    TrunkGeometry tg;
+    trunk_layout(h->plan, tg, h->trunk_smem_bytes);
     TrunkBwdArgs ba;
     trunk_bwd_layout(h->plan, ba, h->bwd_smem_bytes);
-    // k_policy_trunk needs at most 94 KB (G = 16, C = 14); k_policy_trunk_grouped has its shared-memory layout
-    h->trunk_ctas = trunk_ctas(k_policy_trunk, kTrunkThreads, 100 * 1024, h->trunk_smem_bytes);
-    h->grouped_ctas = trunk_ctas(k_policy_trunk_grouped, kTrunkThreads, 100 * 1024, h->trunk_smem_bytes);
+    // k_policy_trunk needs at most 94 KB (G = 16, C = 14)
+    h->trunk_ctas = trunk_ctas(k_policy_trunk<1, 1>, kTrunkThreads, 100 * 1024, h->trunk_smem_bytes);
+    h->grouped_ctas = trunk_ctas(k_policy_trunk<CTF_GROUPED_MAX_POLICIES, CTF_GROUPED_MAX_SEGMENTS>, kTrunkThreads,
+                                 100 * 1024, h->trunk_smem_bytes);
     // k_policy_trunk_backward needs at most 46 KB (G = 16, C = 14)
     h->bwd_ctas = trunk_ctas(k_policy_trunk_backward, kBwdThreads, 64 * 1024, h->bwd_smem_bytes);
 #undef CTF_SET_SMEM_T
@@ -2427,44 +2409,44 @@ static int check_trunk_weights(const char* fn, const ctf_policy_weights_t& w, bo
     return CTF_OK;
 }
 
-extern "C" int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uint32_t* packed, const float* meta,
-                                   int64_t n_envs, int agents_per_env, const uint8_t* agent_ids, int k, void* features,
-                                   int64_t feature_stride, void* stream) {
-    const char* fn = "ctf_policy_features";
-    if (!h || !w || !packed || !meta || !agent_ids || !features) return fail(CTF_ERR_INVALID, "%s: null argument", fn);
-    const DevPlan& P = h->plan;
-    int rc = check_trunk_geometry(fn, P, n_envs, agents_per_env, feature_stride);
-    if (rc == CTF_OK) rc = check_agent_ids(fn, "k", agent_ids, k, agents_per_env);
-    if (rc == CTF_OK) rc = check_trunk_weights(fn, *w, true);
-    if (rc != CTF_OK) return rc;
-    if (reinterpret_cast<uintptr_t>(features) & 15) return fail(CTF_ERR_INVALID, "%s: features must be 16-byte aligned", fn);
-    if ((reinterpret_cast<uintptr_t>(packed) & 3) || (reinterpret_cast<uintptr_t>(meta) & 3))
-        return fail(CTF_ERR_INVALID, "%s: misaligned inputs", fn);
-    const long long n = (long long)n_envs * k;
-    if (n == 0) return CTF_OK;
-    TrunkArgs A;
+// Fills the argument block of one trunk launch from checked arguments with at least one sample and launches
+// k_policy_trunk with that block's table sizes on at most `ctas` CTAs.
+template <int kMaxPolicies, int kMaxSegments>
+static void launch_trunk_table(TrunkLaunch<kMaxPolicies, kMaxSegments>& A, const TrunkGeometry& geo,
+                               const ctf_policy_weights_t* weights, int n_policies, const ctf_policy_segment_t* segments,
+                               int n_segments, int agents_per_env, int ctas, size_t smem, cudaStream_t stream) {
     memset(&A, 0, sizeof(A));
-    size_t smem = 0;
-    trunk_layout(P, A, smem);
-    A.conv1_w = w->conv1_w; A.conv1_b = w->conv1_b; A.conv2_w = static_cast<const uint2*>(w->conv2_w); A.conv2_b = w->conv2_b;
-    A.packed = packed; A.meta = meta; A.features = static_cast<__nv_bfloat16*>(features);
-    A.n_samples = n; A.stride = feature_stride; A.ape = agents_per_env; A.k = k;
-    for (int j = 0; j < k; ++j) A.ids[j] = agent_ids[j];
-    DeviceGuard guard(h->device);
-    CTF_CUDA(guard.err);
-    const long long want = (n + kTrunkWarps - 1) / kTrunkWarps;
-    const unsigned grid = (unsigned)(want < h->trunk_ctas ? want : h->trunk_ctas);
-    k_policy_trunk<<<grid, kTrunkThreads, smem, static_cast<cudaStream_t>(stream)>>>(A);
-    CTF_CUDA(cudaGetLastError());
-    return CTF_OK;
+    A.geo = geo;
+    for (int p = 0; p < n_policies; ++p) {
+        const ctf_policy_weights_t& w = weights[p];
+        A.w[p].conv1_w = w.conv1_w; A.w[p].conv1_b = w.conv1_b;
+        A.w[p].conv2_w = static_cast<const uint2*>(w.conv2_w); A.w[p].conv2_b = w.conv2_b;
+    }
+    long long tiles = 0;
+    for (int i = 0; i < n_segments; ++i) {
+        const ctf_policy_segment_t& g = segments[i];
+        TrunkSegment& T = A.seg[i];
+        T.blk_begin = g.env_begin * agents_per_env;
+        T.row_begin = g.out_row;
+        T.n_samples = g.n_envs * g.k;
+        T.tile_begin = tiles;
+        T.policy = g.policy;
+        T.k = g.k;
+        for (int j = 0; j < g.k; ++j) T.ids[j] = g.agent_ids[j];
+        tiles += (T.n_samples + kTrunkWarps - 1) / kTrunkWarps;
+    }
+    A.n_tiles = tiles;
+    A.n_segments = n_segments;
+    const unsigned grid = (unsigned)(tiles < ctas ? tiles : ctas);
+    k_policy_trunk<kMaxPolicies, kMaxSegments><<<grid, kTrunkThreads, smem, stream>>>(A);
 }
 
-extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weights_t* weights, int n_policies,
-                                           const ctf_policy_segment_t* segments, int n_segments, const uint32_t* packed,
-                                           const float* meta, int64_t n_envs, int agents_per_env, void* features,
-                                           int64_t feature_stride, int64_t n_rows, void* stream) {
-    const char* fn = "ctf_policy_features_grouped";
-    if (!h || !weights || !segments || !packed || !meta || !features) return fail(CTF_ERR_INVALID, "%s: null argument", fn);
+// The forward trunk of both entry points: checks every argument, then launches k_policy_trunk<1, 1> for one policy and
+// one segment, the grouped instantiation otherwise.  Errors name the entry point `fn` and call a segment's k `k_name`.
+static int launch_trunk(const char* fn, const char* k_name, ctf_handle_t h, const ctf_policy_weights_t* weights,
+                        int n_policies, const ctf_policy_segment_t* segments, int n_segments, const uint32_t* packed,
+                        const float* meta, int64_t n_envs, int agents_per_env, void* features, int64_t feature_stride,
+                        int64_t n_rows, void* stream) {
     const DevPlan& P = h->plan;
     int rc = check_trunk_geometry(fn, P, n_envs, agents_per_env, feature_stride);
     if (rc != CTF_OK) return rc;
@@ -2476,57 +2458,72 @@ extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weig
     if (reinterpret_cast<uintptr_t>(features) & 15) return fail(CTF_ERR_INVALID, "%s: features must be 16-byte aligned", fn);
     if ((reinterpret_cast<uintptr_t>(packed) & 3) || (reinterpret_cast<uintptr_t>(meta) & 3))
         return fail(CTF_ERR_INVALID, "%s: misaligned inputs", fn);
-    // the argument block is large (about 26 KB): keep it off the caller's stack
-    static thread_local TrunkGroupedArgs A;
-    memset(&A, 0, sizeof(A));
-    size_t smem = 0;
-    trunk_layout(P, A.geo, smem);
-    for (int p = 0; p < n_policies; ++p) {
-        const ctf_policy_weights_t& w = weights[p];
-        if ((rc = check_trunk_weights(fn, w, true)) != CTF_OK) return rc;
-        A.w[p].conv1_w = w.conv1_w; A.w[p].conv1_b = w.conv1_b;
-        A.w[p].conv2_w = static_cast<const uint2*>(w.conv2_w); A.w[p].conv2_b = w.conv2_b;
-    }
-    long long tiles = 0;
+    for (int p = 0; p < n_policies; ++p)
+        if ((rc = check_trunk_weights(fn, weights[p], true)) != CTF_OK) return rc;
     int order[CTF_GROUPED_MAX_SEGMENTS];
     int n_busy = 0;
     for (int i = 0; i < n_segments; ++i) {
         const ctf_policy_segment_t& g = segments[i];
         if (g.policy < 0 || g.policy >= n_policies)
             return fail(CTF_ERR_INVALID, "%s: a segment's policy index is out of range", fn);
-        if ((rc = check_agent_ids(fn, "a segment's k", g.agent_ids, g.k, agents_per_env)) != CTF_OK) return rc;
+        if ((rc = check_agent_ids(fn, k_name, g.agent_ids, g.k, agents_per_env)) != CTF_OK) return rc;
         if (g.env_begin < 0 || g.n_envs < 0 || g.env_begin > n_envs || g.n_envs > n_envs - g.env_begin)
             return fail(CTF_ERR_INVALID, "%s: a segment's env range is outside [0, n_envs)", fn);
         const long long ns = g.n_envs * g.k;
         if (g.out_row < 0 || g.out_row > n_rows || ns > n_rows - g.out_row)
             return fail(CTF_ERR_INVALID, "%s: a segment's output rows are outside [0, n_rows)", fn);
-        TrunkSegment& S = A.seg[i];
-        S.blk_begin = g.env_begin * agents_per_env;
-        S.row_begin = g.out_row;
-        S.n_samples = ns;
-        S.tile_begin = tiles;
-        S.policy = g.policy;
-        S.k = g.k;
-        for (int j = 0; j < g.k; ++j) S.ids[j] = g.agent_ids[j];
-        tiles += (ns + kTrunkWarps - 1) / kTrunkWarps;
         if (ns > 0) order[n_busy++] = i;
     }
     // no two segments may write the same row (the result would depend on the schedule)
-    std::sort(order, order + n_busy, [&](int a, int b) { return A.seg[a].row_begin < A.seg[b].row_begin; });
-    for (int i = 1; i < n_busy; ++i)
-        if (A.seg[order[i - 1]].row_begin + A.seg[order[i - 1]].n_samples > A.seg[order[i]].row_begin)
+    std::sort(order, order + n_busy, [&](int a, int b) { return segments[a].out_row < segments[b].out_row; });
+    for (int i = 1; i < n_busy; ++i) {
+        const ctf_policy_segment_t& prev = segments[order[i - 1]];
+        if (prev.out_row + prev.n_envs * prev.k > segments[order[i]].out_row)
             return fail(CTF_ERR_INVALID, "%s: the output rows of two segments overlap", fn);
-    if (tiles == 0) return CTF_OK;
-    A.geo.packed = packed; A.geo.meta = meta; A.geo.features = static_cast<__nv_bfloat16*>(features);
-    A.geo.stride = feature_stride; A.geo.ape = agents_per_env;
-    A.n_tiles = tiles;
-    A.n_segments = n_segments;
+    }
+    if (n_busy == 0) return CTF_OK;
+    TrunkGeometry geo;
+    size_t smem = 0;
+    trunk_layout(P, geo, smem);
+    geo.packed = packed; geo.meta = meta; geo.features = static_cast<__nv_bfloat16*>(features);
+    geo.stride = feature_stride; geo.ape = agents_per_env;
     DeviceGuard guard(h->device);
     CTF_CUDA(guard.err);
-    const unsigned grid = (unsigned)(tiles < h->grouped_ctas ? tiles : h->grouped_ctas);
-    k_policy_trunk_grouped<<<grid, kTrunkThreads, smem, static_cast<cudaStream_t>(stream)>>>(A);
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (n_policies == 1 && n_segments == 1) {
+        TrunkLaunchOne A;
+        launch_trunk_table(A, geo, weights, n_policies, segments, n_segments, agents_per_env, h->trunk_ctas, smem, s);
+    } else {
+        // the grouped argument block is large (about 26 KB): keep it off the caller's stack
+        static thread_local TrunkLaunchGrouped A;
+        launch_trunk_table(A, geo, weights, n_policies, segments, n_segments, agents_per_env, h->grouped_ctas, smem, s);
+    }
     CTF_CUDA(cudaGetLastError());
     return CTF_OK;
+}
+
+extern "C" int ctf_policy_features(ctf_handle_t h, const ctf_policy_weights_t* w, const uint32_t* packed, const float* meta,
+                                   int64_t n_envs, int agents_per_env, const uint8_t* agent_ids, int k, void* features,
+                                   int64_t feature_stride, void* stream) {
+    const char* fn = "ctf_policy_features";
+    if (!h || !w || !packed || !meta || !agent_ids || !features) return fail(CTF_ERR_INVALID, "%s: null argument", fn);
+    // one segment over every env whose sample s is feature row s; launch_trunk rejects a k outside 1..8 (the ids are
+    // copied only for a k in range, and n_rows stays >= 0 so that it is k that the error names)
+    ctf_policy_segment_t seg = {0, n_envs, 0, 0, k, {}};
+    if (k >= 1 && k <= CTF_MAX_AGENTS) memcpy(seg.agent_ids, agent_ids, k);
+    const int64_t n_rows = k > 0 ? n_envs * k : 0;
+    return launch_trunk(fn, "k", h, w, 1, &seg, 1, packed, meta, n_envs, agents_per_env, features, feature_stride, n_rows,
+                        stream);
+}
+
+extern "C" int ctf_policy_features_grouped(ctf_handle_t h, const ctf_policy_weights_t* weights, int n_policies,
+                                           const ctf_policy_segment_t* segments, int n_segments, const uint32_t* packed,
+                                           const float* meta, int64_t n_envs, int agents_per_env, void* features,
+                                           int64_t feature_stride, int64_t n_rows, void* stream) {
+    const char* fn = "ctf_policy_features_grouped";
+    if (!h || !weights || !segments || !packed || !meta || !features) return fail(CTF_ERR_INVALID, "%s: null argument", fn);
+    return launch_trunk(fn, "a segment's k", h, weights, n_policies, segments, n_segments, packed, meta, n_envs,
+                        agents_per_env, features, feature_stride, n_rows, stream);
 }
 
 extern "C" int ctf_policy_trunk_ctas(ctf_handle_t h, int* trunk_ctas, int* grouped_ctas) {

@@ -26,8 +26,8 @@ step, agent), like the env's own draws (draws.py), so the actions do not depend 
 envs are batched.  ``seed=None`` keeps torch's ``Categorical``.
 
 Several policies on one env batch: ``PolicyPool(env, policies)`` runs any number of (policy, env slice, agent ids)
-segments with one ``ctf_policy_features_grouped`` launch (``k_policy_trunk_grouped``, the same per-sample code as
-``k_policy_trunk``, so every row is bit-identical to ``FusedPolicy``'s) and one bf16 ``torch.baddbmm`` head chain over
+segments with one ``ctf_policy_features_grouped`` launch (the same ``k_policy_trunk`` kernel with the grouped tables,
+so every row is bit-identical to ``FusedPolicy``'s) and one bf16 ``torch.baddbmm`` head chain over
 all policies; league evaluation uses it (``league.duel_pairs(grouped=True)``).
 """
 from __future__ import annotations
@@ -590,7 +590,7 @@ class PoolPlan:
 
 class PolicyPool:
     """Inference for several policies on one env batch: one grouped trunk launch (``ctf_policy_features_grouped``,
-    ``k_policy_trunk_grouped``) and one bf16 ``torch.baddbmm`` chain for the heads of all policies per forward.
+    ``k_policy_trunk``) and one bf16 ``torch.baddbmm`` chain for the heads of all policies per forward.
 
     ``policies``: ``CtfPolicy`` modules or ``FusedPolicy`` views of them (their ``policy`` is used), each policy once,
     at most ``GROUPED_MAX_POLICIES`` (64).  Every weight lives in stacked persistent buffers: conv1 / conv2 in the
@@ -614,7 +614,7 @@ class PolicyPool:
         self.k1, self.stride = _check_policies(env, mods)
         self.env, self.policies = env, mods
         self._trunk_w = _TrunkWeights(len(mods), env.n_channels, env.device)
-        self._weights = self._trunk_w.native        # the grouped kernel's weight table, one entry per policy
+        self._weights = self._trunk_w.native        # the grouped launch's weight table, one entry per policy
         self._head_w = _HeadWeights(len(mods), self.k1, self.stride, env.device)
         self.refresh()
 
